@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...   # CPU arm (restated oracle; PyBullet is not in the image)
     torchrun --nproc-per-node N bench.py --gpus N ...         # one rank per GPU, weak scaling
+    python bench.py ... --dump-outputs DIR                    # also write the last timed step's outputs (two builds compare)
 
 A "step" is one pass of the hot path over the batch: one agent-visible env step for every env of the batch
 (SwingRacket's 26th step, which fast-forwards up to 776 physics substeps, counts once).  Workload = config 5's
@@ -52,6 +53,7 @@ EPISODE_STEPS = 26
 GROUP = 128
 RING = 32  # pre-drawn action batches: >= 26, so the actions of an episode are i.i.d. (a ring of 4 repeats every 4 steps and
            # drives the racket in one direction: many more racket-ball contacts than action_space.sample() gives)
+DUMP_LIMIT = 64 * 10**6  # bytes of all files --dump-outputs writes; beyond it a seeded sample of envs is written
 
 
 def parse():
@@ -70,7 +72,13 @@ def parse():
     ap.add_argument("--skip-cpu-baseline", action="store_true")
     ap.add_argument("--extras", default="auto", choices=["auto", "on", "off"],
                     help="measure the other BASELINE configs too (auto: at N = 1)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last of them returned (rank 0's envs) as DIR/<name>.npy, "
+                         "at most 64 MB: obs, reward, done, terminal_obs, events, one row per env")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    return args
 
 
 # ---------------------------------------------------------------------------------------------- helpers
@@ -200,6 +208,26 @@ def measured_peak():
     return 6650.0, "fallback"
 
 
+def dump_outputs(out_dir, arrays):
+    """Write {name: array with one row per env} as out_dir/<name>.npy in float32 (float64 arrays stay float64), so that
+    two builds can be compared output for output.  When the files would exceed DUMP_LIMIT, the same seeded sample of envs
+    is taken from every array and the sampled env indices go to env_index.npy."""
+    import numpy as np
+
+    arrays = {k: (v if v.dtype in (np.float32, np.float64) else v.astype(np.float32)) for k, v in arrays.items()}
+    n = len(next(iter(arrays.values())))
+    row_bytes = sum(v.nbytes for v in arrays.values()) // n
+    budget = DUMP_LIMIT - 4096  # room for the .npy headers
+    if n * row_bytes > budget:
+        idx = np.sort(np.random.default_rng(0).choice(n, budget // (row_bytes + 8), replace=False))
+        arrays = {k: v[idx] for k, v in arrays.items()}
+        arrays["env_index"] = idx.astype(np.float64)
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(out / f"{k}.npy", v)
+
+
 class CpuOracleRun:
     """The restated CPU oracle (PyBullet is not installable here) on `threads` host threads: one env batch, one
     pre-drawn action tape; step() timings exclude construction and action generation."""
@@ -216,12 +244,13 @@ class CpuOracleRun:
         rng = np.random.default_rng(0)
         self.acts = rng.uniform(-1, 1, (EPISODE_STEPS, n_envs, self.o.act_dim)).astype(np.float32)
         self.t = 0
+        self.last = None
 
     def run(self, steps):
-        """`steps` env steps for every env of the sample; returns (seconds, env steps done)."""
+        """`steps` env steps for every env of the sample; returns (seconds, env steps done).  self.last: the last step's outputs."""
         t0 = time.perf_counter()
         for _ in range(steps):
-            self.o.step(self.acts[self.t % EPISODE_STEPS])
+            self.last = self.o.step(self.acts[self.t % EPISODE_STEPS])
             self.t += 1
         return time.perf_counter() - t0, self.n * steps
 
@@ -263,15 +292,19 @@ def run_real_reference(args, ref_path):  # pragma: no cover - needs pybullet
     venv.reset()
     rng = np.random.default_rng(0)
     ad = venv.action_space.shape[0]
+    last = {}
     def episode():
         t0 = time.perf_counter()
         for _ in range(EPISODE_STEPS):
-            venv.step(rng.uniform(-1, 1, (cores, ad)).astype(np.float32))
+            obs, reward, done, _ = venv.step(rng.uniform(-1, 1, (cores, ad)).astype(np.float32))
+        last.update(obs=obs, reward=reward, done=done)
         return time.perf_counter() - t0
     for _ in range(max(args.warmup, 0)):
         episode()
     wall = sum(episode() for _ in range(args.steps))
     venv.close()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last)
     return cores * EPISODE_STEPS * args.steps / wall, wall, cores
 
 
@@ -303,6 +336,8 @@ def run_reference(args, rank):
         wall += dt
         total += k
     value = total / wall
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, run.last)
     line = {
         "impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
         "warmup": args.warmup, "ms_per_step": 1e3 * wall / args.steps, "higher_is_better": True, "scaling": "weak",
@@ -421,14 +456,14 @@ def run_extras(args, torch, np):
 
 
 # ---------------------------------------------------------------------------------------------- B200 arm
-def stagger_phases(batch, torch):
+def stagger_phases(batch, torch, gen):
     """Group g (128 envs) starts g mod 26 steps late: step everyone, then restart the groups whose turn it is."""
     n = batch.num_envs
     group = torch.arange(n, device=batch.device) // GROUP % EPISODE_STEPS
     act = torch.zeros((n, batch.act_dim), dtype=torch.float32, device=batch.device)
     batch.reset()
     for p in range(1, EPISODE_STEPS):
-        act.uniform_(-1, 1)
+        act.uniform_(-1, 1, generator=gen)
         batch.step(act)
         batch.reset(mask=(group == p))
     return EPISODE_STEPS - 1
@@ -459,13 +494,14 @@ def run_b200(args, rank, world):
         torch.cuda.synchronize()
 
     # action buffers: a ring of pre-drawn U(-1,1) batches resident in HBM (synthetic actions = action_space.sample())
-    ring = [torch.empty((n, batch.act_dim), dtype=torch.float32, device=dev).uniform_(-1, 1) for _ in range(RING)]
+    gen = torch.Generator(device=dev).manual_seed(0)  # same actions in every run, so that --dump-outputs can be compared
+    ring = [torch.empty((n, batch.act_dim), dtype=torch.float32, device=dev).uniform_(-1, 1, generator=gen) for _ in range(RING)]
     pre_launch = 0
     stagger = args.stagger == "on" and args.env == "SwingRacket-v0"
     if not stagger:
         batch.reset()
     else:
-        pre_launch = stagger_phases(batch, torch)
+        pre_launch = stagger_phases(batch, torch, gen)
     # lock-step: start the timed region at episode phase (-K mod 26) so that it ends right after a fast-forward step
     swing_lockstep = args.env == "SwingRacket-v0" and not stagger
     align = (-args.steps - args.warmup) % EPISODE_STEPS if swing_lockstep else 0
@@ -485,7 +521,7 @@ def run_b200(args, rank, world):
     e0.record()
     n_reductions = 0
     for k in range(args.steps):
-        batch.step(ring[k % len(ring)])
+        out = batch.step(ring[k % len(ring)])
         # the per-iteration reduction of the episode statistics (10 x int64, NCCL) follows every step that ends an episode:
         # in lock step those are the fast-forward steps, and the region ends on one
         if dist is not None and ((args.steps - 1 - k) % EPISODE_STEPS == 0 if swing_lockstep else (k + 1) % EPISODE_STEPS == 0):
@@ -507,6 +543,8 @@ def run_b200(args, rank, world):
         reduced.copy_(stats)
         dist.all_reduce(reduced)
         st = reduced.cpu().numpy()
+    if args.dump_outputs and rank == 0:  # before the steps below overwrite the batch's output buffers
+        dump_outputs(args.dump_outputs, dict(zip(("obs", "reward", "done", "terminal_obs", "events"), (t.cpu().numpy() for t in out))))
 
     # ---- per-kernel device times over one more episode (events inside the library, stream synchronised per step:
     #      outside the timed region by construction)
@@ -633,6 +671,7 @@ def emit(line):
 
 def main():
     global _REAL_STDOUT
+    sys.dont_write_bytecode = True  # the tree may be read-only: bench.py writes nothing there
     args = parse()
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
