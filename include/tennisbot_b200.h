@@ -108,6 +108,7 @@ const char *tb_last_error(void);
 int tb_abi_version(void);
 int tb_obs_dim(int env_kind);   /* observation_space.shape[0]: 6 (swingracket_env.py:34-39) / 12 (tennisbot_env.py:51-55) */
 int tb_act_dim(int env_kind);   /* action_space.shape[0]:      6 (swingracket_env.py:29-31) / 2  (tennisbot_env.py:37-44) */
+int tb_policy_floats(int env_kind); /* floats tb_set_policy expects: TB_POLICY_FLOATS / TB_POLICY_FLOATS_HIT (-1: unknown kind) */
 int tb_num_params(void);
 const char *tb_param_name(int index);
 /* scene constants as compiled into the library (masses, radii, hull outline ...), for the fixture cross-check */
@@ -149,19 +150,26 @@ int tb_rollout(tb_ctx *ctx, int action_mode, int k_steps, float *d_obs, float *d
 
 /* ---- policy rollout (SURVEY 8(f)-1): what SB3's collect_rollouts does around env.step (train_swing.py:83-122), kept on the
  * device.  The policy is the one the reference trains: SB3 MlpPolicy with net_arch pi = vf = [32, 64, 32], tanh, a Gaussian
- * head with state-independent log_std (train_swing.py:80-91; backup_models/ppo_swing.zip).  Parameters, float32, each
- * tensor row-major [out][in] and padded to a multiple of 4 floats:
+ * head with state-independent log_std (train_swing.py:80-91; backup_models/ppo_swing.zip).  Tennisbot-v0 uses the same
+ * towers on its 12 inputs and 2 outputs (train.py's net_arch is not recorded).  Parameters, float32, each tensor row-major
+ * [out][in] and padded to a multiple of 4 floats.  SwingRacket-v0 (obs_dim 6, act_dim 6):
  *   pi tower: W1[32x6] b1[32] W2[64x32] b2[64] W3[32x64] b3[32] action_net W[6x32] b[6 -> 8]                (4616 floats)
  *   vf tower: W1 b1 W2 b2 W3 b3 (same shapes) value_net W[1x32] b[1 -> 4]                                   (4452 floats)
- *   log_std[6 -> 8]                                                                                          (8 floats) */
+ *   log_std[6 -> 8]                                                                                          (8 floats)
+ * Tennisbot-v0 (obs_dim 12, act_dim 2):
+ *   pi tower: W1[32x12] b1[32] W2[64x32] b2[64] W3[32x64] b3[32] action_net W[2x32] b[2 -> 4]               (4676 floats)
+ *   vf tower: W1 b1 W2 b2 W3 b3 (same shapes) value_net W[1x32] b[1 -> 4]                                   (4644 floats)
+ *   log_std[2 -> 4]                                                                                          (4 floats) */
 #define TB_POLICY_FLOATS 9076
+#define TB_POLICY_FLOATS_HIT 9324
+/* count must be tb_policy_floats(env_kind) */
 int tb_set_policy(tb_ctx *ctx, const float *d_params, int64_t count, void *stream);
 /* K env steps with actions sampled from the policy: per step one policy_kernel launch (forward, Philox Gaussian noise,
  * log-density, value) followed by tb_step's launches, all on `stream`, nothing synchronises - capturable in a CUDA graph.
- * d_obs float32 [K, N, 6]: d_obs[0] must hold the current observation (from tb_reset or the previous rollout's
- * d_last_obs); d_obs[t] receives the observation step t acted on.  d_actions float32 [K, N, 6]: the sampled, UNCLIPPED
+ * d_obs float32 [K, N, obs_dim]: d_obs[0] must hold the current observation (from tb_reset or the previous rollout's
+ * d_last_obs); d_obs[t] receives the observation step t acted on.  d_actions float32 [K, N, act_dim]: the sampled, UNCLIPPED
  * action (env.step gets it clipped to the Box, as SB3 does); d_logp, d_value float32 [K, N]; d_reward float32 [K, N];
- * d_done uint8 [K, N]; d_last_obs float32 [N, 6] and d_last_value float32 [N]: observation after the last step and its
+ * d_done uint8 [K, N]; d_last_obs float32 [N, obs_dim] and d_last_value float32 [N]: observation after the last step and its
  * value (GAE bootstrap).  d_actions, d_logp, d_value, d_last_value may be NULL.  deterministic = 1: action = mean
  * (model.predict(deterministic=True)); else stochastic, as validate_swing.py:35 rolls the policy.  The noise streams
  * are keyed (noise_seed, global env id, the context's env-step counter, a device word): independent of the env's own streams

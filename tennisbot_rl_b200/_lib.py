@@ -14,7 +14,8 @@ ENV_SWING, ENV_HIT = 0, 1
 F32, F64 = 0, 1
 STATE_WORDS, INIT_WORDS, NUM_STATS = 32, 8, 10
 ACT_RANDOM, ACT_TRACK = 0, 1
-POLICY_FLOATS = 9076
+POLICY_FLOATS = 9076       # SwingRacket-v0's in-kernel policy (TB_POLICY_FLOATS)
+POLICY_FLOATS_HIT = 9324   # Tennisbot-v0's (TB_POLICY_FLOATS_HIT)
 CONTROL_FORCE, CONTROL_PID = 0, 1
 
 EV_RACKET_BALL, EV_COURT_BALL, EV_GOAL_BALL, EV_TIMEOUT, EV_BALL_PASSED, EV_NET_BALL, EV_RACKET_LOW = 1, 2, 4, 8, 16, 32, 64
@@ -23,7 +24,7 @@ STAT_NAMES = ("episodes", "sum_length", "racket_hits", "goals", "court", "timeou
 
 # every symbol include/tennisbot_b200.h declares (checked by tests/test_abi.py)
 EXPORTS = (
-    "tb_last_error", "tb_abi_version", "tb_obs_dim", "tb_act_dim", "tb_num_params", "tb_param_name",
+    "tb_last_error", "tb_abi_version", "tb_obs_dim", "tb_act_dim", "tb_policy_floats", "tb_num_params", "tb_param_name",
     "tb_scene_constant", "tb_create", "tb_destroy", "tb_set_param", "tb_get_param", "tb_set_control_mode", "tb_reset", "tb_reset_from",
     "tb_step", "tb_rollout", "tb_get_state", "tb_set_state", "tb_stats_device_ptr", "tb_read_stats",
     "tb_reset_host", "tb_step_host", "tb_launch_count", "tb_ff_diagnostics", "tb_set_kernel_timing", "tb_get_kernel_timing",
@@ -60,6 +61,8 @@ def load():
     L.tb_param_name.argtypes = [i32]
     L.tb_obs_dim.argtypes = [i32]
     L.tb_act_dim.argtypes = [i32]
+    if hasattr(L, "tb_policy_floats"):
+        L.tb_policy_floats.argtypes = [i32]
     L.tb_scene_constant.argtypes = [C.c_char_p, i32, C.POINTER(dbl)]
     L.tb_create.argtypes = [C.POINTER(TbConfig), C.POINTER(vp)]
     L.tb_destroy.argtypes = [vp]

@@ -122,17 +122,40 @@ class TennisBatch:
 
     # ------------------------------------------------------------------ policy rollout (tb_set_policy / tb_policy_rollout)
     def set_policy(self, params):
-        """params: float32 CUDA tensor [POLICY_FLOATS] in the layout of include/tennisbot_b200.h (pack_policy builds it)."""
+        """params: float32 CUDA tensor [policy_floats] in the layout of include/tennisbot_b200.h for this batch's env
+        (POLICY_FLOATS for SwingRacket-v0, POLICY_FLOATS_HIT for Tennisbot-v0; pack_policy builds it)."""
         p = params.to(device=self.device, dtype=torch.float32).contiguous()
-        if p.numel() != _lib.POLICY_FLOATS:
-            raise ValueError(f"policy parameter vector must have {_lib.POLICY_FLOATS} floats")
+        want = _lib.POLICY_FLOATS if self.kind == _lib.ENV_SWING else _lib.POLICY_FLOATS_HIT
+        if p.numel() != want:
+            raise ValueError(f"policy parameter vector must have {want} floats for this env, got {p.numel()}")
         _lib.check(self.lib.tb_set_policy(self.h, _dptr(p), p.numel(), self._stream()))
 
     def policy_rollout(self, obs, reward, done, last_obs, actions=None, logp=None, value=None, last_value=None,
                        deterministic=False, noise_seed=0):
         """K = obs.shape[0] env steps with actions sampled in-kernel from the policy set by set_policy.  obs[0] must hold
-        the current observation.  All buffers are float32 CUDA tensors ([K, N, 6] / [K, N]; done uint8)."""
-        k = int(obs.shape[0])
+        the current observation.  obs [K, N, obs_dim], actions [K, N, act_dim], reward / logp / value [K, N], last_obs
+        [N, obs_dim], last_value [N]: contiguous float32 tensors on this batch's device; done [K, N] uint8.  The library
+        writes through raw pointers, so every buffer is checked here."""
+        k, n = int(obs.shape[0]) if obs.dim() == 3 else -1, self.num_envs
+
+        def need(t, name, shape, dtype=torch.float32, optional=False):
+            if t is None and optional:
+                return
+            if (t is None or t.dtype != dtype or t.device != self.device or not t.is_contiguous() or tuple(t.shape) != shape):
+                got = None if t is None else (tuple(t.shape), t.dtype, str(t.device), t.is_contiguous())
+                raise ValueError(f"policy_rollout: {name} must be a contiguous {dtype} tensor of shape {shape} on {self.device}, "
+                                 f"got {got}")
+
+        if k < 1:
+            raise ValueError(f"policy_rollout: obs must have shape (K >= 1, {n}, {self.obs_dim}), got {tuple(obs.shape)}")
+        need(obs, "obs", (k, n, self.obs_dim))
+        need(actions, "actions", (k, n, self.act_dim), optional=True)
+        need(logp, "logp", (k, n), optional=True)
+        need(value, "value", (k, n), optional=True)
+        need(reward, "reward", (k, n))
+        need(done, "done", (k, n), dtype=torch.uint8)
+        need(last_obs, "last_obs", (n, self.obs_dim))
+        need(last_value, "last_value", (n,), optional=True)
         _lib.check(self.lib.tb_policy_rollout(self.h, k, int(bool(deterministic)), int(noise_seed) & (2 ** 64 - 1), _dptr(obs),
                                               _dptr(actions), _dptr(logp), _dptr(value), _dptr(reward), _dptr(done), _dptr(last_obs),
                                               _dptr(last_value), self._stream()))

@@ -172,8 +172,10 @@ struct StepIO {
   unsigned long long *dq_full, *dq_late;  // ff_kernel's dynamic queues (slots tagged with `epoch`): envs parked for a full
                                      // substep; envs whose flight goes on after one.  dq_cap slots each
   long long dq_cap;
-  unsigned *epoch;                   // two device words: [0] steps completed (read by step_kernel, advanced by ff_kernel),
-                                     // [1] = [0] + 1 written by step_kernel = the tag of this step's queue slots
+  unsigned *epoch;                   // three device words: [0] steps completed (read by step_kernel, advanced by ff_kernel),
+                                     // [1] = [0] + 1 written by step_kernel = the tag of this step's queue slots,
+                                     // [2] Tennisbot-v0 steps completed (advanced by step_kernel; no ff_kernel advances [0]
+                                     // there): the noise counter of the policy rollout
   int prefetch_ahead;                // step_kernel: CTAs resident at a time (the L2 prefetch distance), 0 = none
   unsigned long long *fault;         // sticky: non-zero once a wait inside ff_kernel has timed out (every later call on the
                                      // context fails); fault_host: the same word in mapped host memory, read by the host
@@ -543,6 +545,8 @@ __global__ void __launch_bounds__(kBlock, MINB ? MINB : StepMinBlocks<T, KIND>::
     unsigned long long *next = ctr_set(io, e + 1u);
     for (int i = threadIdx.x; i < kCtrWords; i += kBlock) next[i] = 0;
     if (threadIdx.x == 0) io.epoch[1] = e + 1u;  // the tag of this step's queue slots, never 0
+    // (policy_kernel reads [2] after its pdl_wait, i.e. after this grid has finished; nothing in this grid reads it)
+    if (KIND == TB_ENV_HIT && threadIdx.x == 0) io.epoch[2] += 1u;
   }
 
   const int64_t tile0 = io.env_lo + (int64_t)blockIdx.x * kBlock + wib * 32, me = tile0 + lane;
@@ -1466,11 +1470,20 @@ __global__ void __launch_bounds__(kBlock) rollout_kernel(const __grid_constant__
 // SURVEY 8(f)-1: the policy of train_swing.py:80-91 (SB3 MlpPolicy, net_arch pi = vf = [32, 64, 32], tanh, Gaussian head with
 // a state-independent log_std) evaluated on the device, so that a rollout is K x (policy_kernel, step_kernel, ff_kernel) on
 // one stream: observations, actions and the per-step records PPO needs never leave HBM and no host code runs between steps.
-// One thread per env; the 9 076 parameters (36 KB, layout TB_POLICY_* in the header) sit in shared memory and are read as
-// broadcast float4; activations stay in registers (every loop is unrolled).  float32 throughout, like the torch policy.
-constexpr int kPolW1 = 0, kPolB1 = 192, kPolW2 = 224, kPolB2 = 2272, kPolW3 = 2336, kPolB3 = 4384, kPolHead = 4416;
-constexpr int kPolPiTower = 4616, kPolVfTower = 4452, kPolLogStd = kPolPiTower + kPolVfTower;
-static_assert(kPolLogStd + 8 == TB_POLICY_FLOATS, "policy layout / header mismatch");
+// One thread per env; the parameters (layout TB_POLICY_* in the header) sit in shared memory and are read as broadcast
+// float4; activations stay in registers (every loop is unrolled).  float32 throughout, like the torch policy.
+// policy_kernel<OBS, ACT> is instantiated for SwingRacket-v0 (6 -> 6) and Tennisbot-v0 (12 -> 2); both use the same towers.
+__host__ __device__ constexpr int pad4(int x) { return (x + 3) & ~3; }
+template <int OBS, int ACT> struct PolLayout {  // float offsets; every tensor row-major [out][in], padded to 4 floats
+  static constexpr int W1 = 0, B1 = 32 * OBS, W2 = B1 + 32, B2 = W2 + 64 * 32, W3 = B2 + 64, B3 = W3 + 32 * 64, Head = B3 + 32;
+  static constexpr int PiTower = Head + ACT * 32 + pad4(ACT);  // + action_net W [ACT x 32], b
+  static constexpr int VfTower = Head + 32 + 4;                // + value_net W [1 x 32], b
+  static constexpr int LogStd = PiTower + VfTower, Floats = LogStd + pad4(ACT);
+};
+static_assert(PolLayout<6, 6>::Head == 4416 && PolLayout<6, 6>::PiTower == 4616 && PolLayout<6, 6>::VfTower == 4452 &&
+              PolLayout<6, 6>::Floats == TB_POLICY_FLOATS, "policy layout / header mismatch (SwingRacket-v0)");
+static_assert(PolLayout<12, 2>::PiTower == 4676 && PolLayout<12, 2>::VfTower == 4644 && PolLayout<12, 2>::Floats == TB_POLICY_FLOATS_HIT,
+              "policy layout / header mismatch (Tennisbot-v0)");
 
 // tanh(x) = 1 - 2 / (exp(2x) + 1) on the fast exponential: ~1e-6 absolute, a quarter of tanhf's instructions (a thread takes
 // 256 of them per step)
@@ -1506,82 +1519,105 @@ __device__ __forceinline__ void dense_tanh(const float *__restrict__ W, const fl
     for (int k = 0; k < 4; ++k) y[o + k] = tanh_fast(acc[k]);
   }
 }
-// the three tanh layers of one tower: 6 -> 32 -> 64 -> 32
+// the three tanh layers of one tower: OBS -> 32 -> 64 -> 32
+template <int OBS, int ACT>
 __device__ __forceinline__ void tower(const float *P, const float *x, float *h3) {
+  using L = PolLayout<OBS, ACT>;
   float h1[32], h2[64];
-  dense_tanh<6, 32>(P + kPolW1, P + kPolB1, x, h1);
-  dense_tanh<32, 64>(P + kPolW2, P + kPolB2, h1, h2);
-  dense_tanh<64, 32>(P + kPolW3, P + kPolB3, h2, h3);
+  dense_tanh<OBS, 32>(P + L::W1, P + L::B1, x, h1);
+  dense_tanh<32, 64>(P + L::W2, P + L::B2, h1, h2);
+  dense_tanh<64, 32>(P + L::W3, P + L::B3, h2, h3);
 }
 constexpr uint32_t kStreamPolicy = 2u;
 struct PolicyIO {
-  const float *params;     // TB_POLICY_FLOATS floats in HBM
-  const float *obs;        // [N, 6] observation the action is computed from
-  float *act_raw;          // [N, 6] mean + std * eps, NOT clipped (what PPO's ratio is formed with), may be nullptr
-  float *act_env;          // [N, 6] clipped to the Box (what env.step gets: SB3 clips before stepping), may be nullptr
+  const float *params;     // PolLayout<OBS, ACT>::Floats floats in HBM
+  const float *obs;        // [N, OBS] observation the action is computed from
+  float *act_raw;          // [N, ACT] mean + std * eps, NOT clipped (what PPO's ratio is formed with), may be nullptr
+  float *act_env;          // [N, ACT] clipped to the Box (what env.step gets: SB3 clips before stepping), may be nullptr
   float *logp, *value;     // [N] log-density of act_raw; value estimate (either may be nullptr)
   int64_t n, id_offset;
   uint64_t seed;           // noise streams are keyed (seed, global env id, tick): independent of the env's own streams
-  const unsigned *tick;    // device word that advances with every env step (StepIO::epoch[0]): a rollout captured in a CUDA
-                           // graph draws fresh noise on every replay
+  const unsigned *tick;    // device word that advances with every env step (StepIO::epoch[0] for SwingRacket-v0, epoch[2]
+                           // for Tennisbot-v0): a rollout captured in a CUDA graph draws fresh noise on every replay
   int deterministic;       // 1: act_raw = mean (validate_swing.py's predict(deterministic=True) counterpart)
 };
 // grid (ceil(N / 128), 2): blockIdx.y = 0 the policy tower (action, log-density), 1 the value tower
+template <int OBS, int ACT>
 __global__ void __launch_bounds__(kBlock) policy_kernel(const __grid_constant__ PolicyIO io) {
-  __shared__ __align__(16) float P[kPolPiTower + 8];
+  using L = PolLayout<OBS, ACT>;
+  static_assert(OBS % 2 == 0 && ACT % 2 == 0, "observation rows are read as float2 / float4, actions written as float2");
+  __shared__ __align__(16) float P[L::PiTower + pad4(ACT)];
   const bool vf = blockIdx.y != 0;
   pdl_wait();
   if (vf ? io.value == nullptr : (!io.act_raw && !io.act_env && !io.logp)) return;
   {
-    const float4 *src = reinterpret_cast<const float4 *>(io.params + (vf ? kPolPiTower : 0));
-    const int nv = (vf ? kPolVfTower : kPolPiTower) / 4;
+    const float4 *src = reinterpret_cast<const float4 *>(io.params + (vf ? L::PiTower : 0));
+    const int nv = (vf ? L::VfTower : L::PiTower) / 4;
     for (int i = threadIdx.x; i < nv; i += kBlock) reinterpret_cast<float4 *>(P)[i] = src[i];
-    if (!vf && threadIdx.x < 2) reinterpret_cast<float4 *>(P + kPolPiTower)[threadIdx.x] = reinterpret_cast<const float4 *>(io.params + kPolLogStd)[threadIdx.x];
+    if (!vf && threadIdx.x < pad4(ACT) / 4) reinterpret_cast<float4 *>(P + L::PiTower)[threadIdx.x] = reinterpret_cast<const float4 *>(io.params + L::LogStd)[threadIdx.x];
   }
   __syncthreads();
   const int64_t me = (int64_t)blockIdx.x * kBlock + threadIdx.x;
   if (me < io.n) {
-    float x[6];
-    {
-      const float2 *p = reinterpret_cast<const float2 *>(io.obs + me * 6);
-      const float2 a = p[0], b = p[1], c = p[2];
-      x[0] = a.x; x[1] = a.y; x[2] = b.x; x[3] = b.y; x[4] = c.x; x[5] = c.y;
+    float x[OBS];
+    if (OBS % 4 == 0) {  // 48 B rows (Tennisbot-v0): three float4
+#pragma unroll
+      for (int j = 0; j < OBS / 4; ++j) {
+        const float4 a = reinterpret_cast<const float4 *>(io.obs + me * OBS)[j];
+        x[4 * j] = a.x; x[4 * j + 1] = a.y; x[4 * j + 2] = a.z; x[4 * j + 3] = a.w;
+      }
+    } else {  // 24 B rows (SwingRacket-v0): three float2
+#pragma unroll
+      for (int j = 0; j < OBS / 2; ++j) {
+        const float2 a = reinterpret_cast<const float2 *>(io.obs + me * OBS)[j];
+        x[2 * j] = a.x; x[2 * j + 1] = a.y;
+      }
     }
     float h[32];
-    tower(P, x, h);
+    tower<OBS, ACT>(P, x, h);
     if (!vf) {
-      const float *Wa = P + kPolHead, *ba = P + kPolHead + 192, *ls = P + kPolPiTower;
-      uint32_t r0[4], r1[4];
+      const float *Wa = P + L::Head, *ba = P + L::Head + ACT * 32, *ls = P + L::PiTower;
+      // one Box-Muller pair (two uniforms) per two components: one Philox call per four components
+      constexpr int NR = (ACT + 3) / 4;
+      uint32_t rr[4 * NR];
       const uint32_t tick = *io.tick;
-      philox4x32(io.seed, (uint64_t)(io.id_offset + me), tick, stream_word(kStreamPolicy, 0, 0), r0);
-      philox4x32(io.seed, (uint64_t)(io.id_offset + me), tick, stream_word(kStreamPolicy, 0, 1), r1);
-      const uint32_t rr[8] = {r0[0], r0[1], r0[2], r0[3], r1[0], r1[1], r1[2], r1[3]};
-      float raw[6], lp = 0.0f;
 #pragma unroll
-      for (int o = 0; o < 6; ++o) {
+      for (int j = 0; j < NR; ++j) philox4x32(io.seed, (uint64_t)(io.id_offset + me), tick, stream_word(kStreamPolicy, 0, j), rr + 4 * j);
+      float raw[ACT], lp = 0.0f;
+#pragma unroll
+      for (int o = 0; o < ACT; ++o) {
         float mu = ba[o];
 #pragma unroll
         for (int i = 0; i < 32; ++i) mu = fmaf(Wa[o * 32 + i], h[i], mu);
         // Box-Muller on a pair of uniforms: component o takes the cosine (o even) or sine (o odd) branch of pair o / 2
         const float u1 = ((float)(rr[2 * (o / 2)] >> 8) + 0.5f) * (1.0f / 16777216.0f), u2 = (float)(rr[2 * (o / 2) + 1] >> 8) * (1.0f / 16777216.0f);
-        const float rad = sqrtf(-2.0f * logf(u1)), ang = 6.283185307179586f * u2;
-        const float eps = io.deterministic ? 0.0f : rad * ((o & 1) ? sinf(ang) : cosf(ang));
+        const float rad = sqrtf(-2.0f * logf(u1));
+        float sc;
+        if (OBS == 6 && ACT == 6) {  // SwingRacket-v0 keeps sinf / cosf, so its rollouts stay what they were (their
+          const float ang = 6.283185307179586f * u2;  // large-argument range reduction costs a 32-byte stack frame)
+          sc = (o & 1) ? sinf(ang) : cosf(ang);
+        } else {  // sin / cos of pi * 2 u2, 2 u2 in [0, 2): exact range reduction, nothing in local memory
+          sc = (o & 1) ? sinpif(2.0f * u2) : cospif(2.0f * u2);
+        }
+        const float eps = io.deterministic ? 0.0f : rad * sc;
         raw[o] = fmaf(expf(ls[o]), eps, mu);
         lp += -0.5f * eps * eps - ls[o] - 0.9189385332046727f;
       }
       if (io.act_raw) {
-        float2 *q = reinterpret_cast<float2 *>(io.act_raw + me * 6);
-        q[0] = make_float2(raw[0], raw[1]); q[1] = make_float2(raw[2], raw[3]); q[2] = make_float2(raw[4], raw[5]);
+        float2 *q = reinterpret_cast<float2 *>(io.act_raw + me * ACT);
+#pragma unroll
+        for (int j = 0; j < ACT / 2; ++j) q[j] = make_float2(raw[2 * j], raw[2 * j + 1]);
       }
       if (io.act_env) {
-        float2 *q = reinterpret_cast<float2 *>(io.act_env + me * 6);
+        float2 *q = reinterpret_cast<float2 *>(io.act_env + me * ACT);
 #pragma unroll
-        for (int o = 0; o < 6; ++o) raw[o] = fminf(fmaxf(raw[o], -1.0f), 1.0f);
-        q[0] = make_float2(raw[0], raw[1]); q[1] = make_float2(raw[2], raw[3]); q[2] = make_float2(raw[4], raw[5]);
+        for (int o = 0; o < ACT; ++o) raw[o] = fminf(fmaxf(raw[o], -1.0f), 1.0f);
+#pragma unroll
+        for (int j = 0; j < ACT / 2; ++j) q[j] = make_float2(raw[2 * j], raw[2 * j + 1]);
       }
       if (io.logp) io.logp[me] = lp;
     } else {
-      const float *Wv = P + kPolHead;
+      const float *Wv = P + L::Head;
       float v = Wv[32];
 #pragma unroll
       for (int i = 0; i < 32; ++i) v = fmaf(Wv[i], h[i], v);
@@ -2050,8 +2086,8 @@ struct tb_ctx {
   cudaStream_t s_up = nullptr, s_dn = nullptr;
   cudaEvent_t ev_up[kMaxSlices] = {}, ev_k[kMaxSlices] = {};
   unsigned *h_ffran = nullptr, *h_ffran_dev = nullptr;  // mapped host word, see StepIO::ff_ran_host
-  float *policy = nullptr;                   // TB_POLICY_FLOATS parameters (tb_set_policy)
-  float *pol_act = nullptr;                  // [N, 6] clipped actions handed from policy_kernel to step_kernel
+  float *policy = nullptr;                   // tb_policy_floats(env_kind) parameters (tb_set_policy)
+  float *pol_act = nullptr;                  // [N, act_dim] clipped actions handed from policy_kernel to step_kernel
   bool timing = false;                       // tb_set_kernel_timing
   cudaEvent_t ev[3] = {nullptr, nullptr, nullptr};
   double ms_step = 0, ms_ff = 0;
@@ -2245,6 +2281,7 @@ const char *tb_last_error(void) { return g_err; }
 int tb_abi_version(void) { return TB_ABI_VERSION; }
 int tb_obs_dim(int kind) { return kind == TB_ENV_SWING ? 6 : kind == TB_ENV_HIT ? 12 : -1; }
 int tb_act_dim(int kind) { return kind == TB_ENV_SWING ? 6 : kind == TB_ENV_HIT ? 2 : -1; }
+int tb_policy_floats(int kind) { return kind == TB_ENV_SWING ? TB_POLICY_FLOATS : kind == TB_ENV_HIT ? TB_POLICY_FLOATS_HIT : -1; }
 int tb_num_params(void) { return kNumParams; }
 const char *tb_param_name(int i) { return (i >= 0 && i < kNumParams) ? k_param_names[i] : nullptr; }
 
@@ -2343,8 +2380,8 @@ int tb_create(const tb_config *cfg, tb_ctx **out) {
     if (!(limit_ms > 0)) limit_ms = 4000.0;
     c->spin_limit = (long long)(limit_ms * 1e-3 * (double)prop.clockRate * 1e3);  // clockRate is in kHz
   }
-  if (e == cudaSuccess) e = cudaMalloc(&c->epoch, 2 * sizeof(unsigned));
-  if (e == cudaSuccess) e = cudaMemsetAsync(c->epoch, 0, 2 * sizeof(unsigned), c->own_stream);
+  if (e == cudaSuccess) e = cudaMalloc(&c->epoch, 3 * sizeof(unsigned));
+  if (e == cudaSuccess) e = cudaMemsetAsync(c->epoch, 0, 3 * sizeof(unsigned), c->own_stream);
   if (e == cudaSuccess && c->dq) e = cudaMemsetAsync(c->dq, 0, (size_t)c->dq_cap * 2 * sizeof(unsigned long long), c->own_stream);  // tag 0 = no epoch
   if (e == cudaSuccess) {
     // identity quaternion, episode = -1 so the first reset starts episode 0
@@ -2471,11 +2508,15 @@ int tb_rollout(tb_ctx *c, int action_mode, int k_steps, float *d_obs, float *d_r
 
 int tb_set_policy(tb_ctx *c, const float *d_params, int64_t count, void *stream) {
   GUARD(c);
-  if (c->cfg.env_kind != TB_ENV_SWING) return fail("%s", "tb_set_policy: the in-kernel policy is SwingRacket-v0's (6 -> 6)");
-  if (!d_params || count != TB_POLICY_FLOATS) return fail("%s", "tb_set_policy: expected TB_POLICY_FLOATS floats in device memory");
-  if (!c->policy) CU(cudaMalloc(&c->policy, TB_POLICY_FLOATS * sizeof(float)));
-  if (!c->pol_act) CU(cudaMalloc(&c->pol_act, (size_t)c->cfg.num_envs * 6 * sizeof(float)));
-  CU(cudaMemcpyAsync(c->policy, d_params, TB_POLICY_FLOATS * sizeof(float), cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
+  const int64_t want = tb_policy_floats(c->cfg.env_kind);
+  if (!d_params || count != want) {
+    std::snprintf(g_err, sizeof g_err, "tb_set_policy: expected tb_policy_floats(env_kind) = %lld floats in device memory, got %lld",
+                  (long long)want, (long long)count);
+    return 1;
+  }
+  if (!c->policy) CU(cudaMalloc(&c->policy, (size_t)want * sizeof(float)));
+  if (!c->pol_act) CU(cudaMalloc(&c->pol_act, (size_t)c->cfg.num_envs * tb_act_dim(c->cfg.env_kind) * sizeof(float)));
+  CU(cudaMemcpyAsync(c->policy, d_params, (size_t)want * sizeof(float), cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
   return 0;
 }
 
@@ -2487,28 +2528,31 @@ int tb_policy_rollout(tb_ctx *c, int k_steps, int deterministic, uint64_t noise_
   if (k_steps < 1 || !d_obs || !d_reward || !d_done || !d_last_obs) return fail("%s", "tb_policy_rollout: k_steps >= 1, obs, reward, done and last_obs are required");
   if (check_fault(c, "tb_policy_rollout")) return 1;
   const int64_t n = c->cfg.num_envs;
+  const bool swing = c->cfg.env_kind == TB_ENV_SWING;
+  const int od = tb_obs_dim(c->cfg.env_kind), ad = tb_act_dim(c->cfg.env_kind);
+  void (*kernel)(PolicyIO) = swing ? policy_kernel<6, 6> : policy_kernel<12, 2>;
   cudaStream_t s = (cudaStream_t)stream;
   PolicyIO pio;
   std::memset(&pio, 0, sizeof pio);
   pio.params = c->policy; pio.n = n; pio.id_offset = c->cfg.env_id_offset; pio.seed = noise_seed; pio.deterministic = deterministic;
-  pio.act_env = c->pol_act; pio.tick = c->epoch;
+  pio.act_env = c->pol_act; pio.tick = swing ? c->epoch : c->epoch + 2;  // (see StepIO::epoch)
   const unsigned grid = grid_for(n, kBlock);
   for (int t = 0; t < k_steps; ++t) {
-    pio.obs = d_obs + (size_t)t * n * 6;
-    pio.act_raw = d_actions ? d_actions + (size_t)t * n * 6 : nullptr;
+    pio.obs = d_obs + (size_t)t * n * od;
+    pio.act_raw = d_actions ? d_actions + (size_t)t * n * ad : nullptr;
     pio.logp = d_logp ? d_logp + (size_t)t * n : nullptr;
     pio.value = d_value ? d_value + (size_t)t * n : nullptr;
-    CU(launch_pdl(c->pdl, policy_kernel, dim3(grid, 2), s, pio));
+    CU(launch_pdl(c->pdl, kernel, dim3(grid, 2), s, pio));
     c->launches++;
     StepIO io = make_io(c);
     io.actions = c->pol_act;
-    io.obs = t + 1 < k_steps ? d_obs + (size_t)(t + 1) * n * 6 : d_last_obs;
+    io.obs = t + 1 < k_steps ? d_obs + (size_t)(t + 1) * n * od : d_last_obs;
     io.reward = d_reward + (size_t)t * n; io.done = d_done + (size_t)t * n;
     if (launch_step(c, io, s)) return 1;
   }
   if (d_last_value) {  // bootstrap value of the observation the rollout ends with
     pio.obs = d_last_obs; pio.act_raw = nullptr; pio.act_env = nullptr; pio.logp = nullptr; pio.value = d_last_value;
-    CU(launch_pdl(c->pdl, policy_kernel, dim3(grid, 2), s, pio));
+    CU(launch_pdl(c->pdl, kernel, dim3(grid, 2), s, pio));
     c->launches++;
   }
   CU(cudaGetLastError());

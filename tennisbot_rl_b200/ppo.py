@@ -1,4 +1,5 @@
-"""GPU-resident PPO on SwingRacket-v0 (BASELINE config 4: 16 384 envs on one B200) - SURVEY 8(f)-1.
+"""GPU-resident PPO on SwingRacket-v0 (BASELINE config 4: 16 384 envs on one B200) - SURVEY 8(f)-1 - and on Tennisbot-v0
+with train.py's racket-scale curriculum (HitPPO).
 
 The reference trains with SB3 PPO (`train_swing.py:80-91`: MlpPolicy, net_arch pi/vf [32,64,32], tanh, ent_coef
 0.002, gamma .99, gae_lambda .95, clip .2, n_epochs 10, vf_coef .5, max_grad_norm .5) on ONE env, 1100 steps per
@@ -10,6 +11,9 @@ log-density, value), so the 26-step episode is 26 x (policy_kernel, step_kernel,
 is captured once as a CUDA graph and replayed per update (nothing in it synchronises; the queue tags of ff_kernel advance
 on the device).  `fused_policy=False` keeps the eager torch policy of round 1 for comparison.  Target: the mean episodic
 return stored in backup_models/ppo_swing.zip, 31.5.
+
+HitPPO trains Tennisbot-v0 (train.py) the same way with the same hyper-parameters and the same towers on the env's 12
+inputs and 2 outputs (train.py's net_arch is not recorded); its rollouts are K steps of episodes up to 1001 steps long.
 """
 import math
 import time
@@ -19,6 +23,7 @@ import torch.nn as nn
 
 from . import _lib
 from .batch import TennisBatch
+from .playground import curriculum_scale
 
 EPISODE = 26  # agent steps per SwingRacket-v0 episode (swingracket_env.py:85-86: 25 control steps + the fast-forward step)
 
@@ -59,13 +64,21 @@ class ActorCritic(nn.Module):
         return pack_policy(lin(self.pi), (self.mu.weight, self.mu.bias), lin(self.vf), (self.v.weight, self.v.bias), self.log_std)
 
 
+# (obs_dim, act_dim) -> floats of the in-kernel policy (TB_POLICY_FLOATS, TB_POLICY_FLOATS_HIT)
+POLICY_FLOATS_BY_DIMS = {(6, 6): _lib.POLICY_FLOATS, (12, 2): _lib.POLICY_FLOATS_HIT}
+
+
 def pack_policy(pi, mu, vf, v, log_std):
     """Flat float32 parameter vector in tb_set_policy's layout from (weight, bias) lists of the two towers: pi, vf = three
-    (W [out, in], b) pairs each; mu, v = the heads; every tensor padded to a multiple of 4 floats."""
+    (W [out, in], b) pairs each; mu, v = the heads; every tensor padded to a multiple of 4 floats.  The dimensions come from
+    the first layer (obs_dim) and the action head (act_dim)."""
     def pad(t):
         t = t.detach().reshape(-1).to(torch.float32)
         r = (-t.numel()) % 4
         return t if r == 0 else torch.cat([t, t.new_zeros(r)])
+    dims = (int(pi[0][0].shape[1]), int(mu[0].shape[0]))
+    if dims not in POLICY_FLOATS_BY_DIMS:
+        raise ValueError(f"no in-kernel policy for (obs_dim, act_dim) = {dims}; there are {sorted(POLICY_FLOATS_BY_DIMS)}")
     parts = []
     for tower, head in ((pi, mu), (vf, v)):
         for W, b in tower:
@@ -73,53 +86,59 @@ def pack_policy(pi, mu, vf, v, log_std):
         parts += [pad(head[0]), pad(head[1])]
     parts.append(pad(log_std))
     out = torch.cat(parts)
-    assert out.numel() == _lib.POLICY_FLOATS, out.numel()
+    assert out.numel() == POLICY_FLOATS_BY_DIMS[dims], (out.numel(), dims)
     return out
 
 
-class SwingPPO:
-    """PPO learner whose rollouts run on the B200 env batch.  use_graph: replay the rollout as one CUDA graph."""
+class GpuPPO:
+    """PPO learner whose rollouts run on the B200 env batch: rollout_len steps of every env per update, collected by
+    tb_policy_rollout (fused_policy) or by an eager torch policy.  use_graph: replay the rollout as one CUDA graph.
+    GAE masks with the done flags and bootstraps from the value of the observation the rollout ends with, so a rollout
+    need not hold whole episodes."""
 
-    def __init__(self, num_envs=16384, precision="f64", seed=0, lr=3e-4, epochs=10, minibatches=8, device=0, use_graph=True,
-                 fused_policy=True):
+    def __init__(self, env_id, num_envs, rollout_len, precision="f64", seed=0, lr=3e-4, epochs=10, minibatches=8, device=0,
+                 use_graph=True, fused_policy=True):
         torch.manual_seed(seed)
         self.fused_policy = fused_policy
         self.seed = seed
         self.dev = torch.device("cuda", device)
         self.n = n = int(num_envs)
-        self.env = TennisBatch("SwingRacket-v0", n, device=device, seed=seed, precision=precision)
-        self.ac = ActorCritic().to(self.dev)
+        self.K = K = int(rollout_len)
+        self.env = TennisBatch(env_id, n, device=device, seed=seed, precision=precision)
+        self.od, self.ad = od, ad = self.env.obs_dim, self.env.act_dim
+        self.ac = ActorCritic(od, ad).to(self.dev)
         self.opt = torch.optim.Adam(self.ac.parameters(), lr=lr, eps=1e-5, capturable=use_graph)
         self.epochs, self.minibatches = epochs, minibatches
         self.gamma, self.lam, self.clip, self.ent_coef, self.vf_coef, self.max_norm = 0.99, 0.95, 0.2, 0.002, 0.5, 0.5
         z = lambda *s: torch.zeros(s, device=self.dev)  # noqa: E731
-        self.obs_buf, self.act_buf = z(EPISODE, n, 6), z(EPISODE, n, 6)
-        self.logp_buf, self.rew_buf, self.done_buf, self.val_buf = z(EPISODE, n), z(EPISODE, n), z(EPISODE, n), z(EPISODE + 1, n)
-        self.done_u8 = torch.zeros((EPISODE, n), dtype=torch.uint8, device=self.dev)
-        self.params = z(_lib.POLICY_FLOATS)
+        self.obs_buf, self.act_buf = z(K, n, od), z(K, n, ad)
+        self.logp_buf, self.rew_buf, self.done_buf, self.val_buf = z(K, n), z(K, n), z(K, n), z(K + 1, n)
+        self.done_u8 = torch.zeros((K, n), dtype=torch.uint8, device=self.dev)
+        self.params = z(POLICY_FLOATS_BY_DIMS[(od, ad)])
         self.obs = self.env.reset().clone()
         self.graph = None
+        self.warmed_up = False
         self.use_graph = use_graph
         self.rollout_s = 0.0
         # one minibatch update as a CUDA graph over static buffers (the update is ~40 small kernels, 80 times per iteration)
-        self.mb = EPISODE * n // minibatches
+        self.mb = K * n // minibatches
         self.upd_graph = None
-        self.mb_obs, self.mb_act = z(self.mb, 6), z(self.mb, 6)
+        self.mb_obs, self.mb_act = z(self.mb, od), z(self.mb, ad)
         self.mb_logp, self.mb_adv, self.mb_ret = z(self.mb), z(self.mb), z(self.mb)
 
     # ------------------------------------------------------------------ rollout
     def _rollout_body(self):
-        ac, env = self.ac, self.env
+        ac, env, K = self.ac, self.env, self.K
         if self.fused_policy:
             # parameters -> the library's buffer (device to device, inside the graph: every replay sees the current weights)
             self.params.copy_(ac.packed())
             env.set_policy(self.params)
             self.obs_buf[0].copy_(self.obs)
             env.policy_rollout(self.obs_buf, self.rew_buf, self.done_u8, self.obs, actions=self.act_buf, logp=self.logp_buf,
-                               value=self.val_buf[:EPISODE], last_value=self.val_buf[EPISODE], noise_seed=self.seed + 1)
+                               value=self.val_buf[:K], last_value=self.val_buf[K], noise_seed=self.seed + 1)
             self.done_buf.copy_(self.done_u8)
             return
-        for t in range(EPISODE):
+        for t in range(K):
             mu = ac.mean(self.obs)
             a = mu + ac.log_std.exp() * torch.randn_like(mu)
             self.obs_buf[t].copy_(self.obs)
@@ -130,25 +149,27 @@ class SwingPPO:
             self.rew_buf[t].copy_(r)
             self.done_buf[t].copy_(dn)
             self.obs.copy_(o)
-        self.val_buf[EPISODE].copy_(ac.value(self.obs))
+        self.val_buf[K].copy_(ac.value(self.obs))
 
     @torch.no_grad()
     def rollout(self):
-        """One whole episode per env into the buffers; returns the statistics vector of those episodes."""
+        """rollout_len steps of every env into the buffers; returns the statistics vector of the episodes that ended in them."""
         self.env.read_stats(clear=True)
         torch.cuda.synchronize()
         t0 = time.time()
         if not self.use_graph:
             self._rollout_body()
         else:
-            if self.graph is None:  # warm up on a side stream (library state, cuBLAS handles), then capture
-                s = torch.cuda.Stream(self.dev)
-                s.wait_stream(torch.cuda.current_stream(self.dev))
-                with torch.cuda.stream(s):
-                    self._rollout_body()
-                torch.cuda.current_stream(self.dev).wait_stream(s)
-                torch.cuda.synchronize()
-                self.env.read_stats(clear=True)
+            if self.graph is None:
+                if not self.warmed_up:  # warm up on a side stream (library state, cuBLAS handles), then capture
+                    s = torch.cuda.Stream(self.dev)
+                    s.wait_stream(torch.cuda.current_stream(self.dev))
+                    with torch.cuda.stream(s):
+                        self._rollout_body()
+                    torch.cuda.current_stream(self.dev).wait_stream(s)
+                    torch.cuda.synchronize()
+                    self.env.read_stats(clear=True)
+                    self.warmed_up = True
                 self.graph = torch.cuda.CUDAGraph()
                 with torch.cuda.graph(self.graph):
                     self._rollout_body()
@@ -161,17 +182,17 @@ class SwingPPO:
 
     # ------------------------------------------------------------------ update
     def update(self):
-        n, ac = self.n, self.ac
+        n, ac, K = self.n, self.ac, self.K
         adv = torch.zeros_like(self.rew_buf)
         last = torch.zeros(n, device=self.dev)
-        for t in reversed(range(EPISODE)):
+        for t in reversed(range(K)):
             nonterm = 1.0 - self.done_buf[t]
             delta = self.rew_buf[t] + self.gamma * self.val_buf[t + 1] * nonterm - self.val_buf[t]
             last = delta + self.gamma * self.lam * nonterm * last
             adv[t] = last
-        ret = adv + self.val_buf[:EPISODE]
-        B = EPISODE * n
-        fo, fa, fl = self.obs_buf.reshape(B, 6), self.act_buf.reshape(B, 6), self.logp_buf.reshape(B)
+        ret = adv + self.val_buf[:K]
+        B = K * n
+        fo, fa, fl = self.obs_buf.reshape(B, self.od), self.act_buf.reshape(B, self.ad), self.logp_buf.reshape(B)
         fadv, fret = adv.reshape(B), ret.reshape(B)
         mb = self.mb
         for _ in range(self.epochs):
@@ -221,6 +242,15 @@ class SwingPPO:
         nn.utils.clip_grad_norm_(ac.parameters(), self.max_norm)
         self.opt.step()
 
+
+class SwingPPO(GpuPPO):
+    """PPO on SwingRacket-v0, one whole episode (26 steps) per env per update."""
+
+    def __init__(self, num_envs=16384, precision="f64", seed=0, lr=3e-4, epochs=10, minibatches=8, device=0, use_graph=True,
+                 fused_policy=True):
+        super().__init__("SwingRacket-v0", num_envs, EPISODE, precision, seed, lr, epochs, minibatches, device, use_graph,
+                         fused_policy)
+
     def train(self, iters=150, target=31.5, log=None):
         history, reached, t0 = [], None, time.time()
         for it in range(iters):
@@ -240,3 +270,67 @@ class SwingPPO:
                 "final_mean_return": history[-1]["mean_return"], "best_mean_return": max(h["mean_return"] for h in history),
                 "reference_target": target, "first_reached": reached, "wall_s": wall, "rollout_s": self.rollout_s,
                 "rollout_env_steps_per_s": iters * EPISODE * self.n / max(self.rollout_s, 1e-9), "history": history}
+
+
+class HitPPO(GpuPPO):
+    """PPO on Tennisbot-v0 (train.py): rollouts of rollout_len steps per env, not aligned to episodes (up to 1001 steps).
+    A time-out ends an episode like any other done, as in the reference (no bootstrap across it).
+
+    curriculum_total_timesteps: train.py's ProgressCallback (train.py:155-176).  At each rollout start the racket scale is
+    curriculum_scale(env_steps, total); when the stage changes, the library's racket_scale is set, every env is reset (an
+    episode runs wholly at one scale) and the rollout graph is captured again: the scene constants are kernel arguments,
+    which a captured graph holds by value.  None: the env's racket scale is left as it is."""
+
+    def __init__(self, num_envs=16384, rollout_len=128, curriculum_total_timesteps=None, precision="f64", seed=0, lr=3e-4,
+                 epochs=10, minibatches=8, device=0, use_graph=True, fused_policy=True):
+        super().__init__("Tennisbot-v0", num_envs, rollout_len, precision, seed, lr, epochs, minibatches, device, use_graph,
+                         fused_policy)
+        self.curriculum_total = curriculum_total_timesteps
+        self.env_steps = 0   # env steps of the rollouts taken so far (the curriculum's num_timesteps)
+        self.scale = None    # racket scale set by the curriculum
+        self.stages = []     # (env_steps, scale) of every stage change
+
+    def apply_curriculum(self):
+        """Set the curriculum's racket scale for the current env_steps; True when the stage changed (envs reset)."""
+        if not self.curriculum_total:
+            return False
+        s = curriculum_scale(self.env_steps, self.curriculum_total)
+        if s == self.scale:
+            return False
+        self.env.set_param("racket_scale", s)
+        self.obs.copy_(self.env.reset())
+        self.graph = None
+        self.scale = s
+        self.stages.append((self.env_steps, s))
+        return True
+
+    def rollout(self):
+        self.apply_curriculum()
+        st = super().rollout()
+        self.env_steps += self.K * self.n
+        return st
+
+    def train(self, iters=100, log=None):
+        """iters x (rollout, update).  Per iteration: the episodes that ended in the rollout, their mean return and
+        racket-ball contact steps per episode (None when no episode ended), and the racket scale."""
+        history, t0 = [], time.time()
+        for it in range(iters):
+            st = self.rollout()
+            eps = int(st[0])
+            h = {"iter": it, "env_steps": self.env_steps, "racket_scale": self.scale, "episodes": eps,
+                 "mean_return": float(st[6] / 2 ** 20 / eps) if eps else None,
+                 "hits_per_episode": float(st[2] / eps) if eps else None,
+                 "mean_length": float(st[1] / eps) if eps else None}
+            history.append(h)
+            self.update()
+            if log and (it % 10 == 0 or it == iters - 1):
+                log(f"iter {it:4d} env-steps {h['env_steps']:>11d} scale {h['racket_scale']} episodes {eps:8d} "
+                    f"return {h['mean_return']} hits/ep {h['hits_per_episode']} wall {time.time() - t0:6.1f}s")
+        wall = time.time() - t0
+        done = [h for h in history if h["episodes"]]
+        return {"envs": self.n, "rollout_len": self.K, "iters": iters, "cuda_graph_rollout": bool(self.use_graph),
+                "curriculum_total_timesteps": self.curriculum_total, "stages": self.stages,
+                "final_mean_return": done[-1]["mean_return"] if done else None,
+                "best_mean_return": max(h["mean_return"] for h in done) if done else None,
+                "wall_s": wall, "rollout_s": self.rollout_s,
+                "rollout_env_steps_per_s": iters * self.K * self.n / max(self.rollout_s, 1e-9), "history": history}
