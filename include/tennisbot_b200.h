@@ -190,9 +190,9 @@ int tb_read_stats(tb_ctx *ctx, int64_t *h_stats, int clear, void *stream); /* sy
  * HOST arrays, on the context's own stream, synchronised before returning.  Transport, by default: when every buffer is
  * pinned (cudaHostAlloc / torch pin_memory) the kernels address the host buffers themselves - actions are read and results
  * written over PCIe while the step computes, both directions at once (zero copy); pageable buffers are staged (H2D copy,
- * kernels, D2H copies).  TB_HOST_MODE = zero_copy | pipeline | staging selects one explicitly; `pipeline` steps the batch in
- * slices whose uploads, kernels and downloads overlap on the two copy engines (measured slower than zero copy on the B200
- * box, DESIGN.md section 4).  A call fails if a fast-forward launch of the context has timed out (see tb_ff_diagnostics). */
+ * kernels, D2H copies).  TB_HOST_MODE=staging stages pinned buffers too (eight GPUs stepping at once were faster staged,
+ * DESIGN.md section 4); TB_HOST_MODE=zero_copy or unset is the default above, and any other value makes the call fail.
+ * A call also fails if a fast-forward launch of the context has timed out (see tb_ff_diagnostics). */
 int tb_reset_host(tb_ctx *ctx, const uint8_t *h_mask, float *h_obs);
 int tb_step_host(tb_ctx *ctx, const float *h_actions, float *h_obs, float *h_reward, uint8_t *h_done,
                  float *h_terminal_obs, uint8_t *h_events);
@@ -202,8 +202,8 @@ int tb_launch_count(tb_ctx *ctx, int64_t *launches);
 
 /* Diagnostics of the most recent SwingRacket fast-forward (the launch of tb_step's second kernel on an env's 26th
  * step; read it before the next step): out[0] = 1 if one ran, out[1] = visits of envs to the generic full-substep path
- * (server warps), out[2] = nanoseconds until every flight had landed, out[3..13] = reserved (instrumented builds),
- * out[14] = 0 (the finishing pass overlaps the flights since round 2), out[15] = non-zero if a wait inside a fast-forward
+ * (server warps), out[2] = nanoseconds until every flight had landed, out[3..14] = 0 (reserved; the finishing pass
+ * overlaps the flights, so it has no time of its own), out[15] = non-zero if a wait inside a fast-forward
  * launch of this context has ever timed out (sticky; that launch left envs unfinished instead of hanging the device, and
  * EVERY later call on the context - tb_step, tb_step_host, tb_reset, tb_rollout, tb_read_stats - fails from then on: the
  * fault word is mirrored in mapped host memory and checked on entry without synchronising).  A wait gives up after

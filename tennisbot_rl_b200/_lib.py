@@ -8,7 +8,7 @@ import os
 from pathlib import Path
 
 PKG = Path(__file__).resolve().parent
-LIB_PATH = Path(os.environ.get("TB_LIB_PATH", PKG / "libtennisbot_b200.so"))  # override = kernel-variant experiments only
+LIB_PATH = Path(os.environ.get("TB_LIB_PATH", PKG / "libtennisbot_b200.so"))  # override: load another build, e.g. to compare two commits
 
 ENV_SWING, ENV_HIT = 0, 1
 F32, F64 = 0, 1

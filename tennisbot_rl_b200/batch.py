@@ -226,8 +226,8 @@ class TennisBatch:
     def step_host(self, actions=None, want_terminal=True, want_events=True):
         """actions: float32 [N, act_dim] host array (None = already written into host_buffers()['actions']).
         One env step inside the C call, synchronised on return.  The buffers are pinned, so by default the kernels read the
-        actions from and write the results to host memory themselves (zero copy; TB_HOST_MODE selects the sliced
-        copy-engine pipeline or plain staging instead).  Returns the pinned result arrays (overwritten by the next call)."""
+        actions from and write the results to host memory themselves (zero copy; TB_HOST_MODE=staging copies them through
+        device buffers instead).  Returns the pinned result arrays (overwritten by the next call)."""
         hb = self.host_buffers()
         if actions is not None:
             np.copyto(hb["actions"], np.asarray(actions, np.float32).reshape(self.num_envs, self.act_dim))

@@ -95,20 +95,14 @@ template <typename T> __device__ __forceinline__ T norm3(const T *a) { return M<
 template <typename T> __device__ __forceinline__ T norm3_fast(const T *a) { return M<T>::sqrt_fast(dot3(a, a)); }
 
 // ------------------------------------------------------------------------------------------------ scene
-#ifndef TB_EDGE_UNROLL
-#define TB_EDGE_UNROLL 6
-#endif
 // unroll depth of the loops over the edge tables: the entries are constant-bank loads with a lane-dependent index (long
 // latency), and a lone lane of a server warp has nothing else to overlap them with
-constexpr int kEdgeUnroll = TB_EDGE_UNROLL;
+constexpr int kEdgeUnroll = 6;
 constexpr int kBallVzEntries = 32;  // Scene::ball_vz (SwingRacket's control phase is 26 substeps long)
 constexpr int kRacketEdges = TB_RACKET_OUTLINE_N;
 constexpr int kGoalEdges = TB_GOAL_SIDES;
 
-#ifndef TB_COARSE_UNROLL
-#define TB_COARSE_UNROLL 6
-#endif
-constexpr int kCoarseEdges = 18, kCoarseUnroll = TB_COARSE_UNROLL;
+constexpr int kCoarseEdges = 18, kCoarseUnroll = 6;
 template <typename T> struct Edge {
   T ax, ay, ex, ey, inv_len2, nx, ny;
 };
@@ -387,15 +381,9 @@ constexpr int kNeedRacket = 1, kNeedFloor = 2, kNeedNet = 4, kNeedGoal = 8, kNee
 // per episode), kept out of line so the substep loop stays small.  The rows are ALWAYS solved in double, also
 // by the float32 kernel: the residual early exit makes the impulse sensitive to the sweep count, and a float
 // solve that stops one sweep apart from the double oracle moves the ball's exit velocity by ~1e-2 m/s.
-// NC > 0: exactly NC contacts, every loop over contacts and rows unrolled so that the rows live in registers (one
-// contact is the rule: a server lane of ff_kernel working alone through a chain of contact substeps used to spend most of
-// its time on the local-memory round trips of the row table); NC == 0: nc contacts, rows in local memory.  Same
-// operations in the same order either way.
-template <typename T, int NC>
-__device__ __forceinline__ void solve_impl(const Scene<T> &sc, const ContactSet<T> *cs, int nc_dyn, SolveIO<T> *io) {
+template <typename T>
+__device__ __noinline__ void solve_contacts(const Scene<T> &sc, const ContactSet<T> *cs, int nc, SolveIO<T> *io) {
   typedef double S;
-  const int nc = NC ? NC : nc_dyn;
-  constexpr int UK = NC ? NC : 1, UR = NC ? 3 : 1;  // unroll depths
   const Contact<T> *ct = cs->c;
   const S rb = sc.ball_r, inv_mb = sc.ball_inv_m, inv_ib = sc.ball_inv_i, inv_mr = sc.racket_inv_m, dt = sc.dt;
   S R[9], bv[3], bw[3], rv[3], rw[3];
@@ -413,8 +401,8 @@ __device__ __forceinline__ void solve_impl(const Scene<T> &sc, const ContactSet<
 #pragma unroll
   for (int i = 0; i < 3; ++i) { bv[i] = io->bv[i]; bw[i] = io->bw[i]; rv[i] = io->rv[i]; rw[i] = io->rw[i]; }
   S dvb[3] = {0, 0, 0}, dwb[3] = {0, 0, 0}, dva[3] = {0, 0, 0}, dwa[3] = {0, 0, 0};
-  Row<S> rows[NC ? NC : kMaxContacts][3];
-#pragma unroll UK
+  Row<S> rows[kMaxContacts][3];
+#pragma unroll 1
   for (int k = 0; k < nc; ++k) {
     const Contact<T> &c = ct[k];
     S dirs[3][3];
@@ -422,7 +410,7 @@ __device__ __forceinline__ void solve_impl(const Scene<T> &sc, const ContactSet<
     plane_space<S>(dirs[0], dirs[1], dirs[2]);
     S rbv[3] = {-rb * dirs[0][0], -rb * dirs[0][1], -rb * dirs[0][2]};
     S ra[3] = {(S)c.ra[0], (S)c.ra[1], (S)c.ra[2]};
-#pragma unroll UR
+#pragma unroll 1
     for (int r = 0; r < 3; ++r) {
       Row<S> &w = rows[k][r];
       w.u[0] = dirs[r][0]; w.u[1] = dirs[r][1]; w.u[2] = dirs[r][2];
@@ -464,7 +452,7 @@ __device__ __forceinline__ void solve_impl(const Scene<T> &sc, const ContactSet<
 #pragma unroll 1
   for (int it = 0; it < sc.iters; ++it) {
     S resid = 0;
-#pragma unroll UK
+#pragma unroll 1
     for (int k = 0; k < nc; ++k) {
       Row<S> &w = rows[k][0];
       S jd = dot3(w.u, dvb) + dot3(w.rbxu, dwb) - dot3(w.u, dva) - dot3(w.raxu, dwa);
@@ -480,7 +468,7 @@ __device__ __forceinline__ void solve_impl(const Scene<T> &sc, const ContactSet<
       S rr = dl * w.denom;  // (= dl / jinv to an ulp; feeds the early-exit test only: no division on the servers' critical path)
       if (rr * rr > resid) resid = rr * rr;
     }
-#pragma unroll UK
+#pragma unroll 1
     for (int k = 0; k < nc; ++k) {
       S lam_n = rows[k][0].lam;
       if (!(lam_n > 0)) continue;
@@ -515,14 +503,6 @@ __device__ __forceinline__ void solve_impl(const Scene<T> &sc, const ContactSet<
   }
 #pragma unroll
   for (int i = 0; i < 3; ++i) { io->dvb[i] = (T)dvb[i]; io->dwb[i] = (T)dwb[i]; io->dva[i] = (T)dva[i]; io->dwa[i] = (T)dwa[i]; }
-}
-template <typename T>
-__device__ __noinline__ void solve_contacts(const Scene<T> &sc, const ContactSet<T> *cs, int nc, SolveIO<T> *io) {
-#ifdef TB_SOLVE_UNROLL1
-  if (nc == 1) solve_impl<T, 1>(sc, cs, nc, io);
-  else
-#endif
-    solve_impl<T, 0>(sc, cs, nc, io);
 }
 
 // Narrow phase of every pair whose broad-phase test passed, one out-of-line call.  Appends to cs->c[] in the
@@ -978,11 +958,7 @@ __device__ __forceinline__ bool env_substep(const Scene<T> &sc, St<T> &s, const 
     }
     T Fb[3] = {0, 0, 0};
     if (s.step >= sc.shoot_start && s.step < sc.shoot_start + sc.shoot_frames) { Fb[0] = s.aux[0]; Fb[1] = s.aux[1]; Fb[2] = s.aux[2]; }
-#ifdef TB_HIT_GENERIC  // (A/B builds only: the generic step in line, as before hit_fast existed)
-    int bits = physics_step<T, false>(sc, s, F, zero, Fb);
-#else
     int bits = hit_physics<T>(sc, s, F, Fb);
-#endif
     int k = ++s.step;
     c.events = bits;
     if (k < sc.shoot_frames) { c.done = false; return true; }  // returns False regardless of self.done (tennisbot_env.py:138-139)
@@ -1218,9 +1194,6 @@ constexpr int kFfDone = 3;  // (returned by the step functions) the env step is 
 // only, so which path integrates a given substep never depends on the other lanes of the warp.
 // nb, nr, nw: squared speeds of ball, racket and racket spin.
 // QUICK: the outline test with its quick accept / reject first (ff_kernel's loops); else the plain loop (step_kernel).
-#ifdef TB_FF_DIAG
-__device__ unsigned long long g_diag_edge_loops, g_diag_quick_in, g_diag_quick_out, g_diag_edge_in;
-#endif
 // Around the rim: is the ball within `rim` of the hull?  pl0: its face-normal coordinate, max_side: the largest signed
 // distance to an edge line of the outline (a lower bound of the in-plane distance to it).  Beyond the plate's thickness
 // AND beyond the outline the two offsets are orthogonal, so the distance is at least their root sum of squares; taking
@@ -1253,25 +1226,15 @@ __device__ __forceinline__ int ff_classify_core(const Scene<T> &sc, const T *rp,
       // the substep loop's schedule (measured on B200: +7 % on the whole fast-forward launch).
       T q1 = pl1, q2 = pl2;
       opaque(q1); opaque(q2);
-#ifdef TB_FF_DIAG
-      if (prism_inside_fast(sc.racket, q1, q2)) atomicAdd(&g_diag_quick_in, 1ULL);
-      else if (prism_outside_fast(sc.racket, q1, q2, sc.ffp_rim)) atomicAdd(&g_diag_quick_out, 1ULL);
-#endif
       if (prism_inside_fast(sc.racket, q1, q2)) racket = true;
       else if (prism_outside_fast(sc.racket, q1, q2, sc.ffp_rim)) racket = false;
       else {  // the coarse outline decides (it contains the outline: the signed distance to its edge lines is a lower bound too)
-#ifdef TB_FF_DIAG
-        atomicAdd(&g_diag_edge_loops, 1ULL);
-#endif
         T max_side = -M<T>::inf();
 #pragma unroll kCoarseUnroll
         for (int i = 0; i < kCoarseEdges; ++i) {
           T side = (q1 - sc.racket.c_ax[i]) * sc.racket.c_nx[i] + (q2 - sc.racket.c_ay[i]) * sc.racket.c_ny[i];
           max_side = side > max_side ? side : max_side;
         }
-#ifdef TB_FF_DIAG
-        if (!(max_side > sc.ffp_rim)) atomicAdd(&g_diag_edge_in, 1ULL);
-#endif
         // (the in-plane bound alone: ff_rim_within here keeps a ball in the corner band in this lane, where it takes the edge
         // loop above every substep with the other 31 lanes waiting - measured +0.06 ms per launch, more than the servers save)
         racket = !(max_side > sc.ffp_rim);

@@ -24,15 +24,9 @@ namespace tb {
 
 constexpr int kPacks = 8;
 constexpr int kBlock = 128;     // threads per CTA of the step kernel
-#ifndef TB_MINB32
-#define TB_MINB32 5
-#endif
-#ifndef TB_MINB64
-#define TB_MINB64 4
-#endif
 // CTAs per SM ff_kernel's register budget is held to: 5 x 128 threads -> 96 regs/thread (f32), 4 -> 128 (f64); measured best on B200
-template <typename T> struct MinBlocks { static constexpr int v = TB_MINB32; };
-template <> struct MinBlocks<double> { static constexpr int v = TB_MINB64; };
+template <typename T> struct MinBlocks { static constexpr int v = 5; };
+template <> struct MinBlocks<double> { static constexpr int v = 4; };
 
 // ------------------------------------------------------------------------------------------------ pack I/O
 template <typename T> struct Pack { T x, y, z, w; };
@@ -182,11 +176,6 @@ struct StepIO {
                                      // without synchronising
   volatile unsigned long long *fault_host;
   long long spin_limit;              // clock cycles any wait inside ff_kernel may take before the launch gives up
-  int64_t env_lo, env_hi;            // step_kernel: the envs [env_lo, env_hi) of this launch (tb_step_host steps the batch in slices
-                                     // so that uploads, kernels and downloads overlap); the per-step bookkeeping belongs to the
-                                     // slice that starts at env 0
-  volatile unsigned *ff_ran_host;    // mapped host word ff_kernel sets when it had anything to do (it then wrote outputs of envs
-                                     // in any slice), or nullptr
   int server_sm_stride;              // ff_kernel: > 0 = every warp on an SM whose id is a multiple of this is a server warp and
                                      // all others are flight warps (full persistent grids); 0 = one server warp per
                                      // kServerStride CTAs
@@ -260,7 +249,7 @@ constexpr int kFlagFirst = 8;       // the flight's first substep (no external f
 constexpr int kFlagLastShift = 16;  // contact bits of the flight's last substep
 constexpr int kFlagVisitShift = 4;  // 2 bits: visits to the full path during this flight
 // counter words of one step's set
-constexpr int kCtrWords = 512;  // words that are polled never share a 128-byte line with words that are claimed from; words 128.. : TB_FF_DIAG time series
+constexpr int kCtrWords = 512;  // words that are polled never share a 128-byte line with words that are claimed from
 constexpr int kCFront = 0, kCBack = 1, kCSafe = 2, kCError = 3;
 constexpr int kDRounds = 48, kDFullEnvs = 49, kDPhase = 50, kDFinish = 62;  // tb_ff_diagnostics
 constexpr int kCFull0 = 4;        // entries of queue_full (appended by step_kernel)
@@ -364,22 +353,10 @@ __device__ __forceinline__ void finish_api(const Scene<T> &sc, const StepIO &io,
   if (io.events) io.events[me] = (uint8_t)events;
 }
 
-#ifndef TB_STEP_MINB32
-#define TB_STEP_MINB32 3
-#endif
-#ifndef TB_STEP_MINB64
-#define TB_STEP_MINB64 3
-#endif
-#ifndef TB_STEP_SWING_MINB32
-#define TB_STEP_SWING_MINB32 5
-#endif
-#ifndef TB_STEP_SWING_MINB64
-#define TB_STEP_SWING_MINB64 4
-#endif
 // CTAs per SM the register budget of step_kernel is held to.  SwingRacket's instantiation holds the straight-line control
 // substep only (everything else is deferred to ff_kernel), Tennisbot's hit_fast plus the generic physics_step out of line.
-template <typename T, int KIND> struct StepMinBlocks { static constexpr int v = KIND == TB_ENV_SWING ? TB_STEP_SWING_MINB32 : TB_STEP_MINB32; };
-template <int KIND> struct StepMinBlocks<double, KIND> { static constexpr int v = KIND == TB_ENV_SWING ? TB_STEP_SWING_MINB64 : TB_STEP_MINB64; };
+template <typename T, int KIND> struct StepMinBlocks { static constexpr int v = KIND == TB_ENV_SWING ? 5 : 3; };
+template <int KIND> struct StepMinBlocks<double, KIND> { static constexpr int v = KIND == TB_ENV_SWING ? 4 : 3; };
 
 // The counter set of the step with index e (= epoch[0] when its step_kernel starts): sets alternate, and every step_kernel
 // zeroes the set of the step after it.  Indices run 0 .. kEpochLast - 1 and wrap (an even period, so the sets keep
@@ -541,7 +518,7 @@ __global__ void __launch_bounds__(kBlock, MINB ? MINB : StepMinBlocks<T, KIND>::
   ws.init(sacc[wib], lane);
   const unsigned e = io.epoch[0];  // index of this step; constant while this grid runs (ff_kernel advances it)
   unsigned long long *qctr = ctr_set(io, e);
-  if (blockIdx.x == 0 && io.env_lo == 0) {
+  if (blockIdx.x == 0) {
     unsigned long long *next = ctr_set(io, e + 1u);
     for (int i = threadIdx.x; i < kCtrWords; i += kBlock) next[i] = 0;
     if (threadIdx.x == 0) io.epoch[1] = e + 1u;  // the tag of this step's queue slots, never 0
@@ -549,9 +526,9 @@ __global__ void __launch_bounds__(kBlock, MINB ? MINB : StepMinBlocks<T, KIND>::
     if (KIND == TB_ENV_HIT && threadIdx.x == 0) io.epoch[2] += 1u;
   }
 
-  const int64_t tile0 = io.env_lo + (int64_t)blockIdx.x * kBlock + wib * 32, me = tile0 + lane;
-  const bool valid = me < io.env_hi;
-  const int rows = io.env_hi - tile0 >= 32 ? 32 : (io.env_hi > tile0 ? (int)(io.env_hi - tile0) : 0);
+  const int64_t tile0 = (int64_t)blockIdx.x * kBlock + wib * 32, me = tile0 + lane;
+  const bool valid = me < io.n;
+  const int rows = io.n - tile0 >= 32 ? 32 : (io.n > tile0 ? (int)(io.n - tile0) : 0);
   St<T> s;
   float a[8];
   if (STAGE) {
@@ -571,8 +548,8 @@ __global__ void __launch_bounds__(kBlock, MINB ? MINB : StepMinBlocks<T, KIND>::
   // 15 % faster in float32 but slower in float64: two 35 KB stages x 3 CTAs leave almost no L1 for the rare paths'
   // local-memory records.  Measured on B200, see DESIGN.md.)
   if (!STAGE && threadIdx.x == 0 && io.prefetch_ahead > 0) {
-    const int64_t e0 = io.env_lo + ((int64_t)blockIdx.x + io.prefetch_ahead) * kBlock;
-    if (e0 + kBlock <= io.env_hi) {
+    const int64_t e0 = ((int64_t)blockIdx.x + io.prefetch_ahead) * kBlock;
+    if (e0 + kBlock <= io.n) {
       const T *b0 = static_cast<const T *>(io.state);
 #pragma unroll
       for (int p = 0; p < kPacks; ++p)
@@ -615,25 +592,10 @@ __global__ void __launch_bounds__(kBlock, MINB ? MINB : StepMinBlocks<T, KIND>::
 // contact stalled 31 other lanes and streamed ~40 KB of rare code through the instruction caches of the substep
 // loop); the same work in barrier-separated phases 4.6 - 5.0 ms (every round of "contact, then fly on" paid the latency
 // of its longest chain and longest flight); roles: see profiles/.
-#ifndef TB_FF_SERVE_MIN
-#define TB_FF_SERVE_MIN 6
-#endif
-#ifndef TB_FF_SERVE_WAIT
-#define TB_FF_SERVE_WAIT 12
-#endif
-#ifndef TB_FF_SERVER_STRIDE
-#define TB_FF_SERVER_STRIDE 2
-#endif
-#ifndef TB_FF_SERVER_LANES
-#define TB_FF_SERVER_LANES 32
-#endif
-constexpr int kServeMin = TB_FF_SERVE_MIN, kServeWait = TB_FF_SERVE_WAIT, kServerStride = TB_FF_SERVER_STRIDE, kServerLanes = TB_FF_SERVER_LANES;
+constexpr int kServeMin = 6, kServeWait = 12, kServerStride = 2;
 constexpr int kIdle = 4, kWait = 5, kRetired = 6;  // lane states 0..3 = kFfFree, kFfLand (running), kFfFull, kFfDone (leaving);
                                                    // no env; no env, holds a late-queue ticket; no env, never will
-#ifndef TB_FF_MAX_VISITS
-#define TB_FF_MAX_VISITS 3
-#endif
-constexpr int kFfMaxVisits = TB_FF_MAX_VISITS;  // an env that comes to the servers this often finishes its flight there
+constexpr int kFfMaxVisits = 3;  // an env that comes to the servers this often finishes its flight there
 __device__ __forceinline__ unsigned long long ld_ctr(const unsigned long long *p) { return *reinterpret_cast<const volatile unsigned long long *>(p); }
 __device__ __forceinline__ unsigned long long global_ns() {
   unsigned long long t;
@@ -753,18 +715,6 @@ template <typename T> __device__ __forceinline__ void ff_mark_landed(T *base, in
   base[((int64_t)7 * n + me) * 4 + 2] = int_as(T(), flags | kFlagLanded);
 }
 
-#ifdef TB_FF_DIAG
-// log of the last ~100 envs to land: final step count, substeps of the last leg, visits to the servers, where it ended
-// (0 flight warp, 1 server, 2 server running the env to its end), time: words 300.. of the counter set, two per entry
-__device__ __forceinline__ void ff_diag_late(unsigned long long *ctr, int step, int leg, int visits, int where) {
-  unsigned long long i = atomicAdd(ctr + 299, 1ULL);
-  if (i < 100) {
-    ctr[300 + 2 * i] = (unsigned long long)step | ((unsigned long long)leg << 16) | ((unsigned long long)visits << 32) | ((unsigned long long)where << 40);
-    ctr[301 + 2 * i] = global_ns();
-  }
-}
-#endif
-
 // The finishing pass for 32 envs (a tile of consecutive envs in pass 1, entries of the retry list in pass 2): complete the
 // env step of those whose flight has landed - reward (swingracket_env.py:111-126, from the contact bits of the final
 // substep), statistics, terminal observation, outputs, auto-reset - coalesced like step_kernel.  Warps run it whenever
@@ -805,9 +755,6 @@ __device__ __noinline__ void ff_finish_dense(const Scene<T> &sc, const StepIO &i
       s.step = (int)as_int(p7.y);
       s.episode = (uint32_t)as_int(p7.w);
       events = (flags >> kFlagEventShift) & 0xff;
-#ifdef TB_FF_DIAG_VISITS  // (analysis builds only: bit 7 of the events byte = the flight went through the servers)
-      if ((flags >> kFlagVisitShift) & 3) events |= 128;
-#endif
       reward = ff_reward(s, (flags >> kFlagLastShift) & 0xff);
       s.ret = p7.x + (T)reward;
       s.flags = flags & kFlagDone;  // drop every in-flight mark
@@ -898,10 +845,6 @@ __device__ __forceinline__ void ff_flight_warp(const Scene<T> &sc, const StepIO 
   bool exhausted0 = n0 == 0, first = false, first_pending = false, pass1_over = false;
   long long idle_since = 0;
   unsigned nap = 0;  // idle back-off: thousands of warps polling one cache line would starve the servers' atomics on it
-#ifdef TB_FF_DIAG
-  int src = 0;
-  const unsigned long long ts0 = global_ns();
-#endif
   for (;;) {
     // ---- substeps until enough lanes want to leave / claim (no call, no rare code in this loop)
     unsigned run_m, leave_m;
@@ -934,13 +877,7 @@ __device__ __forceinline__ void ff_flight_warp(const Scene<T> &sc, const StepIO 
         nsub += L.step - step0;
         flags = kFlagInFlight | (L.events << kFlagEventShift) | (visits << kFlagVisitShift);
         if (landed) flags |= TB_EV_COURT_BALL << kFlagLastShift;
-#ifdef TB_FF_DIAG
-        if (landed && ld_ctr(ctr + kCLanded) + 100 >= (unsigned long long)total0 + ld_ctr(ctr + kCDynTotal)) ff_diag_late(ctr, L.step, L.step - step0, visits, 0);
-#endif
         ff_store(base, io.n, (int64_t)me, L, flags);
-#ifdef TB_FF_DIAG
-        if (to_full) { atomicAdd(ctr + 92 + src, 1ULL); atomicAdd(ctr + 95 + src, (unsigned long long)(L.step - 26)); }
-#endif
       }
       dq_push(io.dq_full, io.dq_cap, ctr + kCFullTail, epoch, to_full, me, lane, ctr + kCError);
       unsigned done_m = __ballot_sync(full, landed);
@@ -951,30 +888,12 @@ __device__ __forceinline__ void ff_flight_warp(const Scene<T> &sc, const StepIO 
       }
       if (to_full || landed) st = kIdle;
     }
-#ifdef TB_FF_DIAG
-    if (blockIdx.x == 0 && threadIdx.x == 0) {
-      unsigned long long ld = ld_ctr(ctr + kCLanded), t = global_ns(), tot = (unsigned long long)total0 + ld_ctr(ctr + kCDynTotal);
-      if (!ctr[kDPhase + 1] && ld * 2 >= tot) ctr[kDPhase + 1] = t;
-      if (!ctr[kDPhase + 2] && ld * 10 >= tot * 9) ctr[kDPhase + 2] = t;
-      if (!ctr[kDPhase + 3] && ld * 100 >= tot * 99) ctr[kDPhase + 3] = t;
-      int bin = (int)((t - ts0) / 100000ULL);
-      if (bin < 34 && !ctr[128 + 5 * bin]) {
-        ctr[128 + 5 * bin] = ld + 1; ctr[129 + 5 * bin] = ld_ctr(ctr + kCClaim0); ctr[130 + 5 * bin] = ld_ctr(ctr + kCFullTail);
-        ctr[131 + 5 * bin] = ld_ctr(ctr + kCLateTail); ctr[132 + 5 * bin] = ld_ctr(ctr + kCLateHead);
-      }
-    }
-#endif
     // ---- lanes without an env: the next entries of step_kernel's queue (one atomic per warp); once that is empty, a
     //      ticket each for the late queue, polled here every time round
     bool got = false;
     if (st == kWait) {
       int e = dq_poll(io.dq_late, ticket, epoch);
-      if (e >= 0) {
-        me = e; got = true;
-#ifdef TB_FF_DIAG
-        src = 2;
-#endif
-      }
+      if (e >= 0) { me = e; got = true; }
     }
     unsigned idle = __ballot_sync(full, st == kIdle);
     if (idle) {
@@ -1011,9 +930,6 @@ __device__ __forceinline__ void ff_flight_warp(const Scene<T> &sc, const StepIO 
         if (st == kIdle && idx < n0) {
           me = __ldcg(idx < qfront ? io.queue + idx : idx < qmid ? io.queue + (io.n - 1 - (idx - qfront)) : io.queue_full + (io.n - 1 - (idx - qmid)));
           got = true;
-#ifdef TB_FF_DIAG
-          src = idx < qfront ? 0 : 1;  // (last-to-start entries count as back)
-#endif
         }
       }
     }
@@ -1072,9 +988,6 @@ __device__ __noinline__ void ff_server_warp(const Scene<T> &sc, const StepIO &io
   bool exhausted0 = nfull0 == 0, busy = false, to_end = false, waiting = false;
   long long idle_since = 0, ticket = 0;
   unsigned nap = 0;
-#ifdef TB_FF_DIAG
-  int chain = 0;
-#endif
   FfLane<T> L;
   {
     T *z = reinterpret_cast<T *>(&L);
@@ -1083,30 +996,17 @@ __device__ __noinline__ void ff_server_warp(const Scene<T> &sc, const StepIO &io
     L.step = 0; L.events = 0;
   }
   int me = 0, r = kFfDone, phase = 2, last = 0, visits = 0, step0 = 0;
-#ifdef TB_FF_DIAG
-  const unsigned long long ts0 = global_ns();
-#endif
   for (;;) {
-#ifdef TB_FF_DIAG
-    if (blockIdx.x == 0 && lane == 0) {
-      int bin = (int)((global_ns() - ts0) / 100000ULL);
-      if (bin < 34 && !ctr[128 + 5 * bin]) {
-        ctr[128 + 5 * bin] = ld_ctr(ctr + kCLanded) + 1; ctr[129 + 5 * bin] = ld_ctr(ctr + kCClaim0); ctr[130 + 5 * bin] = ld_ctr(ctr + kCFullTail);
-        ctr[131 + 5 * bin] = ld_ctr(ctr + kCLateTail); ctr[132 + 5 * bin] = ld_ctr(ctr + kCLateHead);
-      }
-    }
-#endif
     // ---- lanes without an env: step_kernel's list (envs whose first fast-forward substep is a full one), then a ticket
-    //      each for the full queue.  At most kServerLanes envs at a time: lanes on different rare paths run one after
-    //      the other, so every busy lane lengthens the warp's iteration.
+    //      each for the full queue.
     bool got = false;
     if (waiting) {
       int e = dq_poll(io.dq_full, ticket, epoch);
       if (e >= 0) { me = e; got = true; waiting = false; }
     }
     const unsigned held = __ballot_sync(full, busy || waiting || got);
-    if (__popc(held) < kServerLanes) {
-      const unsigned cand = ~held & (kServerLanes >= 32 ? 0xffffffffu : (1u << (kServerLanes & 31)) - 1u);  // lanes 0 .. kServerLanes-1 only ever hold envs
+    if (held != full) {
+      const unsigned cand = ~held;
       if (!exhausted0) {
         const int want = __popc(cand);
         long long at = 0;
@@ -1120,17 +1020,11 @@ __device__ __noinline__ void ff_server_warp(const Scene<T> &sc, const StepIO &io
         if (((cand >> lane) & 1u) && t < io.dq_cap) { ticket = t; waiting = true; }
       }
     }
-#ifdef TB_FF_DIAG
-    const long long tl0 = clock64();
-#endif
     if (got) {
       int flags = ff_load(base, io.n, (int64_t)me, L);
       phase = (flags & kFlagFirst) ? 1 : 2;
       visits = min(((flags >> kFlagVisitShift) & 3) + 1, 3);
       to_end = visits >= kFfMaxVisits;
-#ifdef TB_FF_DIAG
-      if (to_end) atomicAdd(ctr + kDPhase + 6, 1ULL);
-#endif
       step0 = L.step;
       last = 0;
       // no classification here: the lane that parked the env found it within reach of something, and the substep functions
@@ -1138,9 +1032,6 @@ __device__ __noinline__ void ff_server_warp(const Scene<T> &sc, const StepIO &io
       L.nb = dot3(L.bv, L.bv); L.nr = dot3(L.rv, L.rv); L.nw = dot3(L.wl, L.wl);
       r = kFfFull;
       busy = true;
-#ifdef TB_FF_DIAG
-      atomicAdd(ctr + 108, 1ULL); atomicAdd(ctr + 109, (unsigned long long)(clock64() - tl0));
-#endif
     }
     if (!__any_sync(full, busy)) {  // nothing to do: done when every flight has landed
       if (ff_all_landed(ctr, nctl, total0) || ld_ctr(ctr + kCError) != 0) break;
@@ -1156,38 +1047,10 @@ __device__ __noinline__ void ff_server_warp(const Scene<T> &sc, const StepIO &io
     // ---- one substep per busy lane
     bool leave = false;
     int lflags = 0;
-#ifdef TB_FF_DIAG
-    long long tb0 = clock64();
-    if (busy) ++chain;
-#endif
     if (busy) {
-#ifdef TB_FF_DIAG
-      atomicAdd(ctr + kDPhase + (r == kFfFull ? 4 : 5), 1ULL);
-#endif
       if (r == kFfFull) {
-#ifdef TB_FF_DIAG
-        const long long tc0 = clock64();
-#endif
-#ifndef TB_FF_NO_LEAN
         int rl = ff_contact_lean<T>(sc, &L, phase, &last);  // ball against a racket face, high above the court: the short cut
-#else
-        int rl = -1;
-#endif
-#ifdef TB_FF_DIAG
-        const long long tc1 = clock64();
-        atomicAdd(ctr + (rl < 0 ? 102 : 100), 1ULL); atomicAdd(ctr + (rl < 0 ? 103 : 101), (unsigned long long)(tc1 - tc0));
-#endif
-        if (rl < 0) {
-          rl = ff_full<T>(sc, &L, phase, &last);
-#ifdef TB_FF_DIAG
-          atomicAdd(ctr + 104, (unsigned long long)(clock64() - tc1));
-          if (last & TB_EV_RACKET_BALL) atomicAdd(ctr + 105, 1ULL);
-          if (last & ~(TB_EV_RACKET_BALL | TB_EV_RACKET_LOW)) atomicAdd(ctr + 106, 1ULL);
-#endif
-        }
-#ifdef TB_FF_DIAG
-        else if (last & TB_EV_RACKET_BALL) atomicAdd(ctr + 107, 1ULL);
-#endif
+        if (rl < 0) rl = ff_full<T>(sc, &L, phase, &last);
         r = rl;
       } else {  // (to_end, or a rounding-level disagreement with the classification that queued the env)
         if (phase == 1) {  // the force-free first substep (see ff_flight_warp)
@@ -1206,35 +1069,12 @@ __device__ __noinline__ void ff_server_warp(const Scene<T> &sc, const StepIO &io
       leave = r == kFfDone || (r != kFfFull && !to_end);
       if (leave) {
         *nsub += L.step - step0;
-#ifdef TB_FF_DIAG
-        if (r == kFfDone && ld_ctr(ctr + kCLanded) + 100 >= (unsigned long long)total0 + ld_ctr(ctr + kCDynTotal)) ff_diag_late(ctr, L.step, L.step - step0, visits, 1 + (to_end ? 1 : 0));
-#endif
         lflags = kFlagInFlight | (L.events << kFlagEventShift) | (visits << kFlagVisitShift);
         if (r == kFfDone) lflags |= last << kFlagLastShift;
         ff_store(base, io.n, (int64_t)me, L, lflags);
         busy = false;
-#ifdef TB_FF_DIAG
-        atomicMax(ctr + kDPhase + 8, (unsigned long long)chain);
-        chain = 0;
-#endif
       }
     }
-#ifdef TB_FF_DIAG
-    {
-      const unsigned bm = __ballot_sync(full, busy || leave);
-      if (bm && lane == 0) {
-        const unsigned long long dtc = (unsigned long long)(clock64() - tb0), tn = global_ns();
-        atomicAdd(ctr + kDPhase + 9, 1ULL);
-        atomicAdd(ctr + kDPhase + 10, dtc);
-        atomicMax(ctr + kDPhase + 11, tn);
-        // iteration time by the number of lanes that took a substep (1, 2, 3-4, 5-8, 9-16, 17-32): words 112.. for
-        // the whole launch, 80.. for iterations later than 1.5 ms into it
-        const int nb = __popc(bm), bin = nb <= 1 ? 0 : 32 - __clz(nb - 1);
-        atomicAdd(ctr + 112 + 2 * bin, 1ULL); atomicAdd(ctr + 113 + 2 * bin, dtc);
-        if (tn - ts0 > 1500000ULL) { atomicAdd(ctr + 80 + 2 * bin, 1ULL); atomicAdd(ctr + 81 + 2 * bin, dtc); }
-      }
-    }
-#endif
     const bool landed = leave && r == kFfDone;
     dq_push(io.dq_late, io.dq_cap, ctr + kCLateTail, epoch, leave && r != kFfDone, me, lane, ctr + kCError);
     unsigned done_m = __ballot_sync(full, landed);
@@ -1331,7 +1171,6 @@ __global__ void __launch_bounds__(kBlock, MinBlocks<T>::v) ff_kernel(const __gri
                   qn0 = qmid + (long long)ctr[kCSafe], nfull0 = (long long)ctr[kCFull0];
   const long long total0 = qn0 + nfull0;
   if (nctl == 0 && total0 == 0) return;
-  if (io.ff_ran_host && blockIdx.x == 0 && threadIdx.x == 0) *io.ff_ran_host = 1u;
   WarpStats ws;
   ws.init(sacc[wib], lane);
   // No CTA ever waits for a particular other CTA: all work - deferred control substeps, flights, parked envs - is claimed
@@ -1366,13 +1205,7 @@ __global__ void __launch_bounds__(kBlock, MinBlocks<T>::v) ff_kernel(const __gri
   if (server) ff_server_warp<T>(sc, io, epoch, nfull0, nctl, total0, &ws, &nsub);
   else ff_flight_warp<T>(sc, io, epoch, qn0, qfront, qmid, nctl, total0, ws, nsub);
   if (diag) {
-    unsigned long long t = global_ns();
-#ifdef TB_FF_DIAG
-    for (int i = 1; i <= 3; ++i) ctr[kDPhase + i] = ctr[kDPhase + i] ? ctr[kDPhase + i] - t_mark : 0;
-    ctr[kDPhase + 7] = ld_ctr(ctr + kCLateTail);
-    ctr[kDPhase + 11] = ctr[kDPhase + 11] ? ctr[kDPhase + 11] - t_mark : 0;
-#endif
-    ctr[kDPhase] = t - t_mark;
+    ctr[kDPhase] = global_ns() - t_mark;
     ctr[kDRounds] = 1;
     ctr[kDFullEnvs] = ld_ctr(ctr + kCFullTail) + (unsigned long long)nfull0;
     ctr[kDFinish] = 0;
@@ -2074,18 +1907,11 @@ struct tb_ctx {
   long long spin_limit = 0;                  // clock cycles, see StepIO (TB_FF_SPIN_LIMIT_MS, default 4000 ms)
   unsigned long long *queue_ctrs = nullptr;  // two counter sets (kCtrWords each) used by alternate steps
   unsigned ff_grid = 0;                      // persistent grid of ff_kernel
-  int ff_server_sm_stride = 0;               // see StepIO (set with the grid size; TB_FF_SERVER_SM_STRIDE overrides, 0 = per-CTA roles)
+  int ff_server_sm_stride = 0;               // see StepIO (set with the grid size, 0 = per-CTA roles)
   int step_resident = -1;                    // resident CTAs of step_kernel (its L2 prefetch distance)
   bool one_wave4 = false;                    // Tennisbot-v0: launch the 4-CTAs-per-SM build of step_kernel (see its MINB)
-  bool pdl = std::getenv("TB_NO_PDL") == nullptr;  // programmatic dependent launch of the step's kernels
   int control_mode = TB_CONTROL_FORCE;
   void *pid = nullptr;                       // controller memory, allocated by tb_set_control_mode(TB_CONTROL_PID)
-  bool zero_copy = std::getenv("TB_HOST_STAGING") == nullptr;  // tb_step_host: address pinned host buffers from the kernels
-  // tb_step_host's pipelined mode: the batch in slices, uploads / kernels / downloads of different slices overlapping
-  static constexpr int kMaxSlices = 8;
-  cudaStream_t s_up = nullptr, s_dn = nullptr;
-  cudaEvent_t ev_up[kMaxSlices] = {}, ev_k[kMaxSlices] = {};
-  unsigned *h_ffran = nullptr, *h_ffran_dev = nullptr;  // mapped host word, see StepIO::ff_ran_host
   float *policy = nullptr;                   // tb_policy_floats(env_kind) parameters (tb_set_policy)
   float *pol_act = nullptr;                  // [N, act_dim] clipped actions handed from policy_kernel to step_kernel
   bool timing = false;                       // tb_set_kernel_timing
@@ -2134,7 +1960,6 @@ static StepIO make_io(tb_ctx *c) {
   std::memset(&io, 0, sizeof io);
   io.state = c->state; io.n = c->cfg.num_envs; io.id_offset = c->cfg.env_id_offset; io.seed = c->cfg.seed;
   io.auto_reset = c->cfg.auto_reset; io.stats = c->stats; io.k_steps = 1;
-  io.env_lo = 0; io.env_hi = c->cfg.num_envs;
   io.pid = c->control_mode == TB_CONTROL_PID ? c->pid : nullptr;
   return io;
 }
@@ -2170,11 +1995,9 @@ template <typename T> static int ff_grid_size(tb_ctx *c, unsigned *grid) {
   int64_t resident = (int64_t)sms * (per_sm > 0 ? per_sm : 1);
   int64_t need = (c->cfg.num_envs + kBlock - 1) / kBlock;
   *grid = (unsigned)(need < resident ? need : resident);
-  {
-    const char *e = std::getenv("TB_FF_SERVER_SM_STRIDE");
-    int stride = e ? std::atoi(e) : 12;  // measured on B200 (1 Mi envs, f64): 12 -> 2.46 ms per fast-forward launch, 8 -> 2.59, 16 -> 2.99, per-CTA roles 2.60
-    c->ff_server_sm_stride = (need >= resident && stride > 0 && stride <= sms) ? stride : 0;
-  }
+  // server SMs every 12th: measured on B200 (1 Mi envs, f64) 2.46 ms per fast-forward launch, stride 8 2.59, 16 2.99,
+  // per-CTA roles 2.60
+  c->ff_server_sm_stride = need >= resident ? 12 : 0;
   return 0;
 }
 // CTAs of step_kernel that are resident at a time = how far ahead its L2 prefetch reaches.
@@ -2182,7 +2005,7 @@ template <typename T, int KIND> static int step_resident_ctas(tb_ctx *c) {
   int per_sm = 0, sms = 0;
   CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, step_kernel<T, KIND, false>, kBlock, 0));
   CU(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, c->cfg.device));
-  c->step_resident = std::getenv("TB_NO_PREFETCH") ? 0 : sms * (per_sm > 0 ? per_sm : 1);
+  c->step_resident = sms * (per_sm > 0 ? per_sm : 1);
   if (KIND == TB_ENV_HIT) {  // see step_kernel's MINB
     int per_sm4 = 0;
     CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm4, step_kernel<T, TB_ENV_HIT, false, 4>, kBlock, 0));
@@ -2192,13 +2015,13 @@ template <typename T, int KIND> static int step_resident_ctas(tb_ctx *c) {
   return 0;
 }
 template <typename... KArgs, typename... Args>
-static cudaError_t launch_pdl(bool pdl, void (*kernel)(KArgs...), dim3 grid, cudaStream_t stream, Args &&...args) {
+static cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, cudaStream_t stream, Args &&...args) {
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = grid; cfg.blockDim = dim3(kBlock); cfg.dynamicSmemBytes = 0; cfg.stream = stream;
   cudaLaunchAttribute at[1];
   at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   at[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = at; cfg.numAttrs = pdl ? 1 : 0;
+  cfg.attrs = at; cfg.numAttrs = 1;
   return cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
 }
 // One env step = step_kernel (+ ff_kernel for SwingRacket) on `stream`.
@@ -2210,22 +2033,22 @@ static void fill_io(tb_ctx *c, StepIO &io) {
   io.epoch = c->epoch;  // (a slot written 2^32 steps ago with the same tag would have to survive untouched)
   io.queue_ctrs = c->queue_ctrs;
 }
-// step_kernel for the envs [io.env_lo, io.env_hi) on `stream`
+// step_kernel for the whole batch on `stream`
 static int launch_step_kernel(tb_ctx *c, StepIO &io, cudaStream_t stream, bool stage) {
-  const unsigned grid = grid_for(io.env_hi - io.env_lo, kBlock);
+  const unsigned grid = grid_for(io.n, kBlock);
   const bool swing = c->cfg.env_kind == TB_ENV_SWING;
 #define TB_LAUNCH_STEP(T, K, SC)                                                                           \
   do {                                                                                                    \
     if (stage) {                                                                                          \
-      CU(launch_pdl(c->pdl, step_kernel<T, K, true>, grid, stream, SC, io));                             \
+      CU(launch_pdl(step_kernel<T, K, true>, grid, stream, SC, io));                                      \
     } else {                                                                                              \
       if (c->step_resident < 0 && step_resident_ctas<T, K>(c)) return 1;                                  \
       io.prefetch_ahead = c->step_resident;                                                               \
       if (K == TB_ENV_HIT && c->one_wave4) {                                                              \
         io.prefetch_ahead = 0;                                                                            \
-        CU(launch_pdl(c->pdl, step_kernel<T, TB_ENV_HIT, false, 4>, grid, stream, SC, io));               \
+        CU(launch_pdl(step_kernel<T, TB_ENV_HIT, false, 4>, grid, stream, SC, io));                       \
       } else {                                                                                            \
-        CU(launch_pdl(c->pdl, step_kernel<T, K, false>, grid, stream, SC, io));                          \
+        CU(launch_pdl(step_kernel<T, K, false>, grid, stream, SC, io));                                   \
       }                                                                                                   \
     }                                                                                                     \
   } while (0)
@@ -2247,11 +2070,11 @@ static int launch_ff_kernel(tb_ctx *c, StepIO &io, cudaStream_t stream) {
   if (c->cfg.precision == TB_F64) {
     if (!c->ff_grid && ff_grid_size<double>(c, &c->ff_grid)) return 1;
     io.server_sm_stride = c->ff_server_sm_stride;
-    CU(launch_pdl(c->pdl, ff_kernel<double>, c->ff_grid, stream, c->sc64, io));
+    CU(launch_pdl(ff_kernel<double>, c->ff_grid, stream, c->sc64, io));
   } else {
     if (!c->ff_grid && ff_grid_size<float>(c, &c->ff_grid)) return 1;
     io.server_sm_stride = c->ff_server_sm_stride;
-    CU(launch_pdl(c->pdl, ff_kernel<float>, c->ff_grid, stream, c->sc32, io));
+    CU(launch_pdl(ff_kernel<float>, c->ff_grid, stream, c->sc32, io));
   }
   c->launches++;
   CU(cudaGetLastError());
@@ -2420,10 +2243,6 @@ int tb_destroy(tb_ctx *c) {
   for (int i = 0; i < 3; ++i) if (c->ev[i]) cudaEventDestroy(c->ev[i]);
   cudaFree(c->state); cudaFree(c->stats); cudaFree(c->queue_ctrs); cudaFree(c->queue); cudaFree(c->dq); cudaFree(c->epoch); cudaFree(c->fault); cudaFree(c->queue_full); cudaFree(c->queue_ctl); cudaFree(c->pid); cudaFree(c->policy); cudaFree(c->pol_act);
   if (c->h_fault) cudaFreeHost(c->h_fault);
-  if (c->h_ffran) cudaFreeHost(c->h_ffran);
-  if (c->s_up) cudaStreamDestroy(c->s_up);
-  if (c->s_dn) cudaStreamDestroy(c->s_dn);
-  for (int i = 0; i < tb_ctx::kMaxSlices; ++i) { if (c->ev_up[i]) cudaEventDestroy(c->ev_up[i]); if (c->ev_k[i]) cudaEventDestroy(c->ev_k[i]); }
   cudaFree(c->d_actions); cudaFree(c->d_obs); cudaFree(c->d_reward); cudaFree(c->d_term);
   cudaFree(c->d_done); cudaFree(c->d_events); cudaFree(c->d_mask);
   delete c;
@@ -2488,9 +2307,7 @@ static int step_impl(tb_ctx *c, const float *d_actions, float *d_obs, float *d_r
 }
 int tb_step(tb_ctx *c, const float *d_actions, float *d_obs, float *d_reward, uint8_t *d_done, float *d_terminal_obs,
             uint8_t *d_events, void *stream) {
-  // TB_STEP_STAGE (measurements, tools/e2e_paths_probe.py): the kernel build that tb_step_host's zero copy uses
-  static const bool stage = std::getenv("TB_STEP_STAGE") != nullptr;
-  return step_impl(c, d_actions, d_obs, d_reward, d_done, d_terminal_obs, d_events, stream, stage);
+  return step_impl(c, d_actions, d_obs, d_reward, d_done, d_terminal_obs, d_events, stream, false);
 }
 
 int tb_rollout(tb_ctx *c, int action_mode, int k_steps, float *d_obs, float *d_reward_sum, int32_t *d_done_count, void *stream) {
@@ -2542,7 +2359,7 @@ int tb_policy_rollout(tb_ctx *c, int k_steps, int deterministic, uint64_t noise_
     pio.act_raw = d_actions ? d_actions + (size_t)t * n * ad : nullptr;
     pio.logp = d_logp ? d_logp + (size_t)t * n : nullptr;
     pio.value = d_value ? d_value + (size_t)t * n : nullptr;
-    CU(launch_pdl(c->pdl, kernel, dim3(grid, 2), s, pio));
+    CU(launch_pdl(kernel, dim3(grid, 2), s, pio));
     c->launches++;
     StepIO io = make_io(c);
     io.actions = c->pol_act;
@@ -2552,7 +2369,7 @@ int tb_policy_rollout(tb_ctx *c, int k_steps, int deterministic, uint64_t noise_
   }
   if (d_last_value) {  // bootstrap value of the observation the rollout ends with
     pio.obs = d_last_obs; pio.act_raw = nullptr; pio.act_env = nullptr; pio.logp = nullptr; pio.value = d_last_value;
-    CU(launch_pdl(c->pdl, kernel, dim3(grid, 2), s, pio));
+    CU(launch_pdl(kernel, dim3(grid, 2), s, pio));
     c->launches++;
   }
   CU(cudaGetLastError());
@@ -2635,93 +2452,25 @@ static void *mapped_alias(const void *h) {
   return at.type == cudaMemoryTypeHost ? at.devicePointer : nullptr;
 }
 
-// tb_step_host for large batches and pinned buffers: the batch is stepped in slices.  The actions of every slice go up on
-// the upload stream (copy engine), each slice's step_kernel waits for its own upload, and its outputs go down on the
-// download stream (the other copy engine) while later slices are still uploading and stepping: both directions of the link
-// carry data at the same time (B200 box: 42 GB/s up and 53 GB/s down, 92 GB/s together) instead of the kernels reading and
-// writing host memory themselves (~60 GB/s in both directions together).  ff_kernel follows the last slice; when it had
-// anything to do (deferred control substeps, flights - it says so in a mapped host word) it wrote outputs of envs whose slice
-// may have gone down already, and all outputs are copied once more.
-static int step_host_pipelined(tb_ctx *c, const float *h_actions, float *h_obs, float *h_reward, uint8_t *h_done, float *h_terminal_obs,
-                               uint8_t *h_events, int slices) {
-  const int64_t n = c->cfg.num_envs;
-  const size_t od = (size_t)tb_obs_dim(c->cfg.env_kind), ad = (size_t)tb_act_dim(c->cfg.env_kind);
-  if (ensure_staging(c)) return 1;
-  if (!c->s_up) {
-    CU(cudaStreamCreateWithFlags(&c->s_up, cudaStreamNonBlocking));
-    CU(cudaStreamCreateWithFlags(&c->s_dn, cudaStreamNonBlocking));
-    for (int i = 0; i < tb_ctx::kMaxSlices; ++i) {
-      CU(cudaEventCreateWithFlags(&c->ev_up[i], cudaEventDisableTiming));
-      CU(cudaEventCreateWithFlags(&c->ev_k[i], cudaEventDisableTiming));
-    }
-    CU(cudaHostAlloc((void **)&c->h_ffran, sizeof(unsigned), cudaHostAllocMapped));
-    CU(cudaHostGetDevicePointer((void **)&c->h_ffran_dev, c->h_ffran, 0));
-  }
-  cudaStream_t s = c->own_stream;
-  *c->h_ffran = 0;
-  StepIO io = make_io(c);
-  fill_io(c, io);
-  io.actions = c->d_actions; io.obs = c->d_obs; io.reward = c->d_reward; io.done = c->d_done;
-  io.term_obs = h_terminal_obs ? c->d_term : nullptr; io.events = h_events ? c->d_events : nullptr;
-  io.ff_ran_host = c->h_ffran_dev;
-  const int64_t per = ((n + slices - 1) / slices + kBlock - 1) / kBlock * kBlock;  // whole CTAs per slice
-  for (int k = 0; k < slices; ++k) {
-    const int64_t lo = std::min<int64_t>(n, k * per), hi = std::min<int64_t>(n, lo + per);
-    if (hi > lo) CU(cudaMemcpyAsync(c->d_actions + lo * ad, h_actions + lo * ad, (size_t)(hi - lo) * ad * sizeof(float), cudaMemcpyHostToDevice, c->s_up));
-    CU(cudaEventRecord(c->ev_up[k], c->s_up));
-  }
-  for (int k = 0; k < slices; ++k) {
-    const int64_t lo = std::min<int64_t>(n, k * per), hi = std::min<int64_t>(n, lo + per);
-    if (hi <= lo) continue;
-    CU(cudaStreamWaitEvent(s, c->ev_up[k], 0));
-    io.env_lo = lo; io.env_hi = hi;
-    if (launch_step_kernel(c, io, s, false)) return 1;
-    CU(cudaEventRecord(c->ev_k[k], s));
-    CU(cudaStreamWaitEvent(c->s_dn, c->ev_k[k], 0));
-    const size_t m = (size_t)(hi - lo);
-    CU(cudaMemcpyAsync(h_obs + lo * od, c->d_obs + lo * od, m * od * sizeof(float), cudaMemcpyDeviceToHost, c->s_dn));
-    CU(cudaMemcpyAsync(h_reward + lo, c->d_reward + lo, m * sizeof(float), cudaMemcpyDeviceToHost, c->s_dn));
-    CU(cudaMemcpyAsync(h_done + lo, c->d_done + lo, m, cudaMemcpyDeviceToHost, c->s_dn));
-    if (h_terminal_obs) CU(cudaMemcpyAsync(h_terminal_obs + lo * od, c->d_term + lo * od, m * od * sizeof(float), cudaMemcpyDeviceToHost, c->s_dn));
-    if (h_events) CU(cudaMemcpyAsync(h_events + lo, c->d_events + lo, m, cudaMemcpyDeviceToHost, c->s_dn));
-  }
-  io.env_lo = 0; io.env_hi = n;
-  if (launch_ff_kernel(c, io, s)) return 1;
-  CU(cudaStreamSynchronize(s));
-  CU(cudaStreamSynchronize(c->s_dn));
-  if (*reinterpret_cast<volatile unsigned *>(c->h_ffran)) {
-    const size_t m = (size_t)n;
-    CU(cudaMemcpyAsync(h_obs, c->d_obs, m * od * sizeof(float), cudaMemcpyDeviceToHost, s));
-    CU(cudaMemcpyAsync(h_reward, c->d_reward, m * sizeof(float), cudaMemcpyDeviceToHost, s));
-    CU(cudaMemcpyAsync(h_done, c->d_done, m, cudaMemcpyDeviceToHost, s));
-    if (h_terminal_obs) CU(cudaMemcpyAsync(h_terminal_obs, c->d_term, m * od * sizeof(float), cudaMemcpyDeviceToHost, s));
-    if (h_events) CU(cudaMemcpyAsync(h_events, c->d_events, m, cudaMemcpyDeviceToHost, s));
-    CU(cudaStreamSynchronize(s));
-  }
-  return check_fault(c, "tb_step_host");
-}
-
 int tb_step_host(tb_ctx *c, const float *h_actions, float *h_obs, float *h_reward, uint8_t *h_done, float *h_terminal_obs,
                  uint8_t *h_events) {
   GUARD(c);
   if (!h_actions || !h_obs || !h_reward || !h_done) return fail("%s", "tb_step_host: actions, obs, reward and done are required");
   if (check_fault(c, "tb_step_host")) return 1;
+  // Transport: zero copy for pinned buffers, staging for pageable ones and for pinned ones when TB_HOST_MODE=staging.
+  // Measured on the B200 box, 1 Mi SwingRacket envs, per step averaged over episodes: zero copy 0.92 ms, staging 1.24 ms
+  // (a sliced copy-engine pipeline: 1.19 ms).  The link carries 50 GB/s either way alone and 80-92 GB/s both ways at once
+  // (0.63-0.68 ms for a step's 55.6 MB through the copy engines); a zero-copy light step is 0.77 ms (72 GB/s,
+  // tools/e2e_paths_probe.py).  Reading the actions in place and copying only the results down was measured too: 0.93 ms
+  // per light step.  Staging stays selectable because eight GPUs stepping at once measured 2.91e9 env-steps/s staged
+  // against 2.71e9 zero copy: the host side of PCIe saturates, which the library cannot observe.
+  const char *mode = std::getenv("TB_HOST_MODE");
+  const bool staging = mode && !std::strcmp(mode, "staging");
+  if (mode && *mode && !staging && std::strcmp(mode, "zero_copy"))
+    return fail("tb_step_host: TB_HOST_MODE='%s' is neither zero_copy nor staging", mode);
   size_t n = (size_t)c->cfg.num_envs, od = (size_t)tb_obs_dim(c->cfg.env_kind), ad = (size_t)tb_act_dim(c->cfg.env_kind);
   cudaStream_t s = c->own_stream;
-  // mode: TB_HOST_MODE = zero_copy (default for pinned buffers) | pipeline | staging (pageable memory always takes it).
-  // Measured on the B200 box, 1 Mi SwingRacket envs, per step averaged over episodes: zero copy 0.92 ms, pipeline 1.19 ms,
-  // staging 1.24 ms.  The link carries 50 GB/s either way alone and 80-92 GB/s both ways at once (0.63-0.68 ms for a step's
-  // 55.6 MB through the copy engines); a zero-copy light step is 0.77 ms (72 GB/s, tools/e2e_paths_probe.py).  The pipeline's
-  // device time line (8 slices): uploads slowed to 33 GB/s by the concurrent downloads, 0.72 ms, then 0.16 ms for the last
-  // slice's results - and every fast-forward step copies the outputs twice.  Reading the actions in place and copying only the
-  // results down ("hybrid") was measured too: kernel slices 97 us instead of 63, 0.93 ms per light step.
-  const char *mode = std::getenv("TB_HOST_MODE");
-  const bool pinned = mapped_alias(h_actions) && mapped_alias(h_obs) && mapped_alias(h_reward) && mapped_alias(h_done) &&
-                      (mapped_alias(h_terminal_obs) || !h_terminal_obs) && (mapped_alias(h_events) || !h_events);
-  const bool want_pipeline = mode && !std::strcmp(mode, "pipeline");
-  if (pinned && want_pipeline && c->timing == false)
-    return step_host_pipelined(c, h_actions, h_obs, h_reward, h_done, h_terminal_obs, h_events, n >= 262144 ? 8 : (n >= 65536 ? 4 : 2));
-  if (c->zero_copy && !(mode && !std::strcmp(mode, "staging"))) {
+  if (!staging) {
     // Pinned buffers: the kernels read the actions from and write the results to host memory themselves.  The
     // two PCIe directions then run concurrently and overlap with the compute, instead of H2D -> kernels -> D2H.
     const float *za = (const float *)mapped_alias(h_actions);
@@ -2772,7 +2521,8 @@ int tb_ff_diagnostics(tb_ctx *c, int64_t *h_out) {
   // the set of the most recent step that entered the fast-forward: the one whose round count is non-zero and whose
   // twin was zeroed since (both non-zero cannot happen: every step_kernel zeroes the next step's set)
   const unsigned long long *s = h[kDRounds] ? h : h + kCtrWords;
-  for (int i = 0; i < 14; ++i) h_out[i] = (int64_t)s[kDRounds + i];  // rounds, full-path envs, phase times
+  h_out[0] = (int64_t)s[kDRounds]; h_out[1] = (int64_t)s[kDFullEnvs]; h_out[2] = (int64_t)s[kDPhase];
+  for (int i = 3; i < 14; ++i) h_out[i] = 0;
   h_out[14] = (int64_t)s[kDFinish];
   h_out[15] = (int64_t)s[kCError];
   {
@@ -2780,40 +2530,6 @@ int tb_ff_diagnostics(tb_ctx *c, int64_t *h_out) {
     CU(cudaMemcpy(&fault, c->fault, sizeof fault, cudaMemcpyDeviceToHost));
     if (fault) h_out[15] = (int64_t)fault;
   }
-  if (std::getenv("TB_FF_DIAG_DUMP"))
-    for (int b = 0; b < 6; ++b)
-      std::fprintf(stderr, "server iterations with %d..%d lanes: %llu, mean %llu cycles; after 1.5 ms: %llu, mean %llu cycles\n", b ? (1 << (b - 1)) + 1 : 1,
-                   1 << b, s[112 + 2 * b], s[112 + 2 * b] ? s[113 + 2 * b] / s[112 + 2 * b] : 0ULL, s[80 + 2 * b],
-                   s[80 + 2 * b] ? s[81 + 2 * b] / s[80 + 2 * b] : 0ULL);
-  if (std::getenv("TB_FF_DIAG_DUMP"))
-    std::fprintf(stderr, "server substeps: lean %llu (mean %llu cycles, %llu with contact), handed to ff_full %llu (lean part mean %llu cycles, ff_full mean %llu cycles; "
-                 "%llu with racket contact, %llu with another event); loads %llu (mean %llu cycles)\n", s[100], s[100] ? s[101] / s[100] : 0ULL, s[107], s[102],
-                 s[102] ? s[103] / s[102] : 0ULL, s[102] ? s[104] / s[102] : 0ULL, s[105], s[106], s[108], s[108] ? s[109] / s[108] : 0ULL);
-  if (std::getenv("TB_FF_DIAG_DUMP"))
-    std::fprintf(stderr, "visits to the servers by where the flight lane got the env: front list %llu (mean substep %llu), back list %llu (%llu), late queue %llu (%llu)\n",
-                 s[92], s[92] ? s[95] / s[92] : 0ULL, s[93], s[93] ? s[96] / s[93] : 0ULL, s[94], s[94] ? s[97] / s[94] : 0ULL);
-#ifdef TB_FF_DIAG
-  if (std::getenv("TB_FF_DIAG_DUMP")) {
-    unsigned long long v[4] = {0, 0, 0, 0}, z = 0;
-    cudaMemcpyFromSymbol(&v[0], g_diag_edge_loops, 8); cudaMemcpyFromSymbol(&v[1], g_diag_quick_in, 8);
-    cudaMemcpyFromSymbol(&v[2], g_diag_quick_out, 8); cudaMemcpyFromSymbol(&v[3], g_diag_edge_in, 8);
-    cudaMemcpyToSymbol(g_diag_edge_loops, &z, 8); cudaMemcpyToSymbol(g_diag_quick_in, &z, 8);
-    cudaMemcpyToSymbol(g_diag_quick_out, &z, 8); cudaMemcpyToSymbol(g_diag_edge_in, &z, 8);
-    std::fprintf(stderr, "racket classification inside the slab and the bounding box (since the last dump): quick inside %llu, quick outside %llu, edge loop %llu (within the rim: %llu)\n",
-                 v[1], v[2], v[0], v[3]);
-  }
-#endif
-  if (std::getenv("TB_FF_DIAG_DUMP")) {
-    unsigned long long tmax = 0;
-    for (int i = 0; i < 100 && i < (int)s[299]; ++i) tmax = s[301 + 2 * i] > tmax ? s[301 + 2 * i] : tmax;
-    for (int i = 0; i < 100 && i < (int)s[299]; ++i)
-      std::fprintf(stderr, "late landing: step %llu last leg %llu substeps visits %llu where %llu at -%.1f us\n", s[300 + 2 * i] & 0xffff,
-                   (s[300 + 2 * i] >> 16) & 0xffff, (s[300 + 2 * i] >> 32) & 0xff, s[300 + 2 * i] >> 40, (tmax - s[301 + 2 * i]) * 1e-3);
-  }
-  if (std::getenv("TB_FF_DIAG_DUMP"))
-    for (int b = 0; b < 34 && s[128 + 5 * b]; ++b)
-      std::fprintf(stderr, "t=%.1fms landed %llu claimed %llu full queue tail %llu late queue head / tail %llu / %llu\n", 0.1 * b, s[128 + 5 * b] - 1, s[129 + 5 * b],
-                   s[130 + 5 * b], s[132 + 5 * b], s[131 + 5 * b]);
   return 0;
 }
 

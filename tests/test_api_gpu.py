@@ -136,14 +136,14 @@ def test_full_size_properties(env_id, n, steps):
     assert torch.equal(obs, obs2) and torch.equal(state, state2)  # bit-reproducible
 
 
-@pytest.mark.parametrize("mode", ["pipeline", "zero_copy", "staging"])
+@pytest.mark.parametrize("mode", ["zero_copy", "staging"])
 def test_step_host_modes_match_oracle(oracle_lib, mode, monkeypatch):
-    """tb_step_host's three transports (sliced uploads / kernels / downloads on two copy engines; kernels addressing the pinned
-    host buffers; plain staging) give the oracle's results, through SwingRacket's fast-forward step and the auto-resets."""
+    """tb_step_host's two transports (kernels addressing the pinned host buffers; plain staging) give the oracle's results,
+    through SwingRacket's fast-forward step and the auto-resets."""
     from tennisbot_rl_b200.batch import TennisBatch
 
     monkeypatch.setenv("TB_HOST_MODE", mode)
-    n = 5000  # not a multiple of the slice size
+    n = 5000  # not a multiple of the CTA size
     b = TennisBatch("SwingRacket-v0", n, seed=77)
     o = oracle_lib.OracleEnv("SwingRacket-v0", n, seed=77, threads=8)
     np.testing.assert_array_equal(b.reset_host(), o.reset())
@@ -159,4 +159,18 @@ def test_step_host_modes_match_oracle(oracle_lib, mode, monkeypatch):
         d = ref["done"] != 0
         np.testing.assert_allclose(hb["terminal_obs"][d], ref["terminal_obs"][d], atol=2e-6)
     np.testing.assert_array_equal(b.read_stats(), o.read_stats())
+    b.close()
+
+
+def test_step_host_rejects_unknown_mode(monkeypatch):
+    """A TB_HOST_MODE that names no transport (here the removed `pipeline`) fails the call instead of falling back."""
+    from tennisbot_rl_b200 import _lib
+    from tennisbot_rl_b200.batch import TennisBatch
+
+    monkeypatch.setenv("TB_HOST_MODE", "pipeline")
+    b = TennisBatch("SwingRacket-v0", 256, seed=1)
+    b.reset_host()
+    with pytest.raises(_lib.TennisbotLibraryError, match="pipeline") as err:
+        b.step_host(np.zeros((256, 6), np.float32))
+    assert "zero_copy" in str(err.value) and "staging" in str(err.value)
     b.close()

@@ -151,7 +151,7 @@ def test_f64_parity_hit_env_tracking_policy(oracle_lib):
     ({"racket_scale": 2.5}, TOL_F64_STATE, TOL_F64_OUT),
     ({"lin_damping": 0.0, "ang_damping": 0.0}, TOL_F64_STATE, TOL_F64_OUT),
     # balls come to rest and roll on the court here: hundreds of consecutive contact steps, each turning position
-    # rounding into velocity at 1/dt = 240.  Measured 3.2e-6 (3.8e-6 with the generic step in line, -DTB_HIT_GENERIC):
+    # rounding into velocity at 1/dt = 240.  Measured 3.2e-6 (3.8e-6 with the generic step in line instead of hit_fast):
     # the amplification is the contact model's, not the straight line's, hence the wider bar for this scene only
     ({"gravity_z": -25.0, "racket_scale": 1.6}, 2e-5, 2e-5)])
 def test_f64_parity_hit_env_paths(oracle_lib, params, tol_state, tol_out):

@@ -1,6 +1,6 @@
 """End-to-end (tb_step_host, pinned host buffers) throughput of G ranks stepping at once, with the PCIe traffic nvidia-smi
 sees per GPU meanwhile: what bounds the end-to-end curve at 8 GPUs (VERDICT round 1, item 8).
-    torchrun --nproc-per-node G tools/e2e_scale.py [n_envs] [mode: zero_copy|staging|pipeline]
+    torchrun --nproc-per-node G tools/e2e_scale.py [n_envs] [mode: zero_copy|staging]
 Rank 0 prints one JSON line."""
 import json, os, subprocess, sys, threading, time
 import numpy as np

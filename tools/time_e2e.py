@@ -1,4 +1,4 @@
-"""End-to-end step time through tb_step_host (pinned host buffers in and out) for the three transports.
+"""End-to-end step time through tb_step_host (pinned host buffers in and out) for the two transports.
 usage: time_e2e.py [n_envs] [env] [mode,mode,...]"""
 import os, sys, time
 import numpy as np
@@ -7,7 +7,7 @@ sys.path.insert(0, ".")
 from tennisbot_rl_b200.batch import TennisBatch
 n = int(sys.argv[1]) if len(sys.argv) > 1 else 1 << 20
 env = sys.argv[2] if len(sys.argv) > 2 else "SwingRacket-v0"
-modes = sys.argv[3].split(",") if len(sys.argv) > 3 else ("pipeline", "zero_copy", "staging")
+modes = sys.argv[3].split(",") if len(sys.argv) > 3 else ("zero_copy", "staging")
 for mode in modes:
     os.environ["TB_HOST_MODE"] = mode
     b = TennisBatch(env, n, seed=0)

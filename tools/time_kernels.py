@@ -21,4 +21,4 @@ for t in range(26):
 for t, r in enumerate(rows):
     if t % 26 >= 23 or t % 26 in (0, 12): print(t, "step_kernel %.4f ms ff_kernel %.4f ms" % (r[0], r[1]))
 d = b.ff_diagnostics()
-print("ff diagnostics: ran %d, visits to the server path %d, flights over after %d ns (+ instrumented words %s), finishing pass %d ns, fault %d" % (d[0], d[1], d[2], d[3:14].tolist(), d[14], d[15]))
+print("ff diagnostics: ran %d, visits to the server path %d, flights over after %d ns, fault %d" % (d[0], d[1], d[2], d[15]))
