@@ -178,6 +178,38 @@ int tb_policy_rollout(tb_ctx *ctx, int k_steps, int deterministic, uint64_t nois
                       float *d_logp, float *d_value, float *d_reward, uint8_t *d_done, float *d_last_obs,
                       float *d_last_value, void *stream);
 
+/* ---- ES fitness rollout (SURVEY 8(f)-2): fitness_static (fitness_functions.py:18-158) for a whole population in one context.
+ * Env i evaluates individual i / (N / individuals) with the reference's GatedCNN (policies.py:59-128) on an 8-step history of
+ * observations, each normalised by the env's own float64 running normaliser (evolution_strategy_static.py:25-44); the
+ * action is clipped to [-1, 1].  Parameters per individual, float32, in parameters_to_vector order (each conv weight
+ * [out][in][2]):
+ *   conv_0 W[8 x C x 2] b[8], conv_gate_0 W[8 x C x 2] b[8]          (dilation 1)
+ *   conv_1 W[12 x 8 x 2] b[12], conv_gate_1 W[12 x 8 x 2] b[12]      (dilation 2)
+ *   conv_2 W[A x 12 x 2] b[A]                                       (dilation 4)
+ * with C = obs_dim, A = act_dim: 766 floats for SwingRacket-v0, 858 for Tennisbot-v0. */
+#define TB_ES_FLOATS 766
+#define TB_ES_FLOATS_HIT 858
+#define TB_ES_HISTORY 8
+int tb_es_floats(int env_kind); /* TB_ES_FLOATS / TB_ES_FLOATS_HIT (-1: unknown kind); callable without a GPU */
+/* Start a generation: d_weights float32 [individuals, floats] (floats = tb_es_floats(env_kind), individuals must divide N; the
+ * library keeps its own copy, so the buffer may be reused once the stream has passed this call); d_normalizer double
+ * [3, obs_dim] = the master normaliser's (n, mean, mean_diff), NULL = zeros.  Resets every env from the RNG (a context's first
+ * generation places as tb_reset does on a fresh context; later generations continue the episode counters), observes the reset
+ * observation, fills the history with its normalised value, zeroes the returns and marks every env alive.  Needs
+ * TB_CONTROL_FORCE.  Stream-ordered, never synchronises. */
+int tb_es_begin(tb_ctx *ctx, const float *d_weights, int64_t individuals, int64_t floats, const double *d_normalizer,
+                void *stream);
+/* k_steps >= 1 env steps of the generation: per step one es_kernel launch (fold the previous step's reward, done and observation
+ * into return, alive, normaliser and history; GatedCNN forward) and tb_step's launches, then one fold-only es_kernel launch.
+ * return += reward while alive, then alive &= !done; after an env's first done it acts 0 and its normaliser and history stop.
+ * d_return double [N], d_alive uint8 [N] (required): the state after the last step.  Optional traces (NULL = none):
+ * d_obs float32 [K + 1, N, obs_dim], the raw observation the normaliser consumed before each action (the terminal one when the
+ * step ended an episode; [0] is the one consumed before this call, [K] the last step's); d_actions float32 [K, N, act_dim], the
+ * clipped actions; d_reward float32 [K, N]; d_done uint8 [K, N].  The envs must not be stepped by other calls between
+ * tb_es_begin and the last tb_es_rollout of a generation.  Never synchronises: capturable in a CUDA graph. */
+int tb_es_rollout(tb_ctx *ctx, int k_steps, double *d_return, uint8_t *d_alive, float *d_obs, float *d_actions,
+                  float *d_reward, uint8_t *d_done, void *stream);
+
 /* ---- state dump / injection for the parity harness: double [N, TB_STATE_WORDS] */
 int tb_get_state(tb_ctx *ctx, double *d_state, void *stream);
 int tb_set_state(tb_ctx *ctx, const double *d_state, void *stream);

@@ -16,6 +16,9 @@ STATE_WORDS, INIT_WORDS, NUM_STATS = 32, 8, 10
 ACT_RANDOM, ACT_TRACK = 0, 1
 POLICY_FLOATS = 9076       # SwingRacket-v0's in-kernel policy (TB_POLICY_FLOATS)
 POLICY_FLOATS_HIT = 9324   # Tennisbot-v0's (TB_POLICY_FLOATS_HIT)
+ES_FLOATS = 766            # SwingRacket-v0's GatedCNN (TB_ES_FLOATS)
+ES_FLOATS_HIT = 858        # Tennisbot-v0's (TB_ES_FLOATS_HIT)
+ES_HISTORY = 8             # observations the GatedCNN sees (TB_ES_HISTORY)
 CONTROL_FORCE, CONTROL_PID = 0, 1
 
 EV_RACKET_BALL, EV_COURT_BALL, EV_GOAL_BALL, EV_TIMEOUT, EV_BALL_PASSED, EV_NET_BALL, EV_RACKET_LOW = 1, 2, 4, 8, 16, 32, 64
@@ -28,7 +31,7 @@ EXPORTS = (
     "tb_scene_constant", "tb_create", "tb_destroy", "tb_set_param", "tb_get_param", "tb_set_control_mode", "tb_reset", "tb_reset_from",
     "tb_step", "tb_rollout", "tb_get_state", "tb_set_state", "tb_stats_device_ptr", "tb_read_stats",
     "tb_reset_host", "tb_step_host", "tb_launch_count", "tb_ff_diagnostics", "tb_set_kernel_timing", "tb_get_kernel_timing",
-    "tb_set_policy", "tb_policy_rollout",
+    "tb_set_policy", "tb_policy_rollout", "tb_es_floats", "tb_es_begin", "tb_es_rollout",
 )
 
 
@@ -85,6 +88,10 @@ def load():
     if hasattr(L, "tb_set_policy"):
         L.tb_set_policy.argtypes = [vp, vp, i64, vp]
         L.tb_policy_rollout.argtypes = [vp, i32, i32, C.c_uint64, vp, vp, vp, vp, vp, vp, vp, vp, vp]
+    if hasattr(L, "tb_es_begin"):
+        L.tb_es_floats.argtypes = [i32]
+        L.tb_es_begin.argtypes = [vp, vp, i64, i64, vp, vp]
+        L.tb_es_rollout.argtypes = [vp, i32, vp, vp, vp, vp, vp, vp, vp]
     L.tb_set_kernel_timing.argtypes = [vp, i32]
     L.tb_get_kernel_timing.argtypes = [vp, C.POINTER(dbl), C.POINTER(dbl), C.POINTER(i64)]
     _lib = L

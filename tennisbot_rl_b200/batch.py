@@ -160,6 +160,43 @@ class TennisBatch:
                                               _dptr(actions), _dptr(logp), _dptr(value), _dptr(reward), _dptr(done), _dptr(last_obs),
                                               _dptr(last_value), self._stream()))
 
+    # ------------------------------------------------------------------ ES fitness rollout (tb_es_begin / tb_es_rollout)
+    def _need(self, who, t, name, shape, dtype, optional=False):
+        if t is None and optional:
+            return
+        if t is None or t.dtype != dtype or t.device != self.device or not t.is_contiguous() or tuple(t.shape) != shape:
+            got = None if t is None else (tuple(t.shape), t.dtype, str(t.device), t.is_contiguous())
+            raise ValueError(f"{who}: {name} must be a contiguous {dtype} tensor of shape {shape} on {self.device}, got {got}")
+
+    def es_begin(self, weights, normalizer=None):
+        """Start an ES generation: weights float32 [individuals, es_floats] (individuals divides num_envs; env i evaluates
+        individual i // (num_envs // individuals)), normalizer float64 [3, obs_dim] = the master (n, mean, mean_diff) or None.
+        Resets every env, so a generation always starts new episodes."""
+        floats = _lib.ES_FLOATS if self.kind == _lib.ENV_SWING else _lib.ES_FLOATS_HIT
+        if weights.dim() != 2 or weights.shape[1] != floats or weights.shape[0] < 1 or self.num_envs % weights.shape[0]:
+            raise ValueError(f"es_begin: weights must have shape (individuals, {floats}) with individuals dividing {self.num_envs}, "
+                             f"got {tuple(weights.shape)}")
+        self._need("es_begin", weights, "weights", tuple(weights.shape), torch.float32)
+        self._need("es_begin", normalizer, "normalizer", (3, self.obs_dim), torch.float64, optional=True)
+        _lib.check(self.lib.tb_es_begin(self.h, _dptr(weights), int(weights.shape[0]), floats, _dptr(normalizer), self._stream()))
+
+    def es_rollout(self, k_steps, ret, alive, obs=None, actions=None, reward=None, done=None):
+        """k_steps env steps of the generation with in-kernel GatedCNN actions.  ret float64 [N] and alive uint8 [N] receive the
+        state after the last step.  Optional traces: obs float32 [K+1, N, obs_dim] (the raw observation each normaliser update
+        consumed, [0] the one before this call), actions float32 [K, N, act_dim] (clipped), reward float32 [K, N], done uint8
+        [K, N].  The library writes through raw pointers, so every buffer is checked here."""
+        k, n = int(k_steps), self.num_envs
+        if k < 1:
+            raise ValueError(f"es_rollout: k_steps must be >= 1, got {k}")
+        self._need("es_rollout", ret, "ret", (n,), torch.float64)
+        self._need("es_rollout", alive, "alive", (n,), torch.uint8)
+        self._need("es_rollout", obs, "obs", (k + 1, n, self.obs_dim), torch.float32, optional=True)
+        self._need("es_rollout", actions, "actions", (k, n, self.act_dim), torch.float32, optional=True)
+        self._need("es_rollout", reward, "reward", (k, n), torch.float32, optional=True)
+        self._need("es_rollout", done, "done", (k, n), torch.uint8, optional=True)
+        _lib.check(self.lib.tb_es_rollout(self.h, k, _dptr(ret), _dptr(alive), _dptr(obs), _dptr(actions), _dptr(reward),
+                                          _dptr(done), self._stream()))
+
     def get_state(self):
         s = torch.empty((self.num_envs, _lib.STATE_WORDS), dtype=torch.float64, device=self.device)
         _lib.check(self.lib.tb_get_state(self.h, _dptr(s), self._stream()))

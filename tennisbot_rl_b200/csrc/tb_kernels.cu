@@ -1460,6 +1460,212 @@ __global__ void __launch_bounds__(kBlock) policy_kernel(const __grid_constant__ 
   pdl_trigger();
 }
 
+// ------------------------------------------------------------------------------------------------ ES fitness rollout
+// SURVEY 8(f)-2: fitness_static (fitness_functions.py:18-158) for a whole population on the device.  Env i evaluates
+// individual i / repeats with the reference's GatedCNN (policies.py:59-128) on an 8-step history of observations normalised by
+// the env's own running normaliser (evolution_strategy_static.py:25-44, float64).  A rollout is K x (es_kernel, step_kernel,
+// ff_kernel) on one stream plus one fold-only es_kernel: nothing between two env steps runs on the host.
+// Parameters in parameters_to_vector order (es_eval.gated_cnn_sizes), each conv weight [out][in][2]:
+//   conv_0 W[8 x C x 2] b[8], conv_gate_0 (same), conv_1 W[12 x 8 x 2] b[12] (dilation 2), conv_gate_1 (same),
+//   conv_2 W[A x 12 x 2] b[A] (dilation 4)
+template <int C, int A> struct EsLayout {
+  static constexpr int W0 = 0, B0 = W0 + 16 * C, G0 = B0 + 8, GB0 = G0 + 16 * C, W1 = GB0 + 8, B1 = W1 + 192, G1 = B1 + 12,
+                       GB1 = G1 + 192, W2 = GB1 + 12, B2 = W2 + 24 * A, Floats = B2 + A;
+};
+static_assert(EsLayout<6, 6>::Floats == TB_ES_FLOATS && EsLayout<12, 2>::Floats == TB_ES_FLOATS_HIT, "GatedCNN layout / header mismatch");
+static_assert(TB_ES_HISTORY == 8, "the history ring is indexed with & 7");
+
+struct EsIO {
+  const float *w;               // [Floats][individuals]: the population parameter-major (tb_es_begin transposes the caller's rows),
+                                // so lanes of one individual read one address and neighbouring individuals neighbouring ones
+  int64_t n, individuals;
+  int repeats;                  // env i evaluates individual i / repeats
+  double *norm;                 // [2 OBS][N] normaliser: mean rows, then mean_diff rows
+  double *n0;                   // [OBS] the master normaliser's count; every env has observed the same number of values since
+  float *hist;                  // [8 OBS][N] ring of normalised observations; slot (tick - base) % 8 holds the newest
+  double *ret;                  // [N] return summed while alive
+  uint8_t *alive;               // [N] no done yet
+  const unsigned *tick;         // the env-step counter (StepIO::epoch[0] / [2]): constant while an es_kernel runs
+  unsigned *base;               // its value at tb_es_begin, so tick - base = env steps since then
+  const float *obs, *term, *reward;  // the previous env step's outputs (the context's buffers)
+  const uint8_t *done;
+  int fold;                     // 1: fold the previous step into return, alive, normaliser and history
+  float *act;                   // [N, A] clipped action for step_kernel; nullptr: fold only (the launch ending a rollout)
+  float *obs_trace, *act_trace, *rew_trace;  // optional: step obs consumed [N, C], action [N, A], reward [N]
+  uint8_t *done_trace;          // optional: done [N]
+  double *ret_out;              // optional: return and alive copied out (the launch ending a rollout)
+  uint8_t *alive_out;
+};
+
+// tanh(a) * sigmoid(g), on the accurate tanhf: tanh_fast's ~1e-6 per activation, carried through two layers of 16 and 24
+// weighted terms, can reach ~1e-5 in the action
+__device__ __forceinline__ float es_gate(float a, float g) { return tanhf(a) * fmaf(0.5f, tanhf(0.5f * g), 0.5f); }
+
+// Observe x (float64, no contraction: the same roundings as BatchedNormalizer.observe), return the normalised value.
+__device__ __forceinline__ float es_observe(double x, double nn, double &mean, double &md) {
+  const double last = mean;
+  mean = __dadd_rn(mean, (x - mean) / nn);
+  md = __dadd_rn(md, __dmul_rn(x - last, x - mean));
+  const double var = fmax(md / nn, 1e-2);
+  return (float)((x - mean) / sqrt(var));
+}
+
+// One thread per env.  Only the network's last output position is needed, so conv_0 is evaluated at positions 0, 2, 4, 6
+// and conv_1 at 0 and 4.  After an env's first done nothing it computes matters: it skips the fold and the network and
+// hands a zero action to the env step.
+template <int OBS, int ACT>
+__global__ void __launch_bounds__(kBlock, 4) es_kernel(const __grid_constant__ EsIO io) {
+  using L = EsLayout<OBS, ACT>;
+  static_assert(OBS % 2 == 0 && ACT % 2 == 0, "observation and action rows are accessed as float2");
+  pdl_wait();
+  const int64_t i = (int64_t)blockIdx.x * kBlock + threadIdx.x, n = io.n;
+  if (i < n) {
+    const unsigned s = *io.tick - *io.base;
+    const bool trace = io.obs_trace != nullptr;
+    bool live = io.alive[i] != 0;
+    const bool fold = io.fold && live;
+    const uint8_t d = (trace || fold) ? io.done[i] : 0;
+    if (io.fold) {
+      if (io.rew_trace) io.rew_trace[i] = io.reward[i];
+      if (io.done_trace) io.done_trace[i] = io.done[i];
+    }
+    double ret = 0.0;
+    if (fold) {
+      ret = io.ret[i] + (double)io.reward[i];
+      io.ret[i] = ret;
+      if (d) { live = false; io.alive[i] = 0; }
+    } else if (io.ret_out) {
+      ret = io.ret[i];
+    }
+    if (trace || (fold && live)) {
+      float x[OBS];
+      const float2 *src = reinterpret_cast<const float2 *>((d ? io.term : io.obs) + i * OBS);
+#pragma unroll
+      for (int j = 0; j < OBS / 2; ++j) { const float2 v = src[j]; x[2 * j] = v.x; x[2 * j + 1] = v.y; }
+      if (trace) {
+        float2 *q = reinterpret_cast<float2 *>(io.obs_trace + i * OBS);
+#pragma unroll
+        for (int j = 0; j < OBS / 2; ++j) q[j] = make_float2(x[2 * j], x[2 * j + 1]);
+      }
+      if (fold && live) {
+        const int slot = (int)(s & 7u);
+#pragma unroll
+        for (int c = 0; c < OBS; ++c) {
+          double mean = io.norm[c * n + i], md = io.norm[(OBS + c) * n + i];
+          io.hist[(slot * OBS + c) * n + i] = es_observe((double)x[c], io.n0[c] + (double)(s + 1u), mean, md);
+          io.norm[c * n + i] = mean; io.norm[(OBS + c) * n + i] = md;
+        }
+      }
+    }
+    if (io.act) {
+      float a[ACT];
+#pragma unroll
+      for (int o = 0; o < ACT; ++o) a[o] = 0.0f;
+      if (live) {
+        const float *wp = io.w + i / io.repeats;
+        const unsigned ld = (unsigned)io.individuals;  // (tb_es_begin keeps individuals x floats below 2^32)
+        auto W = [&](int f) { return __ldg(wp + (unsigned)f * ld); };
+        // conv_0 / conv_gate_0 (dilation 1) at positions 0, 2, 4, 6: position p reads history columns p and p + 1
+        float h0[8][4], g0[8][4];
+#pragma unroll
+        for (int o = 0; o < 8; ++o) {
+          const float b = W(L::B0 + o), bg = W(L::GB0 + o);
+#pragma unroll
+          for (int j = 0; j < 4; ++j) { h0[o][j] = b; g0[o][j] = bg; }
+        }
+        // The loops over conv_0's input channels and conv_1's outputs stay rolled: unrolled, ptxas hoists hundreds of
+        // independent weight loads and spills.
+        const int oldest = (int)((s + 1u) & 7u);
+#pragma unroll 1
+        for (int c = 0; c < OBS; ++c) {
+          float x[8];  // channel c, oldest first
+#pragma unroll
+          for (int t = 0; t < 8; ++t) x[t] = io.hist[(((oldest + t) & 7) * OBS + c) * n + i];
+#pragma unroll
+          for (int o = 0; o < 8; ++o)
+#pragma unroll
+            for (int k = 0; k < 2; ++k) {
+              const float wa = W(L::W0 + (o * OBS + c) * 2 + k), wg = W(L::G0 + (o * OBS + c) * 2 + k);
+#pragma unroll
+              for (int j = 0; j < 4; ++j) { h0[o][j] = fmaf(wa, x[2 * j + k], h0[o][j]); g0[o][j] = fmaf(wg, x[2 * j + k], g0[o][j]); }
+            }
+        }
+#pragma unroll
+        for (int o = 0; o < 8; ++o)
+#pragma unroll
+          for (int j = 0; j < 4; ++j) h0[o][j] = es_gate(h0[o][j], g0[o][j]);
+        // conv_1 / conv_gate_1 (dilation 2) at positions 0 and 4 (position 4 m reads conv_0 positions 4 m and 4 m + 2), each
+        // output channel folded straight into conv_2 (dilation 4), whose one output position reads conv_1 positions 0 and 4
+#pragma unroll
+        for (int o = 0; o < ACT; ++o) a[o] = W(L::B2 + o);
+#pragma unroll 1
+        for (int o = 0; o < 12; ++o) {
+          float acc[2], gac[2];
+          acc[0] = acc[1] = W(L::B1 + o);
+          gac[0] = gac[1] = W(L::GB1 + o);
+#pragma unroll
+          for (int c = 0; c < 8; ++c)
+#pragma unroll
+            for (int k = 0; k < 2; ++k) {
+              const float wa = W(L::W1 + (o * 8 + c) * 2 + k), wg = W(L::G1 + (o * 8 + c) * 2 + k);
+#pragma unroll
+              for (int m = 0; m < 2; ++m) { acc[m] = fmaf(wa, h0[c][2 * m + k], acc[m]); gac[m] = fmaf(wg, h0[c][2 * m + k], gac[m]); }
+            }
+          const float h1[2] = {es_gate(acc[0], gac[0]), es_gate(acc[1], gac[1])};
+#pragma unroll
+          for (int q = 0; q < ACT; ++q)
+#pragma unroll
+            for (int k = 0; k < 2; ++k) a[q] = fmaf(W(L::W2 + (q * 12 + o) * 2 + k), h1[k], a[q]);
+        }
+#pragma unroll
+        for (int o = 0; o < ACT; ++o) a[o] = fminf(fmaxf(a[o], -1.0f), 1.0f);
+      }
+      float2 *q = reinterpret_cast<float2 *>(io.act + i * ACT);
+#pragma unroll
+      for (int j = 0; j < ACT / 2; ++j) q[j] = make_float2(a[2 * j], a[2 * j + 1]);
+      if (io.act_trace) {
+        q = reinterpret_cast<float2 *>(io.act_trace + i * ACT);
+#pragma unroll
+        for (int j = 0; j < ACT / 2; ++j) q[j] = make_float2(a[2 * j], a[2 * j + 1]);
+      }
+    }
+    if (io.ret_out) { io.ret_out[i] = ret; io.alive_out[i] = live ? 1 : 0; }
+  }
+  pdl_trigger();
+}
+
+// After the reset of tb_es_begin: seed every env's normaliser from the master state (or zeros), observe the reset observation
+// (io.obs), fill the history with its normalised value, zero the return, mark the env alive.
+template <int OBS>
+__global__ void __launch_bounds__(kBlock) es_begin_kernel(const __grid_constant__ EsIO io, const double *master) {
+  const int64_t i = (int64_t)blockIdx.x * kBlock + threadIdx.x, n = io.n;
+  if (blockIdx.x == 0 && threadIdx.x == 0) *io.base = *io.tick;
+  if (blockIdx.x == 0 && threadIdx.x < OBS) io.n0[threadIdx.x] = master ? master[threadIdx.x] : 0.0;
+  if (i >= n) return;
+#pragma unroll
+  for (int c = 0; c < OBS; ++c) {
+    double mean = master ? master[OBS + c] : 0.0, md = master ? master[2 * OBS + c] : 0.0;
+    const float z = es_observe((double)io.obs[i * OBS + c], (master ? master[c] : 0.0) + 1.0, mean, md);
+    io.norm[c * n + i] = mean; io.norm[(OBS + c) * n + i] = md;
+#pragma unroll
+    for (int t = 0; t < 8; ++t) io.hist[(t * OBS + c) * n + i] = z;
+  }
+  io.ret[i] = 0.0;
+  io.alive[i] = 1;
+}
+
+// [rows][cols] -> [cols][rows] through 32 x 32 shared tiles (block 32 x 8); rows on grid x, cols on grid y
+__global__ void es_transpose_kernel(const float *in, int64_t rows, int cols, float *out) {
+  __shared__ float tile[32][33];
+  const int64_t r0 = (int64_t)blockIdx.x * 32;
+  const int c0 = blockIdx.y * 32;
+  for (int j = threadIdx.y; j < 32; j += 8)
+    if (r0 + j < rows && c0 + (int)threadIdx.x < cols) tile[j][threadIdx.x] = in[(r0 + j) * cols + c0 + threadIdx.x];
+  __syncthreads();
+  for (int j = threadIdx.y; j < 32; j += 8)
+    if (c0 + j < cols && r0 + (int)threadIdx.x < rows) out[(int64_t)(c0 + j) * rows + r0 + threadIdx.x] = tile[threadIdx.x][j];
+}
+
 template <typename T, int KIND>
 __global__ void __launch_bounds__(kBlock) reset_kernel(const __grid_constant__ Scene<T> sc, const __grid_constant__ StepIO io,
                                                        const double *init, const uint8_t *mask) {
@@ -1914,7 +2120,15 @@ struct tb_ctx {
   void *pid = nullptr;                       // controller memory, allocated by tb_set_control_mode(TB_CONTROL_PID)
   float *policy = nullptr;                   // tb_policy_floats(env_kind) parameters (tb_set_policy)
   float *pol_act = nullptr;                  // [N, act_dim] clipped actions handed from policy_kernel to step_kernel
-  bool timing = false;                       // tb_set_kernel_timing
+  // ES fitness rollout (tb_es_begin / tb_es_rollout), allocated by the first tb_es_begin; see EsIO
+  int64_t es_individuals = 0;                // 0: no tb_es_begin yet
+  float *es_w = nullptr;                     // [floats][individuals]
+  int64_t es_w_cap = 0;                      // floats es_w holds
+  double *es_norm = nullptr, *es_n0 = nullptr, *es_ret = nullptr;
+  float *es_hist = nullptr, *es_obs = nullptr, *es_term = nullptr, *es_rew = nullptr, *es_act = nullptr;
+  uint8_t *es_alive = nullptr, *es_done = nullptr;
+  unsigned *es_base = nullptr;
+  bool timing = false;                      // tb_set_kernel_timing
   cudaEvent_t ev[3] = {nullptr, nullptr, nullptr};
   double ms_step = 0, ms_ff = 0;
   int64_t timed_steps = 0;
@@ -2105,6 +2319,7 @@ int tb_abi_version(void) { return TB_ABI_VERSION; }
 int tb_obs_dim(int kind) { return kind == TB_ENV_SWING ? 6 : kind == TB_ENV_HIT ? 12 : -1; }
 int tb_act_dim(int kind) { return kind == TB_ENV_SWING ? 6 : kind == TB_ENV_HIT ? 2 : -1; }
 int tb_policy_floats(int kind) { return kind == TB_ENV_SWING ? TB_POLICY_FLOATS : kind == TB_ENV_HIT ? TB_POLICY_FLOATS_HIT : -1; }
+int tb_es_floats(int kind) { return kind == TB_ENV_SWING ? TB_ES_FLOATS : kind == TB_ENV_HIT ? TB_ES_FLOATS_HIT : -1; }
 int tb_num_params(void) { return kNumParams; }
 const char *tb_param_name(int i) { return (i >= 0 && i < kNumParams) ? k_param_names[i] : nullptr; }
 
@@ -2242,6 +2457,8 @@ int tb_destroy(tb_ctx *c) {
   if (c->own_stream) { cudaStreamSynchronize(c->own_stream); cudaStreamDestroy(c->own_stream); }
   for (int i = 0; i < 3; ++i) if (c->ev[i]) cudaEventDestroy(c->ev[i]);
   cudaFree(c->state); cudaFree(c->stats); cudaFree(c->queue_ctrs); cudaFree(c->queue); cudaFree(c->dq); cudaFree(c->epoch); cudaFree(c->fault); cudaFree(c->queue_full); cudaFree(c->queue_ctl); cudaFree(c->pid); cudaFree(c->policy); cudaFree(c->pol_act);
+  cudaFree(c->es_w); cudaFree(c->es_norm); cudaFree(c->es_n0); cudaFree(c->es_ret); cudaFree(c->es_hist); cudaFree(c->es_obs);
+  cudaFree(c->es_term); cudaFree(c->es_rew); cudaFree(c->es_act); cudaFree(c->es_alive); cudaFree(c->es_done); cudaFree(c->es_base);
   if (c->h_fault) cudaFreeHost(c->h_fault);
   cudaFree(c->d_actions); cudaFree(c->d_obs); cudaFree(c->d_reward); cudaFree(c->d_term);
   cudaFree(c->d_done); cudaFree(c->d_events); cudaFree(c->d_mask);
@@ -2371,6 +2588,107 @@ int tb_policy_rollout(tb_ctx *c, int k_steps, int deterministic, uint64_t noise_
     pio.obs = d_last_obs; pio.act_raw = nullptr; pio.act_env = nullptr; pio.logp = nullptr; pio.value = d_last_value;
     CU(launch_pdl(kernel, dim3(grid, 2), s, pio));
     c->launches++;
+  }
+  CU(cudaGetLastError());
+  return 0;
+}
+
+static EsIO es_io(tb_ctx *c) {
+  EsIO io;
+  std::memset(&io, 0, sizeof io);
+  io.w = c->es_w; io.n = c->cfg.num_envs; io.individuals = c->es_individuals;
+  io.repeats = c->es_individuals ? (int)(c->cfg.num_envs / c->es_individuals) : 0;
+  io.norm = c->es_norm; io.n0 = c->es_n0; io.hist = c->es_hist; io.ret = c->es_ret; io.alive = c->es_alive;
+  io.tick = c->cfg.env_kind == TB_ENV_SWING ? c->epoch : c->epoch + 2;  // (see StepIO::epoch)
+  io.base = c->es_base;
+  io.obs = c->es_obs; io.term = c->es_term; io.reward = c->es_rew; io.done = c->es_done;
+  return io;
+}
+
+int tb_es_begin(tb_ctx *c, const float *d_weights, int64_t individuals, int64_t floats, const double *d_normalizer, void *stream) {
+  if (!d_weights) return fail("%s", "tb_es_begin: d_weights is NULL");
+  if (individuals < 1) return fail("%s", "tb_es_begin: individuals must be >= 1");
+  GUARD(c);
+  const int64_t n = c->cfg.num_envs, want = tb_es_floats(c->cfg.env_kind);
+  if (floats != want) {
+    std::snprintf(g_err, sizeof g_err, "tb_es_begin: expected tb_es_floats(env_kind) = %lld floats per individual, got %lld",
+                  (long long)want, (long long)floats);
+    return 1;
+  }
+  if (n % individuals) {
+    std::snprintf(g_err, sizeof g_err, "tb_es_begin: individuals (%lld) must divide num_envs (%lld)", (long long)individuals, (long long)n);
+    return 1;
+  }
+  if (individuals * floats > 0xffffffffLL) return fail("%s", "tb_es_begin: individuals x floats must be below 2^32 (es_kernel indexes the population with 32 bits)");
+  if (c->control_mode != TB_CONTROL_FORCE) return fail("%s", "tb_es_begin: the GatedCNN's actions are forces (TB_CONTROL_FORCE)");
+  if (check_fault(c, "tb_es_begin")) return 1;
+  cudaStream_t s = (cudaStream_t)stream;
+  const int od = tb_obs_dim(c->cfg.env_kind), ad = tb_act_dim(c->cfg.env_kind);
+  if (!c->es_norm) {  // per-env state, once per context
+    CU(cudaMalloc(&c->es_norm, (size_t)2 * od * n * sizeof(double)));
+    CU(cudaMalloc(&c->es_n0, (size_t)od * sizeof(double)));
+    CU(cudaMalloc(&c->es_ret, (size_t)n * sizeof(double)));
+    CU(cudaMalloc(&c->es_hist, (size_t)TB_ES_HISTORY * od * n * sizeof(float)));
+    CU(cudaMalloc(&c->es_obs, (size_t)od * n * sizeof(float)));
+    CU(cudaMalloc(&c->es_term, (size_t)od * n * sizeof(float)));
+    CU(cudaMalloc(&c->es_rew, (size_t)n * sizeof(float)));
+    CU(cudaMalloc(&c->es_act, (size_t)ad * n * sizeof(float)));
+    CU(cudaMalloc(&c->es_alive, (size_t)n));
+    CU(cudaMalloc(&c->es_done, (size_t)n));
+    CU(cudaMalloc(&c->es_base, sizeof(unsigned)));
+  }
+  if (c->es_w_cap < individuals * floats) {  // stream-ordered: a larger population does not synchronise either
+    if (c->es_w) CU(cudaFreeAsync(c->es_w, s));
+    c->es_w = nullptr; c->es_w_cap = 0;
+    CU(cudaMallocAsync(&c->es_w, (size_t)(individuals * floats) * sizeof(float), s));
+    c->es_w_cap = individuals * floats;
+  }
+  es_transpose_kernel<<<dim3((unsigned)((individuals + 31) / 32), (unsigned)((floats + 31) / 32)), dim3(32, 8), 0, s>>>(
+      d_weights, individuals, (int)floats, c->es_w);
+  c->launches++;
+  StepIO io = make_io(c);
+  io.obs = c->es_obs;
+  DISPATCH(reset_kernel, grid_for(n, kBlock), kBlock, s, io, (const double *)nullptr, (const uint8_t *)nullptr);
+  CU(cudaMemsetAsync(c->es_done, 0, (size_t)n, s));  // the reset observation is the step obs the first action's trace shows
+  c->es_individuals = individuals;
+  const EsIO eio = es_io(c);
+  if (c->cfg.env_kind == TB_ENV_SWING) es_begin_kernel<6><<<grid_for(n, kBlock), kBlock, 0, s>>>(eio, d_normalizer);
+  else es_begin_kernel<12><<<grid_for(n, kBlock), kBlock, 0, s>>>(eio, d_normalizer);
+  c->launches++;
+  CU(cudaGetLastError());
+  return 0;
+}
+
+int tb_es_rollout(tb_ctx *c, int k_steps, double *d_return, uint8_t *d_alive, float *d_obs, float *d_actions, float *d_reward,
+                  uint8_t *d_done, void *stream) {
+  if (k_steps < 1) return fail("%s", "tb_es_rollout: k_steps must be >= 1");
+  if (!d_return || !d_alive) return fail("%s", "tb_es_rollout: d_return and d_alive are required");
+  GUARD(c);
+  if (!c->es_individuals) return fail("%s", "tb_es_rollout: no population (call tb_es_begin first)");
+  if (c->control_mode != TB_CONTROL_FORCE) return fail("%s", "tb_es_rollout: the GatedCNN's actions are forces (TB_CONTROL_FORCE)");
+  if (check_fault(c, "tb_es_rollout")) return 1;
+  const int64_t n = c->cfg.num_envs;
+  const bool swing = c->cfg.env_kind == TB_ENV_SWING;
+  const int od = tb_obs_dim(c->cfg.env_kind), ad = tb_act_dim(c->cfg.env_kind);
+  void (*kernel)(EsIO) = swing ? es_kernel<6, 6> : es_kernel<12, 2>;
+  cudaStream_t s = (cudaStream_t)stream;
+  const unsigned grid = grid_for(n, kBlock);
+  EsIO eio = es_io(c);
+  for (int t = 0; t <= k_steps; ++t) {  // launch t folds step t - 1 (t > 0) and acts for step t (t < K)
+    eio.fold = t > 0;
+    eio.act = t < k_steps ? c->es_act : nullptr;
+    eio.obs_trace = d_obs ? d_obs + (size_t)t * n * od : nullptr;
+    eio.act_trace = d_actions && t < k_steps ? d_actions + (size_t)t * n * ad : nullptr;
+    eio.rew_trace = d_reward && t > 0 ? d_reward + (size_t)(t - 1) * n : nullptr;
+    eio.done_trace = d_done && t > 0 ? d_done + (size_t)(t - 1) * n : nullptr;
+    eio.ret_out = t == k_steps ? d_return : nullptr;
+    eio.alive_out = t == k_steps ? d_alive : nullptr;
+    CU(launch_pdl(kernel, grid, s, eio));
+    c->launches++;
+    if (t == k_steps) break;
+    StepIO io = make_io(c);
+    io.actions = c->es_act; io.obs = c->es_obs; io.reward = c->es_rew; io.done = c->es_done; io.term_obs = c->es_term;
+    if (launch_step(c, io, s)) return 1;
   }
   CU(cudaGetLastError());
   return 0;

@@ -5,7 +5,10 @@
 (individual, repeat) pair is one env of a single CUDA batch: per-env GatedCNN weights (766 parameters for 6 -> 6,
 `policies.py:59-128`), per-env running observation normaliser (`evolution_strategy_static.py:25-44`, each call
 works on its own copy there as well), 8-step history, action clipped to the Box, reward summed until done.
-The policy math is plain torch on the same GPU; observations and actions never leave HBM.
+Two implementations of that evaluation:
+- `EsEvaluator`: the GatedCNN, the normalisers, the history and the returns live in HBM and are advanced by the library's
+  es_kernel between env steps (tb_es_begin / tb_es_rollout); nothing between two env steps runs on the host.
+- `batched_fitness_static`: the same semantics in plain torch around `TennisBatch.step`, kept as the reference.
 """
 import torch
 
@@ -108,3 +111,55 @@ def batched_fitness_static(weights, env_id="SwingRacket-v0", repeats=10, normali
     env.close()
     per_episode = ret.reshape(pop, repeats)
     return per_episode.mean(dim=1), per_episode
+
+
+class EsEvaluator:
+    """batched_fitness_static on the device: the GatedCNN, the normalisers, the history and the returns live in HBM and are
+    advanced by es_kernel between env steps (tb_es_begin / tb_es_rollout), so nothing between two env steps runs on the host.
+    One context is kept across generations; each generation continues the envs' episode counters, so it gets fresh
+    placements.  env_id_offset shards a population over contexts (env i of this one is global env env_id_offset + i)."""
+
+    # env steps per tb_es_rollout call, with one 1-byte read of alive.any() after each: one whole SwingRacket-v0 episode
+    # (every one takes 26 steps), so a SwingRacket-v0 generation is one call; a 1001-step Tennisbot-v0 one is 39
+    CHUNK = 26
+
+    def __init__(self, env_id, individuals, repeats, device=0, seed=0, precision="f64", env_id_offset=0):
+        self.individuals, self.repeats = int(individuals), int(repeats)
+        if self.individuals < 1 or self.repeats < 1:
+            raise ValueError(f"EsEvaluator: individuals and repeats must be >= 1, got {individuals}, {repeats}")
+        self.env = TennisBatch(env_id, self.individuals * self.repeats, device=device, seed=seed, precision=precision,
+                               auto_reset=True, env_id_offset=env_id_offset)
+        n, dev = self.env.num_envs, self.env.device
+        self.num_params = num_params(self.env.obs_dim, self.env.act_dim)
+        self.ret = torch.zeros(n, dtype=torch.float64, device=dev)
+        self.alive = torch.zeros(n, dtype=torch.uint8, device=dev)
+        self.steps_run = 0  # env steps the last evaluate() ran
+
+    def close(self):
+        self.env.close()
+
+    @torch.no_grad()
+    def evaluate(self, weights, normalizer_state=None, max_steps=1001):
+        """weights [individuals, num_params]; normalizer_state: the master's (n, mean, mean_diff, var) as BatchedNormalizer takes
+        it (var is ignored: observe overwrites it).  Returns (fitness [individuals], returns [individuals, repeats]) like
+        batched_fitness_static: the return of every env summed until its first done or max_steps."""
+        if int(max_steps) < 1:
+            raise ValueError(f"EsEvaluator.evaluate: max_steps must be >= 1, got {max_steps}")
+        dev, od = self.env.device, self.env.obs_dim
+        w = torch.as_tensor(weights, dtype=torch.float32, device=dev).contiguous()
+        if tuple(w.shape) != (self.individuals, self.num_params):
+            raise ValueError(f"weights must have shape ({self.individuals}, {self.num_params}), got {tuple(w.shape)}")
+        norm = None
+        if normalizer_state is not None:
+            norm = torch.stack([torch.as_tensor(x, dtype=torch.float64, device=dev).reshape(od) for x in normalizer_state[:3]])
+        self.env.es_begin(w, norm)
+        steps = 0
+        while steps < max_steps:
+            k = min(self.CHUNK, int(max_steps) - steps)
+            self.env.es_rollout(k, self.ret, self.alive)
+            steps += k
+            if not bool(self.alive.any()):
+                break
+        self.steps_run = steps
+        per_episode = self.ret.reshape(self.individuals, self.repeats).clone()
+        return per_episode.mean(dim=1), per_episode
