@@ -210,6 +210,29 @@ int tb_es_begin(tb_ctx *ctx, const float *d_weights, int64_t individuals, int64_
 int tb_es_rollout(tb_ctx *ctx, int k_steps, double *d_return, uint8_t *d_alive, float *d_obs, float *d_actions,
                   float *d_reward, uint8_t *d_done, void *stream);
 
+/* ---- ES population and update (ARS V2-t with seeded perturbations).  Direction j's noise in generation g is a float32 vector
+ * eps_j drawn from Philox, so any shard can regenerate it:
+ *   r = Philox4x32-10(key = noise_seed, counter = (j lo, j hi, g, (3 << 28) | ((f / 4) << 4))),  q = f / 4, k = 0, 1:
+ *   u1 = (r[2k] + 0.5) / 2^32, u2 = r[2k + 1] / 2^32, rho = sqrt(-2 ln u1) (float64),
+ *   eps_j[4q + 2k] = float32(rho cos(2 pi u2)), eps_j[4q + 2k + 1] = float32(rho sin(2 pi u2)).
+ * Global individual g = env_id_offset / repeats + p (p local) belongs to direction j = g / 2 and is theta + d for even g,
+ * theta - d for odd g, with d = float32(sigma * eps_j) and one float32 rounding per add (no fused multiply-add).
+ * tb_es_begin_noise is tb_es_begin with that population drawn in the library from d_theta float32 [floats]; it also fails when
+ * individuals is odd, env_id_offset is not a multiple of 2 x repeats (a shard holds whole pairs), sigma is not a finite number
+ * above 0 or d_theta is NULL.  Stream-ordered, never synchronises. */
+int tb_es_begin_noise(tb_ctx *ctx, const float *d_theta, int64_t individuals, int64_t floats, float sigma, uint64_t noise_seed,
+                      uint32_t generation, const double *d_normalizer, void *stream);
+/* d_out float32 [tb_es_floats(env_kind)] = sum_k d_coef[k] * eps_{d_dirs[k]} of generation `generation`, accumulated in float64 in
+ * the order k = 0 .. count - 1 and rounded once.  d_dirs int64 [count] are global direction indices, d_coef float32 [count];
+ * count may be 0 (d_out = 0).  Stream-ordered, never synchronises. */
+int tb_es_noise_combine(tb_ctx *ctx, const int64_t *d_dirs, const float *d_coef, int64_t count, uint64_t noise_seed,
+                        uint32_t generation, float *d_out, void *stream);
+/* d_out double [3, obs_dim] = (count, mean, M2) of the observations this context's normalisers took since the last
+ * tb_es_begin* (the master's share excluded): each env's reset observation and one per step until its first done (the
+ * terminal observation is not taken).  Combine shards and the master with Chan's formula.  A deterministic two-pass
+ * reduction, no atomics.  Fails before the first tb_es_begin*.  Stream-ordered, never synchronises. */
+int tb_es_normalizer_stats(tb_ctx *ctx, double *d_out, void *stream);
+
 /* ---- state dump / injection for the parity harness: double [N, TB_STATE_WORDS] */
 int tb_get_state(tb_ctx *ctx, double *d_state, void *stream);
 int tb_set_state(tb_ctx *ctx, const double *d_state, void *stream);

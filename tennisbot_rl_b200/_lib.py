@@ -32,6 +32,7 @@ EXPORTS = (
     "tb_step", "tb_rollout", "tb_get_state", "tb_set_state", "tb_stats_device_ptr", "tb_read_stats",
     "tb_reset_host", "tb_step_host", "tb_launch_count", "tb_ff_diagnostics", "tb_set_kernel_timing", "tb_get_kernel_timing",
     "tb_set_policy", "tb_policy_rollout", "tb_es_floats", "tb_es_begin", "tb_es_rollout",
+    "tb_es_begin_noise", "tb_es_noise_combine", "tb_es_normalizer_stats",
 )
 
 
@@ -92,6 +93,11 @@ def load():
         L.tb_es_floats.argtypes = [i32]
         L.tb_es_begin.argtypes = [vp, vp, i64, i64, vp, vp]
         L.tb_es_rollout.argtypes = [vp, i32, vp, vp, vp, vp, vp, vp, vp]
+    if hasattr(L, "tb_es_begin_noise"):
+        u32, u64 = C.c_uint32, C.c_uint64
+        L.tb_es_begin_noise.argtypes = [vp, vp, i64, i64, C.c_float, u64, u32, vp, vp]
+        L.tb_es_noise_combine.argtypes = [vp, vp, vp, i64, u64, u32, vp, vp]
+        L.tb_es_normalizer_stats.argtypes = [vp, vp, vp]
     L.tb_set_kernel_timing.argtypes = [vp, i32]
     L.tb_get_kernel_timing.argtypes = [vp, C.POINTER(dbl), C.POINTER(dbl), C.POINTER(i64)]
     _lib = L

@@ -197,6 +197,46 @@ class TennisBatch:
         _lib.check(self.lib.tb_es_rollout(self.h, k, _dptr(ret), _dptr(alive), _dptr(obs), _dptr(actions), _dptr(reward),
                                           _dptr(done), self._stream()))
 
+    # ------------------------------------------------------------------ ES population and update (seeded perturbations)
+    def _es_floats(self):
+        return _lib.ES_FLOATS if self.kind == _lib.ENV_SWING else _lib.ES_FLOATS_HIT
+
+    def es_begin_noise(self, theta, individuals, sigma, noise_seed, generation, normalizer=None):
+        """es_begin with the antithetic population drawn in the library: global individual g = env_id_offset // repeats + p is
+        theta + sigma * eps_{g // 2} for even g and theta - sigma * eps_{g // 2} for odd g (tb_es_begin_noise documents eps).
+        theta float32 [es_floats]; individuals even and dividing num_envs; env_id_offset a multiple of 2 x repeats."""
+        floats, individuals = self._es_floats(), int(individuals)
+        if individuals < 2 or individuals % 2 or self.num_envs % individuals:
+            raise ValueError(f"es_begin_noise: individuals must be even and divide {self.num_envs}, got {individuals}")
+        self._need("es_begin_noise", theta, "theta", (floats,), torch.float32)
+        self._need("es_begin_noise", normalizer, "normalizer", (3, self.obs_dim), torch.float64, optional=True)
+        _lib.check(self.lib.tb_es_begin_noise(self.h, _dptr(theta), individuals, floats, float(sigma), int(noise_seed) & (2 ** 64 - 1),
+                                              int(generation) & (2 ** 32 - 1), _dptr(normalizer), self._stream()))
+
+    def es_noise_combine(self, dirs, coef, noise_seed, generation, out=None):
+        """out float32 [es_floats] = sum_k coef[k] * eps_{dirs[k]} of `generation` (float64 sum in order k), regenerated from the
+        seed.  dirs int64 [count] (global direction indices), coef float32 [count]."""
+        count = int(dirs.shape[0]) if dirs is not None and dirs.dim() == 1 else -1
+        if count < 0:
+            raise ValueError(f"es_noise_combine: dirs must be a 1-d int64 tensor, got {None if dirs is None else tuple(dirs.shape)}")
+        self._need("es_noise_combine", dirs, "dirs", (count,), torch.int64)
+        self._need("es_noise_combine", coef, "coef", (count,), torch.float32)
+        if out is None:
+            out = torch.empty(self._es_floats(), dtype=torch.float32, device=self.device)
+        self._need("es_noise_combine", out, "out", (self._es_floats(),), torch.float32)
+        _lib.check(self.lib.tb_es_noise_combine(self.h, _dptr(dirs), _dptr(coef), count, int(noise_seed) & (2 ** 64 - 1),
+                                                int(generation) & (2 ** 32 - 1), _dptr(out), self._stream()))
+        return out
+
+    def es_normalizer_stats(self, out=None):
+        """float64 [3, obs_dim] = (count, mean, M2) of the observations this batch's normalisers took since the last
+        es_begin*, without the master's share.  Merge with the master (and other shards) by Chan's formula."""
+        if out is None:
+            out = torch.empty((3, self.obs_dim), dtype=torch.float64, device=self.device)
+        self._need("es_normalizer_stats", out, "out", (3, self.obs_dim), torch.float64)
+        _lib.check(self.lib.tb_es_normalizer_stats(self.h, _dptr(out), self._stream()))
+        return out
+
     def get_state(self):
         s = torch.empty((self.num_envs, _lib.STATE_WORDS), dtype=torch.float64, device=self.device)
         _lib.check(self.lib.tb_get_state(self.h, _dptr(s), self._stream()))

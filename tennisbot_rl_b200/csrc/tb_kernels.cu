@@ -1485,6 +1485,7 @@ struct EsIO {
   float *hist;                  // [8 OBS][N] ring of normalised observations; slot (tick - base) % 8 holds the newest
   double *ret;                  // [N] return summed while alive
   uint8_t *alive;               // [N] no done yet
+  unsigned *stop;               // [N] tick - base when alive flipped: the observations the env's normaliser took (valid once dead)
   const unsigned *tick;         // the env-step counter (StepIO::epoch[0] / [2]): constant while an es_kernel runs
   unsigned *base;               // its value at tb_es_begin, so tick - base = env steps since then
   const float *obs, *term, *reward;  // the previous env step's outputs (the context's buffers)
@@ -1533,7 +1534,7 @@ __global__ void __launch_bounds__(kBlock, 4) es_kernel(const __grid_constant__ E
     if (fold) {
       ret = io.ret[i] + (double)io.reward[i];
       io.ret[i] = ret;
-      if (d) { live = false; io.alive[i] = 0; }
+      if (d) { live = false; io.alive[i] = 0; io.stop[i] = s; }
     } else if (io.ret_out) {
       ret = io.ret[i];
     }
@@ -1664,6 +1665,149 @@ __global__ void es_transpose_kernel(const float *in, int64_t rows, int cols, flo
   __syncthreads();
   for (int j = threadIdx.y; j < 32; j += 8)
     if (c0 + j < cols && r0 + (int)threadIdx.x < rows) out[(int64_t)(c0 + j) * rows + r0 + threadIdx.x] = tile[threadIdx.x][j];
+}
+
+// ------------------------------------------------------------------------------------------------ ES population and update
+// ARS V2-t (Mania, Guy and Recht 2018) with the perturbations keyed by seed, as OpenAI-ES does: nothing of size
+// [individuals x floats] exists outside es_w, and every shard regenerates any direction it needs.
+// Noise of direction j (a global index), parameter f, generation g, noise seed s: one Philox call per four parameters,
+//   r = philox4x32(seed = s, id = j, episode = g, word = stream_word(kStreamEsNoise, f / 4, 0)),
+// and Box-Muller in float64 on the pairs (r[0], r[1]) -> parameters 4q, 4q + 1 and (r[2], r[3]) -> 4q + 2, 4q + 3 (q = f / 4):
+//   u1 = (r[2k] + 0.5) / 2^32,  u2 = r[2k + 1] / 2^32,  rho = sqrt(-2 ln u1),
+//   eps[4q + 2k] = float32(rho cos(2 pi u2)),  eps[4q + 2k + 1] = float32(rho sin(2 pi u2))   (one rounding, to nearest)
+// The stream id sits beside kStreamReset (0), kStreamAction (1) and kStreamPolicy (2); the env and policy streams are keyed by
+// env ids, this one by direction ids, so they never share a counter.
+constexpr uint32_t kStreamEsNoise = 3u;
+__device__ __forceinline__ void es_noise4(uint64_t seed, int64_t j, uint32_t gen, int q, float eps[4]) {
+  uint32_t r[4];
+  philox4x32(seed, (uint64_t)j, gen, stream_word(kStreamEsNoise, (uint32_t)q, 0), r);
+#pragma unroll
+  for (int k = 0; k < 2; ++k) {
+    const double u1 = ((double)r[2 * k] + 0.5) * 0x1p-32, u2 = (double)r[2 * k + 1] * 0x1p-32;
+    const double rho = sqrt(-2.0 * log(u1));
+    double sn, cs;
+    sincospi(2.0 * u2, &sn, &cs);
+    eps[2 * k] = __double2float_rn(rho * cs);
+    eps[2 * k + 1] = __double2float_rn(rho * sn);
+  }
+}
+
+// The population of tb_es_begin_noise straight into es_w [floats][2 pairs]: local individual p is global individual
+// g = g0 + p (g0 even), of direction j = g >> 1, with w = theta + d for even g and theta - d for odd g, d = sigma * eps_j
+// (each rounded on its own: no contraction).  Thread t makes the pair (2t, 2t + 1) of direction j0 + t and stores it as one
+// float2, so stores are coalesced along individuals; grid y runs over the quads of parameters.
+__global__ void __launch_bounds__(kBlock) es_perturb_kernel(const float *theta, int64_t pairs, int floats, float sigma,
+                                                            uint64_t seed, uint32_t gen, int64_t j0, float *w) {
+  const int64_t t = (int64_t)blockIdx.x * kBlock + threadIdx.x;
+  const int q = blockIdx.y;
+  if (t >= pairs) return;
+  float eps[4];
+  es_noise4(seed, j0 + t, gen, q, eps);
+#pragma unroll
+  for (int k = 0; k < 4; ++k) {
+    const int f = 4 * q + k;
+    if (f < floats) {
+      const float th = __ldg(theta + f), d = __fmul_rn(sigma, eps[k]);
+      reinterpret_cast<float2 *>(w + (int64_t)f * 2 * pairs)[t] = make_float2(__fadd_rn(th, d), __fsub_rn(th, d));
+    }
+  }
+}
+
+// out[f] = sum_k coef[k] * eps_{dirs[k]}[f], accumulated in float64 in the order k = 0, 1, ... and rounded to float32 once, so
+// the result depends on the inputs only.  One CTA per quad of parameters: its threads regenerate the terms of kBlock
+// directions at a time (each product of two float32 values is exact in float64), threads 0..3 add them in order.
+__global__ void __launch_bounds__(kBlock) es_combine_kernel(const int64_t *dirs, const float *coef, int64_t count, uint64_t seed,
+                                                            uint32_t gen, int floats, float *out) {
+  __shared__ double term[4][kBlock];
+  const int q = blockIdx.x;
+  double acc = 0.0;
+  for (int64_t k0 = 0; k0 < count; k0 += kBlock) {
+    const int64_t k = k0 + threadIdx.x;
+    if (k < count) {
+      float eps[4];
+      es_noise4(seed, dirs[k], gen, q, eps);
+      const double c = (double)coef[k];
+#pragma unroll
+      for (int m = 0; m < 4; ++m) term[m][threadIdx.x] = c * (double)eps[m];
+    }
+    __syncthreads();
+    if (threadIdx.x < 4) {
+      const int m = count - k0 < kBlock ? (int)(count - k0) : kBlock;
+      for (int i = 0; i < m; ++i) acc += term[threadIdx.x][i];
+    }
+    __syncthreads();
+  }
+  const int f = 4 * q + (int)threadIdx.x;
+  if (threadIdx.x < 4 && f < floats) out[f] = __double2float_rn(acc);
+}
+
+// Count, mean and M2 of a set of observations, the mean kept as its offset from the master's mean (small, well-conditioned).
+struct EsMoments { double n, d, m2; };
+// Chan, Golub and LeVeque's pairwise merge
+__device__ __forceinline__ EsMoments es_merge(EsMoments a, EsMoments b) {
+  if (b.n == 0.0) return a;
+  if (a.n == 0.0) return b;
+  const double n = a.n + b.n, delta = b.d - a.d;
+  return {n, a.d + delta * (b.n / n), a.m2 + b.m2 + delta * delta * (a.n * (b.n / n))};
+}
+constexpr int kEsStatsPer = 8;  // envs per thread of es_norm_partial_kernel
+
+// CTA-wide merge of one EsMoments per thread in a fixed tree; thread 0 gets the result
+__device__ __forceinline__ EsMoments es_merge_cta(EsMoments v) {
+  __shared__ double sh[3][kBlock];
+  __syncthreads();
+  sh[0][threadIdx.x] = v.n; sh[1][threadIdx.x] = v.d; sh[2][threadIdx.x] = v.m2;
+  for (int h = kBlock / 2; h > 0; h >>= 1) {
+    __syncthreads();
+    if ((int)threadIdx.x < h) {
+      const EsMoments r = es_merge({sh[0][threadIdx.x], sh[1][threadIdx.x], sh[2][threadIdx.x]},
+                                   {sh[0][threadIdx.x + h], sh[1][threadIdx.x + h], sh[2][threadIdx.x + h]});
+      sh[0][threadIdx.x] = r.n; sh[1][threadIdx.x] = r.d; sh[2][threadIdx.x] = r.m2;
+    }
+  }
+  __syncthreads();
+  return {sh[0][0], sh[1][0], sh[2][0]};
+}
+
+// Pass 1 of tb_es_normalizer_stats: each env's own share of its normaliser, the observations since tb_es_begin*, split off
+// the master's (n0, mu0, M0).  Env e took m_e observations (tick - base + 1 while alive: the reset observation and one per
+// step; io.stop once dead) and holds N = n0 + m_e, mean mu_e and mean_diff D_e, so its own observations have
+//   mean - mu0 = (mu_e - mu0) N / m_e,   M2 = (D_e - M0) - (mean - mu0)^2 n0 m_e / N.
+// Each thread merges kEsStatsPer envs in order, the CTA merges its threads in a fixed tree: part[blockIdx.x][3][OBS].
+template <int OBS>
+__global__ void __launch_bounds__(kBlock) es_norm_partial_kernel(const __grid_constant__ EsIO io, const double *m0, double *part) {
+  const int64_t n = io.n, e0 = (int64_t)blockIdx.x * kBlock * kEsStatsPer + threadIdx.x;
+  const unsigned s = *io.tick - *io.base;
+  for (int c = 0; c < OBS; ++c) {
+    const double n0 = m0[c], mu0 = m0[OBS + c], M0 = m0[2 * OBS + c];
+    EsMoments v = {0.0, 0.0, 0.0};
+    for (int r = 0; r < kEsStatsPer; ++r) {
+      const int64_t e = e0 + (int64_t)r * kBlock;
+      if (e >= n) break;
+      const double m = io.alive[e] ? (double)(s + 1u) : (double)io.stop[e], nn = n0 + m;
+      const double d = (io.norm[c * n + e] - mu0) * (nn / m);
+      v = es_merge(v, {m, d, (io.norm[(OBS + c) * n + e] - M0) - d * d * (n0 * (m / nn))});
+    }
+    v = es_merge_cta(v);
+    if (threadIdx.x == 0) {
+      double *p = part + (int64_t)blockIdx.x * 3 * OBS;
+      p[c] = v.n; p[OBS + c] = v.d; p[2 * OBS + c] = v.m2;
+    }
+  }
+}
+
+// Pass 2: one CTA per observation channel merges the `blocks` partials (each thread a strided subset in order, then the
+// fixed tree) and writes out [3][OBS] = (count, mean, M2).
+__global__ void __launch_bounds__(kBlock) es_norm_final_kernel(const double *part, int64_t blocks, int obs, const double *m0,
+                                                               double *out) {
+  const int c = blockIdx.x;
+  EsMoments v = {0.0, 0.0, 0.0};
+  for (int64_t b = threadIdx.x; b < blocks; b += kBlock) {
+    const double *p = part + b * 3 * obs;
+    v = es_merge(v, {p[c], p[obs + c], p[2 * obs + c]});
+  }
+  v = es_merge_cta(v);
+  if (threadIdx.x == 0) { out[c] = v.n; out[obs + c] = m0[obs + c] + v.d; out[2 * obs + c] = v.m2; }
 }
 
 template <typename T, int KIND>
@@ -2128,6 +2272,9 @@ struct tb_ctx {
   float *es_hist = nullptr, *es_obs = nullptr, *es_term = nullptr, *es_rew = nullptr, *es_act = nullptr;
   uint8_t *es_alive = nullptr, *es_done = nullptr;
   unsigned *es_base = nullptr;
+  unsigned *es_stop = nullptr;               // [N] see EsIO::stop
+  double *es_master = nullptr;               // [3, obs_dim] the generation's master normaliser (zeros for NULL)
+  double *es_part = nullptr;                 // es_norm_partial_kernel's per-CTA moments
   bool timing = false;                      // tb_set_kernel_timing
   cudaEvent_t ev[3] = {nullptr, nullptr, nullptr};
   double ms_step = 0, ms_ff = 0;
@@ -2459,6 +2606,7 @@ int tb_destroy(tb_ctx *c) {
   cudaFree(c->state); cudaFree(c->stats); cudaFree(c->queue_ctrs); cudaFree(c->queue); cudaFree(c->dq); cudaFree(c->epoch); cudaFree(c->fault); cudaFree(c->queue_full); cudaFree(c->queue_ctl); cudaFree(c->pid); cudaFree(c->policy); cudaFree(c->pol_act);
   cudaFree(c->es_w); cudaFree(c->es_norm); cudaFree(c->es_n0); cudaFree(c->es_ret); cudaFree(c->es_hist); cudaFree(c->es_obs);
   cudaFree(c->es_term); cudaFree(c->es_rew); cudaFree(c->es_act); cudaFree(c->es_alive); cudaFree(c->es_done); cudaFree(c->es_base);
+  cudaFree(c->es_stop); cudaFree(c->es_master); cudaFree(c->es_part);
   if (c->h_fault) cudaFreeHost(c->h_fault);
   cudaFree(c->d_actions); cudaFree(c->d_obs); cudaFree(c->d_reward); cudaFree(c->d_term);
   cudaFree(c->d_done); cudaFree(c->d_events); cudaFree(c->d_mask);
@@ -2598,31 +2746,37 @@ static EsIO es_io(tb_ctx *c) {
   std::memset(&io, 0, sizeof io);
   io.w = c->es_w; io.n = c->cfg.num_envs; io.individuals = c->es_individuals;
   io.repeats = c->es_individuals ? (int)(c->cfg.num_envs / c->es_individuals) : 0;
-  io.norm = c->es_norm; io.n0 = c->es_n0; io.hist = c->es_hist; io.ret = c->es_ret; io.alive = c->es_alive;
+  io.norm = c->es_norm; io.n0 = c->es_n0; io.hist = c->es_hist; io.ret = c->es_ret; io.alive = c->es_alive; io.stop = c->es_stop;
   io.tick = c->cfg.env_kind == TB_ENV_SWING ? c->epoch : c->epoch + 2;  // (see StepIO::epoch)
   io.base = c->es_base;
   io.obs = c->es_obs; io.term = c->es_term; io.reward = c->es_rew; io.done = c->es_done;
   return io;
 }
 
-int tb_es_begin(tb_ctx *c, const float *d_weights, int64_t individuals, int64_t floats, const double *d_normalizer, void *stream) {
-  if (!d_weights) return fail("%s", "tb_es_begin: d_weights is NULL");
-  if (individuals < 1) return fail("%s", "tb_es_begin: individuals must be >= 1");
-  GUARD(c);
+static int64_t es_norm_blocks(int64_t n) { return (n + kBlock * kEsStatsPer - 1) / (kBlock * kEsStatsPer); }
+
+// The checks tb_es_begin and tb_es_begin_noise share once the context is current, then the per-env state (once per context)
+// and room for the population in es_w.
+static int es_prepare(tb_ctx *c, const char *who, int64_t individuals, int64_t floats, cudaStream_t s) {
   const int64_t n = c->cfg.num_envs, want = tb_es_floats(c->cfg.env_kind);
   if (floats != want) {
-    std::snprintf(g_err, sizeof g_err, "tb_es_begin: expected tb_es_floats(env_kind) = %lld floats per individual, got %lld",
+    std::snprintf(g_err, sizeof g_err, "%s: expected tb_es_floats(env_kind) = %lld floats per individual, got %lld", who,
                   (long long)want, (long long)floats);
     return 1;
   }
   if (n % individuals) {
-    std::snprintf(g_err, sizeof g_err, "tb_es_begin: individuals (%lld) must divide num_envs (%lld)", (long long)individuals, (long long)n);
+    std::snprintf(g_err, sizeof g_err, "%s: individuals (%lld) must divide num_envs (%lld)", who, (long long)individuals, (long long)n);
     return 1;
   }
-  if (individuals * floats > 0xffffffffLL) return fail("%s", "tb_es_begin: individuals x floats must be below 2^32 (es_kernel indexes the population with 32 bits)");
-  if (c->control_mode != TB_CONTROL_FORCE) return fail("%s", "tb_es_begin: the GatedCNN's actions are forces (TB_CONTROL_FORCE)");
-  if (check_fault(c, "tb_es_begin")) return 1;
-  cudaStream_t s = (cudaStream_t)stream;
+  if (individuals * floats > 0xffffffffLL) {
+    std::snprintf(g_err, sizeof g_err, "%s: individuals x floats must be below 2^32 (es_kernel indexes the population with 32 bits)", who);
+    return 1;
+  }
+  if (c->control_mode != TB_CONTROL_FORCE) {
+    std::snprintf(g_err, sizeof g_err, "%s: the GatedCNN's actions are forces (TB_CONTROL_FORCE)", who);
+    return 1;
+  }
+  if (check_fault(c, who)) return 1;
   const int od = tb_obs_dim(c->cfg.env_kind), ad = tb_act_dim(c->cfg.env_kind);
   if (!c->es_norm) {  // per-env state, once per context
     CU(cudaMalloc(&c->es_norm, (size_t)2 * od * n * sizeof(double)));
@@ -2636,6 +2790,9 @@ int tb_es_begin(tb_ctx *c, const float *d_weights, int64_t individuals, int64_t 
     CU(cudaMalloc(&c->es_alive, (size_t)n));
     CU(cudaMalloc(&c->es_done, (size_t)n));
     CU(cudaMalloc(&c->es_base, sizeof(unsigned)));
+    CU(cudaMalloc(&c->es_stop, (size_t)n * sizeof(unsigned)));
+    CU(cudaMalloc(&c->es_master, (size_t)3 * od * sizeof(double)));
+    CU(cudaMalloc(&c->es_part, (size_t)es_norm_blocks(n) * 3 * od * sizeof(double)));
   }
   if (c->es_w_cap < individuals * floats) {  // stream-ordered: a larger population does not synchronise either
     if (c->es_w) CU(cudaFreeAsync(c->es_w, s));
@@ -2643,9 +2800,15 @@ int tb_es_begin(tb_ctx *c, const float *d_weights, int64_t individuals, int64_t 
     CU(cudaMallocAsync(&c->es_w, (size_t)(individuals * floats) * sizeof(float), s));
     c->es_w_cap = individuals * floats;
   }
-  es_transpose_kernel<<<dim3((unsigned)((individuals + 31) / 32), (unsigned)((floats + 31) / 32)), dim3(32, 8), 0, s>>>(
-      d_weights, individuals, (int)floats, c->es_w);
-  c->launches++;
+  return 0;
+}
+
+// Once es_w holds the population: reset every env, seed the normalisers from the master (kept for tb_es_normalizer_stats).
+static int es_start(tb_ctx *c, int64_t individuals, const double *d_normalizer, cudaStream_t s) {
+  const int64_t n = c->cfg.num_envs;
+  const size_t master_bytes = (size_t)3 * tb_obs_dim(c->cfg.env_kind) * sizeof(double);
+  if (d_normalizer) CU(cudaMemcpyAsync(c->es_master, d_normalizer, master_bytes, cudaMemcpyDeviceToDevice, s));
+  else CU(cudaMemsetAsync(c->es_master, 0, master_bytes, s));
   StepIO io = make_io(c);
   io.obs = c->es_obs;
   DISPATCH(reset_kernel, grid_for(n, kBlock), kBlock, s, io, (const double *)nullptr, (const uint8_t *)nullptr);
@@ -2655,6 +2818,72 @@ int tb_es_begin(tb_ctx *c, const float *d_weights, int64_t individuals, int64_t 
   if (c->cfg.env_kind == TB_ENV_SWING) es_begin_kernel<6><<<grid_for(n, kBlock), kBlock, 0, s>>>(eio, d_normalizer);
   else es_begin_kernel<12><<<grid_for(n, kBlock), kBlock, 0, s>>>(eio, d_normalizer);
   c->launches++;
+  CU(cudaGetLastError());
+  return 0;
+}
+
+int tb_es_begin(tb_ctx *c, const float *d_weights, int64_t individuals, int64_t floats, const double *d_normalizer, void *stream) {
+  if (!d_weights) return fail("%s", "tb_es_begin: d_weights is NULL");
+  if (individuals < 1) return fail("%s", "tb_es_begin: individuals must be >= 1");
+  GUARD(c);
+  cudaStream_t s = (cudaStream_t)stream;
+  if (es_prepare(c, "tb_es_begin", individuals, floats, s)) return 1;
+  es_transpose_kernel<<<dim3((unsigned)((individuals + 31) / 32), (unsigned)((floats + 31) / 32)), dim3(32, 8), 0, s>>>(
+      d_weights, individuals, (int)floats, c->es_w);
+  c->launches++;
+  return es_start(c, individuals, d_normalizer, s);
+}
+
+int tb_es_begin_noise(tb_ctx *c, const float *d_theta, int64_t individuals, int64_t floats, float sigma, uint64_t noise_seed,
+                      uint32_t generation, const double *d_normalizer, void *stream) {
+  if (!d_theta) return fail("%s", "tb_es_begin_noise: d_theta is NULL");
+  if (individuals < 1) return fail("%s", "tb_es_begin_noise: individuals must be >= 1");
+  if (individuals % 2) return fail("%s", "tb_es_begin_noise: individuals must be even (antithetic pairs)");
+  if (!(sigma > 0.0f) || !std::isfinite(sigma)) return fail("%s", "tb_es_begin_noise: sigma must be a finite number above 0");
+  GUARD(c);
+  const int64_t repeats = individuals > 0 && c->cfg.num_envs % individuals == 0 ? c->cfg.num_envs / individuals : 0;
+  if (repeats && c->cfg.env_id_offset % (2 * repeats)) {
+    std::snprintf(g_err, sizeof g_err, "tb_es_begin_noise: env_id_offset (%lld) must be a multiple of 2 x repeats (%lld), so a shard "
+                  "holds whole antithetic pairs", (long long)c->cfg.env_id_offset, (long long)(2 * repeats));
+    return 1;
+  }
+  cudaStream_t s = (cudaStream_t)stream;
+  if (es_prepare(c, "tb_es_begin_noise", individuals, floats, s)) return 1;
+  const int64_t pairs = individuals / 2, j0 = c->cfg.env_id_offset / (2 * repeats);
+  es_perturb_kernel<<<dim3(grid_for(pairs, kBlock), (unsigned)((floats + 3) / 4)), kBlock, 0, s>>>(
+      d_theta, pairs, (int)floats, sigma, noise_seed, generation, j0, c->es_w);
+  c->launches++;
+  return es_start(c, individuals, d_normalizer, s);
+}
+
+int tb_es_noise_combine(tb_ctx *c, const int64_t *d_dirs, const float *d_coef, int64_t count, uint64_t noise_seed, uint32_t generation,
+                        float *d_out, void *stream) {
+  if (count < 0) return fail("%s", "tb_es_noise_combine: count must be >= 0");
+  if (count > 0 && (!d_dirs || !d_coef)) return fail("%s", "tb_es_noise_combine: d_dirs and d_coef are required when count > 0");
+  if (!d_out) return fail("%s", "tb_es_noise_combine: d_out is NULL");
+  GUARD(c);
+  if (check_fault(c, "tb_es_noise_combine")) return 1;
+  const int floats = tb_es_floats(c->cfg.env_kind);
+  es_combine_kernel<<<(unsigned)((floats + 3) / 4), kBlock, 0, (cudaStream_t)stream>>>(d_dirs, d_coef, count, noise_seed,
+                                                                                         generation, floats, d_out);
+  c->launches++;
+  CU(cudaGetLastError());
+  return 0;
+}
+
+int tb_es_normalizer_stats(tb_ctx *c, double *d_out, void *stream) {
+  if (!d_out) return fail("%s", "tb_es_normalizer_stats: d_out is NULL");
+  GUARD(c);
+  if (!c->es_individuals) return fail("%s", "tb_es_normalizer_stats: no generation (call tb_es_begin or tb_es_begin_noise first)");
+  if (check_fault(c, "tb_es_normalizer_stats")) return 1;
+  cudaStream_t s = (cudaStream_t)stream;
+  const int64_t blocks = es_norm_blocks(c->cfg.num_envs);
+  const EsIO eio = es_io(c);
+  const int od = tb_obs_dim(c->cfg.env_kind);
+  if (c->cfg.env_kind == TB_ENV_SWING) es_norm_partial_kernel<6><<<(unsigned)blocks, kBlock, 0, s>>>(eio, c->es_master, c->es_part);
+  else es_norm_partial_kernel<12><<<(unsigned)blocks, kBlock, 0, s>>>(eio, c->es_master, c->es_part);
+  es_norm_final_kernel<<<(unsigned)od, kBlock, 0, s>>>(c->es_part, blocks, od, c->es_master, d_out);
+  c->launches += 2;
   CU(cudaGetLastError());
   return 0;
 }

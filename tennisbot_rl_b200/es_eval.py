@@ -138,6 +138,12 @@ class EsEvaluator:
     def close(self):
         self.env.close()
 
+    def _normalizer(self, normalizer_state):
+        if normalizer_state is None:
+            return None
+        dev, od = self.env.device, self.env.obs_dim
+        return torch.stack([torch.as_tensor(x, dtype=torch.float64, device=dev).reshape(od) for x in normalizer_state[:3]])
+
     @torch.no_grad()
     def evaluate(self, weights, normalizer_state=None, max_steps=1001):
         """weights [individuals, num_params]; normalizer_state: the master's (n, mean, mean_diff, var) as BatchedNormalizer takes
@@ -145,14 +151,33 @@ class EsEvaluator:
         batched_fitness_static: the return of every env summed until its first done or max_steps."""
         if int(max_steps) < 1:
             raise ValueError(f"EsEvaluator.evaluate: max_steps must be >= 1, got {max_steps}")
-        dev, od = self.env.device, self.env.obs_dim
-        w = torch.as_tensor(weights, dtype=torch.float32, device=dev).contiguous()
+        w = torch.as_tensor(weights, dtype=torch.float32, device=self.env.device).contiguous()
         if tuple(w.shape) != (self.individuals, self.num_params):
             raise ValueError(f"weights must have shape ({self.individuals}, {self.num_params}), got {tuple(w.shape)}")
-        norm = None
-        if normalizer_state is not None:
-            norm = torch.stack([torch.as_tensor(x, dtype=torch.float64, device=dev).reshape(od) for x in normalizer_state[:3]])
-        self.env.es_begin(w, norm)
+        self.env.es_begin(w, self._normalizer(normalizer_state))
+        return self.run(max_steps)
+
+    @torch.no_grad()
+    def evaluate_noise(self, theta, sigma, noise_seed, generation, normalizer_state=None, max_steps=1001):
+        """evaluate() on the antithetic population the library draws around theta [num_params]: global individual
+        g = env_id_offset // repeats + p is theta + sigma * eps_{g // 2} (g even) or theta - sigma * eps_{g // 2} (g odd), eps
+        keyed by (noise_seed, direction, generation) as tb_es_begin_noise documents.  individuals must be even."""
+        self.begin_noise(theta, sigma, noise_seed, generation, normalizer_state)
+        return self.run(max_steps)
+
+    def begin_noise(self, theta, sigma, noise_seed, generation, normalizer_state=None):
+        """The first half of evaluate_noise: draw the population and start the generation (no synchronisation)."""
+        th = torch.as_tensor(theta, dtype=torch.float32, device=self.env.device).reshape(-1).contiguous()
+        if th.numel() != self.num_params:
+            raise ValueError(f"theta must have {self.num_params} entries, got {th.numel()}")
+        self.env.es_begin_noise(th, self.individuals, sigma, noise_seed, generation, self._normalizer(normalizer_state))
+
+    @torch.no_grad()
+    def run(self, max_steps=1001):
+        """Roll the started generation out in CHUNK-step calls until every env is done or max_steps; returns
+        (fitness [individuals], returns [individuals, repeats])."""
+        if int(max_steps) < 1:
+            raise ValueError(f"EsEvaluator.run: max_steps must be >= 1, got {max_steps}")
         steps = 0
         while steps < max_steps:
             k = min(self.CHUNK, int(max_steps) - steps)

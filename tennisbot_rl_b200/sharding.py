@@ -27,6 +27,18 @@ def all_reduce_stats(stats, group=None):
     return stats
 
 
+def all_gather(t, group=None):
+    """Concatenate every rank's `t` along dim 0 in rank order (EsTrainer's `gather`: each rank evaluates an equal, contiguous
+    shard of the directions).  Identity without an initialised process group of more than one rank."""
+    import torch.distributed as dist
+
+    if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size(group) == 1:
+        return t
+    parts = [torch.empty_like(t) for _ in range(dist.get_world_size(group))]
+    dist.all_gather(parts, t.contiguous(), group=group)
+    return torch.cat(parts)
+
+
 def make_shard(env_id, total_envs, rank, world, device=None, seed=0, precision="f64"):
     """TennisBatch for this rank's shard of a `total_envs` batch."""
     from .batch import TennisBatch
