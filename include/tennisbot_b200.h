@@ -252,7 +252,7 @@ int tb_reset_host(tb_ctx *ctx, const uint8_t *h_mask, float *h_obs);
 int tb_step_host(tb_ctx *ctx, const float *h_actions, float *h_obs, float *h_reward, uint8_t *h_done,
                  float *h_terminal_obs, uint8_t *h_events);
 
-/* number of kernels this context has launched (bench.py's gpu_launches) */
+/* number of kernels this context has launched, tb_create's and tb_set_param's included (bench.py's gpu_launches) */
 int tb_launch_count(tb_ctx *ctx, int64_t *launches);
 
 /* Diagnostics of the most recent SwingRacket fast-forward (the launch of tb_step's second kernel on an env's 26th

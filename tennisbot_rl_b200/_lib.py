@@ -25,21 +25,36 @@ EV_RACKET_BALL, EV_COURT_BALL, EV_GOAL_BALL, EV_TIMEOUT, EV_BALL_PASSED, EV_NET_
 STAT_NAMES = ("episodes", "sum_length", "racket_hits", "goals", "court", "timeouts", "sum_return_q20",
               "sum_return2_q10", "physics_steps", "env_steps")
 
-# every symbol include/tennisbot_b200.h declares (checked by tests/test_abi.py)
-EXPORTS = (
-    "tb_last_error", "tb_abi_version", "tb_obs_dim", "tb_act_dim", "tb_policy_floats", "tb_num_params", "tb_param_name",
-    "tb_scene_constant", "tb_create", "tb_destroy", "tb_set_param", "tb_get_param", "tb_set_control_mode", "tb_reset", "tb_reset_from",
-    "tb_step", "tb_rollout", "tb_get_state", "tb_set_state", "tb_stats_device_ptr", "tb_read_stats",
-    "tb_reset_host", "tb_step_host", "tb_launch_count", "tb_ff_diagnostics", "tb_set_kernel_timing", "tb_get_kernel_timing",
-    "tb_set_policy", "tb_policy_rollout", "tb_es_floats", "tb_es_begin", "tb_es_rollout",
-    "tb_es_begin_noise", "tb_es_noise_combine", "tb_es_normalizer_stats",
-)
-
-
 class TbConfig(C.Structure):
     _fields_ = [("struct_size", C.c_uint32), ("env_kind", C.c_int32), ("precision", C.c_int32), ("device", C.c_int32),
                 ("num_envs", C.c_int64), ("env_id_offset", C.c_int64), ("seed", C.c_uint64),
                 ("auto_reset", C.c_int32), ("reserved", C.c_int32)]
+
+
+_vp, _i32, _u32, _i64, _u64, _dbl = C.c_void_p, C.c_int, C.c_uint32, C.c_int64, C.c_uint64, C.c_double
+_str, _dblp, _i64p = C.c_char_p, C.POINTER(C.c_double), C.POINTER(C.c_int64)
+# argument types of every entry point include/tennisbot_b200.h declares (tests/test_abi.py checks the names); all return int
+# except those in _STRING_RESULTS
+SIGNATURES = {
+    "tb_last_error": [], "tb_abi_version": [], "tb_obs_dim": [_i32], "tb_act_dim": [_i32], "tb_policy_floats": [_i32],
+    "tb_es_floats": [_i32], "tb_num_params": [], "tb_param_name": [_i32], "tb_scene_constant": [_str, _i32, _dblp],
+    "tb_create": [C.POINTER(TbConfig), C.POINTER(_vp)], "tb_destroy": [_vp],
+    "tb_set_param": [_vp, _str, _dbl], "tb_get_param": [_vp, _str, _dblp], "tb_set_control_mode": [_vp, _i32],
+    "tb_reset": [_vp, _vp, _vp, _vp], "tb_reset_from": [_vp, _vp, _vp, _vp, _vp],
+    "tb_step": [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp], "tb_rollout": [_vp, _i32, _i32, _vp, _vp, _vp, _vp],
+    "tb_set_policy": [_vp, _vp, _i64, _vp],
+    "tb_policy_rollout": [_vp, _i32, _i32, _u64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
+    "tb_es_begin": [_vp, _vp, _i64, _i64, _vp, _vp], "tb_es_rollout": [_vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
+    "tb_es_begin_noise": [_vp, _vp, _i64, _i64, C.c_float, _u64, _u32, _vp, _vp],
+    "tb_es_noise_combine": [_vp, _vp, _vp, _i64, _u64, _u32, _vp, _vp], "tb_es_normalizer_stats": [_vp, _vp, _vp],
+    "tb_get_state": [_vp, _vp, _vp], "tb_set_state": [_vp, _vp, _vp],
+    "tb_stats_device_ptr": [_vp, C.POINTER(_vp)], "tb_read_stats": [_vp, _vp, _i32, _vp],
+    "tb_reset_host": [_vp, _vp, _vp], "tb_step_host": [_vp, _vp, _vp, _vp, _vp, _vp, _vp],
+    "tb_launch_count": [_vp, _i64p], "tb_ff_diagnostics": [_vp, _i64p],
+    "tb_set_kernel_timing": [_vp, _i32], "tb_get_kernel_timing": [_vp, _dblp, _dblp, _i64p],
+}
+_STRING_RESULTS = ("tb_last_error", "tb_param_name")
+EXPORTS = tuple(SIGNATURES)
 
 
 class TennisbotLibraryError(RuntimeError):
@@ -59,47 +74,13 @@ def load():
             f"{LIB_PATH} is missing: build it with `python -m tennisbot_rl_b200.build` "
             "(needs nvcc; there is no CPU fallback for the env step)")
     L = C.CDLL(str(LIB_PATH))
-    vp, i32, i64, dbl = C.c_void_p, C.c_int, C.c_int64, C.c_double
-    L.tb_last_error.restype = C.c_char_p
-    L.tb_param_name.restype = C.c_char_p
-    L.tb_param_name.argtypes = [i32]
-    L.tb_obs_dim.argtypes = [i32]
-    L.tb_act_dim.argtypes = [i32]
-    if hasattr(L, "tb_policy_floats"):
-        L.tb_policy_floats.argtypes = [i32]
-    L.tb_scene_constant.argtypes = [C.c_char_p, i32, C.POINTER(dbl)]
-    L.tb_create.argtypes = [C.POINTER(TbConfig), C.POINTER(vp)]
-    L.tb_destroy.argtypes = [vp]
-    L.tb_set_param.argtypes = [vp, C.c_char_p, dbl]
-    L.tb_get_param.argtypes = [vp, C.c_char_p, C.POINTER(dbl)]
-    L.tb_set_control_mode.argtypes = [vp, i32]
-    L.tb_reset.argtypes = [vp, vp, vp, vp]
-    L.tb_reset_from.argtypes = [vp, vp, vp, vp, vp]
-    L.tb_step.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp]
-    L.tb_rollout.argtypes = [vp, i32, i32, vp, vp, vp, vp]
-    L.tb_get_state.argtypes = [vp, vp, vp]
-    L.tb_set_state.argtypes = [vp, vp, vp]
-    L.tb_stats_device_ptr.argtypes = [vp, C.POINTER(vp)]
-    L.tb_read_stats.argtypes = [vp, vp, i32, vp]
-    L.tb_reset_host.argtypes = [vp, vp, vp]
-    L.tb_step_host.argtypes = [vp, vp, vp, vp, vp, vp, vp]
-    L.tb_launch_count.argtypes = [vp, C.POINTER(i64)]
-    if hasattr(L, "tb_ff_diagnostics"):  # absent from older builds loaded through TB_LIB_PATH for comparisons
-        L.tb_ff_diagnostics.argtypes = [vp, C.POINTER(i64)]
-    if hasattr(L, "tb_set_policy"):
-        L.tb_set_policy.argtypes = [vp, vp, i64, vp]
-        L.tb_policy_rollout.argtypes = [vp, i32, i32, C.c_uint64, vp, vp, vp, vp, vp, vp, vp, vp, vp]
-    if hasattr(L, "tb_es_begin"):
-        L.tb_es_floats.argtypes = [i32]
-        L.tb_es_begin.argtypes = [vp, vp, i64, i64, vp, vp]
-        L.tb_es_rollout.argtypes = [vp, i32, vp, vp, vp, vp, vp, vp, vp]
-    if hasattr(L, "tb_es_begin_noise"):
-        u32, u64 = C.c_uint32, C.c_uint64
-        L.tb_es_begin_noise.argtypes = [vp, vp, i64, i64, C.c_float, u64, u32, vp, vp]
-        L.tb_es_noise_combine.argtypes = [vp, vp, vp, i64, u64, u32, vp, vp]
-        L.tb_es_normalizer_stats.argtypes = [vp, vp, vp]
-    L.tb_set_kernel_timing.argtypes = [vp, i32]
-    L.tb_get_kernel_timing.argtypes = [vp, C.POINTER(dbl), C.POINTER(dbl), C.POINTER(i64)]
+    for name, argtypes in SIGNATURES.items():
+        f = getattr(L, name, None)
+        if f is None:  # absent from older builds loaded through TB_LIB_PATH for comparisons
+            continue
+        f.argtypes = argtypes
+        if name in _STRING_RESULTS:
+            f.restype = C.c_char_p
     _lib = L
     return L
 

@@ -5,6 +5,7 @@ libtennisbot_b200.so (csrc/tb_kernels.cu).  Replaces, for a batch, what one refe
 p.connect / loadURDF / stepSimulation / getContactPoints (tennisbot/envs/*.py, tennisbot/resources/*.py).
 """
 import ctypes as C
+import functools
 
 import numpy as np
 import torch
@@ -120,6 +121,14 @@ class TennisBatch:
         _lib.check(self.lib.tb_rollout(self.h, int(action_mode), int(k_steps), *args, self._stream()))
         return (self.obs, self._rsum, self._dcount) if want_outputs else None
 
+    def _need(self, who, t, name, shape, dtype=torch.float32, optional=False):
+        """The library writes through raw pointers: a buffer must be a contiguous tensor of this shape and dtype on this device."""
+        if t is None and optional:
+            return
+        if t is None or t.dtype != dtype or t.device != self.device or not t.is_contiguous() or tuple(t.shape) != shape:
+            got = None if t is None else (tuple(t.shape), t.dtype, str(t.device), t.is_contiguous())
+            raise ValueError(f"{who}: {name} must be a contiguous {dtype} tensor of shape {shape} on {self.device}, got {got}")
+
     # ------------------------------------------------------------------ policy rollout (tb_set_policy / tb_policy_rollout)
     def set_policy(self, params):
         """params: float32 CUDA tensor [policy_floats] in the layout of include/tennisbot_b200.h for this batch's env
@@ -137,17 +146,9 @@ class TennisBatch:
         [N, obs_dim], last_value [N]: contiguous float32 tensors on this batch's device; done [K, N] uint8.  The library
         writes through raw pointers, so every buffer is checked here."""
         k, n = int(obs.shape[0]) if obs.dim() == 3 else -1, self.num_envs
-
-        def need(t, name, shape, dtype=torch.float32, optional=False):
-            if t is None and optional:
-                return
-            if (t is None or t.dtype != dtype or t.device != self.device or not t.is_contiguous() or tuple(t.shape) != shape):
-                got = None if t is None else (tuple(t.shape), t.dtype, str(t.device), t.is_contiguous())
-                raise ValueError(f"policy_rollout: {name} must be a contiguous {dtype} tensor of shape {shape} on {self.device}, "
-                                 f"got {got}")
-
         if k < 1:
             raise ValueError(f"policy_rollout: obs must have shape (K >= 1, {n}, {self.obs_dim}), got {tuple(obs.shape)}")
+        need = functools.partial(self._need, "policy_rollout")
         need(obs, "obs", (k, n, self.obs_dim))
         need(actions, "actions", (k, n, self.act_dim), optional=True)
         need(logp, "logp", (k, n), optional=True)
@@ -161,18 +162,11 @@ class TennisBatch:
                                               _dptr(last_value), self._stream()))
 
     # ------------------------------------------------------------------ ES fitness rollout (tb_es_begin / tb_es_rollout)
-    def _need(self, who, t, name, shape, dtype, optional=False):
-        if t is None and optional:
-            return
-        if t is None or t.dtype != dtype or t.device != self.device or not t.is_contiguous() or tuple(t.shape) != shape:
-            got = None if t is None else (tuple(t.shape), t.dtype, str(t.device), t.is_contiguous())
-            raise ValueError(f"{who}: {name} must be a contiguous {dtype} tensor of shape {shape} on {self.device}, got {got}")
-
     def es_begin(self, weights, normalizer=None):
         """Start an ES generation: weights float32 [individuals, es_floats] (individuals divides num_envs; env i evaluates
         individual i // (num_envs // individuals)), normalizer float64 [3, obs_dim] = the master (n, mean, mean_diff) or None.
         Resets every env, so a generation always starts new episodes."""
-        floats = _lib.ES_FLOATS if self.kind == _lib.ENV_SWING else _lib.ES_FLOATS_HIT
+        floats = self._es_floats()
         if weights.dim() != 2 or weights.shape[1] != floats or weights.shape[0] < 1 or self.num_envs % weights.shape[0]:
             raise ValueError(f"es_begin: weights must have shape (individuals, {floats}) with individuals dividing {self.num_envs}, "
                              f"got {tuple(weights.shape)}")

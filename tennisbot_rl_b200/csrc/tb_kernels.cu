@@ -11,11 +11,14 @@
 
 #include <algorithm>
 #include <cmath>
+#include <cstdarg>
 #include <cstddef>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <memory>
 #include <new>
+#include <type_traits>
 #include <utility>
 
 #include "tb_device.cuh"
@@ -2221,64 +2224,94 @@ template <typename T> static void build_scene(const Params &p, Scene<T> &sc) {
 using namespace tb;
 
 static thread_local char g_err[512];
-static int fail(const char *fmt, const char *detail = "") {
-  std::snprintf(g_err, sizeof g_err, fmt, detail);
+__attribute__((format(printf, 1, 2))) static int fail(const char *fmt, ...) {
+  va_list ap;
+  va_start(ap, fmt);
+  std::vsnprintf(g_err, sizeof g_err, fmt, ap);
+  va_end(ap);
   return 1;
 }
-#define CU(call)                                                                     \
-  do {                                                                               \
-    cudaError_t e_ = (call);                                                         \
-    if (e_ != cudaSuccess) {                                                         \
-      std::snprintf(g_err, sizeof g_err, "%s failed: %s", #call, cudaGetErrorString(e_)); \
-      return 1;                                                                      \
-    }                                                                                \
+#define CU(call)                                                                          \
+  do {                                                                                    \
+    const cudaError_t e_ = (call);                                                        \
+    if (e_ != cudaSuccess) return fail("%s failed: %s", #call, cudaGetErrorString(e_));  \
   } while (0)
+
+// Device memory owned by a context: freed with it, and on the error paths that leave a buffer or a partly built group behind.
+struct CudaFree { void operator()(void *p) const { cudaFree(p); } };
+struct CudaFreeHost { void operator()(void *p) const { cudaFreeHost(p); } };
+template <typename T> using DevPtr = std::unique_ptr<T, CudaFree>;
+template <typename T> static cudaError_t dev_alloc(DevPtr<T> &p, size_t bytes) {
+  void *raw = nullptr;
+  const cudaError_t e = cudaMalloc(&raw, bytes);
+  p.reset(static_cast<T *>(raw));
+  return e;
+}
+
+// The groups allocated on first use.  Each is built in a local and moved into the context once all of it exists, so a call
+// that fails part-way leaves the group absent and the next call builds it again.
+struct EsBufs {               // per-env state of the ES rollout (see EsIO), from the first tb_es_begin*
+  DevPtr<double> norm, n0, ret;
+  DevPtr<float> hist, obs, term, rew, act;
+  DevPtr<uint8_t> alive, done;
+  DevPtr<unsigned> base;
+  DevPtr<unsigned> stop;      // [N] see EsIO::stop
+  DevPtr<double> master;      // [3, obs_dim] the generation's master normaliser (zeros for NULL)
+  DevPtr<double> part;        // es_norm_partial_kernel's per-CTA moments
+};
+struct StagingBufs {          // device copies of the host-buffer entry points' arrays
+  DevPtr<float> actions, obs, reward, term;
+  DevPtr<uint8_t> done, events, mask;
+};
+struct PolicyBufs {           // tb_set_policy
+  DevPtr<float> params;       // tb_policy_floats(env_kind) parameters
+  DevPtr<float> act;          // [N, act_dim] clipped actions handed from policy_kernel to step_kernel
+};
 
 struct tb_ctx {
   tb_config cfg;
   Params params;
-  Scene<float> sc32;
+  Scene<float> sc32;                         // the scene of the context's precision (rebuild)
   Scene<double> sc64;
-  void *state = nullptr;
-  unsigned long long *stats = nullptr;
+  DevPtr<void> state;
+  DevPtr<unsigned long long> stats;
   cudaStream_t own_stream = nullptr;
-  // device staging for the host-buffer entry points
-  float *d_actions = nullptr, *d_obs = nullptr, *d_reward = nullptr, *d_term = nullptr;
-  uint8_t *d_done = nullptr, *d_events = nullptr, *d_mask = nullptr;
+  StagingBufs staging;
   int64_t launches = 0;
-  int *queue = nullptr;                      // fast-forward work queue (env indices), num_envs entries
-  int *queue_full = nullptr, *queue_ctl = nullptr;
-  unsigned long long *dq = nullptr;          // the two dynamic queues of ff_kernel, dq_cap tagged slots each
+  DevPtr<int> queue;                         // fast-forward work queue (env indices), num_envs entries
+  DevPtr<int> queue_full, queue_ctl;
+  DevPtr<unsigned long long> dq;             // the two dynamic queues of ff_kernel, dq_cap tagged slots each
   long long dq_cap = 0;
-  unsigned *epoch = nullptr;                 // device word, see StepIO
-  unsigned long long *fault = nullptr;       // device word, see StepIO
-  unsigned long long *h_fault = nullptr;     // the same word in mapped host memory (checked on entry of every call, no sync)
+  DevPtr<unsigned> epoch;                    // device word, see StepIO
+  DevPtr<unsigned long long> fault;          // device word, see StepIO
+  std::unique_ptr<unsigned long long, CudaFreeHost> h_fault;  // the same word in mapped host memory (checked on entry of
+                                                              // every call, no sync)
   unsigned long long *h_fault_dev = nullptr; // its device alias
   long long spin_limit = 0;                  // clock cycles, see StepIO (TB_FF_SPIN_LIMIT_MS, default 4000 ms)
-  unsigned long long *queue_ctrs = nullptr;  // two counter sets (kCtrWords each) used by alternate steps
+  DevPtr<unsigned long long> queue_ctrs;     // two counter sets (kCtrWords each) used by alternate steps
   unsigned ff_grid = 0;                      // persistent grid of ff_kernel
   int ff_server_sm_stride = 0;               // see StepIO (set with the grid size, 0 = per-CTA roles)
   int step_resident = -1;                    // resident CTAs of step_kernel (its L2 prefetch distance)
   bool one_wave4 = false;                    // Tennisbot-v0: launch the 4-CTAs-per-SM build of step_kernel (see its MINB)
   int control_mode = TB_CONTROL_FORCE;
-  void *pid = nullptr;                       // controller memory, allocated by tb_set_control_mode(TB_CONTROL_PID)
-  float *policy = nullptr;                   // tb_policy_floats(env_kind) parameters (tb_set_policy)
-  float *pol_act = nullptr;                  // [N, act_dim] clipped actions handed from policy_kernel to step_kernel
-  // ES fitness rollout (tb_es_begin / tb_es_rollout), allocated by the first tb_es_begin; see EsIO
+  DevPtr<void> pid;                          // controller memory, allocated by tb_set_control_mode(TB_CONTROL_PID)
+  PolicyBufs policy;
+  // ES fitness rollout (tb_es_begin / tb_es_rollout); see EsIO
   int64_t es_individuals = 0;                // 0: no tb_es_begin yet
-  float *es_w = nullptr;                     // [floats][individuals]
+  DevPtr<float> es_w;                        // [floats][individuals], stream-ordered allocation
   int64_t es_w_cap = 0;                      // floats es_w holds
-  double *es_norm = nullptr, *es_n0 = nullptr, *es_ret = nullptr;
-  float *es_hist = nullptr, *es_obs = nullptr, *es_term = nullptr, *es_rew = nullptr, *es_act = nullptr;
-  uint8_t *es_alive = nullptr, *es_done = nullptr;
-  unsigned *es_base = nullptr;
-  unsigned *es_stop = nullptr;               // [N] see EsIO::stop
-  double *es_master = nullptr;               // [3, obs_dim] the generation's master normaliser (zeros for NULL)
-  double *es_part = nullptr;                 // es_norm_partial_kernel's per-CTA moments
-  bool timing = false;                      // tb_set_kernel_timing
+  EsBufs es;
+  bool timing = false;                       // tb_set_kernel_timing
   cudaEvent_t ev[3] = {nullptr, nullptr, nullptr};
   double ms_step = 0, ms_ff = 0;
   int64_t timed_steps = 0;
+
+  // runs with the context's device current; the owners free the buffers after it, once the own stream has drained
+  ~tb_ctx() {
+    if (own_stream) { cudaStreamSynchronize(own_stream); cudaStreamDestroy(own_stream); }
+    for (cudaEvent_t e : ev)
+      if (e) cudaEventDestroy(e);
+  }
 };
 
 struct DeviceGuard {
@@ -2288,74 +2321,99 @@ struct DeviceGuard {
   ~DeviceGuard() { if (prev >= 0) cudaSetDevice(prev); }
 };
 #define GUARD(ctx)                                               \
-  if (!(ctx)) return fail("%s", "context is NULL");              \
+  if (!(ctx)) return fail("context is NULL");                    \
   DeviceGuard guard_((ctx)->cfg.device);                         \
-  if (!guard_.ok) return fail("%s", "cudaSetDevice failed")
+  if (!guard_.ok) return fail("cudaSetDevice failed")
+
+template <int KIND> using Kind = std::integral_constant<int, KIND>;
+// f(Kind<env_kind>()), or -1 for an unknown kind
+template <typename F> static int with_kind(int env_kind, F &&f) {
+  return env_kind == TB_ENV_SWING ? f(Kind<TB_ENV_SWING>()) : env_kind == TB_ENV_HIT ? f(Kind<TB_ENV_HIT>()) : -1;
+}
+// The one place a context's precision and env kind become the compile-time T and KIND of its kernels:
+// f(Scene<T> &scene, T *state, Kind<KIND>()).
+template <typename F> static int with_env(tb_ctx *c, F &&f) {
+  if (c->cfg.precision == TB_F64)
+    return with_kind(c->cfg.env_kind, [&](auto kind) { return f(c->sc64, static_cast<double *>(c->state.get()), kind); });
+  return with_kind(c->cfg.env_kind, [&](auto kind) { return f(c->sc32, static_cast<float *>(c->state.get()), kind); });
+}
+// bytes of one state scalar
+static size_t state_word(tb_ctx *c) { return with_env(c, [](auto &, auto *state, auto) { return (int)sizeof *state; }); }
+
+// Every kernel launch of the library: plain, or with programmatic stream serialisation (pdl), counted and checked.
+constexpr bool kPlain = false, kPdl = true;
+template <typename... KArgs, typename... Args>
+static int launch(tb_ctx *c, bool pdl, void (*kernel)(KArgs...), dim3 grid, dim3 block, cudaStream_t stream, Args &&...args) {
+  if (pdl) {
+    cudaLaunchConfig_t cfg{};
+    cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = 0; cfg.stream = stream;
+    cudaLaunchAttribute at[1];
+    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    at[0].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = at; cfg.numAttrs = 1;
+    CU(cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...));
+  } else {
+    kernel<<<grid, block, 0, stream>>>(std::forward<Args>(args)...);
+  }
+  c->launches++;
+  CU(cudaGetLastError());
+  return 0;
+}
 
 // A fast-forward launch of this context gave up on a wait (ff_give_up): its batch state is incomplete.  Sticky; every
 // later call fails loudly instead of handing stale observations on.
+static unsigned long long fault_word(const tb_ctx *c) { return *reinterpret_cast<volatile unsigned long long *>(c->h_fault.get()); }
 static int check_fault(tb_ctx *c, const char *who) {
-  const unsigned long long f = c->h_fault ? *reinterpret_cast<volatile unsigned long long *>(c->h_fault) : 0ULL;
+  const unsigned long long f = fault_word(c);
   if (!f) return 0;
-  std::snprintf(g_err, sizeof g_err, "%s: an earlier fast-forward launch of this context timed out waiting on its work queues (code %llu); "
-                "the batch state is incomplete - destroy the context", who, f);
-  return 1;
+  return fail("%s: an earlier fast-forward launch of this context timed out waiting on its work queues (code %llu); "
+              "the batch state is incomplete - destroy the context", who, f);
 }
-template <typename T> static bool fill_ball_vz(Scene<T> &sc) {
-  T *d = nullptr;
-  if (cudaMalloc(&d, kBallVzEntries * sizeof(T)) != cudaSuccess) return false;
-  ball_vz_kernel<T><<<1, 1>>>(sc, d);
-  bool ok = cudaMemcpy(sc.ball_vz, d, kBallVzEntries * sizeof(T), cudaMemcpyDeviceToHost) == cudaSuccess;
-  cudaFree(d);
-  return ok;
-}
-// (needs the context's device current: the ball_vz tables are computed there)
-static bool rebuild(tb_ctx *c) {
-  build_scene<float>(c->params, c->sc32);
-  build_scene<double>(c->params, c->sc64);
-  return fill_ball_vz(c->sc32) && fill_ball_vz(c->sc64);
+// The scene of the context's precision and its ball_vz table, which is computed on the context's device (it must be current).
+static int rebuild(tb_ctx *c) {
+  return with_env(c, [c](auto &sc, auto *state, auto) {
+    using T = std::remove_pointer_t<decltype(state)>;
+    build_scene<T>(c->params, sc);
+    DevPtr<T> d;
+    CU(dev_alloc(d, kBallVzEntries * sizeof(T)));
+    if (launch(c, kPlain, ball_vz_kernel<T>, 1, 1, nullptr, sc, d.get())) return 1;
+    CU(cudaMemcpy(sc.ball_vz, d.get(), kBallVzEntries * sizeof(T), cudaMemcpyDeviceToHost));
+    return 0;
+  });
 }
 static unsigned grid_for(int64_t n, int block) { return (unsigned)((n + block - 1) / block); }
 static StepIO make_io(tb_ctx *c) {
   StepIO io;
   std::memset(&io, 0, sizeof io);
-  io.state = c->state; io.n = c->cfg.num_envs; io.id_offset = c->cfg.env_id_offset; io.seed = c->cfg.seed;
-  io.auto_reset = c->cfg.auto_reset; io.stats = c->stats; io.k_steps = 1;
-  io.pid = c->control_mode == TB_CONTROL_PID ? c->pid : nullptr;
+  io.state = c->state.get(); io.n = c->cfg.num_envs; io.id_offset = c->cfg.env_id_offset; io.seed = c->cfg.seed;
+  io.auto_reset = c->cfg.auto_reset; io.stats = c->stats.get(); io.k_steps = 1;
+  io.pid = c->control_mode == TB_CONTROL_PID ? c->pid.get() : nullptr;
   return io;
 }
+// The env-step counter the policy noise and the ES history are keyed by (see StepIO::epoch).
+static const unsigned *step_counter(tb_ctx *c) { return c->cfg.env_kind == TB_ENV_SWING ? c->epoch.get() : c->epoch.get() + 2; }
 
 static int set_control_mode(tb_ctx *c, int mode) {
-  if (mode != TB_CONTROL_FORCE && mode != TB_CONTROL_PID) return fail("%s", "tb_set_control_mode: unknown mode");
+  if (mode != TB_CONTROL_FORCE && mode != TB_CONTROL_PID) return fail("tb_set_control_mode: unknown mode");
   if (mode == TB_CONTROL_PID && !c->pid) {
-    size_t bytes = (size_t)c->cfg.num_envs * 8 * (c->cfg.precision == TB_F64 ? 8 : 4);
-    CU(cudaMalloc(&c->pid, bytes));
-    CU(cudaMemset(c->pid, 0, bytes));
+    const size_t bytes = (size_t)c->cfg.num_envs * 8 * state_word(c);
+    DevPtr<void> pid;
+    CU(dev_alloc(pid, bytes));
+    CU(cudaMemset(pid.get(), 0, bytes));
+    c->pid = std::move(pid);
   }
   c->control_mode = mode;
   return 0;
 }
 
-#define DISPATCH(KERNEL, grid, block, stream, ...)                                                          \
-  do {                                                                                                      \
-    if (c->cfg.precision == TB_F64) {                                                                       \
-      if (c->cfg.env_kind == TB_ENV_SWING) KERNEL<double, TB_ENV_SWING><<<grid, block, 0, stream>>>(c->sc64, __VA_ARGS__); \
-      else KERNEL<double, TB_ENV_HIT><<<grid, block, 0, stream>>>(c->sc64, __VA_ARGS__);                      \
-    } else {                                                                                                \
-      if (c->cfg.env_kind == TB_ENV_SWING) KERNEL<float, TB_ENV_SWING><<<grid, block, 0, stream>>>(c->sc32, __VA_ARGS__); \
-      else KERNEL<float, TB_ENV_HIT><<<grid, block, 0, stream>>>(c->sc32, __VA_ARGS__);                       \
-    }                                                                                                       \
-    c->launches++;                                                                                          \
-  } while (0)
-
 // ff_kernel is persistent: one CTA per resident slot (SMs x CTAs/SM from the occupancy calculator).
-template <typename T> static int ff_grid_size(tb_ctx *c, unsigned *grid) {
+template <typename T> static int ff_grid_size(tb_ctx *c) {
   int per_sm = 0, sms = 0;
   CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ff_kernel<T>, kBlock, 0));
   CU(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, c->cfg.device));
   int64_t resident = (int64_t)sms * (per_sm > 0 ? per_sm : 1);
   int64_t need = (c->cfg.num_envs + kBlock - 1) / kBlock;
-  *grid = (unsigned)(need < resident ? need : resident);
+  c->ff_grid = (unsigned)(need < resident ? need : resident);
   // server SMs every 12th: measured on B200 (1 Mi envs, f64) 2.46 ms per fast-forward launch, stride 8 2.59, 16 2.99,
   // per-CTA roles 2.60
   c->ff_server_sm_stride = need >= resident ? 12 : 0;
@@ -2367,7 +2425,7 @@ template <typename T, int KIND> static int step_resident_ctas(tb_ctx *c) {
   CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, step_kernel<T, KIND, false>, kBlock, 0));
   CU(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, c->cfg.device));
   c->step_resident = sms * (per_sm > 0 ? per_sm : 1);
-  if (KIND == TB_ENV_HIT) {  // see step_kernel's MINB
+  if constexpr (KIND == TB_ENV_HIT) {  // see step_kernel's MINB
     int per_sm4 = 0;
     CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm4, step_kernel<T, TB_ENV_HIT, false, 4>, kBlock, 0));
     const int64_t grid = (c->cfg.num_envs + kBlock - 1) / kBlock;
@@ -2375,103 +2433,68 @@ template <typename T, int KIND> static int step_resident_ctas(tb_ctx *c) {
   }
   return 0;
 }
-template <typename... KArgs, typename... Args>
-static cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, cudaStream_t stream, Args &&...args) {
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = grid; cfg.blockDim = dim3(kBlock); cfg.dynamicSmemBytes = 0; cfg.stream = stream;
-  cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  at[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = at; cfg.numAttrs = 1;
-  return cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
-}
-// One env step = step_kernel (+ ff_kernel for SwingRacket) on `stream`.
 static void fill_io(tb_ctx *c, StepIO &io) {
-  io.queue = c->queue; io.queue_full = c->queue_full; io.queue_ctl = c->queue_ctl;
-  io.fault = c->fault; io.fault_host = c->h_fault_dev; io.spin_limit = c->spin_limit;
+  io.queue = c->queue.get(); io.queue_full = c->queue_full.get(); io.queue_ctl = c->queue_ctl.get();
+  io.fault = c->fault.get(); io.fault_host = c->h_fault_dev; io.spin_limit = c->spin_limit;
   io.server_sm_stride = c->ff_server_sm_stride;
-  io.dq_full = c->dq; io.dq_late = c->dq ? c->dq + c->dq_cap : nullptr; io.dq_cap = c->dq_cap;
-  io.epoch = c->epoch;  // (a slot written 2^32 steps ago with the same tag would have to survive untouched)
-  io.queue_ctrs = c->queue_ctrs;
-}
-// step_kernel for the whole batch on `stream`
-static int launch_step_kernel(tb_ctx *c, StepIO &io, cudaStream_t stream, bool stage) {
-  const unsigned grid = grid_for(io.n, kBlock);
-  const bool swing = c->cfg.env_kind == TB_ENV_SWING;
-#define TB_LAUNCH_STEP(T, K, SC)                                                                           \
-  do {                                                                                                    \
-    if (stage) {                                                                                          \
-      CU(launch_pdl(step_kernel<T, K, true>, grid, stream, SC, io));                                      \
-    } else {                                                                                              \
-      if (c->step_resident < 0 && step_resident_ctas<T, K>(c)) return 1;                                  \
-      io.prefetch_ahead = c->step_resident;                                                               \
-      if (K == TB_ENV_HIT && c->one_wave4) {                                                              \
-        io.prefetch_ahead = 0;                                                                            \
-        CU(launch_pdl(step_kernel<T, TB_ENV_HIT, false, 4>, grid, stream, SC, io));                       \
-      } else {                                                                                            \
-        CU(launch_pdl(step_kernel<T, K, false>, grid, stream, SC, io));                                   \
-      }                                                                                                   \
-    }                                                                                                     \
-  } while (0)
-  if (c->cfg.precision == TB_F64) {
-    if (swing) TB_LAUNCH_STEP(double, TB_ENV_SWING, c->sc64);
-    else TB_LAUNCH_STEP(double, TB_ENV_HIT, c->sc64);
-  } else {
-    if (swing) TB_LAUNCH_STEP(float, TB_ENV_SWING, c->sc32);
-    else TB_LAUNCH_STEP(float, TB_ENV_HIT, c->sc32);
-  }
-#undef TB_LAUNCH_STEP
-  c->launches++;
-  CU(cudaGetLastError());
-  return 0;
-}
-// ff_kernel (SwingRacket-v0) for the whole batch on `stream`
-static int launch_ff_kernel(tb_ctx *c, StepIO &io, cudaStream_t stream) {
-  if (c->cfg.env_kind != TB_ENV_SWING) return 0;
-  if (c->cfg.precision == TB_F64) {
-    if (!c->ff_grid && ff_grid_size<double>(c, &c->ff_grid)) return 1;
-    io.server_sm_stride = c->ff_server_sm_stride;
-    CU(launch_pdl(ff_kernel<double>, c->ff_grid, stream, c->sc64, io));
-  } else {
-    if (!c->ff_grid && ff_grid_size<float>(c, &c->ff_grid)) return 1;
-    io.server_sm_stride = c->ff_server_sm_stride;
-    CU(launch_pdl(ff_kernel<float>, c->ff_grid, stream, c->sc32, io));
-  }
-  c->launches++;
-  CU(cudaGetLastError());
-  return 0;
+  io.dq_full = c->dq.get(); io.dq_late = c->dq ? c->dq.get() + c->dq_cap : nullptr; io.dq_cap = c->dq_cap;
+  io.epoch = c->epoch.get();  // (a slot written 2^32 steps ago with the same tag would have to survive untouched)
+  io.queue_ctrs = c->queue_ctrs.get();
 }
 // One env step = step_kernel (+ ff_kernel for SwingRacket) on `stream`.
 static int launch_step(tb_ctx *c, StepIO &io, cudaStream_t stream, bool stage = false) {
   fill_io(c, io);
-  if (c->timing) CU(cudaEventRecord(c->ev[0], stream));
-  if (launch_step_kernel(c, io, stream, stage)) return 1;
-  if (c->timing) CU(cudaEventRecord(c->ev[1], stream));
-  if (launch_ff_kernel(c, io, stream)) return 1;
-  if (c->timing) {
-    float a = 0, b = 0;
-    CU(cudaEventRecord(c->ev[2], stream));
-    CU(cudaEventSynchronize(c->ev[2]));
-    CU(cudaEventElapsedTime(&a, c->ev[0], c->ev[1]));
-    CU(cudaEventElapsedTime(&b, c->ev[1], c->ev[2]));
-    c->ms_step += a; c->ms_ff += b; c->timed_steps++;
-  }
-  return 0;
+  return with_env(c, [&](auto &sc, auto *state, auto kind) {
+    using T = std::remove_pointer_t<decltype(state)>;
+    const unsigned grid = grid_for(io.n, kBlock);
+    if (c->timing) CU(cudaEventRecord(c->ev[0], stream));
+    auto kernel = step_kernel<T, kind, true>;
+    if (!stage) {
+      if (c->step_resident < 0 && step_resident_ctas<T, kind>(c)) return 1;
+      io.prefetch_ahead = c->step_resident;
+      kernel = step_kernel<T, kind, false>;
+      if constexpr (kind == TB_ENV_HIT) {
+        if (c->one_wave4) { io.prefetch_ahead = 0; kernel = step_kernel<T, TB_ENV_HIT, false, 4>; }
+      }
+    }
+    if (launch(c, kPdl, kernel, grid, kBlock, stream, sc, io)) return 1;
+    if (c->timing) CU(cudaEventRecord(c->ev[1], stream));
+    if constexpr (kind == TB_ENV_SWING) {
+      if (!c->ff_grid && ff_grid_size<T>(c)) return 1;
+      io.server_sm_stride = c->ff_server_sm_stride;
+      if (launch(c, kPdl, ff_kernel<T>, c->ff_grid, kBlock, stream, sc, io)) return 1;
+    }
+    if (c->timing) {
+      float a = 0, b = 0;
+      CU(cudaEventRecord(c->ev[2], stream));
+      CU(cudaEventSynchronize(c->ev[2]));
+      CU(cudaEventElapsedTime(&a, c->ev[0], c->ev[1]));
+      CU(cudaEventElapsedTime(&b, c->ev[1], c->ev[2]));
+      c->ms_step += a; c->ms_ff += b; c->timed_steps++;
+    }
+    return 0;
+  });
+}
+static int launch_reset(tb_ctx *c, const StepIO &io, const double *d_init, const uint8_t *d_mask, cudaStream_t stream) {
+  return with_env(c, [&](auto &sc, auto *state, auto kind) {
+    using T = std::remove_pointer_t<decltype(state)>;
+    return launch(c, kPlain, reset_kernel<T, kind>, grid_for(io.n, kBlock), kBlock, stream, sc, io, d_init, d_mask);
+  });
 }
 
 extern "C" {
 
 const char *tb_last_error(void) { return g_err; }
 int tb_abi_version(void) { return TB_ABI_VERSION; }
-int tb_obs_dim(int kind) { return kind == TB_ENV_SWING ? 6 : kind == TB_ENV_HIT ? 12 : -1; }
-int tb_act_dim(int kind) { return kind == TB_ENV_SWING ? 6 : kind == TB_ENV_HIT ? 2 : -1; }
-int tb_policy_floats(int kind) { return kind == TB_ENV_SWING ? TB_POLICY_FLOATS : kind == TB_ENV_HIT ? TB_POLICY_FLOATS_HIT : -1; }
-int tb_es_floats(int kind) { return kind == TB_ENV_SWING ? TB_ES_FLOATS : kind == TB_ENV_HIT ? TB_ES_FLOATS_HIT : -1; }
+int tb_obs_dim(int kind) { return with_kind(kind, [](auto k) { return Dims<k>::obs; }); }
+int tb_act_dim(int kind) { return with_kind(kind, [](auto k) { return Dims<k>::act; }); }
+int tb_policy_floats(int kind) { return with_kind(kind, [](auto k) { return PolLayout<Dims<k>::obs, Dims<k>::act>::Floats; }); }
+int tb_es_floats(int kind) { return with_kind(kind, [](auto k) { return EsLayout<Dims<k>::obs, Dims<k>::act>::Floats; }); }
 int tb_num_params(void) { return kNumParams; }
 const char *tb_param_name(int i) { return (i >= 0 && i < kNumParams) ? k_param_names[i] : nullptr; }
 
 int tb_scene_constant(const char *name, int index, double *value) {
-  if (!name || !value) return fail("%s", "tb_scene_constant: bad argument");
+  if (!name || !value) return fail("tb_scene_constant: bad argument");
   Params p;
   params_default(p);
   HostScene h;
@@ -2514,108 +2537,91 @@ int tb_scene_constant(const char *name, int index, double *value) {
 }
 
 int tb_create(const tb_config *cfg, tb_ctx **out) {
-  if (!cfg || !out) return fail("%s", "tb_create: bad argument");
-  if (cfg->struct_size != sizeof(tb_config)) return fail("%s", "tb_create: tb_config.struct_size mismatch");
-  if (cfg->env_kind != TB_ENV_SWING && cfg->env_kind != TB_ENV_HIT) return fail("%s", "tb_create: unknown env_kind");
-  if (cfg->precision != TB_F32 && cfg->precision != TB_F64) return fail("%s", "tb_create: unknown precision");
-  if (cfg->num_envs <= 0 || cfg->num_envs > 0x7fffffffLL) return fail("%s", "tb_create: num_envs must be in [1, 2^31)");
+  if (!cfg || !out) return fail("tb_create: bad argument");
+  if (cfg->struct_size != sizeof(tb_config)) return fail("tb_create: tb_config.struct_size mismatch");
+  if (cfg->env_kind != TB_ENV_SWING && cfg->env_kind != TB_ENV_HIT) return fail("tb_create: unknown env_kind");
+  if (cfg->precision != TB_F32 && cfg->precision != TB_F64) return fail("tb_create: unknown precision");
+  if (cfg->num_envs <= 0 || cfg->num_envs > 0x7fffffffLL) return fail("tb_create: num_envs must be in [1, 2^31)");
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
-    return fail("%s", "tb_create: no CUDA device (this library has no CPU fallback)");
-  if (cfg->device < 0 || cfg->device >= ndev) return fail("%s", "tb_create: device ordinal out of range");
+    return fail("tb_create: no CUDA device (this library has no CPU fallback)");
+  if (cfg->device < 0 || cfg->device >= ndev) return fail("tb_create: device ordinal out of range");
   cudaDeviceProp prop;
   CU(cudaGetDeviceProperties(&prop, cfg->device));
-  if (prop.major != 10) return fail("%s", "tb_create: device is not sm_100 (library is built for sm_100a only)");
-  tb_ctx *c = new (std::nothrow) tb_ctx();
-  if (!c) return fail("%s", "tb_create: out of memory");
+  if (prop.major != 10) return fail("tb_create: device is not sm_100 (library is built for sm_100a only)");
+  DeviceGuard g(cfg->device);  // (declared first: the context's buffers are freed with its device current)
+  if (!g.ok) return fail("tb_create: cudaSetDevice failed");
+  std::unique_ptr<tb_ctx> c(new (std::nothrow) tb_ctx());
+  if (!c) return fail("tb_create: out of memory");
   c->cfg = *cfg;
   params_default(c->params);
-  DeviceGuard g(cfg->device);
-  if (!g.ok) { delete c; return fail("%s", "tb_create: cudaSetDevice failed"); }
-  if (!rebuild(c)) { delete c; return fail("%s", "tb_create: could not build the scene tables on the device"); }
-  size_t word = cfg->precision == TB_F64 ? 8 : 4;
-  size_t bytes = (size_t)cfg->num_envs * kPacks * 4 * word;
-  cudaError_t e = cudaMalloc(&c->state, bytes);
-  if (e == cudaSuccess) e = cudaMalloc(&c->stats, TB_NUM_STATS * sizeof(unsigned long long));
-  if (e == cudaSuccess) e = cudaMalloc(&c->queue_ctrs, 2 * kCtrWords * sizeof(unsigned long long));
-  if (e == cudaSuccess && cfg->env_kind == TB_ENV_SWING) e = cudaMalloc(&c->queue, (size_t)cfg->num_envs * sizeof(int));
-  if (e == cudaSuccess && cfg->env_kind == TB_ENV_SWING) {
-    // every env is pushed to either dynamic queue at most kFfMaxVisits times per launch
-    {
-      // + a ticket for every lane that may end up waiting: ff_kernel's grid is at most ceil(n / 128) CTAs and never more
-      // than fit the device (<= 2048 CTAs of 128 threads on any sm_100 part)
-      long long ctas = (cfg->num_envs + kBlock - 1) / kBlock;
-      c->dq_cap = (long long)cfg->num_envs * (kFfMaxVisits + 1) + (ctas < 2048 ? ctas : 2048) * kBlock;
-    }
-    e = cudaMalloc(&c->dq, (size_t)c->dq_cap * 2 * sizeof(unsigned long long));
+  if (rebuild(c.get())) return fail("tb_create: could not build the scene tables on the device");
+  const int64_t n = cfg->num_envs;
+  const size_t bytes = (size_t)n * kPacks * 4 * state_word(c.get());
+  CU(dev_alloc(c->state, bytes));
+  CU(dev_alloc(c->stats, TB_NUM_STATS * sizeof(unsigned long long)));
+  CU(dev_alloc(c->queue_ctrs, 2 * kCtrWords * sizeof(unsigned long long)));
+  if (cfg->env_kind == TB_ENV_SWING) {
+    // every env is pushed to either dynamic queue at most kFfMaxVisits times per launch, + a ticket for every lane that may
+    // end up waiting: ff_kernel's grid is at most ceil(n / 128) CTAs and never more than fit the device (<= 2048 CTAs of 128
+    // threads on any sm_100 part)
+    const long long ctas = (n + kBlock - 1) / kBlock;
+    c->dq_cap = (long long)n * (kFfMaxVisits + 1) + (ctas < 2048 ? ctas : 2048) * kBlock;
+    CU(dev_alloc(c->queue, (size_t)n * sizeof(int)));
+    CU(dev_alloc(c->dq, (size_t)c->dq_cap * 2 * sizeof(unsigned long long)));
+    CU(dev_alloc(c->queue_full, (size_t)n * sizeof(int)));
+    CU(dev_alloc(c->queue_ctl, (size_t)n * sizeof(int)));
   }
-  if (e == cudaSuccess && cfg->env_kind == TB_ENV_SWING) e = cudaMalloc(&c->queue_full, (size_t)cfg->num_envs * sizeof(int));
-  if (e == cudaSuccess && cfg->env_kind == TB_ENV_SWING) e = cudaMalloc(&c->queue_ctl, (size_t)cfg->num_envs * sizeof(int));
-  if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&c->own_stream, cudaStreamNonBlocking);
-  if (e == cudaSuccess) e = cudaMemsetAsync(c->state, 0, bytes, c->own_stream);
-  if (e == cudaSuccess) e = cudaMemsetAsync(c->stats, 0, TB_NUM_STATS * sizeof(unsigned long long), c->own_stream);
-  if (e == cudaSuccess) e = cudaMemsetAsync(c->queue_ctrs, 0, 2 * kCtrWords * sizeof(unsigned long long), c->own_stream);
-  if (e == cudaSuccess) e = cudaMalloc(&c->fault, sizeof(unsigned long long));
-  if (e == cudaSuccess) e = cudaMemsetAsync(c->fault, 0, sizeof(unsigned long long), c->own_stream);
-  if (e == cudaSuccess) e = cudaHostAlloc((void **)&c->h_fault, sizeof(unsigned long long), cudaHostAllocMapped);
-  if (e == cudaSuccess) { *c->h_fault = 0; e = cudaHostGetDevicePointer((void **)&c->h_fault_dev, c->h_fault, 0); }
+  CU(cudaStreamCreateWithFlags(&c->own_stream, cudaStreamNonBlocking));
+  const cudaStream_t s = c->own_stream;
+  CU(cudaMemsetAsync(c->state.get(), 0, bytes, s));
+  CU(cudaMemsetAsync(c->stats.get(), 0, TB_NUM_STATS * sizeof(unsigned long long), s));
+  CU(cudaMemsetAsync(c->queue_ctrs.get(), 0, 2 * kCtrWords * sizeof(unsigned long long), s));
+  CU(dev_alloc(c->fault, sizeof(unsigned long long)));
+  CU(cudaMemsetAsync(c->fault.get(), 0, sizeof(unsigned long long), s));
+  {
+    void *h = nullptr;
+    CU(cudaHostAlloc(&h, sizeof(unsigned long long), cudaHostAllocMapped));
+    c->h_fault.reset(static_cast<unsigned long long *>(h));
+  }
+  *c->h_fault = 0;
+  CU(cudaHostGetDevicePointer((void **)&c->h_fault_dev, c->h_fault.get(), 0));
   {
     const char *ms = std::getenv("TB_FF_SPIN_LIMIT_MS");
     double limit_ms = ms ? std::atof(ms) : 4000.0;
     if (!(limit_ms > 0)) limit_ms = 4000.0;
     c->spin_limit = (long long)(limit_ms * 1e-3 * (double)prop.clockRate * 1e3);  // clockRate is in kHz
   }
-  if (e == cudaSuccess) e = cudaMalloc(&c->epoch, 3 * sizeof(unsigned));
-  if (e == cudaSuccess) e = cudaMemsetAsync(c->epoch, 0, 3 * sizeof(unsigned), c->own_stream);
-  if (e == cudaSuccess && c->dq) e = cudaMemsetAsync(c->dq, 0, (size_t)c->dq_cap * 2 * sizeof(unsigned long long), c->own_stream);  // tag 0 = no epoch
-  if (e == cudaSuccess) {
-    // identity quaternion, episode = -1 so the first reset starts episode 0
-    std::size_t n = (size_t)cfg->num_envs;
-    double *tmp = (double *)std::calloc(n * TB_STATE_WORDS, sizeof(double));
-    double *dtmp = nullptr;
-    if (!tmp) e = cudaErrorMemoryAllocation;
-    if (e == cudaSuccess) {
-      for (size_t i = 0; i < n; ++i) { tmp[i * TB_STATE_WORDS + TB_S_RACKET_QUAT + 3] = 1.0; tmp[i * TB_STATE_WORDS + TB_S_EPISODE] = -1.0; }
-      e = cudaMalloc(&dtmp, n * TB_STATE_WORDS * sizeof(double));
-    }
-    if (e == cudaSuccess) e = cudaMemcpyAsync(dtmp, tmp, n * TB_STATE_WORDS * sizeof(double), cudaMemcpyHostToDevice, c->own_stream);
-    if (e == cudaSuccess) {
-      if (cfg->precision == TB_F64) set_state_kernel<double><<<grid_for(cfg->num_envs, 256), 256, 0, c->own_stream>>>((double *)c->state, cfg->num_envs, dtmp);
-      else set_state_kernel<float><<<grid_for(cfg->num_envs, 256), 256, 0, c->own_stream>>>((float *)c->state, cfg->num_envs, dtmp);
-      e = cudaGetLastError();
-      c->launches++;
-    }
-    if (e == cudaSuccess) e = cudaStreamSynchronize(c->own_stream);
-    if (dtmp) cudaFree(dtmp);
-    std::free(tmp);
-  }
-  if (e != cudaSuccess) {
-    std::snprintf(g_err, sizeof g_err, "tb_create: %s", cudaGetErrorString(e));
-    tb_destroy(c);
+  CU(dev_alloc(c->epoch, 3 * sizeof(unsigned)));
+  CU(cudaMemsetAsync(c->epoch.get(), 0, 3 * sizeof(unsigned), s));
+  if (c->dq) CU(cudaMemsetAsync(c->dq.get(), 0, (size_t)c->dq_cap * 2 * sizeof(unsigned long long), s));  // tag 0 = no epoch
+  // identity quaternion, episode = -1 so the first reset starts episode 0
+  const size_t words = (size_t)n * TB_STATE_WORDS;
+  std::unique_ptr<double[]> init(new (std::nothrow) double[words]());
+  if (!init) return fail("tb_create: out of memory");
+  for (size_t i = 0; i < (size_t)n; ++i) { init[i * TB_STATE_WORDS + TB_S_RACKET_QUAT + 3] = 1.0; init[i * TB_STATE_WORDS + TB_S_EPISODE] = -1.0; }
+  DevPtr<double> d_init;
+  CU(dev_alloc(d_init, words * sizeof(double)));
+  CU(cudaMemcpyAsync(d_init.get(), init.get(), words * sizeof(double), cudaMemcpyHostToDevice, s));
+  if (with_env(c.get(), [&](auto &, auto *state, auto) {
+        using T = std::remove_pointer_t<decltype(state)>;
+        return launch(c.get(), kPlain, set_state_kernel<T>, grid_for(n, 256), 256, s, state, n, d_init.get());
+      }))
     return 1;
-  }
-  *out = c;
+  CU(cudaStreamSynchronize(s));
+  *out = c.release();
   return 0;
 }
 
 int tb_destroy(tb_ctx *c) {
   if (!c) return 0;
   DeviceGuard g(c->cfg.device);
-  if (c->own_stream) { cudaStreamSynchronize(c->own_stream); cudaStreamDestroy(c->own_stream); }
-  for (int i = 0; i < 3; ++i) if (c->ev[i]) cudaEventDestroy(c->ev[i]);
-  cudaFree(c->state); cudaFree(c->stats); cudaFree(c->queue_ctrs); cudaFree(c->queue); cudaFree(c->dq); cudaFree(c->epoch); cudaFree(c->fault); cudaFree(c->queue_full); cudaFree(c->queue_ctl); cudaFree(c->pid); cudaFree(c->policy); cudaFree(c->pol_act);
-  cudaFree(c->es_w); cudaFree(c->es_norm); cudaFree(c->es_n0); cudaFree(c->es_ret); cudaFree(c->es_hist); cudaFree(c->es_obs);
-  cudaFree(c->es_term); cudaFree(c->es_rew); cudaFree(c->es_act); cudaFree(c->es_alive); cudaFree(c->es_done); cudaFree(c->es_base);
-  cudaFree(c->es_stop); cudaFree(c->es_master); cudaFree(c->es_part);
-  if (c->h_fault) cudaFreeHost(c->h_fault);
-  cudaFree(c->d_actions); cudaFree(c->d_obs); cudaFree(c->d_reward); cudaFree(c->d_term);
-  cudaFree(c->d_done); cudaFree(c->d_events); cudaFree(c->d_mask);
   delete c;
   return 0;
 }
 
 int tb_set_param(tb_ctx *c, const char *name, double value) {
-  if (!name) return fail("%s", "tb_set_param: bad argument");
+  if (!name) return fail("tb_set_param: bad argument");
   GUARD(c);
   double *slots = reinterpret_cast<double *>(&c->params);
   for (int i = 0; i < kNumParams; ++i)
@@ -2624,11 +2630,14 @@ int tb_set_param(tb_ctx *c, const char *name, double value) {
       // first; a configuration call, so it simply waits for everything the device has in flight
       CU(cudaDeviceSynchronize());
       const int64_t n = c->cfg.num_envs;
-      if (c->cfg.precision == TB_F64) materialise_kernel<double><<<grid_for(n, 256), 256, 0, c->own_stream>>>(c->sc64, (double *)c->state, n);
-      else materialise_kernel<float><<<grid_for(n, 256), 256, 0, c->own_stream>>>(c->sc32, (float *)c->state, n);
+      if (with_env(c, [&](auto &sc, auto *state, auto) {
+            using T = std::remove_pointer_t<decltype(state)>;
+            return launch(c, kPlain, materialise_kernel<T>, grid_for(n, 256), 256, c->own_stream, sc, state, n);
+          }))
+        return 1;
       CU(cudaStreamSynchronize(c->own_stream));
       slots[i] = value;
-      if (!rebuild(c)) return fail("%s", "tb_set_param: could not rebuild the scene tables on the device");
+      if (rebuild(c)) return fail("tb_set_param: could not rebuild the scene tables on the device");
       return 0;
     }
   return fail("tb_set_param: unknown parameter '%s'", name);
@@ -2638,7 +2647,7 @@ int tb_set_control_mode(tb_ctx *c, int mode) {
   return set_control_mode(c, mode);
 }
 int tb_get_param(tb_ctx *c, const char *name, double *value) {
-  if (!c || !name || !value) return fail("%s", "tb_get_param: bad argument");
+  if (!c || !name || !value) return fail("tb_get_param: bad argument");
   const double *slots = reinterpret_cast<const double *>(&c->params);
   for (int i = 0; i < kNumParams; ++i)
     if (!std::strcmp(name, k_param_names[i])) { *value = slots[i]; return 0; }
@@ -2650,20 +2659,18 @@ static int reset_impl(tb_ctx *c, const double *d_init, const uint8_t *d_mask, fl
   if (check_fault(c, "tb_reset")) return 1;
   StepIO io = make_io(c);
   io.obs = d_obs;
-  DISPATCH(reset_kernel, grid_for(io.n, kBlock), kBlock, (cudaStream_t)stream, io, d_init, d_mask);
-  CU(cudaGetLastError());
-  return 0;
+  return launch_reset(c, io, d_init, d_mask, (cudaStream_t)stream);
 }
 int tb_reset(tb_ctx *c, const uint8_t *d_mask, float *d_obs, void *stream) { return reset_impl(c, nullptr, d_mask, d_obs, stream); }
 int tb_reset_from(tb_ctx *c, const double *d_init, const uint8_t *d_mask, float *d_obs, void *stream) {
-  if (!d_init) return fail("%s", "tb_reset_from: d_init is NULL");
+  if (!d_init) return fail("tb_reset_from: d_init is NULL");
   return reset_impl(c, d_init, d_mask, d_obs, stream);
 }
 
 static int step_impl(tb_ctx *c, const float *d_actions, float *d_obs, float *d_reward, uint8_t *d_done,
                      float *d_terminal_obs, uint8_t *d_events, void *stream, bool stage) {
   GUARD(c);
-  if (!d_actions || !d_obs || !d_reward || !d_done) return fail("%s", "tb_step: actions, obs, reward and done are required");
+  if (!d_actions || !d_obs || !d_reward || !d_done) return fail("tb_step: actions, obs, reward and done are required");
   if (check_fault(c, "tb_step")) return 1;
   StepIO io = make_io(c);
   io.actions = d_actions; io.obs = d_obs; io.reward = d_reward; io.done = d_done; io.term_obs = d_terminal_obs;
@@ -2678,78 +2685,79 @@ int tb_step(tb_ctx *c, const float *d_actions, float *d_obs, float *d_reward, ui
 int tb_rollout(tb_ctx *c, int action_mode, int k_steps, float *d_obs, float *d_reward_sum, int32_t *d_done_count, void *stream) {
   GUARD(c);
   if (action_mode != TB_ACT_RANDOM && !(action_mode == TB_ACT_TRACK && c->cfg.env_kind == TB_ENV_HIT))
-    return fail("%s", "tb_rollout: unknown action mode (TB_ACT_TRACK is Tennisbot-v0's)");
-  if (c->control_mode != TB_CONTROL_FORCE) return fail("%s", "tb_rollout: in-kernel random actions need TB_CONTROL_FORCE");
-  if (k_steps < 0) return fail("%s", "tb_rollout: k_steps must be >= 0");
+    return fail("tb_rollout: unknown action mode (TB_ACT_TRACK is Tennisbot-v0's)");
+  if (c->control_mode != TB_CONTROL_FORCE) return fail("tb_rollout: in-kernel random actions need TB_CONTROL_FORCE");
+  if (k_steps < 0) return fail("tb_rollout: k_steps must be >= 0");
   StepIO io = make_io(c);
   io.k_steps = k_steps; io.action_mode = action_mode; io.obs = d_obs; io.reward_sum = d_reward_sum; io.done_count = d_done_count;
-  DISPATCH(rollout_kernel, grid_for(io.n, kBlock), kBlock, (cudaStream_t)stream, io);
-  CU(cudaGetLastError());
-  return 0;
+  return with_env(c, [&](auto &sc, auto *state, auto kind) {
+    using T = std::remove_pointer_t<decltype(state)>;
+    return launch(c, kPlain, rollout_kernel<T, kind>, grid_for(io.n, kBlock), kBlock, (cudaStream_t)stream, sc, io);
+  });
 }
 
 int tb_set_policy(tb_ctx *c, const float *d_params, int64_t count, void *stream) {
   GUARD(c);
   const int64_t want = tb_policy_floats(c->cfg.env_kind);
-  if (!d_params || count != want) {
-    std::snprintf(g_err, sizeof g_err, "tb_set_policy: expected tb_policy_floats(env_kind) = %lld floats in device memory, got %lld",
-                  (long long)want, (long long)count);
-    return 1;
+  if (!d_params || count != want)
+    return fail("tb_set_policy: expected tb_policy_floats(env_kind) = %lld floats in device memory, got %lld", (long long)want,
+                (long long)count);
+  if (!c->policy.params) {
+    PolicyBufs p;
+    CU(dev_alloc(p.params, (size_t)want * sizeof(float)));
+    CU(dev_alloc(p.act, (size_t)c->cfg.num_envs * tb_act_dim(c->cfg.env_kind) * sizeof(float)));
+    c->policy = std::move(p);
   }
-  if (!c->policy) CU(cudaMalloc(&c->policy, (size_t)want * sizeof(float)));
-  if (!c->pol_act) CU(cudaMalloc(&c->pol_act, (size_t)c->cfg.num_envs * tb_act_dim(c->cfg.env_kind) * sizeof(float)));
-  CU(cudaMemcpyAsync(c->policy, d_params, (size_t)want * sizeof(float), cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
+  CU(cudaMemcpyAsync(c->policy.params.get(), d_params, (size_t)want * sizeof(float), cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
   return 0;
 }
 
 int tb_policy_rollout(tb_ctx *c, int k_steps, int deterministic, uint64_t noise_seed, float *d_obs, float *d_actions, float *d_logp,
                       float *d_value, float *d_reward, uint8_t *d_done, float *d_last_obs, float *d_last_value, void *stream) {
   GUARD(c);
-  if (!c->policy) return fail("%s", "tb_policy_rollout: no policy (tb_set_policy)");
-  if (c->control_mode != TB_CONTROL_FORCE) return fail("%s", "tb_policy_rollout: the policy's actions are forces (TB_CONTROL_FORCE)");
-  if (k_steps < 1 || !d_obs || !d_reward || !d_done || !d_last_obs) return fail("%s", "tb_policy_rollout: k_steps >= 1, obs, reward, done and last_obs are required");
+  if (!c->policy.params) return fail("tb_policy_rollout: no policy (tb_set_policy)");
+  if (c->control_mode != TB_CONTROL_FORCE) return fail("tb_policy_rollout: the policy's actions are forces (TB_CONTROL_FORCE)");
+  if (k_steps < 1 || !d_obs || !d_reward || !d_done || !d_last_obs) return fail("tb_policy_rollout: k_steps >= 1, obs, reward, done and last_obs are required");
   if (check_fault(c, "tb_policy_rollout")) return 1;
   const int64_t n = c->cfg.num_envs;
-  const bool swing = c->cfg.env_kind == TB_ENV_SWING;
   const int od = tb_obs_dim(c->cfg.env_kind), ad = tb_act_dim(c->cfg.env_kind);
-  void (*kernel)(PolicyIO) = swing ? policy_kernel<6, 6> : policy_kernel<12, 2>;
+  void (*kernel)(PolicyIO) = nullptr;
+  with_kind(c->cfg.env_kind, [&](auto kind) { kernel = policy_kernel<Dims<kind>::obs, Dims<kind>::act>; return 0; });
   cudaStream_t s = (cudaStream_t)stream;
   PolicyIO pio;
   std::memset(&pio, 0, sizeof pio);
-  pio.params = c->policy; pio.n = n; pio.id_offset = c->cfg.env_id_offset; pio.seed = noise_seed; pio.deterministic = deterministic;
-  pio.act_env = c->pol_act; pio.tick = swing ? c->epoch : c->epoch + 2;  // (see StepIO::epoch)
+  pio.params = c->policy.params.get(); pio.n = n; pio.id_offset = c->cfg.env_id_offset; pio.seed = noise_seed; pio.deterministic = deterministic;
+  pio.act_env = c->policy.act.get(); pio.tick = step_counter(c);
   const unsigned grid = grid_for(n, kBlock);
   for (int t = 0; t < k_steps; ++t) {
     pio.obs = d_obs + (size_t)t * n * od;
     pio.act_raw = d_actions ? d_actions + (size_t)t * n * ad : nullptr;
     pio.logp = d_logp ? d_logp + (size_t)t * n : nullptr;
     pio.value = d_value ? d_value + (size_t)t * n : nullptr;
-    CU(launch_pdl(kernel, dim3(grid, 2), s, pio));
-    c->launches++;
+    if (launch(c, kPdl, kernel, dim3(grid, 2), kBlock, s, pio)) return 1;
     StepIO io = make_io(c);
-    io.actions = c->pol_act;
+    io.actions = c->policy.act.get();
     io.obs = t + 1 < k_steps ? d_obs + (size_t)(t + 1) * n * od : d_last_obs;
     io.reward = d_reward + (size_t)t * n; io.done = d_done + (size_t)t * n;
     if (launch_step(c, io, s)) return 1;
   }
   if (d_last_value) {  // bootstrap value of the observation the rollout ends with
     pio.obs = d_last_obs; pio.act_raw = nullptr; pio.act_env = nullptr; pio.logp = nullptr; pio.value = d_last_value;
-    CU(launch_pdl(kernel, dim3(grid, 2), s, pio));
-    c->launches++;
+    if (launch(c, kPdl, kernel, dim3(grid, 2), kBlock, s, pio)) return 1;
   }
-  CU(cudaGetLastError());
   return 0;
 }
 
 static EsIO es_io(tb_ctx *c) {
   EsIO io;
   std::memset(&io, 0, sizeof io);
-  io.w = c->es_w; io.n = c->cfg.num_envs; io.individuals = c->es_individuals;
+  io.w = c->es_w.get(); io.n = c->cfg.num_envs; io.individuals = c->es_individuals;
   io.repeats = c->es_individuals ? (int)(c->cfg.num_envs / c->es_individuals) : 0;
-  io.norm = c->es_norm; io.n0 = c->es_n0; io.hist = c->es_hist; io.ret = c->es_ret; io.alive = c->es_alive; io.stop = c->es_stop;
-  io.tick = c->cfg.env_kind == TB_ENV_SWING ? c->epoch : c->epoch + 2;  // (see StepIO::epoch)
-  io.base = c->es_base;
-  io.obs = c->es_obs; io.term = c->es_term; io.reward = c->es_rew; io.done = c->es_done;
+  io.norm = c->es.norm.get(); io.n0 = c->es.n0.get(); io.hist = c->es.hist.get(); io.ret = c->es.ret.get();
+  io.alive = c->es.alive.get(); io.stop = c->es.stop.get();
+  io.tick = step_counter(c);
+  io.base = c->es.base.get();
+  io.obs = c->es.obs.get(); io.term = c->es.term.get(); io.reward = c->es.rew.get(); io.done = c->es.done.get();
   return io;
 }
 
@@ -2759,45 +2767,38 @@ static int64_t es_norm_blocks(int64_t n) { return (n + kBlock * kEsStatsPer - 1)
 // and room for the population in es_w.
 static int es_prepare(tb_ctx *c, const char *who, int64_t individuals, int64_t floats, cudaStream_t s) {
   const int64_t n = c->cfg.num_envs, want = tb_es_floats(c->cfg.env_kind);
-  if (floats != want) {
-    std::snprintf(g_err, sizeof g_err, "%s: expected tb_es_floats(env_kind) = %lld floats per individual, got %lld", who,
-                  (long long)want, (long long)floats);
-    return 1;
-  }
-  if (n % individuals) {
-    std::snprintf(g_err, sizeof g_err, "%s: individuals (%lld) must divide num_envs (%lld)", who, (long long)individuals, (long long)n);
-    return 1;
-  }
-  if (individuals * floats > 0xffffffffLL) {
-    std::snprintf(g_err, sizeof g_err, "%s: individuals x floats must be below 2^32 (es_kernel indexes the population with 32 bits)", who);
-    return 1;
-  }
-  if (c->control_mode != TB_CONTROL_FORCE) {
-    std::snprintf(g_err, sizeof g_err, "%s: the GatedCNN's actions are forces (TB_CONTROL_FORCE)", who);
-    return 1;
-  }
+  if (floats != want)
+    return fail("%s: expected tb_es_floats(env_kind) = %lld floats per individual, got %lld", who, (long long)want, (long long)floats);
+  if (n % individuals) return fail("%s: individuals (%lld) must divide num_envs (%lld)", who, (long long)individuals, (long long)n);
+  if (individuals * floats > 0xffffffffLL)
+    return fail("%s: individuals x floats must be below 2^32 (es_kernel indexes the population with 32 bits)", who);
+  if (c->control_mode != TB_CONTROL_FORCE) return fail("%s: the GatedCNN's actions are forces (TB_CONTROL_FORCE)", who);
   if (check_fault(c, who)) return 1;
-  const int od = tb_obs_dim(c->cfg.env_kind), ad = tb_act_dim(c->cfg.env_kind);
-  if (!c->es_norm) {  // per-env state, once per context
-    CU(cudaMalloc(&c->es_norm, (size_t)2 * od * n * sizeof(double)));
-    CU(cudaMalloc(&c->es_n0, (size_t)od * sizeof(double)));
-    CU(cudaMalloc(&c->es_ret, (size_t)n * sizeof(double)));
-    CU(cudaMalloc(&c->es_hist, (size_t)TB_ES_HISTORY * od * n * sizeof(float)));
-    CU(cudaMalloc(&c->es_obs, (size_t)od * n * sizeof(float)));
-    CU(cudaMalloc(&c->es_term, (size_t)od * n * sizeof(float)));
-    CU(cudaMalloc(&c->es_rew, (size_t)n * sizeof(float)));
-    CU(cudaMalloc(&c->es_act, (size_t)ad * n * sizeof(float)));
-    CU(cudaMalloc(&c->es_alive, (size_t)n));
-    CU(cudaMalloc(&c->es_done, (size_t)n));
-    CU(cudaMalloc(&c->es_base, sizeof(unsigned)));
-    CU(cudaMalloc(&c->es_stop, (size_t)n * sizeof(unsigned)));
-    CU(cudaMalloc(&c->es_master, (size_t)3 * od * sizeof(double)));
-    CU(cudaMalloc(&c->es_part, (size_t)es_norm_blocks(n) * 3 * od * sizeof(double)));
+  if (!c->es.norm) {
+    const size_t od = tb_obs_dim(c->cfg.env_kind), ad = tb_act_dim(c->cfg.env_kind);
+    EsBufs e;
+    CU(dev_alloc(e.norm, 2 * od * n * sizeof(double)));
+    CU(dev_alloc(e.n0, od * sizeof(double)));
+    CU(dev_alloc(e.ret, n * sizeof(double)));
+    CU(dev_alloc(e.hist, TB_ES_HISTORY * od * n * sizeof(float)));
+    CU(dev_alloc(e.obs, od * n * sizeof(float)));
+    CU(dev_alloc(e.term, od * n * sizeof(float)));
+    CU(dev_alloc(e.rew, n * sizeof(float)));
+    CU(dev_alloc(e.act, ad * n * sizeof(float)));
+    CU(dev_alloc(e.alive, n));
+    CU(dev_alloc(e.done, n));
+    CU(dev_alloc(e.base, sizeof(unsigned)));
+    CU(dev_alloc(e.stop, n * sizeof(unsigned)));
+    CU(dev_alloc(e.master, 3 * od * sizeof(double)));
+    CU(dev_alloc(e.part, es_norm_blocks(n) * 3 * od * sizeof(double)));
+    c->es = std::move(e);
   }
   if (c->es_w_cap < individuals * floats) {  // stream-ordered: a larger population does not synchronise either
-    if (c->es_w) CU(cudaFreeAsync(c->es_w, s));
-    c->es_w = nullptr; c->es_w_cap = 0;
-    CU(cudaMallocAsync(&c->es_w, (size_t)(individuals * floats) * sizeof(float), s));
+    c->es_w_cap = 0;
+    if (c->es_w) CU(cudaFreeAsync(c->es_w.release(), s));
+    void *w = nullptr;
+    CU(cudaMallocAsync(&w, (size_t)(individuals * floats) * sizeof(float), s));
+    c->es_w.reset(static_cast<float *>(w));
     c->es_w_cap = individuals * floats;
   }
   return 0;
@@ -2807,185 +2808,172 @@ static int es_prepare(tb_ctx *c, const char *who, int64_t individuals, int64_t f
 static int es_start(tb_ctx *c, int64_t individuals, const double *d_normalizer, cudaStream_t s) {
   const int64_t n = c->cfg.num_envs;
   const size_t master_bytes = (size_t)3 * tb_obs_dim(c->cfg.env_kind) * sizeof(double);
-  if (d_normalizer) CU(cudaMemcpyAsync(c->es_master, d_normalizer, master_bytes, cudaMemcpyDeviceToDevice, s));
-  else CU(cudaMemsetAsync(c->es_master, 0, master_bytes, s));
+  if (d_normalizer) CU(cudaMemcpyAsync(c->es.master.get(), d_normalizer, master_bytes, cudaMemcpyDeviceToDevice, s));
+  else CU(cudaMemsetAsync(c->es.master.get(), 0, master_bytes, s));
   StepIO io = make_io(c);
-  io.obs = c->es_obs;
-  DISPATCH(reset_kernel, grid_for(n, kBlock), kBlock, s, io, (const double *)nullptr, (const uint8_t *)nullptr);
-  CU(cudaMemsetAsync(c->es_done, 0, (size_t)n, s));  // the reset observation is the step obs the first action's trace shows
+  io.obs = c->es.obs.get();
+  if (launch_reset(c, io, nullptr, nullptr, s)) return 1;
+  CU(cudaMemsetAsync(c->es.done.get(), 0, (size_t)n, s));  // the reset observation is the step obs the first action's trace shows
   c->es_individuals = individuals;
   const EsIO eio = es_io(c);
-  if (c->cfg.env_kind == TB_ENV_SWING) es_begin_kernel<6><<<grid_for(n, kBlock), kBlock, 0, s>>>(eio, d_normalizer);
-  else es_begin_kernel<12><<<grid_for(n, kBlock), kBlock, 0, s>>>(eio, d_normalizer);
-  c->launches++;
-  CU(cudaGetLastError());
-  return 0;
+  return with_kind(c->cfg.env_kind, [&](auto kind) {
+    return launch(c, kPlain, es_begin_kernel<Dims<kind>::obs>, grid_for(n, kBlock), kBlock, s, eio, d_normalizer);
+  });
 }
 
 int tb_es_begin(tb_ctx *c, const float *d_weights, int64_t individuals, int64_t floats, const double *d_normalizer, void *stream) {
-  if (!d_weights) return fail("%s", "tb_es_begin: d_weights is NULL");
-  if (individuals < 1) return fail("%s", "tb_es_begin: individuals must be >= 1");
+  if (!d_weights) return fail("tb_es_begin: d_weights is NULL");
+  if (individuals < 1) return fail("tb_es_begin: individuals must be >= 1");
   GUARD(c);
   cudaStream_t s = (cudaStream_t)stream;
   if (es_prepare(c, "tb_es_begin", individuals, floats, s)) return 1;
-  es_transpose_kernel<<<dim3((unsigned)((individuals + 31) / 32), (unsigned)((floats + 31) / 32)), dim3(32, 8), 0, s>>>(
-      d_weights, individuals, (int)floats, c->es_w);
-  c->launches++;
+  if (launch(c, kPlain, es_transpose_kernel, dim3((unsigned)((individuals + 31) / 32), (unsigned)((floats + 31) / 32)), dim3(32, 8), s,
+             d_weights, individuals, (int)floats, c->es_w.get()))
+    return 1;
   return es_start(c, individuals, d_normalizer, s);
 }
 
 int tb_es_begin_noise(tb_ctx *c, const float *d_theta, int64_t individuals, int64_t floats, float sigma, uint64_t noise_seed,
                       uint32_t generation, const double *d_normalizer, void *stream) {
-  if (!d_theta) return fail("%s", "tb_es_begin_noise: d_theta is NULL");
-  if (individuals < 1) return fail("%s", "tb_es_begin_noise: individuals must be >= 1");
-  if (individuals % 2) return fail("%s", "tb_es_begin_noise: individuals must be even (antithetic pairs)");
-  if (!(sigma > 0.0f) || !std::isfinite(sigma)) return fail("%s", "tb_es_begin_noise: sigma must be a finite number above 0");
+  if (!d_theta) return fail("tb_es_begin_noise: d_theta is NULL");
+  if (individuals < 1) return fail("tb_es_begin_noise: individuals must be >= 1");
+  if (individuals % 2) return fail("tb_es_begin_noise: individuals must be even (antithetic pairs)");
+  if (!(sigma > 0.0f) || !std::isfinite(sigma)) return fail("tb_es_begin_noise: sigma must be a finite number above 0");
   GUARD(c);
   const int64_t repeats = individuals > 0 && c->cfg.num_envs % individuals == 0 ? c->cfg.num_envs / individuals : 0;
-  if (repeats && c->cfg.env_id_offset % (2 * repeats)) {
-    std::snprintf(g_err, sizeof g_err, "tb_es_begin_noise: env_id_offset (%lld) must be a multiple of 2 x repeats (%lld), so a shard "
-                  "holds whole antithetic pairs", (long long)c->cfg.env_id_offset, (long long)(2 * repeats));
-    return 1;
-  }
+  if (repeats && c->cfg.env_id_offset % (2 * repeats))
+    return fail("tb_es_begin_noise: env_id_offset (%lld) must be a multiple of 2 x repeats (%lld), so a shard holds whole "
+                "antithetic pairs", (long long)c->cfg.env_id_offset, (long long)(2 * repeats));
   cudaStream_t s = (cudaStream_t)stream;
   if (es_prepare(c, "tb_es_begin_noise", individuals, floats, s)) return 1;
   const int64_t pairs = individuals / 2, j0 = c->cfg.env_id_offset / (2 * repeats);
-  es_perturb_kernel<<<dim3(grid_for(pairs, kBlock), (unsigned)((floats + 3) / 4)), kBlock, 0, s>>>(
-      d_theta, pairs, (int)floats, sigma, noise_seed, generation, j0, c->es_w);
-  c->launches++;
+  if (launch(c, kPlain, es_perturb_kernel, dim3(grid_for(pairs, kBlock), (unsigned)((floats + 3) / 4)), kBlock, s, d_theta, pairs,
+             (int)floats, sigma, noise_seed, generation, j0, c->es_w.get()))
+    return 1;
   return es_start(c, individuals, d_normalizer, s);
 }
 
 int tb_es_noise_combine(tb_ctx *c, const int64_t *d_dirs, const float *d_coef, int64_t count, uint64_t noise_seed, uint32_t generation,
                         float *d_out, void *stream) {
-  if (count < 0) return fail("%s", "tb_es_noise_combine: count must be >= 0");
-  if (count > 0 && (!d_dirs || !d_coef)) return fail("%s", "tb_es_noise_combine: d_dirs and d_coef are required when count > 0");
-  if (!d_out) return fail("%s", "tb_es_noise_combine: d_out is NULL");
+  if (count < 0) return fail("tb_es_noise_combine: count must be >= 0");
+  if (count > 0 && (!d_dirs || !d_coef)) return fail("tb_es_noise_combine: d_dirs and d_coef are required when count > 0");
+  if (!d_out) return fail("tb_es_noise_combine: d_out is NULL");
   GUARD(c);
   if (check_fault(c, "tb_es_noise_combine")) return 1;
   const int floats = tb_es_floats(c->cfg.env_kind);
-  es_combine_kernel<<<(unsigned)((floats + 3) / 4), kBlock, 0, (cudaStream_t)stream>>>(d_dirs, d_coef, count, noise_seed,
-                                                                                         generation, floats, d_out);
-  c->launches++;
-  CU(cudaGetLastError());
-  return 0;
+  return launch(c, kPlain, es_combine_kernel, (unsigned)((floats + 3) / 4), kBlock, (cudaStream_t)stream, d_dirs, d_coef, count,
+                noise_seed, generation, floats, d_out);
 }
 
 int tb_es_normalizer_stats(tb_ctx *c, double *d_out, void *stream) {
-  if (!d_out) return fail("%s", "tb_es_normalizer_stats: d_out is NULL");
+  if (!d_out) return fail("tb_es_normalizer_stats: d_out is NULL");
   GUARD(c);
-  if (!c->es_individuals) return fail("%s", "tb_es_normalizer_stats: no generation (call tb_es_begin or tb_es_begin_noise first)");
+  if (!c->es_individuals) return fail("tb_es_normalizer_stats: no generation (call tb_es_begin or tb_es_begin_noise first)");
   if (check_fault(c, "tb_es_normalizer_stats")) return 1;
   cudaStream_t s = (cudaStream_t)stream;
   const int64_t blocks = es_norm_blocks(c->cfg.num_envs);
   const EsIO eio = es_io(c);
   const int od = tb_obs_dim(c->cfg.env_kind);
-  if (c->cfg.env_kind == TB_ENV_SWING) es_norm_partial_kernel<6><<<(unsigned)blocks, kBlock, 0, s>>>(eio, c->es_master, c->es_part);
-  else es_norm_partial_kernel<12><<<(unsigned)blocks, kBlock, 0, s>>>(eio, c->es_master, c->es_part);
-  es_norm_final_kernel<<<(unsigned)od, kBlock, 0, s>>>(c->es_part, blocks, od, c->es_master, d_out);
-  c->launches += 2;
-  CU(cudaGetLastError());
-  return 0;
+  if (with_kind(c->cfg.env_kind, [&](auto kind) {
+        return launch(c, kPlain, es_norm_partial_kernel<Dims<kind>::obs>, (unsigned)blocks, kBlock, s, eio, c->es.master.get(),
+                      c->es.part.get());
+      }))
+    return 1;
+  return launch(c, kPlain, es_norm_final_kernel, (unsigned)od, kBlock, s, c->es.part.get(), blocks, od, c->es.master.get(), d_out);
 }
 
 int tb_es_rollout(tb_ctx *c, int k_steps, double *d_return, uint8_t *d_alive, float *d_obs, float *d_actions, float *d_reward,
                   uint8_t *d_done, void *stream) {
-  if (k_steps < 1) return fail("%s", "tb_es_rollout: k_steps must be >= 1");
-  if (!d_return || !d_alive) return fail("%s", "tb_es_rollout: d_return and d_alive are required");
+  if (k_steps < 1) return fail("tb_es_rollout: k_steps must be >= 1");
+  if (!d_return || !d_alive) return fail("tb_es_rollout: d_return and d_alive are required");
   GUARD(c);
-  if (!c->es_individuals) return fail("%s", "tb_es_rollout: no population (call tb_es_begin first)");
-  if (c->control_mode != TB_CONTROL_FORCE) return fail("%s", "tb_es_rollout: the GatedCNN's actions are forces (TB_CONTROL_FORCE)");
+  if (!c->es_individuals) return fail("tb_es_rollout: no population (call tb_es_begin first)");
+  if (c->control_mode != TB_CONTROL_FORCE) return fail("tb_es_rollout: the GatedCNN's actions are forces (TB_CONTROL_FORCE)");
   if (check_fault(c, "tb_es_rollout")) return 1;
   const int64_t n = c->cfg.num_envs;
-  const bool swing = c->cfg.env_kind == TB_ENV_SWING;
   const int od = tb_obs_dim(c->cfg.env_kind), ad = tb_act_dim(c->cfg.env_kind);
-  void (*kernel)(EsIO) = swing ? es_kernel<6, 6> : es_kernel<12, 2>;
+  void (*kernel)(EsIO) = nullptr;
+  with_kind(c->cfg.env_kind, [&](auto kind) { kernel = es_kernel<Dims<kind>::obs, Dims<kind>::act>; return 0; });
   cudaStream_t s = (cudaStream_t)stream;
   const unsigned grid = grid_for(n, kBlock);
   EsIO eio = es_io(c);
   for (int t = 0; t <= k_steps; ++t) {  // launch t folds step t - 1 (t > 0) and acts for step t (t < K)
     eio.fold = t > 0;
-    eio.act = t < k_steps ? c->es_act : nullptr;
+    eio.act = t < k_steps ? c->es.act.get() : nullptr;
     eio.obs_trace = d_obs ? d_obs + (size_t)t * n * od : nullptr;
     eio.act_trace = d_actions && t < k_steps ? d_actions + (size_t)t * n * ad : nullptr;
     eio.rew_trace = d_reward && t > 0 ? d_reward + (size_t)(t - 1) * n : nullptr;
     eio.done_trace = d_done && t > 0 ? d_done + (size_t)(t - 1) * n : nullptr;
     eio.ret_out = t == k_steps ? d_return : nullptr;
     eio.alive_out = t == k_steps ? d_alive : nullptr;
-    CU(launch_pdl(kernel, grid, s, eio));
-    c->launches++;
+    if (launch(c, kPdl, kernel, grid, kBlock, s, eio)) return 1;
     if (t == k_steps) break;
     StepIO io = make_io(c);
-    io.actions = c->es_act; io.obs = c->es_obs; io.reward = c->es_rew; io.done = c->es_done; io.term_obs = c->es_term;
+    io.actions = c->es.act.get(); io.obs = c->es.obs.get(); io.reward = c->es.rew.get(); io.done = c->es.done.get();
+    io.term_obs = c->es.term.get();
     if (launch_step(c, io, s)) return 1;
   }
-  CU(cudaGetLastError());
   return 0;
 }
 
 int tb_get_state(tb_ctx *c, double *d_state, void *stream) {
   GUARD(c);
-  if (!d_state) return fail("%s", "tb_get_state: d_state is NULL");
-  int64_t n = c->cfg.num_envs;
-  if (c->cfg.precision == TB_F64) get_state_kernel<double><<<grid_for(n, 256), 256, 0, (cudaStream_t)stream>>>(c->sc64, (const double *)c->state, n, d_state);
-  else get_state_kernel<float><<<grid_for(n, 256), 256, 0, (cudaStream_t)stream>>>(c->sc32, (const float *)c->state, n, d_state);
-  c->launches++;
-  CU(cudaGetLastError());
-  return 0;
+  if (!d_state) return fail("tb_get_state: d_state is NULL");
+  const int64_t n = c->cfg.num_envs;
+  return with_env(c, [&](auto &sc, auto *state, auto) {
+    using T = std::remove_pointer_t<decltype(state)>;
+    return launch(c, kPlain, get_state_kernel<T>, grid_for(n, 256), 256, (cudaStream_t)stream, sc, state, n, d_state);
+  });
 }
 int tb_set_state(tb_ctx *c, const double *d_state, void *stream) {
   GUARD(c);
-  if (!d_state) return fail("%s", "tb_set_state: d_state is NULL");
-  int64_t n = c->cfg.num_envs;
-  if (c->cfg.precision == TB_F64) set_state_kernel<double><<<grid_for(n, 256), 256, 0, (cudaStream_t)stream>>>((double *)c->state, n, d_state);
-  else set_state_kernel<float><<<grid_for(n, 256), 256, 0, (cudaStream_t)stream>>>((float *)c->state, n, d_state);
-  c->launches++;
-  CU(cudaGetLastError());
-  return 0;
+  if (!d_state) return fail("tb_set_state: d_state is NULL");
+  const int64_t n = c->cfg.num_envs;
+  return with_env(c, [&](auto &, auto *state, auto) {
+    using T = std::remove_pointer_t<decltype(state)>;
+    return launch(c, kPlain, set_state_kernel<T>, grid_for(n, 256), 256, (cudaStream_t)stream, state, n, d_state);
+  });
 }
 
 int tb_stats_device_ptr(tb_ctx *c, int64_t **d_stats) {
-  if (!c || !d_stats) return fail("%s", "tb_stats_device_ptr: bad argument");
-  *d_stats = reinterpret_cast<int64_t *>(c->stats);
+  if (!c || !d_stats) return fail("tb_stats_device_ptr: bad argument");
+  *d_stats = reinterpret_cast<int64_t *>(c->stats.get());
   return 0;
 }
 int tb_read_stats(tb_ctx *c, int64_t *h_stats, int clear, void *stream) {
   GUARD(c);
-  if (!h_stats) return fail("%s", "tb_read_stats: h_stats is NULL");
+  if (!h_stats) return fail("tb_read_stats: h_stats is NULL");
   cudaStream_t s = (cudaStream_t)stream;
-  unsigned long long fault = 0;
-  CU(cudaMemcpyAsync(h_stats, c->stats, TB_NUM_STATS * sizeof(int64_t), cudaMemcpyDeviceToHost, s));
-  CU(cudaMemcpyAsync(&fault, c->fault, sizeof fault, cudaMemcpyDeviceToHost, s));
-  if (clear) CU(cudaMemsetAsync(c->stats, 0, TB_NUM_STATS * sizeof(int64_t), s));
+  CU(cudaMemcpyAsync(h_stats, c->stats.get(), TB_NUM_STATS * sizeof(int64_t), cudaMemcpyDeviceToHost, s));
+  if (clear) CU(cudaMemsetAsync(c->stats.get(), 0, TB_NUM_STATS * sizeof(int64_t), s));
   CU(cudaStreamSynchronize(s));
-  if (fault) {  // never seen; a wait in ff_kernel gave up (kSpinLimit) and that launch left envs unfinished
-    std::snprintf(g_err, sizeof g_err, "tb_read_stats: a fast-forward launch timed out waiting on its work queues (code %llu); the batch state is incomplete", fault);
-    return 1;
-  }
-  return 0;
+  return check_fault(c, "tb_read_stats");  // never seen; a wait in ff_kernel gave up (kSpinLimit) and left envs unfinished
 }
 
 static int ensure_staging(tb_ctx *c) {
-  if (c->d_actions) return 0;
-  size_t n = (size_t)c->cfg.num_envs, od = (size_t)tb_obs_dim(c->cfg.env_kind), ad = (size_t)tb_act_dim(c->cfg.env_kind);
-  CU(cudaMalloc(&c->d_actions, n * ad * sizeof(float)));
-  CU(cudaMalloc(&c->d_obs, n * od * sizeof(float)));
-  CU(cudaMalloc(&c->d_term, n * od * sizeof(float)));
-  CU(cudaMalloc(&c->d_reward, n * sizeof(float)));
-  CU(cudaMalloc(&c->d_done, n));
-  CU(cudaMalloc(&c->d_events, n));
-  CU(cudaMalloc(&c->d_mask, n));
+  if (c->staging.actions) return 0;
+  const size_t n = (size_t)c->cfg.num_envs, od = (size_t)tb_obs_dim(c->cfg.env_kind), ad = (size_t)tb_act_dim(c->cfg.env_kind);
+  StagingBufs b;
+  CU(dev_alloc(b.actions, n * ad * sizeof(float)));
+  CU(dev_alloc(b.obs, n * od * sizeof(float)));
+  CU(dev_alloc(b.term, n * od * sizeof(float)));
+  CU(dev_alloc(b.reward, n * sizeof(float)));
+  CU(dev_alloc(b.done, n));
+  CU(dev_alloc(b.events, n));
+  CU(dev_alloc(b.mask, n));
+  c->staging = std::move(b);
   return 0;
 }
 
 int tb_reset_host(tb_ctx *c, const uint8_t *h_mask, float *h_obs) {
   GUARD(c);
   if (ensure_staging(c)) return 1;
+  const StagingBufs &b = c->staging;
   size_t n = (size_t)c->cfg.num_envs, od = (size_t)tb_obs_dim(c->cfg.env_kind);
   cudaStream_t s = c->own_stream;
-  if (h_mask) CU(cudaMemcpyAsync(c->d_mask, h_mask, n, cudaMemcpyHostToDevice, s));
-  if (reset_impl(c, nullptr, h_mask ? c->d_mask : nullptr, c->d_obs, s)) return 1;
-  if (h_obs) CU(cudaMemcpyAsync(h_obs, c->d_obs, n * od * sizeof(float), cudaMemcpyDeviceToHost, s));
+  if (h_mask) CU(cudaMemcpyAsync(b.mask.get(), h_mask, n, cudaMemcpyHostToDevice, s));
+  if (reset_impl(c, nullptr, h_mask ? b.mask.get() : nullptr, b.obs.get(), s)) return 1;
+  if (h_obs) CU(cudaMemcpyAsync(h_obs, b.obs.get(), n * od * sizeof(float), cudaMemcpyDeviceToHost, s));
   CU(cudaStreamSynchronize(s));
   return 0;
 }
@@ -3002,7 +2990,7 @@ static void *mapped_alias(const void *h) {
 int tb_step_host(tb_ctx *c, const float *h_actions, float *h_obs, float *h_reward, uint8_t *h_done, float *h_terminal_obs,
                  uint8_t *h_events) {
   GUARD(c);
-  if (!h_actions || !h_obs || !h_reward || !h_done) return fail("%s", "tb_step_host: actions, obs, reward and done are required");
+  if (!h_actions || !h_obs || !h_reward || !h_done) return fail("tb_step_host: actions, obs, reward and done are required");
   if (check_fault(c, "tb_step_host")) return 1;
   // Transport: zero copy for pinned buffers, staging for pageable ones and for pinned ones when TB_HOST_MODE=staging.
   // Measured on the B200 box, 1 Mi SwingRacket envs, per step averaged over episodes: zero copy 0.92 ms, staging 1.24 ms
@@ -3032,15 +3020,16 @@ int tb_step_host(tb_ctx *c, const float *h_actions, float *h_obs, float *h_rewar
     }
   }
   if (ensure_staging(c)) return 1;
-  CU(cudaMemcpyAsync(c->d_actions, h_actions, n * ad * sizeof(float), cudaMemcpyHostToDevice, s));
-  if (tb_step(c, c->d_actions, c->d_obs, c->d_reward, c->d_done, h_terminal_obs ? c->d_term : nullptr,
-              h_events ? c->d_events : nullptr, s))
+  const StagingBufs &b = c->staging;
+  CU(cudaMemcpyAsync(b.actions.get(), h_actions, n * ad * sizeof(float), cudaMemcpyHostToDevice, s));
+  if (tb_step(c, b.actions.get(), b.obs.get(), b.reward.get(), b.done.get(), h_terminal_obs ? b.term.get() : nullptr,
+              h_events ? b.events.get() : nullptr, s))
     return 1;
-  CU(cudaMemcpyAsync(h_obs, c->d_obs, n * od * sizeof(float), cudaMemcpyDeviceToHost, s));
-  CU(cudaMemcpyAsync(h_reward, c->d_reward, n * sizeof(float), cudaMemcpyDeviceToHost, s));
-  CU(cudaMemcpyAsync(h_done, c->d_done, n, cudaMemcpyDeviceToHost, s));
-  if (h_terminal_obs) CU(cudaMemcpyAsync(h_terminal_obs, c->d_term, n * od * sizeof(float), cudaMemcpyDeviceToHost, s));
-  if (h_events) CU(cudaMemcpyAsync(h_events, c->d_events, n, cudaMemcpyDeviceToHost, s));
+  CU(cudaMemcpyAsync(h_obs, b.obs.get(), n * od * sizeof(float), cudaMemcpyDeviceToHost, s));
+  CU(cudaMemcpyAsync(h_reward, b.reward.get(), n * sizeof(float), cudaMemcpyDeviceToHost, s));
+  CU(cudaMemcpyAsync(h_done, b.done.get(), n, cudaMemcpyDeviceToHost, s));
+  if (h_terminal_obs) CU(cudaMemcpyAsync(h_terminal_obs, b.term.get(), n * od * sizeof(float), cudaMemcpyDeviceToHost, s));
+  if (h_events) CU(cudaMemcpyAsync(h_events, b.events.get(), n, cudaMemcpyDeviceToHost, s));
   CU(cudaStreamSynchronize(s));
   return check_fault(c, "tb_step_host");
 }
@@ -3053,7 +3042,7 @@ int tb_set_kernel_timing(tb_ctx *c, int enabled) {
   return 0;
 }
 int tb_get_kernel_timing(tb_ctx *c, double *ms_step_kernel, double *ms_ff_kernel, int64_t *steps) {
-  if (!c || !ms_step_kernel || !ms_ff_kernel || !steps) return fail("%s", "tb_get_kernel_timing: bad argument");
+  if (!c || !ms_step_kernel || !ms_ff_kernel || !steps) return fail("tb_get_kernel_timing: bad argument");
   *ms_step_kernel = c->ms_step; *ms_ff_kernel = c->ms_ff; *steps = c->timed_steps;
   c->ms_step = c->ms_ff = 0; c->timed_steps = 0;
   return 0;
@@ -3061,27 +3050,22 @@ int tb_get_kernel_timing(tb_ctx *c, double *ms_step_kernel, double *ms_ff_kernel
 
 int tb_ff_diagnostics(tb_ctx *c, int64_t *h_out) {
   GUARD(c);
-  if (!h_out) return fail("%s", "tb_ff_diagnostics: h_out is NULL");
+  if (!h_out) return fail("tb_ff_diagnostics: h_out is NULL");
   CU(cudaDeviceSynchronize());
   unsigned long long h[2 * kCtrWords];
-  CU(cudaMemcpy(h, c->queue_ctrs, sizeof h, cudaMemcpyDeviceToHost));
+  CU(cudaMemcpy(h, c->queue_ctrs.get(), sizeof h, cudaMemcpyDeviceToHost));
   // the set of the most recent step that entered the fast-forward: the one whose round count is non-zero and whose
   // twin was zeroed since (both non-zero cannot happen: every step_kernel zeroes the next step's set)
   const unsigned long long *s = h[kDRounds] ? h : h + kCtrWords;
   h_out[0] = (int64_t)s[kDRounds]; h_out[1] = (int64_t)s[kDFullEnvs]; h_out[2] = (int64_t)s[kDPhase];
-  for (int i = 3; i < 14; ++i) h_out[i] = 0;
-  h_out[14] = (int64_t)s[kDFinish];
-  h_out[15] = (int64_t)s[kCError];
-  {
-    unsigned long long fault = 0;
-    CU(cudaMemcpy(&fault, c->fault, sizeof fault, cudaMemcpyDeviceToHost));
-    if (fault) h_out[15] = (int64_t)fault;
-  }
+  for (int i = 3; i < 15; ++i) h_out[i] = 0;  // (ff_kernel stores kDFinish = 0)
+  const unsigned long long fault = fault_word(c);
+  h_out[15] = (int64_t)(fault ? fault : s[kCError]);
   return 0;
 }
 
 int tb_launch_count(tb_ctx *c, int64_t *launches) {
-  if (!c || !launches) return fail("%s", "tb_launch_count: bad argument");
+  if (!c || !launches) return fail("tb_launch_count: bad argument");
   *launches = c->launches;
   return 0;
 }
