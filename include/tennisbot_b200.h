@@ -233,6 +233,55 @@ int tb_es_noise_combine(tb_ctx *ctx, const int64_t *d_dirs, const float *d_coef,
  * reduction, no atomics.  Fails before the first tb_es_begin*.  Stream-ordered, never synchronises. */
 int tb_es_normalizer_stats(tb_ctx *ctx, double *d_out, void *stream);
 
+/* ---- SAC actor and replay ring (SURVEY 8(f)-5): what SB3 SAC's collect_rollouts does around env.step (train_swing.py's and
+ * train.py's SAC option), kept on the device.  The actor is SB3 1.8 SAC MlpPolicy's: latent_pi = Linear(obs, 256), ReLU,
+ * Linear(256, 256), ReLU; heads mu and log_std = Linear(256, act); log_std clamped to [-20, 2]; action = tanh(mu + exp(log_std)
+ * eps) (TB_SAC_SAMPLE) or tanh(mu) (TB_SAC_MEAN).  Both action spaces are Box(-1, 1), so SB3's unscaling is the identity.
+ * Parameters, float32, in SB3 state-dict order, each tensor row-major [out][in] and padded to a multiple of 4 floats:
+ *   actor.latent_pi.0 W[256 x obs] b[256], actor.latent_pi.2 W[256 x 256] b[256], actor.mu W[act x 256] b[act],
+ *   actor.log_std W[act x 256] b[act]:  70672 floats for SwingRacket-v0 (obs 6, act 6), 70152 for Tennisbot-v0 (obs 12, act 2).
+ * Numerics: layer 1 in float32 (each product and sum rounded, in input order, starting from the bias), ReLU, rounded to BF16;
+ * layer 2 on the tensor cores with W2 rounded to BF16 and FP32 accumulation; b2, ReLU, the heads, exp and tanh in float32.
+ * Noise: r = Philox4x32-10(key = noise_seed, counter = (global env id lo, hi, tick, (4 << 28) | q)), q = o / 4, where tick is
+ * the context's env-step counter when the action is taken (so every replay of a captured graph draws fresh noise, and
+ * shards reproduce the full batch).  With v(x) = (x >> 8) / 2^24:
+ *   TB_SAC_UNIFORM: action[o] = 2 v(r[o mod 4]) - 1 (SB3's learning_starts warm-up; the network is not evaluated);
+ *   TB_SAC_SAMPLE: pair p = o / 2 of words w = r[(2p) mod 4], r[(2p + 1) mod 4]: u1 = v(w0) + 2^-25, u2 = v(w1),
+ *     eps[o] = sqrtf(-2 logf(u1)) * (o even ? cospif(2 u2) : sinpif(2 u2)), all float32. */
+#define TB_SAC_FLOATS 70672
+#define TB_SAC_FLOATS_HIT 70152
+#define TB_SAC_HIDDEN 256
+#define TB_SAC_SAMPLE 0
+#define TB_SAC_MEAN 1
+#define TB_SAC_UNIFORM 2
+int tb_sac_floats(int env_kind); /* TB_SAC_FLOATS / TB_SAC_FLOATS_HIT (-1: unknown kind); callable without a GPU */
+/* Converts d_params (count = tb_sac_floats(env_kind)) on the device into the library's own image of the actor (W2 as BF16 in
+ * the tensor cores' shared-memory layout): one kernel on `stream`, so it is capturable and a replayed graph sees the weights the
+ * buffer holds at replay time. */
+int tb_set_sac_actor(tb_ctx *ctx, const float *d_params, int64_t count, void *stream);
+/* Replay ring, caller-owned device arrays: obs, next_obs float32 [slots, N, obs_dim]; act float32 [slots, N, act_dim]; reward
+ * float32 [slots, N]; done uint8 [slots, N]. */
+typedef struct tb_sac_ring {
+  uint32_t struct_size; /* sizeof(tb_sac_ring) */
+  int32_t reserved;
+  int64_t slots;
+  float *obs, *act, *reward, *next_obs;
+  uint8_t *done;
+} tb_sac_ring;
+/* Needs TB_CONTROL_FORCE and auto_reset = 1.  Resets every env from the RNG, keeps the reset observation in the context and
+ * records the env-step counter as the ring's base.  One kernel launch. */
+int tb_sac_begin(tb_ctx *ctx, void *stream);
+/* k_steps >= 1 env steps: per step one sac_kernel launch (fold the previous step into the ring, then act) and tb_step's
+ * launches, then one fold-only sac_kernel launch: (K + 1) + K s launches, s = 2 for SwingRacket-v0 and 1 for Tennisbot-v0.
+ * The j-th env step since tb_sac_begin writes ring slot j mod slots (j is read on the device, so a captured graph appends at
+ * new slots on every replay): obs = the observation the action was computed from, act = the squashed action step_kernel
+ * received, reward, done (a time-out is a done like any other: the reference returns {} and SB3 does not bootstrap), next_obs
+ * = the terminal observation when done, else the step's observation.  ring = NULL stores nothing (evaluation).  d_last_obs
+ * float32 [N, obs_dim] (may be NULL) receives the observation after the last step.  mode TB_SAC_SAMPLE and TB_SAC_MEAN need
+ * tb_set_sac_actor.  Never synchronises: capturable in a CUDA graph. */
+int tb_sac_rollout(tb_ctx *ctx, int k_steps, int mode, uint64_t noise_seed, const tb_sac_ring *ring, float *d_last_obs,
+                   void *stream);
+
 /* ---- state dump / injection for the parity harness: double [N, TB_STATE_WORDS] */
 int tb_get_state(tb_ctx *ctx, double *d_state, void *stream);
 int tb_set_state(tb_ctx *ctx, const double *d_state, void *stream);

@@ -19,11 +19,20 @@ POLICY_FLOATS_HIT = 9324   # Tennisbot-v0's (TB_POLICY_FLOATS_HIT)
 ES_FLOATS = 766            # SwingRacket-v0's GatedCNN (TB_ES_FLOATS)
 ES_FLOATS_HIT = 858        # Tennisbot-v0's (TB_ES_FLOATS_HIT)
 ES_HISTORY = 8             # observations the GatedCNN sees (TB_ES_HISTORY)
+SAC_FLOATS = 70672         # SwingRacket-v0's SAC actor (TB_SAC_FLOATS)
+SAC_FLOATS_HIT = 70152     # Tennisbot-v0's (TB_SAC_FLOATS_HIT)
+SAC_HIDDEN = 256           # TB_SAC_HIDDEN
+SAC_SAMPLE, SAC_MEAN, SAC_UNIFORM = 0, 1, 2
 CONTROL_FORCE, CONTROL_PID = 0, 1
 
 EV_RACKET_BALL, EV_COURT_BALL, EV_GOAL_BALL, EV_TIMEOUT, EV_BALL_PASSED, EV_NET_BALL, EV_RACKET_LOW = 1, 2, 4, 8, 16, 32, 64
 STAT_NAMES = ("episodes", "sum_length", "racket_hits", "goals", "court", "timeouts", "sum_return_q20",
               "sum_return2_q10", "physics_steps", "env_steps")
+
+class TbSacRing(C.Structure):
+    _fields_ = [("struct_size", C.c_uint32), ("reserved", C.c_int32), ("slots", C.c_int64), ("obs", C.c_void_p),
+                ("act", C.c_void_p), ("reward", C.c_void_p), ("next_obs", C.c_void_p), ("done", C.c_void_p)]
+
 
 class TbConfig(C.Structure):
     _fields_ = [("struct_size", C.c_uint32), ("env_kind", C.c_int32), ("precision", C.c_int32), ("device", C.c_int32),
@@ -47,6 +56,8 @@ SIGNATURES = {
     "tb_es_begin": [_vp, _vp, _i64, _i64, _vp, _vp], "tb_es_rollout": [_vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
     "tb_es_begin_noise": [_vp, _vp, _i64, _i64, C.c_float, _u64, _u32, _vp, _vp],
     "tb_es_noise_combine": [_vp, _vp, _vp, _i64, _u64, _u32, _vp, _vp], "tb_es_normalizer_stats": [_vp, _vp, _vp],
+    "tb_sac_floats": [_i32], "tb_set_sac_actor": [_vp, _vp, _i64, _vp], "tb_sac_begin": [_vp, _vp],
+    "tb_sac_rollout": [_vp, _i32, _i32, _u64, C.POINTER(TbSacRing), _vp, _vp],
     "tb_get_state": [_vp, _vp, _vp], "tb_set_state": [_vp, _vp, _vp],
     "tb_stats_device_ptr": [_vp, C.POINTER(_vp)], "tb_read_stats": [_vp, _vp, _i32, _vp],
     "tb_reset_host": [_vp, _vp, _vp], "tb_step_host": [_vp, _vp, _vp, _vp, _vp, _vp, _vp],

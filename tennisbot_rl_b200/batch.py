@@ -231,6 +231,44 @@ class TennisBatch:
         _lib.check(self.lib.tb_es_normalizer_stats(self.h, _dptr(out), self._stream()))
         return out
 
+    # ------------------------------------------------------------------ SAC actor and replay ring (tb_set_sac_actor / tb_sac_*)
+    def set_sac_actor(self, params):
+        """params: float32 CUDA tensor [sac_floats] in the layout of include/tennisbot_b200.h for this batch's env
+        (SAC_FLOATS for SwingRacket-v0, SAC_FLOATS_HIT for Tennisbot-v0; sac.pack_sac_actor builds it)."""
+        want = _lib.SAC_FLOATS if self.kind == _lib.ENV_SWING else _lib.SAC_FLOATS_HIT
+        self._need("set_sac_actor", params, "params", (want,))
+        _lib.check(self.lib.tb_set_sac_actor(self.h, _dptr(params), want, self._stream()))
+
+    def sac_begin(self):
+        """Reset every env and start the ring at slot 0 (needs force control and auto_reset)."""
+        _lib.check(self.lib.tb_sac_begin(self.h, self._stream()))
+
+    def sac_rollout(self, k, mode=_lib.SAC_SAMPLE, ring=None, noise_seed=0, last_obs=None):
+        """k env steps with in-kernel SAC actions.  mode: SAC_SAMPLE, SAC_MEAN or SAC_UNIFORM (or 'sample', 'mean', 'uniform').
+        ring: None or a dict of tensors obs / next_obs float32 [slots, N, obs_dim], act float32 [slots, N, act_dim], reward
+        float32 [slots, N], done uint8 [slots, N]; step j since sac_begin goes to slot j % slots.  last_obs float32 [N, obs_dim]
+        receives the observation after the last step.  The library writes through raw pointers, so every buffer is checked here."""
+        k, n = int(k), self.num_envs
+        if k < 1:
+            raise ValueError(f"sac_rollout: k must be >= 1, got {k}")
+        mode = {"sample": _lib.SAC_SAMPLE, "mean": _lib.SAC_MEAN, "uniform": _lib.SAC_UNIFORM}.get(mode, mode)
+        need = functools.partial(self._need, "sac_rollout")
+        need(last_obs, "last_obs", (n, self.obs_dim), optional=True)
+        r = None
+        if ring is not None:
+            slots = int(ring["obs"].shape[0]) if torch.is_tensor(ring.get("obs")) and ring["obs"].dim() == 3 else -1
+            if slots < 1:
+                raise ValueError(f"sac_rollout: ring['obs'] must have shape (slots >= 1, {n}, {self.obs_dim})")
+            need(ring.get("obs"), "ring['obs']", (slots, n, self.obs_dim))
+            need(ring.get("next_obs"), "ring['next_obs']", (slots, n, self.obs_dim))
+            need(ring.get("act"), "ring['act']", (slots, n, self.act_dim))
+            need(ring.get("reward"), "ring['reward']", (slots, n))
+            need(ring.get("done"), "ring['done']", (slots, n), dtype=torch.uint8)
+            r = _lib.TbSacRing(C.sizeof(_lib.TbSacRing), 0, slots, *(ring[key].data_ptr() for key in
+                                                                     ("obs", "act", "reward", "next_obs", "done")))
+        _lib.check(self.lib.tb_sac_rollout(self.h, k, int(mode), int(noise_seed) & (2 ** 64 - 1), None if r is None else C.byref(r),
+                                           _dptr(last_obs), self._stream()))
+
     def get_state(self):
         s = torch.empty((self.num_envs, _lib.STATE_WORDS), dtype=torch.float64, device=self.device)
         _lib.check(self.lib.tb_get_state(self.h, _dptr(s), self._stream()))

@@ -1813,6 +1813,271 @@ __global__ void __launch_bounds__(kBlock) es_norm_final_kernel(const double *par
   if (threadIdx.x == 0) { out[c] = v.n; out[obs + c] = m0[obs + c] + v.d; out[2 * obs + c] = v.m2; }
 }
 
+// ------------------------------------------------------------------------------------------------ SAC actor and replay ring
+// SURVEY 8(f)-5: the actor of SB3 SAC's MlpPolicy (latent_pi = Linear(obs, 256), ReLU, Linear(256, 256), ReLU; mu and log_std
+// heads Linear(256, act); log_std clamped to [-20, 2]; action tanh(mu + exp(log_std) eps)) evaluated on the device, and every
+// transition folded into a caller-owned replay ring.  A rollout is K x (sac_kernel, step_kernel, ff_kernel) + one fold-only
+// sac_kernel, as the ES rollout.  Layer 2 (256 x 256) is the one dense contraction of the library: it runs on the tensor cores
+// (tcgen05.mma, BF16 operands, FP32 accumulate in tensor memory); layer 1 and the heads stay float32 on the CUDA cores.
+template <int OBS, int ACT> struct SacLayout {  // the caller's vector (header TB_SAC_*): float offsets, row-major [out][in]
+  static constexpr int H = 256;
+  static constexpr int W1 = 0, B1 = H * OBS, W2 = B1 + H, B2 = W2 + H * H, MuW = B2 + H, MuB = MuW + ACT * H,
+                       LsW = MuB + pad4(ACT), LsB = LsW + ACT * H, Floats = LsB + pad4(ACT);
+  // the image tb_set_sac_actor builds: W2 as BF16 in the canonical layout below (128 KB), then every other tensor in float32
+  // in the same order and padding ("small" offsets = the vector's offsets with W2 taken out)
+  static constexpr int SW1 = W1, SB1 = B1, SB2 = W2, SMuW = SB2 + H, SMuB = SMuW + ACT * H, SLsW = SMuB + pad4(ACT),
+                       SLsB = SLsW + ACT * H, Small = SLsB + pad4(ACT);
+  static constexpr int W2Bytes = H * H * 2, ABytes = 128 * H * 2;
+  static constexpr int Smem = W2Bytes + ABytes + Small * 4 + 16;  // + mbarrier, TMEM address
+};
+static_assert(SacLayout<6, 6>::Floats == TB_SAC_FLOATS && SacLayout<12, 2>::Floats == TB_SAC_FLOATS_HIT, "SAC layout / header mismatch");
+static_assert(SacLayout<6, 6>::Smem <= 227 * 1024 && SacLayout<12, 2>::Smem <= 227 * 1024, "SAC shared memory above 227 KB");
+
+// UMMA canonical K-major layout without swizzle: 8 x 16-byte "core matrices" (8 rows x 8 BF16 along K, 128 contiguous bytes).
+// Core matrix (row group g, K group kc) of an operand with R rows sits at byte (kc * R / 8 + g) * 128: one K = 16 step of the
+// MMA reads K groups 2s and 2s + 1, i.e. leading byte offset (K direction) R * 16, stride byte offset (rows) 128.
+__host__ __device__ constexpr uint32_t umma_offset(int row, int k, int rows) {
+  return (uint32_t)(((k >> 3) * (rows >> 3) + (row >> 3)) * 128 + (row & 7) * 16 + (k & 7) * 2);
+}
+__device__ __forceinline__ uint64_t umma_desc(uint32_t saddr, uint32_t lbo, uint32_t sbo) {
+  return (uint64_t)((saddr & 0x3FFFFu) >> 4) | ((uint64_t)(lbo >> 4) << 16) | ((uint64_t)(sbo >> 4) << 32) |
+         (1ull << 46);  // bits 46-48 = 0b001 (sm_100 descriptor), base offset 0, swizzle none (bits 61-63 = 0)
+}
+// kind::f16 instruction descriptor: D FP32 (bits 4-5 = 1), A and B BF16 (bits 7-9, 10-12 = 1), both K-major, N >> 3 at bit 17,
+// M >> 4 at bit 24
+constexpr uint32_t kSacIdesc = (1u << 4) | (1u << 7) | (1u << 10) | ((256u >> 3) << 17) | ((128u >> 4) << 24);
+__device__ __forceinline__ uint32_t bf16x2(float lo, float hi) {  // round to nearest even, lo in the low half
+  uint32_t r;
+  asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));
+  return r;
+}
+__device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
+
+constexpr uint32_t kStreamSac = 4u;  // beside kStreamReset (0), kStreamAction (1), kStreamPolicy (2), kStreamEsNoise (3)
+struct SacIO {
+  const uint4 *w2;              // [8192] W2 image (BF16, canonical layout)
+  const float *small;           // SacLayout::Small floats
+  int64_t n, id_offset;
+  uint64_t seed;
+  const unsigned *tick;         // the env-step counter (StepIO::epoch[0] / [2]): constant while a sac_kernel runs
+  const unsigned *base;         // its value at tb_sac_begin: step j since then writes ring slot j mod slots
+  int mode;                     // TB_SAC_*
+  int fold;                     // 1: fold the previous step into the ring and `cur`
+  float *act;                   // [N, A] action for step_kernel; nullptr: fold only (the launch ending a rollout)
+  const float *act_prev;        // the same buffer: the action the previous step took
+  float *cur;                   // [N, C] the observation the next action is computed from
+  const float *obs, *term, *reward;  // the previous env step's outputs (the context's buffers)
+  const uint8_t *done;
+  int64_t slots;                // ring (all nullptr: nothing stored)
+  float *r_obs, *r_act, *r_reward, *r_next;
+  uint8_t *r_done;
+  float *last_obs;              // optional: `cur` after the fold (the launch ending a rollout)
+};
+
+// Fold step j = tick - base - 1 of env i into the ring and `cur`; x receives the observation the next action is computed from.
+template <int OBS, int ACT>
+__device__ __forceinline__ void sac_fold(const SacIO &io, int64_t i, float *x) {
+  const float2 *src = reinterpret_cast<const float2 *>((io.fold ? io.obs : io.cur) + i * OBS);
+#pragma unroll
+  for (int j = 0; j < OBS / 2; ++j) { const float2 v = src[j]; x[2 * j] = v.x; x[2 * j + 1] = v.y; }
+  if (!io.fold) return;
+  const int64_t n = io.n;
+  if (io.r_obs) {
+    const int64_t row = (int64_t)((uint64_t)(*io.tick - *io.base - 1u) % (uint64_t)io.slots) * n + i;
+    const uint8_t d = io.done[i];
+    const float2 *prev = reinterpret_cast<const float2 *>(io.cur + i * OBS);
+    const float2 *nxt = reinterpret_cast<const float2 *>((d ? io.term : io.obs) + i * OBS);
+    float2 *ro = reinterpret_cast<float2 *>(io.r_obs + row * OBS), *rn = reinterpret_cast<float2 *>(io.r_next + row * OBS);
+#pragma unroll
+    for (int j = 0; j < OBS / 2; ++j) { ro[j] = prev[j]; rn[j] = nxt[j]; }
+    const float2 *a = reinterpret_cast<const float2 *>(io.act_prev + i * ACT);
+    float2 *ra = reinterpret_cast<float2 *>(io.r_act + row * ACT);
+#pragma unroll
+    for (int j = 0; j < ACT / 2; ++j) ra[j] = a[j];
+    io.r_reward[row] = io.reward[i];
+    io.r_done[row] = d;
+  }
+  float2 *cur = reinterpret_cast<float2 *>(io.cur + i * OBS);
+#pragma unroll
+  for (int j = 0; j < OBS / 2; ++j) cur[j] = make_float2(x[2 * j], x[2 * j + 1]);
+  if (io.last_obs) {
+    float2 *q = reinterpret_cast<float2 *>(io.last_obs + i * OBS);
+#pragma unroll
+    for (int j = 0; j < OBS / 2; ++j) q[j] = make_float2(x[2 * j], x[2 * j + 1]);
+  }
+}
+
+// The Philox words of env i at the current tick: uniform a = 2 u - 1 (TB_SAC_UNIFORM), or Gaussian eps (TB_SAC_SAMPLE).
+template <int ACT> __device__ __forceinline__ void sac_noise(const SacIO &io, int64_t i, float *v, bool gaussian) {
+  constexpr int NR = (ACT + 3) / 4;
+  uint32_t rr[4 * NR];
+  const uint32_t tick = *io.tick;
+#pragma unroll
+  for (int j = 0; j < NR; ++j) philox4x32(io.seed, (uint64_t)(io.id_offset + i), tick, stream_word(kStreamSac, 0, j), rr + 4 * j);
+#pragma unroll
+  for (int o = 0; o < ACT; ++o) {
+    if (!gaussian) {
+      v[o] = 2.0f * u01<float>(rr[o]) - 1.0f;
+    } else {  // Box-Muller on pair o / 2: cosine branch for even o, sine for odd (policy_kernel<12, 2>'s formula)
+      const float u1 = ((float)(rr[2 * (o / 2)] >> 8) + 0.5f) * (1.0f / 16777216.0f), u2 = (float)(rr[2 * (o / 2) + 1] >> 8) * (1.0f / 16777216.0f);
+      v[o] = sqrtf(-2.0f * logf(u1)) * ((o & 1) ? sinpif(2.0f * u2) : cospif(2.0f * u2));
+    }
+  }
+}
+
+template <int ACT> __device__ __forceinline__ void sac_store_act(const SacIO &io, int64_t i, const float *a) {
+  float2 *q = reinterpret_cast<float2 *>(io.act + i * ACT);
+#pragma unroll
+  for (int j = 0; j < ACT / 2; ++j) q[j] = make_float2(a[2 * j], a[2 * j + 1]);
+}
+
+// Two launch shapes.  Fold only, or TB_SAC_UNIFORM: one thread per env, no dynamic shared memory.  With the network: a
+// persistent grid of min(tiles, SMs) CTAs with SacLayout::Smem bytes of dynamic shared memory (one CTA per SM), each looping
+// over 128-env tiles, one env per thread and per TMEM lane:
+//   layer 1 float32 (no contraction, so torch restates it exactly), ReLU, rounded to BF16 into the A tile (128 x 256);
+//   thread 0 issues 16 x tcgen05.mma (M 128, N 256, K 16) into 256 TMEM columns and commits to an mbarrier;
+//   each warp reads its 32 lanes back (tcgen05.ld 32x32b), adds b2, ReLU, and forms both heads in float32;
+//   clamp, noise, accurate tanhf.
+template <int OBS, int ACT>
+__global__ void __launch_bounds__(kBlock, 1) sac_kernel(const __grid_constant__ SacIO io) {
+  using L = SacLayout<OBS, ACT>;
+  static_assert(OBS % 2 == 0 && ACT % 2 == 0, "observation and action rows are accessed as float2");
+  extern __shared__ __align__(1024) uint8_t sac_smem[];
+  pdl_wait();
+  const int64_t n = io.n;
+  if (!io.act || io.mode == TB_SAC_UNIFORM) {
+    const int64_t i = (int64_t)blockIdx.x * kBlock + threadIdx.x;
+    if (i < n) {
+      float x[OBS];
+      sac_fold<OBS, ACT>(io, i, x);
+      if (io.act) {
+        float a[ACT];
+        sac_noise<ACT>(io, i, a, false);
+        sac_store_act<ACT>(io, i, a);
+      }
+    }
+    pdl_trigger();
+    return;
+  }
+  uint8_t *W2 = sac_smem, *A = sac_smem + L::W2Bytes;
+  float *S = reinterpret_cast<float *>(sac_smem + L::W2Bytes + L::ABytes);
+  uint64_t *bar = reinterpret_cast<uint64_t *>(S + L::Small);
+  uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(bar + 1);
+  const int tid = threadIdx.x, warp = tid >> 5;
+  {
+    uint4 *w = reinterpret_cast<uint4 *>(W2);
+    for (int q = tid; q < L::W2Bytes / 16; q += kBlock) w[q] = io.w2[q];
+    for (int q = tid; q < L::Small; q += kBlock) S[q] = io.small[q];
+  }
+  if (warp == 0) {
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 256;" ::"r"(smem_u32(tmem_slot)));
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
+  }
+  if (tid == 0) {
+    asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_u32(bar)));
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+  }
+  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // W2 written by plain stores, read by the tensor cores
+  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  __syncthreads();
+  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  const uint32_t tmem = *tmem_slot, a_base = smem_u32(A), b_base = smem_u32(W2), bar_a = smem_u32(bar);
+  const int64_t tiles = (n + kBlock - 1) / kBlock;
+  uint32_t phase = 0;
+  for (int64_t tile = blockIdx.x; tile < tiles; tile += gridDim.x, phase ^= 1u) {
+    const int64_t i = tile * kBlock + tid;
+    const bool mine = i < n;
+    float x[OBS];
+#pragma unroll
+    for (int c = 0; c < OBS; ++c) x[c] = 0.0f;
+    if (mine) sac_fold<OBS, ACT>(io, i, x);
+    // layer 1: acc = b1, then + W1[j][c] x[c] for c = 0 .. OBS - 1, each product and sum rounded (no fused multiply-add)
+#pragma unroll 1
+    for (int kc = 0; kc < L::H / 8; ++kc) {
+      float h[8];
+#pragma unroll
+      for (int u = 0; u < 8; ++u) {
+        const int j = kc * 8 + u;
+        float acc = S[L::SB1 + j];
+#pragma unroll
+        for (int c = 0; c < OBS; ++c) acc = __fadd_rn(acc, __fmul_rn(S[L::SW1 + j * OBS + c], x[c]));
+        h[u] = fmaxf(acc, 0.0f);
+      }
+      *reinterpret_cast<uint4 *>(A + umma_offset(tid, kc * 8, 128)) =
+          make_uint4(bf16x2(h[0], h[1]), bf16x2(h[2], h[3]), bf16x2(h[4], h[5]), bf16x2(h[6], h[7]));
+    }
+    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    __syncthreads();
+    if (tid == 0) {
+      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+#pragma unroll
+      for (int s = 0; s < L::H / 16; ++s) {
+        const uint64_t ad = umma_desc(a_base + s * 2 * 16 * 128, 16 * 128, 128), bd = umma_desc(b_base + s * 2 * 32 * 128, 32 * 128, 128);
+        asm volatile("{\n.reg .pred p;\nsetp.ne.b32 p, %4, 0;\ntcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n}" ::"r"(tmem),
+                     "l"(ad), "l"(bd), "r"(kSacIdesc), "r"(s));
+      }
+      asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar_a) : "memory");
+    }
+    asm volatile("{\n.reg .pred P;\nSAC_WAIT:\nmbarrier.try_wait.parity.shared::cta.b64 P, [%0], %1;\n@!P bra SAC_WAIT;\n}" ::"r"(bar_a),
+                 "r"(phase) : "memory");
+    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    float mu[ACT], ls[ACT];
+#pragma unroll
+    for (int o = 0; o < ACT; ++o) { mu[o] = S[L::SMuB + o]; ls[o] = S[L::SLsB + o]; }
+#pragma unroll 1
+    for (int q = 0; q < L::H / 32; ++q) {
+      uint32_t r[32];
+      asm volatile(
+          "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,%21,%22,"
+          "%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
+          : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]), "=r"(r[9]),
+            "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]), "=r"(r[17]), "=r"(r[18]),
+            "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]), "=r"(r[25]), "=r"(r[26]), "=r"(r[27]),
+            "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
+          : "r"(tmem + ((uint32_t)(warp * 32) << 16) + (uint32_t)(q * 32)));
+      asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+#pragma unroll
+      for (int u = 0; u < 32; ++u) {
+        const int j = q * 32 + u;
+        const float h = fmaxf(__uint_as_float(r[u]) + S[L::SB2 + j], 0.0f);
+#pragma unroll
+        for (int o = 0; o < ACT; ++o) {
+          mu[o] = fmaf(S[L::SMuW + o * L::H + j], h, mu[o]);
+          ls[o] = fmaf(S[L::SLsW + o * L::H + j], h, ls[o]);
+        }
+      }
+    }
+    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");  // the next tile's MMA overwrites these columns
+    if (mine) {
+      float a[ACT], eps[ACT];
+      const bool sample = io.mode == TB_SAC_SAMPLE;
+      if (sample) sac_noise<ACT>(io, i, eps, true);
+#pragma unroll
+      for (int o = 0; o < ACT; ++o) {
+        const float l = fminf(fmaxf(ls[o], -20.0f), 2.0f);
+        a[o] = tanhf(sample ? fmaf(expf(l), eps[o], mu[o]) : mu[o]);
+      }
+      sac_store_act<ACT>(io, i, a);
+    }
+  }
+  __syncthreads();
+  if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 256;" ::"r"(tmem));
+  pdl_trigger();
+}
+
+// tb_set_sac_actor: the caller's float32 vector -> W2 in BF16 at its canonical-layout offset, everything else to `small`.
+template <int OBS, int ACT> __global__ void __launch_bounds__(256) sac_image_kernel(const float *p, uint16_t *w2, float *small) {
+  using L = SacLayout<OBS, ACT>;
+  const int f = blockIdx.x * 256 + threadIdx.x;
+  if (f >= L::Floats) return;
+  if (f < L::W2) small[f] = p[f];
+  else if (f < L::B2) {
+    const int e = f - L::W2;
+    w2[umma_offset(e / L::H, e % L::H, L::H) / 2] = (uint16_t)(bf16x2(p[f], 0.0f) & 0xFFFFu);
+  } else small[f - L::H * L::H] = p[f];
+}
+
 template <typename T, int KIND>
 __global__ void __launch_bounds__(kBlock) reset_kernel(const __grid_constant__ Scene<T> sc, const __grid_constant__ StepIO io,
                                                        const double *init, const uint8_t *mask) {
@@ -2263,6 +2528,15 @@ struct StagingBufs {          // device copies of the host-buffer entry points' 
   DevPtr<float> actions, obs, reward, term;
   DevPtr<uint8_t> done, events, mask;
 };
+struct SacActorBufs {         // tb_set_sac_actor: the actor's image (see SacLayout)
+  DevPtr<uint4> w2;           // W2, 128 KB
+  DevPtr<float> small;        // the other tensors
+};
+struct SacBufs {              // tb_sac_begin: per-env staging between sac_kernel and the env step (see SacIO)
+  DevPtr<float> cur, act, obs, term, rew;
+  DevPtr<uint8_t> done;
+  DevPtr<unsigned> base;
+};
 struct PolicyBufs {           // tb_set_policy
   DevPtr<float> params;       // tb_policy_floats(env_kind) parameters
   DevPtr<float> act;          // [N, act_dim] clipped actions handed from policy_kernel to step_kernel
@@ -2296,6 +2570,9 @@ struct tb_ctx {
   int control_mode = TB_CONTROL_FORCE;
   DevPtr<void> pid;                          // controller memory, allocated by tb_set_control_mode(TB_CONTROL_PID)
   PolicyBufs policy;
+  SacActorBufs sac_actor;                    // SAC actor and ring (tb_set_sac_actor / tb_sac_begin / tb_sac_rollout)
+  SacBufs sac;
+  int sac_grid = 0;                          // persistent grid of sac_kernel: SMs
   // ES fitness rollout (tb_es_begin / tb_es_rollout); see EsIO
   int64_t es_individuals = 0;                // 0: no tb_es_begin yet
   DevPtr<float> es_w;                        // [floats][individuals], stream-ordered allocation
@@ -2343,21 +2620,26 @@ static size_t state_word(tb_ctx *c) { return with_env(c, [](auto &, auto *state,
 // Every kernel launch of the library: plain, or with programmatic stream serialisation (pdl), counted and checked.
 constexpr bool kPlain = false, kPdl = true;
 template <typename... KArgs, typename... Args>
-static int launch(tb_ctx *c, bool pdl, void (*kernel)(KArgs...), dim3 grid, dim3 block, cudaStream_t stream, Args &&...args) {
+static int launch_smem(tb_ctx *c, bool pdl, void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream,
+                       Args &&...args) {
   if (pdl) {
     cudaLaunchConfig_t cfg{};
-    cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = 0; cfg.stream = stream;
+    cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = stream;
     cudaLaunchAttribute at[1];
     at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     at[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = at; cfg.numAttrs = 1;
     CU(cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...));
   } else {
-    kernel<<<grid, block, 0, stream>>>(std::forward<Args>(args)...);
+    kernel<<<grid, block, smem, stream>>>(std::forward<Args>(args)...);
   }
   c->launches++;
   CU(cudaGetLastError());
   return 0;
+}
+template <typename... KArgs, typename... Args>
+static int launch(tb_ctx *c, bool pdl, void (*kernel)(KArgs...), dim3 grid, dim3 block, cudaStream_t stream, Args &&...args) {
+  return launch_smem(c, pdl, kernel, grid, block, 0, stream, std::forward<Args>(args)...);
 }
 
 // A fast-forward launch of this context gave up on a wait (ff_give_up): its batch state is incomplete.  Sticky; every
@@ -2490,6 +2772,7 @@ int tb_obs_dim(int kind) { return with_kind(kind, [](auto k) { return Dims<k>::o
 int tb_act_dim(int kind) { return with_kind(kind, [](auto k) { return Dims<k>::act; }); }
 int tb_policy_floats(int kind) { return with_kind(kind, [](auto k) { return PolLayout<Dims<k>::obs, Dims<k>::act>::Floats; }); }
 int tb_es_floats(int kind) { return with_kind(kind, [](auto k) { return EsLayout<Dims<k>::obs, Dims<k>::act>::Floats; }); }
+int tb_sac_floats(int kind) { return with_kind(kind, [](auto k) { return SacLayout<Dims<k>::obs, Dims<k>::act>::Floats; }); }
 int tb_num_params(void) { return kNumParams; }
 const char *tb_param_name(int i) { return (i >= 0 && i < kNumParams) ? k_param_names[i] : nullptr; }
 
@@ -2914,6 +3197,108 @@ int tb_es_rollout(tb_ctx *c, int k_steps, double *d_return, uint8_t *d_alive, fl
     if (launch_step(c, io, s)) return 1;
   }
   return 0;
+}
+
+int tb_set_sac_actor(tb_ctx *c, const float *d_params, int64_t count, void *stream) {
+  GUARD(c);
+  const int64_t want = tb_sac_floats(c->cfg.env_kind);
+  if (!d_params || count != want)
+    return fail("tb_set_sac_actor: expected tb_sac_floats(env_kind) = %lld floats in device memory, got %lld", (long long)want,
+                (long long)count);
+  if (!c->sac_actor.w2) {
+    SacActorBufs b;
+    CU(dev_alloc(b.w2, TB_SAC_HIDDEN * TB_SAC_HIDDEN * 2));
+    CU(dev_alloc(b.small, (size_t)(want - TB_SAC_HIDDEN * TB_SAC_HIDDEN) * sizeof(float)));
+    c->sac_actor = std::move(b);
+  }
+  if (with_kind(c->cfg.env_kind, [&](auto kind) {
+        return launch(c, kPlain, sac_image_kernel<Dims<kind>::obs, Dims<kind>::act>, grid_for(want, 256), 256, (cudaStream_t)stream,
+                      d_params, reinterpret_cast<uint16_t *>(c->sac_actor.w2.get()), c->sac_actor.small.get());
+      }))
+    return 1;
+  return 0;
+}
+
+int tb_sac_begin(tb_ctx *c, void *stream) {
+  GUARD(c);
+  if (c->control_mode != TB_CONTROL_FORCE) return fail("tb_sac_begin: the actor's actions are forces (TB_CONTROL_FORCE)");
+  if (!c->cfg.auto_reset) return fail("tb_sac_begin: the ring needs auto_reset = 1 (a done env starts its next episode in the step)");
+  if (check_fault(c, "tb_sac_begin")) return 1;
+  const size_t n = c->cfg.num_envs, od = tb_obs_dim(c->cfg.env_kind), ad = tb_act_dim(c->cfg.env_kind);
+  if (!c->sac.cur) {
+    SacBufs b;
+    CU(dev_alloc(b.cur, od * n * sizeof(float)));
+    CU(dev_alloc(b.obs, od * n * sizeof(float)));
+    CU(dev_alloc(b.term, od * n * sizeof(float)));
+    CU(dev_alloc(b.act, ad * n * sizeof(float)));
+    CU(dev_alloc(b.rew, n * sizeof(float)));
+    CU(dev_alloc(b.done, n));
+    CU(dev_alloc(b.base, sizeof(unsigned)));
+    c->sac = std::move(b);
+  }
+  if (!c->sac_grid) {  // (configuration calls, kept out of tb_sac_rollout so that it can be captured in any capture mode)
+    CU(cudaDeviceGetAttribute(&c->sac_grid, cudaDevAttrMultiProcessorCount, c->cfg.device));
+    if (with_kind(c->cfg.env_kind, [&](auto kind) {
+          constexpr int OBS = Dims<kind>::obs, ACT = Dims<kind>::act;
+          CU(cudaFuncSetAttribute(sac_kernel<OBS, ACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, SacLayout<OBS, ACT>::Smem));
+          return 0;
+        }))
+      return 1;
+  }
+  cudaStream_t s = (cudaStream_t)stream;
+  StepIO io = make_io(c);
+  io.obs = c->sac.cur.get();
+  if (launch_reset(c, io, nullptr, nullptr, s)) return 1;
+  CU(cudaMemcpyAsync(c->sac.base.get(), step_counter(c), sizeof(unsigned), cudaMemcpyDeviceToDevice, s));
+  return 0;
+}
+
+int tb_sac_rollout(tb_ctx *c, int k_steps, int mode, uint64_t noise_seed, const tb_sac_ring *ring, float *d_last_obs, void *stream) {
+  if (k_steps < 1) return fail("tb_sac_rollout: k_steps must be >= 1");
+  if (mode != TB_SAC_SAMPLE && mode != TB_SAC_MEAN && mode != TB_SAC_UNIFORM) return fail("tb_sac_rollout: unknown mode %d", mode);
+  if (ring) {
+    if (ring->struct_size != sizeof(tb_sac_ring)) return fail("tb_sac_rollout: tb_sac_ring.struct_size mismatch");
+    if (ring->slots < 1) return fail("tb_sac_rollout: ring slots must be >= 1");
+    if (!ring->obs || !ring->act || !ring->reward || !ring->next_obs || !ring->done)
+      return fail("tb_sac_rollout: every ring array (obs, act, reward, next_obs, done) is required");
+  }
+  GUARD(c);
+  if (c->control_mode != TB_CONTROL_FORCE) return fail("tb_sac_rollout: the actor's actions are forces (TB_CONTROL_FORCE)");
+  if (!c->cfg.auto_reset) return fail("tb_sac_rollout: the ring needs auto_reset = 1");
+  if (!c->sac.cur) return fail("tb_sac_rollout: no tb_sac_begin on this context");
+  if (mode != TB_SAC_UNIFORM && !c->sac_actor.w2) return fail("tb_sac_rollout: no actor (tb_set_sac_actor)");
+  if (check_fault(c, "tb_sac_rollout")) return 1;
+  const int64_t n = c->cfg.num_envs;
+  cudaStream_t s = (cudaStream_t)stream;
+  SacIO sio;
+  std::memset(&sio, 0, sizeof sio);
+  sio.w2 = c->sac_actor.w2.get(); sio.small = c->sac_actor.small.get(); sio.n = n; sio.id_offset = c->cfg.env_id_offset; sio.seed = noise_seed;
+  sio.tick = step_counter(c); sio.base = c->sac.base.get(); sio.mode = mode; sio.act_prev = c->sac.act.get(); sio.cur = c->sac.cur.get();
+  sio.obs = c->sac.obs.get(); sio.term = c->sac.term.get(); sio.reward = c->sac.rew.get(); sio.done = c->sac.done.get();
+  if (ring) {
+    sio.slots = ring->slots; sio.r_obs = ring->obs; sio.r_act = ring->act; sio.r_reward = ring->reward; sio.r_next = ring->next_obs;
+    sio.r_done = ring->done;
+  }
+  return with_kind(c->cfg.env_kind, [&](auto kind) {
+    constexpr int OBS = Dims<kind>::obs, ACT = Dims<kind>::act;
+    auto kernel = sac_kernel<OBS, ACT>;
+    constexpr int smem = SacLayout<OBS, ACT>::Smem;
+    const int64_t tiles = (n + kBlock - 1) / kBlock;
+    for (int t = 0; t <= k_steps; ++t) {  // launch t folds step t - 1 (t > 0) and acts for step t (t < K)
+      sio.fold = t > 0;
+      sio.act = t < k_steps ? c->sac.act.get() : nullptr;
+      sio.last_obs = t == k_steps ? d_last_obs : nullptr;
+      const bool net = sio.act && mode != TB_SAC_UNIFORM;
+      const unsigned grid = net ? (unsigned)std::min<int64_t>(tiles, c->sac_grid) : (unsigned)tiles;
+      if (launch_smem(c, kPdl, kernel, grid, kBlock, net ? smem : 0, s, sio)) return 1;
+      if (t == k_steps) break;
+      StepIO io = make_io(c);
+      io.actions = c->sac.act.get(); io.obs = c->sac.obs.get(); io.reward = c->sac.rew.get(); io.done = c->sac.done.get();
+      io.term_obs = c->sac.term.get();
+      if (launch_step(c, io, s)) return 1;
+    }
+    return 0;
+  });
 }
 
 int tb_get_state(tb_ctx *c, double *d_state, void *stream) {
