@@ -282,6 +282,58 @@ int tb_sac_begin(tb_ctx *ctx, void *stream);
 int tb_sac_rollout(tb_ctx *ctx, int k_steps, int mode, uint64_t noise_seed, const tb_sac_ring *ring, float *d_last_obs,
                    void *stream);
 
+/* ---- frames rendered on the device: one ray per pixel against the scene's collision shapes.  No GUI; the reference's
+ * PyBullet camera (tennisbot_env.py:269-279) is not recorded, so cameras are the caller's.
+ *
+ * Geometry: the collision shapes as the physics sees them, without the collision margins (hull_margin, box_margin), all in
+ * the world frame (metres):
+ *   TB_BODY_COURT   the floor box |x| <= floor_hx, |y| <= floor_hy, |z| <= floor_hz (centred on the origin, as physics_step has it);
+ *   TB_BODY_NET     the net box   |x| <= net_hx,   |y| <= net_hy,   |z| <= net_hz;
+ *   TB_BODY_GOAL    SwingRacket-v0 contexts only (the hit env has no goal): the goal prism, the 32-gon of goal_vertex_x/y
+ *                   (tb_scene_constant) about the record's goal x, y (TB_S_GOAL), |z| <= goal_half_z;
+ *   TB_BODY_RACKET  the racket's outline prism in its COM frame: |x| <= racket_scale * racket_half_x, polygon (y, z) =
+ *                   racket_scale * (racket_outline_y, racket_outline_z - racket_com_z); placed at the record's COM position
+ *                   (TB_S_RACKET_POS) and quaternion (TB_S_RACKET_QUAT, x,y,z,w, used as the physics uses it: unnormalised);
+ *                   the convex hull the physics uses, not the STL mesh;
+ *   TB_BODY_BALL    the sphere of radius ball_radius at TB_S_BALL_POS.
+ * The context's current scene is used, so racket_scale applies.  There are no court lines (the court texture is not part of
+ * this repository).  A shape is seen where the ray enters it at a positive distance (an eye inside a shape does not see it);
+ * the nearest entry wins, equal distances go to the lower TB_BODY_* value.
+ * Camera: f = normalize(target - eye), r = normalize(f x up), u = r x f, t = tan(fov_y / 2).  Pixel (x, y), x = column,
+ * y = row with row 0 at the top (gym's rgb_array layout), casts the ray direction
+ *   d = normalize(f + ((2 (x + 0.5) / W - 1) t W / H) r + ((1 - 2 (y + 0.5) / H) t) u).
+ * Shading: n = the unit outward normal of the surface the ray enters (for a box or a prism: the entry plane's), flipped to
+ * face the eye (n.d <= 0); channel k = floor(c_body[k] (0.35 + 0.65 max(0, n.L)) + 0.5) with L = TB_RENDER_LIGHT
+ * normalised; a ray that meets nothing gets TB_RENDER_SKY.  No shadows, no anti-aliasing.  The kernel computes in float32
+ * with coordinates relative to the eye (the per-frame plane offsets in float64, rounded once). */
+#define TB_BODY_NONE 0
+#define TB_BODY_COURT 1 /* the floor box */
+#define TB_BODY_NET 2
+#define TB_BODY_GOAL 3  /* SwingRacket-v0 only */
+#define TB_BODY_RACKET 4
+#define TB_BODY_BALL 5
+#define TB_RENDER_SKY {170, 200, 235}
+#define TB_RENDER_COLORS {{0, 0, 0}, {70, 140, 95}, {235, 235, 235}, {215, 60, 50}, {40, 80, 200}, {225, 240, 60}} /* by TB_BODY_* */
+#define TB_RENDER_LIGHT {-0.3, 0.4, 1.0} /* towards the light, before normalisation */
+#define TB_RENDER_MAX_SIZE 4096
+typedef struct tb_camera {
+  uint32_t struct_size;            /* sizeof(tb_camera) */
+  int32_t width, height;           /* pixels, 1 .. TB_RENDER_MAX_SIZE each */
+  int32_t reserved;
+  double eye[3], target[3], up[3]; /* world frame, metres */
+  double fov_y_deg;                /* vertical field of view, (0, 180) */
+} tb_camera;
+/* d_states double [count, TB_STATE_WORDS]: canonical records (tb_get_state rows, a trajectory file, or the caller's).
+ * d_rgb uint8 [count, H, W, 3]; d_depth float32 [count, H, W], the distance from the eye along the ray, +inf where the ray
+ * meets nothing (may be NULL); d_body uint8 [count, H, W], TB_BODY_* (may be NULL).  One kernel launch on `stream`, never
+ * synchronises (capturable in a CUDA graph).  Reads only the context's scene parameters and writes nothing of the context
+ * (env state, RNG counters, statistics and fast-forward queues are untouched; tb_launch_count rises by 1).  Fails when cam,
+ * d_states or d_rgb is NULL, count < 1, struct_size is wrong, width or height is outside 1 .. 4096, fov_y_deg is not finite
+ * or outside (0, 180), eye == target, up is parallel to the view direction (|f x up| <= 1e-9 |up|, a zero up included), an
+ * output's size in bytes overflows int64, or the context is faulted. */
+int tb_render(tb_ctx *ctx, const tb_camera *cam, const double *d_states, int64_t count, uint8_t *d_rgb, float *d_depth,
+              uint8_t *d_body, void *stream);
+
 /* ---- state dump / injection for the parity harness: double [N, TB_STATE_WORDS] */
 int tb_get_state(tb_ctx *ctx, double *d_state, void *stream);
 int tb_set_state(tb_ctx *ctx, const double *d_state, void *stream);

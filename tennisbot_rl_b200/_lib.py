@@ -24,6 +24,11 @@ SAC_FLOATS_HIT = 70152     # Tennisbot-v0's (TB_SAC_FLOATS_HIT)
 SAC_HIDDEN = 256           # TB_SAC_HIDDEN
 SAC_SAMPLE, SAC_MEAN, SAC_UNIFORM = 0, 1, 2
 CONTROL_FORCE, CONTROL_PID = 0, 1
+BODY_NONE, BODY_COURT, BODY_NET, BODY_GOAL, BODY_RACKET, BODY_BALL = 0, 1, 2, 3, 4, 5  # TB_BODY_*
+RENDER_SKY = (170, 200, 235)                                                           # TB_RENDER_SKY
+RENDER_COLORS = ((0, 0, 0), (70, 140, 95), (235, 235, 235), (215, 60, 50), (40, 80, 200), (225, 240, 60))  # by TB_BODY_*
+RENDER_LIGHT = (-0.3, 0.4, 1.0)                                                        # TB_RENDER_LIGHT, not normalised
+RENDER_MAX_SIZE = 4096
 
 EV_RACKET_BALL, EV_COURT_BALL, EV_GOAL_BALL, EV_TIMEOUT, EV_BALL_PASSED, EV_NET_BALL, EV_RACKET_LOW = 1, 2, 4, 8, 16, 32, 64
 STAT_NAMES = ("episodes", "sum_length", "racket_hits", "goals", "court", "timeouts", "sum_return_q20",
@@ -32,6 +37,11 @@ STAT_NAMES = ("episodes", "sum_length", "racket_hits", "goals", "court", "timeou
 class TbSacRing(C.Structure):
     _fields_ = [("struct_size", C.c_uint32), ("reserved", C.c_int32), ("slots", C.c_int64), ("obs", C.c_void_p),
                 ("act", C.c_void_p), ("reward", C.c_void_p), ("next_obs", C.c_void_p), ("done", C.c_void_p)]
+
+
+class TbCamera(C.Structure):
+    _fields_ = [("struct_size", C.c_uint32), ("width", C.c_int32), ("height", C.c_int32), ("reserved", C.c_int32),
+                ("eye", C.c_double * 3), ("target", C.c_double * 3), ("up", C.c_double * 3), ("fov_y_deg", C.c_double)]
 
 
 class TbConfig(C.Structure):
@@ -58,6 +68,7 @@ SIGNATURES = {
     "tb_es_noise_combine": [_vp, _vp, _vp, _i64, _u64, _u32, _vp, _vp], "tb_es_normalizer_stats": [_vp, _vp, _vp],
     "tb_sac_floats": [_i32], "tb_set_sac_actor": [_vp, _vp, _i64, _vp], "tb_sac_begin": [_vp, _vp],
     "tb_sac_rollout": [_vp, _i32, _i32, _u64, C.POINTER(TbSacRing), _vp, _vp],
+    "tb_render": [_vp, C.POINTER(TbCamera), _vp, _i64, _vp, _vp, _vp, _vp],
     "tb_get_state": [_vp, _vp, _vp], "tb_set_state": [_vp, _vp, _vp],
     "tb_stats_device_ptr": [_vp, C.POINTER(_vp)], "tb_read_stats": [_vp, _vp, _i32, _vp],
     "tb_reset_host": [_vp, _vp, _vp], "tb_step_host": [_vp, _vp, _vp, _vp, _vp, _vp, _vp],

@@ -269,6 +269,26 @@ class TennisBatch:
         _lib.check(self.lib.tb_sac_rollout(self.h, k, int(mode), int(noise_seed) & (2 ** 64 - 1), None if r is None else C.byref(r),
                                            _dptr(last_obs), self._stream()))
 
+    # ------------------------------------------------------------------ frames (tb_render)
+    def render(self, camera, states=None, depth=False, body=False):
+        """Frames of canonical state records through `camera` (render.Camera), one kernel launch on the current stream.
+        states: None renders every env of this batch from a fresh get_state(); else a float64 [M, 32] tensor on this batch's
+        device.  Returns (rgb uint8 [M, H, W, 3], depth float32 [M, H, W] or None, body uint8 [M, H, W] or None): device
+        tensors, row 0 at the top; depth is the distance from the eye (+inf: sky), body holds _lib.BODY_*."""
+        if states is None:
+            states = self.get_state()
+        m = int(states.shape[0]) if states.dim() == 2 else -1
+        if m < 1:
+            raise ValueError(f"render: states must have shape (M >= 1, {_lib.STATE_WORDS}), got {tuple(states.shape)}")
+        self._need("render", states, "states", (m, _lib.STATE_WORDS), torch.float64)
+        h, w = int(camera.height), int(camera.width)
+        rgb = torch.empty((m, h, w, 3), dtype=torch.uint8, device=self.device)
+        dep = torch.empty((m, h, w), dtype=torch.float32, device=self.device) if depth else None
+        bod = torch.empty((m, h, w), dtype=torch.uint8, device=self.device) if body else None
+        _lib.check(self.lib.tb_render(self.h, C.byref(camera.to_c()), _dptr(states), m, _dptr(rgb), _dptr(dep), _dptr(bod),
+                                      self._stream()))
+        return rgb, dep, bod
+
     def get_state(self):
         s = torch.empty((self.num_envs, _lib.STATE_WORDS), dtype=torch.float64, device=self.device)
         _lib.check(self.lib.tb_get_state(self.h, _dptr(s), self._stream()))

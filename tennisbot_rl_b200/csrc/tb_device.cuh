@@ -350,6 +350,64 @@ template <typename T, int NE> __device__ __forceinline__ bool prism_outside_fast
                   ((u - pr.t_ax[1]) * pr.t_nx[1] + (v - pr.t_ay[1]) * pr.t_ny[1] > rim);
   return far_head & far_quad;
 }
+
+// ------------------------------------------------------------------------------------------------ ray casting (tb_render)
+// float32, coordinates relative to the eye: the ray is s -> s d with |d| = 1, and a shape counts where it is entered at s > 0.
+// A convex body is the intersection of planes n.p <= h; with c = n.(eye) - h and den = n.d the ray crosses a plane at
+// s = -c / den, entering where den < 0 and leaving where den > 0 (a parallel ray outside a plane misses the body): the
+// Cyrus-Beck clip.  f0 is the entry plane.
+__device__ __forceinline__ void clip_plane(float c, float den, int face, float &s0, float &s1, int &f0) {
+  if (den < 0.f) {
+    const float s = -c / den;
+    if (s > s0) { s0 = s; f0 = face; }
+  } else if (den > 0.f) {
+    s1 = fminf(s1, -c / den);
+  } else if (c > 0.f) {
+    s1 = -M<float>::inf();
+  }
+}
+__device__ __forceinline__ float clip_entry(float s0, float s1) { return s0 > 0.f && s0 < s1 ? s0 : M<float>::inf(); }
+// Box |p_k| <= h_k about the origin; cb[2k] = eye_k - h_k, cb[2k + 1] = -eye_k - h_k.  face 2k: +axis k, 2k + 1: -axis k.
+__device__ __forceinline__ float ray_box(const float *cb, const float *d, int &face) {
+  float s0 = -M<float>::inf(), s1 = M<float>::inf();
+  face = 0;
+#pragma unroll
+  for (int k = 0; k < 3; ++k) {
+    clip_plane(cb[2 * k], d[k], 2 * k, s0, s1, face);
+    clip_plane(cb[2 * k + 1], -d[k], 2 * k + 1, s0, s1, face);
+  }
+  return clip_entry(s0, s1);
+}
+// Prism of the narrow phase in its own frame (t; u, v): |t| <= half_thick, inside every outline edge.  o_t = the eye's t,
+// ce[i] = the eye's c of edge i (formed per frame), dl = the direction in that frame.  face 0: +t, 1: -t, 2 + i: edge i.
+template <typename T, int NE>
+__device__ __forceinline__ float ray_prism(const Prism<T, NE> &pr, const float *ce, float o_t, const float *dl, int &face) {
+  const float ht = (float)pr.half_thick;
+  float s0 = -M<float>::inf(), s1 = M<float>::inf();
+  face = 0;
+  clip_plane(o_t - ht, dl[0], 0, s0, s1, face);
+  clip_plane(-o_t - ht, -dl[0], 1, s0, s1, face);
+#pragma unroll 2
+  for (int i = 0; i < NE; ++i) clip_plane(ce[i], (float)pr.e[i].nx * dl[1] + (float)pr.e[i].ny * dl[2], 2 + i, s0, s1, face);
+  return clip_entry(s0, s1);
+}
+// Sphere of radius r about c (relative to the eye), through the perpendicular from c to the ray (no cancellation of |c|^2
+// against (c.d)^2 for a small sphere far away).
+__device__ __forceinline__ float ray_sphere(const float *c, float r, const float *d) {
+  const float b = c[0] * d[0] + c[1] * d[1] + c[2] * d[2];
+  const float q0 = c[0] - b * d[0], q1 = c[1] - b * d[1], q2 = c[2] - b * d[2];
+  const float h = r * r - (q0 * q0 + q1 * q1 + q2 * q2);
+  if (h < 0.f) return M<float>::inf();
+  return clip_entry(b - sqrtf(h), M<float>::inf());
+}
+// true: the ray passes the bounding sphere (c, r) for certain, or reaches it only beyond `best` (reject only: grown)
+__device__ __forceinline__ bool ray_skips(const float *c, float r, const float *d, float best) {
+  const float b = c[0] * d[0] + c[1] * d[1] + c[2] * d[2];
+  const float q0 = c[0] - b * d[0], q1 = c[1] - b * d[1], q2 = c[2] - b * d[2];
+  const float rr = r * 1.001f + 1e-4f;
+  return q0 * q0 + q1 * q1 + q2 * q2 > rr * rr || b + rr < 0.f || b - rr > best;
+}
+
 // ------------------------------------------------------------------------------------------------ contacts
 constexpr int kMaxContacts = 8;  // the ball's (racket, floor, net, goal) + up to four racket-floor points
 template <typename T> struct Contact {

@@ -2165,6 +2165,131 @@ template <typename T> __global__ void set_state_kernel(T *base, int64_t n, const
   store_state(base, n, i, s);
 }
 
+// ------------------------------------------------------------------------------------------------ tb_render
+// One thread per pixel; a CTA covers kRenderBlock consecutive pixels (row-major) of one frame at a time and walks the frames
+// blockIdx.y, blockIdx.y + gridDim.y, ...  Per frame, 71 threads stage what every ray of it shares: the racket's rotation,
+// the shapes' centres relative to the eye, and the eye's offset c from every prism edge plane, formed in float64 from the
+// record and rounded once (the rays then clip in float32).
+constexpr int kRenderBlock = 256;
+struct RenderIO {
+  const double *states;
+  int64_t count;
+  uint8_t *rgb, *body;
+  float *depth;
+  int width, height;
+  double eye[3];
+  float f[3], r[3], u[3];  // view direction; r scaled by t W / H, u by t (the camera of tb_render)
+  float light[3];          // TB_RENDER_LIGHT normalised
+  float box_c[2][6];       // floor, net: ray_box's cb for this eye
+};
+__constant__ uint8_t k_render_color[6][3] = TB_RENDER_COLORS;
+enum { kRfR = 0, kRfRp = 9, kRfOt = 12, kRfBall = 13, kRfGoal = 16, kRfGoalT = 19, kRfWords = 20 };
+
+template <typename T, int KIND>
+__global__ void __launch_bounds__(kRenderBlock) render_kernel(const __grid_constant__ Scene<T> sc, const __grid_constant__ RenderIO io) {
+  constexpr bool kGoal = KIND == TB_ENV_SWING;
+  __shared__ float s_rc[kRacketEdges], s_gc[kGoalEdges], s_f[kRfWords];
+  const int64_t npix = (int64_t)io.width * io.height;
+  const int64_t pix = (int64_t)blockIdx.x * kRenderBlock + threadIdx.x;
+  const int px = (int)(pix % io.width), py = (int)(pix / io.width);
+  float d[3];
+  {
+    const float a = (float)(2 * px + 1 - io.width) / (float)io.width, b = (float)(io.height - 2 * py - 1) / (float)io.height;
+#pragma unroll
+    for (int k = 0; k < 3; ++k) d[k] = io.f[k] + a * io.r[k] + b * io.u[k];
+    const float inv = 1.f / sqrtf(d[0] * d[0] + d[1] * d[1] + d[2] * d[2]);
+#pragma unroll
+    for (int k = 0; k < 3; ++k) d[k] *= inv;
+  }
+  for (int64_t fr = blockIdx.y; fr < io.count; fr += gridDim.y) {
+    const double *rec = io.states + fr * TB_STATE_WORDS;
+    const int i = threadIdx.x;
+    __syncthreads();  // the previous frame's rays are done with the staged words
+    if (i <= kRacketEdges) {
+      double R[9], rel[3], ol[3];
+      quat_to_mat(rec + TB_S_RACKET_QUAT, R);
+      for (int k = 0; k < 3; ++k) rel[k] = io.eye[k] - rec[TB_S_RACKET_POS + k];
+      matT_vec(R, rel, ol);
+      if (i < kRacketEdges) {
+        const Edge<T> &e = sc.racket.e[i];
+        s_rc[i] = (float)((ol[1] - (double)e.ax) * (double)e.nx + (ol[2] - (double)e.ay) * (double)e.ny);
+      } else {
+        for (int k = 0; k < 9; ++k) s_f[kRfR + k] = (float)R[k];
+        for (int k = 0; k < 3; ++k) {
+          s_f[kRfRp + k] = (float)-rel[k];
+          s_f[kRfBall + k] = (float)(rec[TB_S_BALL_POS + k] - io.eye[k]);
+        }
+        s_f[kRfOt] = (float)ol[0];
+        s_f[kRfGoal] = (float)(rec[TB_S_GOAL] - io.eye[0]);
+        s_f[kRfGoal + 1] = (float)(rec[TB_S_GOAL + 1] - io.eye[1]);
+        s_f[kRfGoal + 2] = (float)-io.eye[2];
+        s_f[kRfGoalT] = (float)io.eye[2];
+      }
+    } else if (kGoal && i <= kRacketEdges + kGoalEdges) {
+      const Edge<T> &e = sc.goal.e[i - kRacketEdges - 1];
+      const double ou = io.eye[0] - rec[TB_S_GOAL], ov = io.eye[1] - rec[TB_S_GOAL + 1];
+      s_gc[i - kRacketEdges - 1] = (float)((ou - (double)e.ax) * (double)e.nx + (ov - (double)e.ay) * (double)e.ny);
+    }
+    __syncthreads();
+    if (pix >= npix) continue;
+    float best = M<float>::inf(), n[3] = {0.f, 0.f, 0.f};
+    int body = TB_BODY_NONE, face;
+#pragma unroll
+    for (int b = 0; b < 2; ++b) {
+      const float s = ray_box(io.box_c[b], d, face);
+      if (s < best) {
+        best = s; body = b ? TB_BODY_NET : TB_BODY_COURT;
+        n[0] = n[1] = n[2] = 0.f;
+        n[face >> 1] = (face & 1) ? -1.f : 1.f;
+      }
+    }
+    if (kGoal && !ray_skips(s_f + kRfGoal, (float)sc.goal.bound_radius, d, best)) {
+      const float dl[3] = {d[2], d[0], d[1]};
+      const float s = ray_prism(sc.goal, s_gc, s_f[kRfGoalT], dl, face);
+      if (s < best) {
+        best = s; body = TB_BODY_GOAL;
+        if (face < 2) { n[0] = n[1] = 0.f; n[2] = face ? -1.f : 1.f; }
+        else { n[0] = (float)sc.goal.e[face - 2].nx; n[1] = (float)sc.goal.e[face - 2].ny; n[2] = 0.f; }
+      }
+    }
+    if (!ray_skips(s_f + kRfRp, (float)sc.racket.bound_radius, d, best)) {
+      const float *R = s_f + kRfR;
+      float dl[3];
+      matT_vec(R, d, dl);
+      const float s = ray_prism(sc.racket, s_rc, s_f[kRfOt], dl, face);
+      if (s < best) {
+        best = s; body = TB_BODY_RACKET;
+        float nl[3] = {face == 0 ? 1.f : (face == 1 ? -1.f : 0.f), 0.f, 0.f};
+        if (face >= 2) { nl[1] = (float)sc.racket.e[face - 2].nx; nl[2] = (float)sc.racket.e[face - 2].ny; }
+        mat_vec(R, nl, n);
+      }
+    }
+    {
+      const float *c = s_f + kRfBall, r = (float)sc.ball_r;
+      const float s = ray_sphere(c, r, d);
+      if (s < best) {
+        best = s; body = TB_BODY_BALL;
+#pragma unroll
+        for (int k = 0; k < 3; ++k) n[k] = (s * d[k] - c[k]) / r;
+      }
+    }
+    const int64_t o = fr * npix + pix;
+    if (io.depth) io.depth[o] = best;
+    if (io.body) io.body[o] = (uint8_t)body;
+    uint8_t *px_rgb = io.rgb + 3 * o;
+    if (body == TB_BODY_NONE) {
+      const uint8_t sky[3] = TB_RENDER_SKY;
+      px_rgb[0] = sky[0]; px_rgb[1] = sky[1]; px_rgb[2] = sky[2];
+    } else {
+      float nl = n[0] * io.light[0] + n[1] * io.light[1] + n[2] * io.light[2];
+      if (n[0] * d[0] + n[1] * d[1] + n[2] * d[2] > 0.f) nl = -nl;
+      const float k = 0.35f + 0.65f * fmaxf(0.f, nl);
+#pragma unroll
+      for (int ch = 0; ch < 3; ++ch) px_rgb[ch] = (uint8_t)floorf((float)k_render_color[body][ch] * k + 0.5f);
+    }
+  }
+}
+
 // ------------------------------------------------------------------------------------------------ host side
 struct Params {  // order matches k_param_names
   double dt, gravity_z, lin_damping, ang_damping, max_coord_vel, rest_ball_racket, rest_ball_court, rest_ball_goal,
@@ -3298,6 +3423,54 @@ int tb_sac_rollout(tb_ctx *c, int k_steps, int mode, uint64_t noise_seed, const 
       if (launch_step(c, io, s)) return 1;
     }
     return 0;
+  });
+}
+
+int tb_render(tb_ctx *c, const tb_camera *cam, const double *d_states, int64_t count, uint8_t *d_rgb, float *d_depth,
+              uint8_t *d_body, void *stream) {
+  GUARD(c);
+  if (!cam || !d_states || !d_rgb) return fail("tb_render: cam, d_states and d_rgb are required");
+  if (count < 1) return fail("tb_render: count must be >= 1, got %lld", (long long)count);
+  if (cam->struct_size != sizeof(tb_camera)) return fail("tb_render: tb_camera.struct_size mismatch");
+  const int w = cam->width, h = cam->height;
+  if (w < 1 || w > TB_RENDER_MAX_SIZE || h < 1 || h > TB_RENDER_MAX_SIZE)
+    return fail("tb_render: width and height must be in 1 .. %d, got %d x %d", TB_RENDER_MAX_SIZE, w, h);
+  if (!(std::isfinite(cam->fov_y_deg) && cam->fov_y_deg > 0 && cam->fov_y_deg < 180))
+    return fail("tb_render: fov_y_deg must be a finite number in (0, 180), got %g", cam->fov_y_deg);
+  double f[3], r[3], u[3];
+  for (int k = 0; k < 3; ++k) f[k] = cam->target[k] - cam->eye[k];
+  const double fl = std::sqrt(f[0] * f[0] + f[1] * f[1] + f[2] * f[2]);
+  if (!(fl > 0)) return fail("tb_render: eye and target coincide");
+  for (int k = 0; k < 3; ++k) f[k] /= fl;
+  const double *up = cam->up;
+  r[0] = f[1] * up[2] - f[2] * up[1]; r[1] = f[2] * up[0] - f[0] * up[2]; r[2] = f[0] * up[1] - f[1] * up[0];
+  const double rl = std::sqrt(r[0] * r[0] + r[1] * r[1] + r[2] * r[2]), ul = std::sqrt(up[0] * up[0] + up[1] * up[1] + up[2] * up[2]);
+  if (!(rl > 1e-9 * ul) || !(ul > 0)) return fail("tb_render: up is parallel to the view direction");
+  for (int k = 0; k < 3; ++k) r[k] /= rl;
+  u[0] = r[1] * f[2] - r[2] * f[1]; u[1] = r[2] * f[0] - r[0] * f[2]; u[2] = r[0] * f[1] - r[1] * f[0];
+  const int64_t px4 = (int64_t)w * h * 4;  // bytes of the largest output per frame (depth; rgb is 3)
+  if (count > INT64_MAX / px4) return fail("tb_render: %lld frames of %d x %d overflow int64", (long long)count, w, h);
+  if (check_fault(c, "tb_render")) return 1;
+  RenderIO io;
+  std::memset(&io, 0, sizeof io);
+  io.states = d_states; io.count = count; io.rgb = d_rgb; io.depth = d_depth; io.body = d_body; io.width = w; io.height = h;
+  const double t = std::tan(cam->fov_y_deg * (M_PI / 360.0)), light[3] = TB_RENDER_LIGHT;
+  const double ll = std::sqrt(light[0] * light[0] + light[1] * light[1] + light[2] * light[2]);
+  for (int k = 0; k < 3; ++k) {
+    io.eye[k] = cam->eye[k];
+    io.f[k] = (float)f[k]; io.r[k] = (float)(r[k] * t * w / h); io.u[k] = (float)(u[k] * t);
+    io.light[k] = (float)(light[k] / ll);
+  }
+  const double boxes[2][3] = {{TB_FLOOR_HX, TB_FLOOR_HY, TB_FLOOR_HZ}, {TB_NET_HX, TB_NET_HY, TB_NET_HZ}};
+  for (int b = 0; b < 2; ++b)
+    for (int k = 0; k < 3; ++k) {
+      io.box_c[b][2 * k] = (float)(cam->eye[k] - boxes[b][k]);
+      io.box_c[b][2 * k + 1] = (float)(-cam->eye[k] - boxes[b][k]);
+    }
+  const dim3 grid((unsigned)(((int64_t)w * h + kRenderBlock - 1) / kRenderBlock), (unsigned)std::min<int64_t>(count, 65535));
+  return with_env(c, [&](auto &sc, auto *state, auto kind) {
+    using T = std::remove_pointer_t<decltype(state)>;
+    return launch(c, kPlain, render_kernel<T, kind>, grid, kRenderBlock, (cudaStream_t)stream, sc, io);
   });
 }
 

@@ -2,8 +2,9 @@
 
 Mirrors `tennisbot/envs/swingracket_env.py` and `tennisbot/envs/tennisbot_env.py` of the reference: same class
 names, constructor kwargs, spaces, `reset()` -> obs, `step(a)` -> (obs, reward, done, {}), `seed`, `close`,
-`render`, `metadata`, and `TennisbotEnv.set_racket_scale`.  Every number comes from the sm_100a kernel through
-the C ABI; without the compiled library or a B200 the constructor raises.
+`render`, `metadata`, and `TennisbotEnv.set_racket_scale`.  `render("rgb_array")` returns a frame drawn on the device
+(tb_render); `render()` / `render("human")` return None, since there is no GUI.  Every number comes from the sm_100a
+kernel through the C ABI; without the compiled library or a B200 the constructor raises.
 """
 import numpy as np
 
@@ -47,8 +48,15 @@ class _SingleEnv(_EnvBase):
             self._batch.close()
             self._batch = None
 
-    def render(self, mode="human"):
-        return None
+    def render(self, mode="human", camera=None):
+        """mode "rgb_array": uint8 [H, W, 3] of the current state through `camera` (default: render.default_camera of this env,
+        320 x 240), drawn on the device.  Any other mode returns None: the env is headless."""
+        if mode != "rgb_array":
+            return None
+        from .render import default_camera
+
+        rgb, _, _ = self._batch.render(camera or default_camera(self._env_id))
+        return rgb[0].cpu().numpy()
 
     @property
     def step_count(self):

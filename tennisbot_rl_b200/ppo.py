@@ -334,3 +334,15 @@ class HitPPO(GpuPPO):
                 "best_mean_return": max(h["mean_return"] for h in done) if done else None,
                 "wall_s": wall, "rollout_s": self.rollout_s,
                 "rollout_env_steps_per_s": iters * self.K * self.n / max(self.rollout_s, 1e-9), "history": history}
+
+
+def load_sb3_policy_npz(path):
+    """tb_set_policy's parameter vector from an npz of an SB3 MlpPolicy state dict with '.' written as '__' (the layout of
+    tests/golden/ppo_swing_policy.npz: mlp_extractor__policy_net__0__weight, ..., action_net__weight, log_std)."""
+    import numpy as np
+
+    w = np.load(path)
+    t = lambda key: torch.from_numpy(np.ascontiguousarray(w[key], np.float32))  # noqa: E731
+    tower = lambda net: [(t(f"mlp_extractor__{net}__{i}__weight"), t(f"mlp_extractor__{net}__{i}__bias")) for i in (0, 2, 4)]  # noqa: E731
+    return pack_policy(tower("policy_net"), (t("action_net__weight"), t("action_net__bias")), tower("value_net"),
+                       (t("value_net__weight"), t("value_net__bias")), t("log_std"))

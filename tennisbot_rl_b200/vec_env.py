@@ -11,6 +11,9 @@ Contract kept (SB3 1.8, the version recorded in backup_models/ppo_swing.zip):
   the 800 / 1000-step time-outs as terminations (no bootstrap from the terminal value); infos[i]["TimeLimit.truncated"] is
   therefore only emitted on request (report_truncation=True).  infos[i]["events"] always carries the event bits.
 Returned arrays are fresh copies (SB3 keeps `_last_obs` across the next step).
+Frames: get_images() renders every env on the device through the `camera` constructor keyword (default:
+render.default_camera(env_id), 320 x 240) and copies them to the host, so its cost grows with N; render("rgb_array") tiles
+them as SB3's VecEnv.render does, which is what VecVideoRecorder records.
 """
 import time
 
@@ -18,6 +21,7 @@ import numpy as np
 
 from . import _lib
 from .batch import TennisBatch
+from .render import default_camera, tile_images
 from .spaces import spaces_for
 
 try:
@@ -52,7 +56,7 @@ except Exception:
 
 class TennisVecEnv(_VecEnvBase):
     def __init__(self, env_id="SwingRacket-v0", num_envs=4096, device=0, seed=0, precision="f64", env_id_offset=0,
-                 report_truncation=False):
+                 report_truncation=False, camera=None):
         obs_space, act_space = spaces_for(env_id)
         self.report_truncation = bool(report_truncation)
         self._pending_scale = None
@@ -65,7 +69,8 @@ class TennisVecEnv(_VecEnvBase):
         self._ep_len = np.zeros(num_envs, np.int64)
         self._t0 = time.time()
         self.racket_scale = 1.0
-        self.metadata = {"render.modes": ["human"]}
+        self.metadata = {"render.modes": ["human", "rgb_array"]}
+        self.camera = camera or default_camera(env_id)
 
     # ---------------------------------------------------------------- VecEnv API
     def reset(self):
@@ -132,10 +137,16 @@ class TennisVecEnv(_VecEnvBase):
         return [False] * len(self._get_indices(indices))
 
     def get_images(self):
-        return [None] * self.num_envs
+        """N uint8 [H, W, 3] frames of the envs' current states, rendered on the device (one launch for all N) and copied to
+        the host once."""
+        rgb, _, _ = self.batch.render(self.camera)
+        return list(rgb.cpu().numpy())
 
     def render(self, mode="human"):
-        return None
+        """mode "rgb_array": get_images() tiled into one image (SB3's VecEnv.render); "human" returns None (no GUI)."""
+        if mode != "rgb_array":
+            return None
+        return tile_images(self.get_images())
 
     # ---------------------------------------------------------------- reference-specific hooks
     def set_racket_scale(self, scale, apply_now=False):
