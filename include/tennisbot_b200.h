@@ -334,6 +334,33 @@ typedef struct tb_camera {
 int tb_render(tb_ctx *ctx, const tb_camera *cam, const double *d_states, int64_t count, uint8_t *d_rgb, float *d_depth,
               uint8_t *d_body, void *stream);
 
+/* ---- one env step traced substep by substep: what tb_step does to a record, with the record kept after every physics
+ * substep.  SwingRacket-v0's 26th step fast-forwards the ball's whole flight inside one env step; the trace shows it (pass
+ * trace rows to tb_render for frames of the flight).
+ * Bound: a step stops after its first substep when that substep's step counter k (the counter after it) is <= 25 or the env
+ * is done (phase 0); otherwise it runs until a landing or the time-out k > 800, which ends it at k = 801 at the latest.  So a
+ * step that starts from a step counter s0 >= 25 takes at most max(801 - s0, 2) <= 801 - 25 = 776 substeps, and any smaller s0
+ * takes 1.  Tennisbot-v0's step is always one substep. */
+#define TB_TRACE_MAX_SUBSTEPS 776
+int tb_trace_max_substeps(int env_kind); /* TB_TRACE_MAX_SUBSTEPS for SwingRacket-v0, 1 for Tennisbot-v0, -1 unknown; no GPU needed */
+/* d_states double [count, TB_STATE_WORDS]: canonical records from any source (copies: the context's envs are not involved);
+ * d_actions float32 [count, act_dim], the actions as tb_step receives them (clipping to the Box is the caller's job).
+ * d_trace double [max_substeps, count, TB_STATE_WORDS]: [k, i] is record i after substep k + 1.  The step counter advances every
+ * substep; the return and the done bit change at the final substep only, as tb_step leaves them.  Records from substeps up to
+ * max_substeps - 1 repeat the final record, which is the terminal state (no auto-reset: what tb_get_state shows after tb_step
+ * with auto_reset = 0).  A step longer than max_substeps stores its first max_substeps records and still runs to its end.
+ * d_bits uint8 [max_substeps, count] (may be NULL): the contact bits of that substep alone, TB_EV_RACKET_BALL | COURT_BALL |
+ * GOAL_BALL | NET_BALL | RACKET_LOW; 0 in the repeated records.  d_substeps int32 [count]: substeps the step took.
+ * d_reward float32, d_done uint8, d_events uint8, each [count] (may be NULL): what tb_step returns for that record and action
+ * (events: the OR of the substep bits, plus TB_EV_TIMEOUT / TB_EV_BALL_PASSED).  The kernel computes in the context's
+ * precision, reads only its scene parameters and writes nothing of the context.  One kernel launch on `stream`, never
+ * synchronises (capturable in a CUDA graph).  Fails when d_states, d_actions, d_trace or d_substeps is NULL, count < 1,
+ * max_substeps is outside 1 .. tb_trace_max_substeps(env_kind), the context is in TB_CONTROL_PID (its controller memory is
+ * not part of the record), count x max_substeps x 256 bytes overflows int64, or the context is faulted. */
+int tb_trace_step(tb_ctx *ctx, const double *d_states, const float *d_actions, int64_t count, int32_t max_substeps,
+                  double *d_trace, uint8_t *d_bits, int32_t *d_substeps, float *d_reward, uint8_t *d_done,
+                  uint8_t *d_events, void *stream);
+
 /* ---- state dump / injection for the parity harness: double [N, TB_STATE_WORDS] */
 int tb_get_state(tb_ctx *ctx, double *d_state, void *stream);
 int tb_set_state(tb_ctx *ctx, const double *d_state, void *stream);

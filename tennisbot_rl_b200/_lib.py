@@ -29,6 +29,7 @@ RENDER_SKY = (170, 200, 235)                                                    
 RENDER_COLORS = ((0, 0, 0), (70, 140, 95), (235, 235, 235), (215, 60, 50), (40, 80, 200), (225, 240, 60))  # by TB_BODY_*
 RENDER_LIGHT = (-0.3, 0.4, 1.0)                                                        # TB_RENDER_LIGHT, not normalised
 RENDER_MAX_SIZE = 4096
+TRACE_MAX_SUBSTEPS = 776   # TB_TRACE_MAX_SUBSTEPS: substeps of SwingRacket-v0's longest env step (Tennisbot-v0's: 1)
 
 EV_RACKET_BALL, EV_COURT_BALL, EV_GOAL_BALL, EV_TIMEOUT, EV_BALL_PASSED, EV_NET_BALL, EV_RACKET_LOW = 1, 2, 4, 8, 16, 32, 64
 STAT_NAMES = ("episodes", "sum_length", "racket_hits", "goals", "court", "timeouts", "sum_return_q20",
@@ -69,6 +70,7 @@ SIGNATURES = {
     "tb_sac_floats": [_i32], "tb_set_sac_actor": [_vp, _vp, _i64, _vp], "tb_sac_begin": [_vp, _vp],
     "tb_sac_rollout": [_vp, _i32, _i32, _u64, C.POINTER(TbSacRing), _vp, _vp],
     "tb_render": [_vp, C.POINTER(TbCamera), _vp, _i64, _vp, _vp, _vp, _vp],
+    "tb_trace_max_substeps": [_i32], "tb_trace_step": [_vp, _vp, _vp, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
     "tb_get_state": [_vp, _vp, _vp], "tb_set_state": [_vp, _vp, _vp],
     "tb_stats_device_ptr": [_vp, C.POINTER(_vp)], "tb_read_stats": [_vp, _vp, _i32, _vp],
     "tb_reset_host": [_vp, _vp, _vp], "tb_step_host": [_vp, _vp, _vp, _vp, _vp, _vp, _vp],

@@ -289,6 +289,39 @@ class TennisBatch:
                                       self._stream()))
         return rgb, dep, bod
 
+    # ------------------------------------------------------------------ substep trace (tb_trace_step)
+    def trace_step(self, actions, states=None, max_substeps=None):
+        """One env step of canonical state records taken substep by substep, one kernel launch on the current stream; the
+        batch's own envs are not stepped.  actions: float32 [M, act_dim] on this batch's device, as step() receives them
+        (clip them to the Box yourself).  states: None traces every env of this batch from a fresh get_state(); else a
+        float64 [M, 32] tensor on this batch's device.  max_substeps: records kept per env (None: the env's bound,
+        _lib.TRACE_MAX_SUBSTEPS for SwingRacket-v0, 1 for Tennisbot-v0).  Returns device tensors (trace float64 [S, M, 32],
+        bits uint8 [S, M], substeps int32 [M], reward float32 [M], done uint8 [M], events uint8 [M]): trace[k, i] is record i
+        after substep k + 1, padded with the final record; bits are the contacts of that substep alone.  Frames of the
+        flight: render(camera, states=trace[::k].reshape(-1, 32))."""
+        if states is None:
+            states = self.get_state()
+        m = int(states.shape[0]) if states.dim() == 2 else -1
+        if m < 1:
+            raise ValueError(f"trace_step: states must have shape (M >= 1, {_lib.STATE_WORDS}), got {tuple(states.shape)}")
+        need = functools.partial(self._need, "trace_step")
+        need(states, "states", (m, _lib.STATE_WORDS), torch.float64)
+        need(actions, "actions", (m, self.act_dim))
+        bound = self.lib.tb_trace_max_substeps(self.kind)
+        s = bound if max_substeps is None else int(max_substeps)
+        if not 1 <= s <= bound:
+            raise ValueError(f"trace_step: max_substeps must be in 1 .. {bound} for this env, got {s}")
+        dev = self.device
+        trace = torch.empty((s, m, _lib.STATE_WORDS), dtype=torch.float64, device=dev)
+        bits = torch.empty((s, m), dtype=torch.uint8, device=dev)
+        substeps = torch.empty(m, dtype=torch.int32, device=dev)
+        reward = torch.empty(m, dtype=torch.float32, device=dev)
+        done = torch.empty(m, dtype=torch.uint8, device=dev)
+        events = torch.empty(m, dtype=torch.uint8, device=dev)
+        _lib.check(self.lib.tb_trace_step(self.h, _dptr(states), _dptr(actions), m, s, _dptr(trace), _dptr(bits), _dptr(substeps),
+                                          _dptr(reward), _dptr(done), _dptr(events), self._stream()))
+        return trace, bits, substeps, reward, done, events
+
     def get_state(self):
         s = torch.empty((self.num_envs, _lib.STATE_WORDS), dtype=torch.float64, device=self.device)
         _lib.check(self.lib.tb_get_state(self.h, _dptr(s), self._stream()))

@@ -973,8 +973,10 @@ struct StepCtl {
 // One physics substep of the env step in flight plus the env logic that follows it.  Returns true when the
 // env step is complete (reward / done / events are final).
 // pid: this env's controller memory when the context runs TB_CONTROL_PID, else nullptr.
+// bits_out: receives the contact bits physics_step / hit_physics returned for this substep alone (trace_kernel), or nullptr.
 template <typename T, int KIND>
-__device__ __forceinline__ bool env_substep(const Scene<T> &sc, St<T> &s, const float *a, StepCtl &c, T *pid = nullptr) {
+__device__ __forceinline__ bool env_substep(const Scene<T> &sc, St<T> &s, const float *a, StepCtl &c, T *pid = nullptr,
+                                            int *bits_out = nullptr) {
   T zero[3] = {0, 0, 0};
   if (KIND == TB_ENV_SWING) {
     T F[3], Tq[3] = {0, 0, 0};
@@ -994,6 +996,7 @@ __device__ __forceinline__ bool env_substep(const Scene<T> &sc, St<T> &s, const 
       F[2] = -2 * (s.rp[2] - s.aux[2] - 4);
     }
     int bits = physics_step<T, true>(sc, s, F, Tq, zero);
+    if (bits_out) *bits_out = bits;
     int k = ++s.step;
     c.events |= bits;
     if (c.phase == 0) {
@@ -1017,6 +1020,7 @@ __device__ __forceinline__ bool env_substep(const Scene<T> &sc, St<T> &s, const 
     T Fb[3] = {0, 0, 0};
     if (s.step >= sc.shoot_start && s.step < sc.shoot_start + sc.shoot_frames) { Fb[0] = s.aux[0]; Fb[1] = s.aux[1]; Fb[2] = s.aux[2]; }
     int bits = hit_physics<T>(sc, s, F, Fb);
+    if (bits_out) *bits_out = bits;
     int k = ++s.step;
     c.events = bits;
     if (k < sc.shoot_frames) { c.done = false; return true; }  // returns False regardless of self.done (tennisbot_env.py:138-139)

@@ -2132,14 +2132,8 @@ template <typename T> __global__ void materialise_kernel(const __grid_constant__
   base[((int64_t)7 * n + i) * 4 + 2] = int_as(T(), flags & ~kStPristine);
 }
 
-// canonical double [N, 32] record <-> packed state
-template <typename T> __global__ void get_state_kernel(const __grid_constant__ Scene<T> sc, const T *base, int64_t n, double *out) {
-  int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  St<T> s;
-  load_state(base, n, i, s);
-  materialise_ball(sc, s);
-  double *o = out + i * TB_STATE_WORDS;
+// canonical double [TB_STATE_WORDS] record <-> St<T> (a materialised state: no kStPristine, no stale pack 4)
+template <typename T> __device__ __forceinline__ void state_to_record(const St<T> &s, double *o) {
   for (int j = 0; j < 3; ++j) {
     o[TB_S_RACKET_POS + j] = s.rp[j]; o[TB_S_RACKET_VEL + j] = s.rv[j]; o[TB_S_RACKET_ANGVEL + j] = s.rw[j];
     o[TB_S_BALL_POS + j] = s.bp[j]; o[TB_S_BALL_VEL + j] = s.bv[j]; o[TB_S_BALL_ANGVEL + j] = s.bw[j];
@@ -2149,11 +2143,7 @@ template <typename T> __global__ void get_state_kernel(const __grid_constant__ S
   o[TB_S_GOAL] = s.goal[0]; o[TB_S_GOAL + 1] = s.goal[1]; o[TB_S_D0] = s.d0; o[TB_S_RETURN] = s.ret;
   o[TB_S_STEP] = s.step; o[TB_S_FLAGS] = s.flags & kFlagDone; o[TB_S_EPISODE] = (double)(int32_t)s.episode;
 }
-template <typename T> __global__ void set_state_kernel(T *base, int64_t n, const double *in) {
-  int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  St<T> s;
-  const double *o = in + i * TB_STATE_WORDS;
+template <typename T> __device__ __forceinline__ void record_to_state(const double *o, St<T> &s) {
   for (int j = 0; j < 3; ++j) {
     s.rp[j] = (T)o[TB_S_RACKET_POS + j]; s.rv[j] = (T)o[TB_S_RACKET_VEL + j]; s.rw[j] = (T)o[TB_S_RACKET_ANGVEL + j];
     s.bp[j] = (T)o[TB_S_BALL_POS + j]; s.bv[j] = (T)o[TB_S_BALL_VEL + j]; s.bw[j] = (T)o[TB_S_BALL_ANGVEL + j];
@@ -2162,7 +2152,85 @@ template <typename T> __global__ void set_state_kernel(T *base, int64_t n, const
   for (int j = 0; j < 4; ++j) s.rq[j] = (T)o[TB_S_RACKET_QUAT + j];
   s.goal[0] = (T)o[TB_S_GOAL]; s.goal[1] = (T)o[TB_S_GOAL + 1]; s.d0 = (T)o[TB_S_D0]; s.ret = (T)o[TB_S_RETURN];
   s.step = (int)o[TB_S_STEP]; s.flags = (int)o[TB_S_FLAGS] & kFlagDone; s.episode = (uint32_t)(int32_t)o[TB_S_EPISODE];
+}
+
+// canonical double [N, 32] record <-> packed state
+template <typename T> __global__ void get_state_kernel(const __grid_constant__ Scene<T> sc, const T *base, int64_t n, double *out) {
+  int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  St<T> s;
+  load_state(base, n, i, s);
+  materialise_ball(sc, s);
+  state_to_record(s, out + i * TB_STATE_WORDS);
+}
+template <typename T> __global__ void set_state_kernel(T *base, int64_t n, const double *in) {
+  int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  St<T> s;
+  record_to_state(in + i * TB_STATE_WORDS, s);
   store_state(base, n, i, s);
+}
+
+// ------------------------------------------------------------------------------------------------ tb_trace_step
+// One thread per traced record: the record's env step taken as rollout_kernel takes it (env_substep until the step is
+// complete), with the canonical record stored after every substep.  A trace is a diagnostic of a few envs, not a
+// throughput path: a lane runs its flight alone, so a warp takes as long as its longest flight.
+struct TraceIO {
+  const double *states;
+  const float *actions;
+  int64_t count;
+  int max_substeps;
+  double *trace;  // [max_substeps, count, TB_STATE_WORDS]
+  uint8_t *bits;  // [max_substeps, count] or nullptr
+  int32_t *substeps;
+  float *reward;
+  uint8_t *done, *events;
+};
+constexpr int kTraceBlock = 128;
+__device__ __forceinline__ void store_record(double *dst, const double *r) {
+  double2 *p = reinterpret_cast<double2 *>(dst);
+#pragma unroll
+  for (int j = 0; j < TB_STATE_WORDS / 2; ++j) p[j] = make_double2(r[2 * j], r[2 * j + 1]);
+}
+
+template <typename T, int KIND>
+__global__ void __launch_bounds__(kTraceBlock) trace_kernel(const __grid_constant__ Scene<T> sc, const __grid_constant__ TraceIO io) {
+  const int64_t i = (int64_t)blockIdx.x * kTraceBlock + threadIdx.x;
+  if (i >= io.count) return;
+  St<T> s;
+  record_to_state(io.states + i * TB_STATE_WORDS, s);
+  float a[8];
+  load_action<KIND>(io.actions, i, a);
+  StepCtl c = {0, 0, 0, 0.0f, false};
+  c.done = s.flags & kFlagDone;
+  double r[TB_STATE_WORDS];
+  int k = 0;
+  bool fin = false;
+#pragma unroll 1
+  while (!fin) {
+    int bits = 0;
+    fin = env_substep<T, KIND>(sc, s, a, c, nullptr, &bits);
+    if (fin) {
+      s.ret += (T)c.reward;
+      if (c.done) s.flags |= kFlagDone;
+    }
+    if (k < io.max_substeps) {  // a longer step still runs to its end: substeps, reward, done and events stay complete
+      state_to_record(s, r);
+      store_record(io.trace + ((int64_t)k * io.count + i) * TB_STATE_WORDS, r);
+      if (io.bits) io.bits[(int64_t)k * io.count + i] = (uint8_t)bits;
+    }
+    ++k;
+  }
+  // the rest of the block repeats the final record (r holds it whenever k < max_substeps)
+#pragma unroll 1
+  for (int j = k; j < io.max_substeps; ++j) {
+    store_record(io.trace + ((int64_t)j * io.count + i) * TB_STATE_WORDS, r);
+    if (io.bits) io.bits[(int64_t)j * io.count + i] = 0;
+  }
+  io.substeps[i] = k;
+  if (io.reward) io.reward[i] = c.reward;
+  if (io.done) io.done[i] = c.done ? 1 : 0;
+  if (io.events) io.events[i] = (uint8_t)c.events;
 }
 
 // ------------------------------------------------------------------------------------------------ tb_render
@@ -3471,6 +3539,35 @@ int tb_render(tb_ctx *c, const tb_camera *cam, const double *d_states, int64_t c
   return with_env(c, [&](auto &sc, auto *state, auto kind) {
     using T = std::remove_pointer_t<decltype(state)>;
     return launch(c, kPlain, render_kernel<T, kind>, grid, kRenderBlock, (cudaStream_t)stream, sc, io);
+  });
+}
+
+int tb_trace_max_substeps(int env_kind) {
+  return with_kind(env_kind, [](auto kind) { return kind == TB_ENV_SWING ? TB_TRACE_MAX_SUBSTEPS : 1; });
+}
+
+int tb_trace_step(tb_ctx *c, const double *d_states, const float *d_actions, int64_t count, int32_t max_substeps,
+                  double *d_trace, uint8_t *d_bits, int32_t *d_substeps, float *d_reward, uint8_t *d_done,
+                  uint8_t *d_events, void *stream) {
+  GUARD(c);
+  if (!d_states || !d_actions || !d_trace || !d_substeps)
+    return fail("tb_trace_step: d_states, d_actions, d_trace and d_substeps are required");
+  if (count < 1) return fail("tb_trace_step: count must be >= 1, got %lld", (long long)count);
+  const int bound = tb_trace_max_substeps(c->cfg.env_kind);
+  if (max_substeps < 1 || max_substeps > bound)
+    return fail("tb_trace_step: max_substeps must be in 1 .. %d for this env, got %d", bound, (int)max_substeps);
+  if (c->control_mode == TB_CONTROL_PID)
+    return fail("tb_trace_step: TB_CONTROL_PID contexts cannot be traced (the controller memory is not part of the record)");
+  const int64_t rec = (int64_t)max_substeps * TB_STATE_WORDS * (int64_t)sizeof(double);  // bytes of one record's trace
+  if (count > INT64_MAX / rec) return fail("tb_trace_step: %lld records x %d substeps overflow int64", (long long)count, (int)max_substeps);
+  if (check_fault(c, "tb_trace_step")) return 1;
+  TraceIO io;
+  std::memset(&io, 0, sizeof io);
+  io.states = d_states; io.actions = d_actions; io.count = count; io.max_substeps = max_substeps; io.trace = d_trace;
+  io.bits = d_bits; io.substeps = d_substeps; io.reward = d_reward; io.done = d_done; io.events = d_events;
+  return with_env(c, [&](auto &sc, auto *state, auto kind) {
+    using T = std::remove_pointer_t<decltype(state)>;
+    return launch(c, kPlain, trace_kernel<T, kind>, grid_for(count, kTraceBlock), kTraceBlock, (cudaStream_t)stream, sc, io);
   });
 }
 

@@ -4,9 +4,12 @@
 Action sources: uniform random (default); the scripted ball tracker (--tracker, Tennisbot-v0); or a policy in tb_set_policy's
 layout, rolled by tb_policy_rollout with K = 1 (--policy: a .npy flat vector, or an .npz of an SB3 MlpPolicy state dict such
 as the reference's trained policy tests/golden/ppo_swing_policy.npz).  Frames exist per env step: a SwingRacket-v0 episode is
-26 frames, and its 26th step fast-forwards the ball's whole flight, which is not drawn.
+26 frames, and its 26th step fast-forwards the ball's whole flight (about 106 physics substeps, at most 776).  With
+--flight-every K that step is also traced substep by substep (tb_trace_step, from the states saved before it and the actions
+it took), and every K-th flight substep plus the last is drawn between frame 25 and the episode's final frame.
 
   python tools/record_episode.py SwingRacket-v0 --policy tests/golden/ppo_swing_policy.npz --out frames/swing
+  python tools/record_episode.py SwingRacket-v0 --policy tests/golden/ppo_swing_policy.npz --flight-every 4 --out frames/shot
   python tools/record_episode.py Tennisbot-v0 --tracker --out frames/hit
 """
 import argparse
@@ -62,7 +65,11 @@ def main():
     ap.add_argument("--racket-scale", type=float, default=1.0)
     ap.add_argument("--out", type=Path, default=Path("frames"))
     ap.add_argument("--sheet-every", type=int, default=0, help="contact sheet: every k-th frame (0: about 13 rows)")
+    ap.add_argument("--flight-every", type=int, default=0,
+                    help="SwingRacket-v0: also draw every k-th substep of the ball's flight in the 26th step (0: none)")
     a = ap.parse_args()
+    if a.flight_every < 0:
+        ap.error("--flight-every must be >= 0")
     if a.tracker and a.env_id != "Tennisbot-v0":
         ap.error("--tracker is Tennisbot-v0's scripted tracker")
     if a.tracker and a.policy:
@@ -76,31 +83,42 @@ def main():
     cam = default_camera(a.env_id, a.width, a.height)
     per_episode = SWING_STEPS if swing else a.steps
     T = a.episodes * per_episode
-    frames = torch.empty((T + a.episodes, m, a.height, a.width, 3), dtype=torch.uint8, device=b.device)
+    frames = []  # device frames [M, H, W, 3], copied to the host together at the end
     obs = torch.zeros((1, m, b.obs_dim), device=b.device)
     if a.policy:
         b.set_policy(load_policy(a.policy).to(b.device))
         rew, done = torch.zeros((1, m), device=b.device), torch.zeros((1, m), dtype=torch.uint8, device=b.device)
         last = torch.zeros((m, b.obs_dim), device=b.device)
+        act = torch.zeros((1, m, b.act_dim), device=b.device)
     gen = torch.Generator(b.device).manual_seed(a.seed)
-    f = 0
+    flight_frames = 0
     for t in range(T):
         if t == 0 or (swing and t % per_episode == 0):  # a new episode: its first frame is the placement
             obs[0].copy_(b.reset())
-            frames[f] = b.render(cam)[0]
-            f += 1
+            frames.append(b.render(cam)[0])
+        flight = swing and a.flight_every > 0 and t % per_episode == per_episode - 1
+        if flight:
+            before = b.get_state()
         if a.policy:
-            b.policy_rollout(obs, rew, done, last, deterministic=not a.stochastic, noise_seed=a.seed)
+            b.policy_rollout(obs, rew, done, last, actions=act, deterministic=not a.stochastic, noise_seed=a.seed)
             obs[0].copy_(last)
+            taken = act[0].clamp(-1, 1)  # policy_rollout returns the unclipped action; the env step took it clipped
         elif a.tracker:
             b.rollout(1, _lib.ACT_TRACK)
         else:
-            b.step(torch.empty((m, b.act_dim), device=b.device).uniform_(-1, 1, generator=gen))
-        frames[f] = b.render(cam)[0]
-        f += 1
+            taken = torch.empty((m, b.act_dim), device=b.device).uniform_(-1, 1, generator=gen)
+            b.step(taken)
+        if flight:  # the flight inside this step: every k-th substep and the last (the landed ball, = the frame below)
+            trace, _, substeps = b.trace_step(taken, before)[:3]
+            last_k = int(substeps.max()) - 1
+            ks = list(range(a.flight_every - 1, last_k, a.flight_every)) + [last_k]
+            frames.extend(b.render(cam, trace[ks].reshape(-1, _lib.STATE_WORDS))[0].reshape(len(ks), m, a.height, a.width, 3))
+            flight_frames += len(ks)
+        frames.append(b.render(cam)[0])
     stats = b.read_stats()
     hits = int(stats[_lib.STAT_NAMES.index("racket_hits")])
-    host = frames[:f].cpu().numpy()  # the one copy to the host
+    host = torch.stack(frames).cpu().numpy()  # the one copy to the host
+    f = len(host)
     a.out.mkdir(parents=True, exist_ok=True)
     for t in range(f):
         for i in range(m):
@@ -111,7 +129,8 @@ def main():
     src = "policy " + str(a.policy) if a.policy else ("tracker" if a.tracker else "uniform random")
     print(f"{a.env_id}: {m} envs x {T} env steps ({src}), {f} frames of {a.width}x{a.height} each -> {a.out}/; "
           f"rewarded racket-ball contact steps {hits}, episodes {int(stats[0])}, "
-          f"mean return {stats[6] / 2 ** 20 / max(int(stats[0]), 1):.3f}; contact sheet: every {every} frames, one env per column")
+          f"mean return {stats[6] / 2 ** 20 / max(int(stats[0]), 1):.3f}; contact sheet: every {every} frames, one env per column"
+          + (f"; {flight_frames} of the frames show flight substeps" if flight_frames else ""))
     b.close()
 
 
