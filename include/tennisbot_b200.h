@@ -178,6 +178,50 @@ int tb_policy_rollout(tb_ctx *ctx, int k_steps, int deterministic, uint64_t nois
                       float *d_logp, float *d_value, float *d_reward, uint8_t *d_done, float *d_last_obs,
                       float *d_last_value, void *stream);
 
+/* ---- observation and reward normalisation of the policy rollout: SB3 1.8 VecNormalize, on the device.
+ * Statistics, float64, RunningMeanStd layout: obs mean [obs_dim], obs var [obs_dim], obs count, ret mean, ret var, ret count
+ * (TB_VECNORM_WORDS doubles); fresh: means 0, variances 1, counts 1e-4 (RunningMeanStd(epsilon=1e-4)).  Per-env discounted
+ * returns, float64 [N], belong to the context and are not part of the record (SB3 drops `returns` when it pickles).
+ * An update with the N envs' values of a batch (population variance b_var, mean b_mean, count N) is Chan's merge, as
+ * RunningMeanStd.update_from_moments: delta = b_mean - mean, tot = count + N, mean += delta N / tot,
+ * var = (var count + b_var N + delta^2 count N / tot) / tot, count = tot.  The batch moments are formed in float64 from the
+ * float32 values in a fixed reduction order (the ES normaliser's pairwise merges); SB3's np.mean of a float32 array sums in
+ * float32, so the library deliberately differs from SB3 in that rounding.
+ * With a normaliser attached, env step t of tb_policy_rollout (raw observation o_t, action, raw r_t, done_t, raw o_{t+1}):
+ *   1. training && norm_obs: fold o_{t+1} of all N envs (an auto-reset env's reset observation included) into the obs stats;
+ *   2. training: returns = returns * gamma + r_t, folded into the return stats;
+ *   3. r^_t = clip(r_t / sqrt(ret_var + epsilon), +-clip_reward) if norm_reward, else r_t; then returns[done_t] = 0;
+ *   4. o^ = clip((o - obs_mean) / sqrt(obs_var + epsilon), +-clip_obs) if norm_obs, else o: float64 with every operation
+ *      rounded (no contraction), rounded once to float32, so numpy float64 on the same statistics reproduces it bit for bit.
+ *      The policy acts on o^ (and the value is that of o^).
+ * The first rollout after tb_set_vecnorm, or after a tb_reset / tb_reset_from of all envs (mask NULL), first folds its
+ * d_obs[0] (SB3's reset() does); those calls zero the returns, a masked reset zeroes the returns of the envs it resets and
+ * folds nothing.  training = 0: the statistics and returns never change (deployment).
+ * tb_policy_rollout's buffers change meaning with a normaliser only: d_obs[0] holds the RAW current observation on entry;
+ * on return d_obs[t] holds the normalised observation step t acted on (t = 0 included), d_reward[t] = r^_t, d_last_obs the
+ * RAW observation after the last step (the next call's d_obs[0]) and d_last_value the value of its normalised form.
+ * Kernel launches of tb_policy_rollout with a normaliser: K (3 + s) + 3 when training (an entry pass of 2 launches that folds
+ * d_obs[0] when armed, and two statistics launches after each step), K (1 + s) + 2 when not; s = 2 for SwingRacket-v0 and 1 for
+ * Tennisbot-v0 (tb_step's launches), and the last launch (bootstrap value, last normalised reward) always runs.  tb_reset /
+ * tb_reset_from add one launch while a training normaliser is attached.  The int64 statistics (tb_read_stats) stay raw;
+ * tb_step, tb_rollout, tb_reset_host, tb_step_host and the ES and SAC entry points ignore the normaliser.  Each context keeps its
+ * own statistics: shards with env_id_offset do not reproduce the statistics of one batch. */
+typedef struct tb_vecnorm {
+  uint32_t struct_size; /* sizeof(tb_vecnorm) */
+  int32_t training, norm_obs, norm_reward;
+  double clip_obs, clip_reward, gamma, epsilon; /* SB3's defaults: 10, 10, 0.99, 1e-8 */
+} tb_vecnorm;
+#define TB_VECNORM_WORDS(obs_dim) (2 * (obs_dim) + 4) /* obs mean, obs var, obs count, ret mean, ret var, ret count */
+/* Attach (cfg) or detach (cfg NULL) the normaliser.  d_stats double [TB_VECNORM_WORDS(obs_dim)]: the record to start from (NULL:
+ * fresh); the call copies it to the host and checks it, so with d_stats it synchronises `stream`; otherwise it is one kernel
+ * launch and never synchronises.  Zeroes the returns and arms the reset fold.  Fails on a wrong struct_size, clip_obs or
+ * clip_reward or epsilon that is not finite and above 0, gamma outside [0, 1], stats with a count <= 0, a variance < 0 or an
+ * entry that is not finite, and on a faulted context.  Detaching keeps the buffers; attaching again starts from d_stats. */
+int tb_set_vecnorm(tb_ctx *ctx, const tb_vecnorm *cfg, const double *d_stats, void *stream);
+/* d_stats double [TB_VECNORM_WORDS(obs_dim)] = the current record (stream-ordered copy, never synchronises).  Fails when no
+ * normaliser is attached. */
+int tb_get_vecnorm(tb_ctx *ctx, double *d_stats, void *stream);
+
 /* ---- ES fitness rollout (SURVEY 8(f)-2): fitness_static (fitness_functions.py:18-158) for a whole population in one context.
  * Env i evaluates individual i / (N / individuals) with the reference's GatedCNN (policies.py:59-128) on an 8-step history of
  * observations, each normalised by the env's own float64 running normaliser (evolution_strategy_static.py:25-44); the

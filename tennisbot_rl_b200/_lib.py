@@ -45,6 +45,16 @@ class TbCamera(C.Structure):
                 ("eye", C.c_double * 3), ("target", C.c_double * 3), ("up", C.c_double * 3), ("fov_y_deg", C.c_double)]
 
 
+class TbVecNorm(C.Structure):
+    _fields_ = [("struct_size", C.c_uint32), ("training", C.c_int32), ("norm_obs", C.c_int32), ("norm_reward", C.c_int32),
+                ("clip_obs", C.c_double), ("clip_reward", C.c_double), ("gamma", C.c_double), ("epsilon", C.c_double)]
+
+
+def vecnorm_words(obs_dim):
+    """TB_VECNORM_WORDS: obs mean [obs_dim], obs var [obs_dim], obs count, ret mean, ret var, ret count."""
+    return 2 * obs_dim + 4
+
+
 class TbConfig(C.Structure):
     _fields_ = [("struct_size", C.c_uint32), ("env_kind", C.c_int32), ("precision", C.c_int32), ("device", C.c_int32),
                 ("num_envs", C.c_int64), ("env_id_offset", C.c_int64), ("seed", C.c_uint64),
@@ -64,6 +74,7 @@ SIGNATURES = {
     "tb_step": [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp], "tb_rollout": [_vp, _i32, _i32, _vp, _vp, _vp, _vp],
     "tb_set_policy": [_vp, _vp, _i64, _vp],
     "tb_policy_rollout": [_vp, _i32, _i32, _u64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
+    "tb_set_vecnorm": [_vp, C.POINTER(TbVecNorm), _vp, _vp], "tb_get_vecnorm": [_vp, _vp, _vp],
     "tb_es_begin": [_vp, _vp, _i64, _i64, _vp, _vp], "tb_es_rollout": [_vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
     "tb_es_begin_noise": [_vp, _vp, _i64, _i64, C.c_float, _u64, _u32, _vp, _vp],
     "tb_es_noise_combine": [_vp, _vp, _vp, _i64, _u64, _u32, _vp, _vp], "tb_es_normalizer_stats": [_vp, _vp, _vp],

@@ -161,6 +161,29 @@ class TennisBatch:
                                               _dptr(actions), _dptr(logp), _dptr(value), _dptr(reward), _dptr(done), _dptr(last_obs),
                                               _dptr(last_value), self._stream()))
 
+    # ------------------------------------------------------------------ normaliser of the policy rollout (tb_set_vecnorm)
+    def set_vecnorm(self, training=True, norm_obs=True, norm_reward=True, clip_obs=10.0, clip_reward=10.0, gamma=0.99,
+                    epsilon=1e-8, stats=None):
+        """Attach SB3 VecNormalize's observation / reward normalisation to policy_rollout (semantics in the header at
+        tb_set_vecnorm).  stats: float64 [2 obs_dim + 4] to start from (obs mean, obs var, obs count, ret mean, ret var, ret
+        count), None = fresh; a given record is checked on the host, which synchronises the stream."""
+        self._need("set_vecnorm", stats, "stats", (_lib.vecnorm_words(self.obs_dim),), torch.float64, optional=True)
+        cfg = _lib.TbVecNorm(C.sizeof(_lib.TbVecNorm), int(bool(training)), int(bool(norm_obs)), int(bool(norm_reward)),
+                             float(clip_obs), float(clip_reward), float(gamma), float(epsilon))
+        _lib.check(self.lib.tb_set_vecnorm(self.h, C.byref(cfg), _dptr(stats), self._stream()))
+
+    def clear_vecnorm(self):
+        """Detach the normaliser: policy_rollout behaves as if none had been attached."""
+        _lib.check(self.lib.tb_set_vecnorm(self.h, None, None, self._stream()))
+
+    def vecnorm_stats(self, out=None):
+        """float64 device tensor [2 obs_dim + 4]: the normaliser's current record (stream-ordered copy)."""
+        if out is None:
+            out = torch.empty(_lib.vecnorm_words(self.obs_dim), dtype=torch.float64, device=self.device)
+        self._need("vecnorm_stats", out, "out", (_lib.vecnorm_words(self.obs_dim),), torch.float64)
+        _lib.check(self.lib.tb_get_vecnorm(self.h, _dptr(out), self._stream()))
+        return out
+
     # ------------------------------------------------------------------ ES fitness rollout (tb_es_begin / tb_es_rollout)
     def es_begin(self, weights, normalizer=None):
         """Start an ES generation: weights float32 [individuals, es_floats] (individuals divides num_envs; env i evaluates

@@ -1376,16 +1376,29 @@ struct PolicyIO {
   const unsigned *tick;    // device word that advances with every env step (StepIO::epoch[0] for SwingRacket-v0, epoch[2]
                            // for Tennisbot-v0): a rollout captured in a CUDA graph draws fresh noise on every replay
   int deterministic;       // 1: act_raw = mean (validate_swing.py's predict(deterministic=True) counterpart)
+  // NORM instances only (VecNormalize, header tb_set_vecnorm): obs holds RAW rows, which both towers normalise in registers
+  const double *vn_stats;  // the running record, TB_VECNORM_WORDS(OBS) doubles
+  float *vn_obs;           // [N, OBS] receives the normalised row (policy tower), may be nullptr
+  float *vn_reward;        // [N] the previous step's raw reward, replaced by its normalised value (policy tower), may be nullptr
+  double vn_clip_obs, vn_clip_reward, vn_eps;
+  int vn_norm_obs, vn_norm_reward;
 };
-// grid (ceil(N / 128), 2): blockIdx.y = 0 the policy tower (action, log-density), 1 the value tower
-template <int OBS, int ACT>
+// VecNormalize's two formulas in float64 with each operation rounded (no contraction), so that numpy reproduces them bit for
+// bit: clip((o - mean) / sqrt(var + eps), -clip, clip), and the same for a reward with mean 0
+__device__ __forceinline__ float vn_apply(float v, double mean, double var, double eps, double clip) {
+  const double d = __ddiv_rn(__dsub_rn((double)v, mean), __dsqrt_rn(__dadd_rn(var, eps)));
+  return __double2float_rn(fmin(fmax(d, -clip), clip));
+}
+// grid (ceil(N / 128), 2): blockIdx.y = 0 the policy tower (action, log-density), 1 the value tower.  NORM: the normalising
+// instance of tb_policy_rollout with a normaliser attached; the policy tower also writes vn_obs and vn_reward.
+template <int OBS, int ACT, bool NORM>
 __global__ void __launch_bounds__(kBlock) policy_kernel(const __grid_constant__ PolicyIO io) {
   using L = PolLayout<OBS, ACT>;
   static_assert(OBS % 2 == 0 && ACT % 2 == 0, "observation rows are read as float2 / float4, actions written as float2");
   __shared__ __align__(16) float P[L::PiTower + pad4(ACT)];
   const bool vf = blockIdx.y != 0;
   pdl_wait();
-  if (vf ? io.value == nullptr : (!io.act_raw && !io.act_env && !io.logp)) return;
+  if (vf ? io.value == nullptr : (!io.act_raw && !io.act_env && !io.logp) && !(NORM && (io.vn_obs || io.vn_reward))) return;
   {
     const float4 *src = reinterpret_cast<const float4 *>(io.params + (vf ? L::PiTower : 0));
     const int nv = (vf ? L::VfTower : L::PiTower) / 4;
@@ -1408,6 +1421,20 @@ __global__ void __launch_bounds__(kBlock) policy_kernel(const __grid_constant__ 
         const float2 a = reinterpret_cast<const float2 *>(io.obs + me * OBS)[j];
         x[2 * j] = a.x; x[2 * j + 1] = a.y;
       }
+    }
+    if (NORM) {
+      if (io.vn_norm_obs) {
+#pragma unroll
+        for (int c = 0; c < OBS; ++c) x[c] = vn_apply(x[c], io.vn_stats[c], io.vn_stats[OBS + c], io.vn_eps, io.vn_clip_obs);
+      }
+      if (!vf && io.vn_obs) {
+        float2 *q = reinterpret_cast<float2 *>(io.vn_obs + me * OBS);
+#pragma unroll
+        for (int j = 0; j < OBS / 2; ++j) q[j] = make_float2(x[2 * j], x[2 * j + 1]);
+      }
+      if (!vf && io.vn_reward && io.vn_norm_reward)
+        io.vn_reward[me] = vn_apply(io.vn_reward[me], 0.0, io.vn_stats[2 * OBS + 2], io.vn_eps, io.vn_clip_reward);
+      if (!vf && !io.act_raw && !io.act_env && !io.logp) return;  // the last launch: normalised reward only
     }
     float h[32];
     tower<OBS, ACT>(P, x, h);
@@ -1811,6 +1838,109 @@ __global__ void __launch_bounds__(kBlock) es_norm_final_kernel(const double *par
   }
   v = es_merge_cta(v);
   if (threadIdx.x == 0) { out[c] = v.n; out[obs + c] = m0[obs + c] + v.d; out[2 * obs + c] = v.m2; }
+}
+
+// ------------------------------------------------------------------------------------------------ VecNormalize (policy rollout)
+// SB3 VecNormalize's running statistics (header tb_set_vecnorm), folded on the device after every env step of
+// tb_policy_rollout in two launches: vecnorm_partial_kernel forms per-CTA moments of the N envs' observations (one channel
+// each) and of their discounted returns, in the fixed order of es_norm_partial_kernel (kEsStatsPer envs per thread in order,
+// then es_merge_cta); vecnorm_final_kernel merges the partials in one CTA and updates the record in place.  The moments are
+// kept as offsets from the record's current mean, so the batch's delta of Chan's update is the merged offset itself.
+struct VecNormIO {
+  double *stats;           // the running record, TB_VECNORM_WORDS(OBS) doubles
+  double *ret;             // [N] discounted returns
+  const float *obs;        // [N, OBS] raw observations to fold
+  float *copy;             // entry pass: obs is copied here (the library's raw buffer); else nullptr
+  const float *reward;     // [N] the step's raw reward; nullptr = entry pass (obs only, and only while *armed)
+  const uint8_t *done;     // [N] the step's done flags (step pass)
+  double *part;            // [blocks][OBS + 1][3] per-CTA (count, mean offset, M2)
+  uint8_t *armed;          // 1 until the entry pass after tb_set_vecnorm / a full reset has folded its observation
+  int64_t n;
+  double gamma;
+  int fold_obs;            // training && norm_obs
+};
+template <int OBS>
+__global__ void __launch_bounds__(kBlock) vecnorm_partial_kernel(const __grid_constant__ VecNormIO io) {
+  const int64_t n = io.n, e0 = (int64_t)blockIdx.x * kBlock * kEsStatsPer + threadIdx.x;
+  const bool fold_obs = io.fold_obs && (io.reward || *io.armed), fold_ret = io.reward != nullptr;
+  double m0[OBS + 1];
+  EsMoments v[OBS + 1];
+#pragma unroll
+  for (int c = 0; c <= OBS; ++c) { m0[c] = io.stats[c < OBS ? c : 2 * OBS + 1]; v[c] = {0.0, 0.0, 0.0}; }
+  for (int r = 0; r < kEsStatsPer; ++r) {
+    const int64_t e = e0 + (int64_t)r * kBlock;
+    if (e >= n) break;
+    float x[OBS];
+#pragma unroll
+    for (int j = 0; j < OBS / 2; ++j) {
+      const float2 a = reinterpret_cast<const float2 *>(io.obs + e * OBS)[j];
+      x[2 * j] = a.x; x[2 * j + 1] = a.y;
+      if (io.copy) reinterpret_cast<float2 *>(io.copy + e * OBS)[j] = a;
+    }
+    if (fold_obs) {
+#pragma unroll
+      for (int c = 0; c < OBS; ++c) v[c] = es_merge(v[c], {1.0, __dsub_rn((double)x[c], m0[c]), 0.0});
+    }
+    if (fold_ret) {  // returns = returns * gamma + reward, folded; then returns[done] = 0
+      const double R = __dadd_rn(__dmul_rn(io.ret[e], io.gamma), (double)io.reward[e]);
+      v[OBS] = es_merge(v[OBS], {1.0, __dsub_rn(R, m0[OBS]), 0.0});
+      io.ret[e] = io.done[e] ? 0.0 : R;
+    }
+  }
+  double *p = io.part + (int64_t)blockIdx.x * (OBS + 1) * 3;
+#pragma unroll
+  for (int c = 0; c <= OBS; ++c) {
+    if (c < OBS ? !fold_obs : !fold_ret) continue;  // (uniform over the CTA)
+    const EsMoments s = es_merge_cta(v[c]);
+    if (threadIdx.x == 0) { p[3 * c] = s.n; p[3 * c + 1] = s.d; p[3 * c + 2] = s.m2; }
+  }
+}
+// One CTA: merge the `blocks` partials of each channel (each thread a strided subset in order, then the fixed tree) and apply
+// RunningMeanStd.update_from_moments with batch mean = mean + d, batch variance M2 / N, batch count N:
+//   tot = count + N, mean += d N / tot, var = (var count + M2 / N N + d^2 count N / tot) / tot, count = tot.
+template <int OBS>
+__global__ void __launch_bounds__(kBlock) vecnorm_final_kernel(const __grid_constant__ VecNormIO io, int64_t blocks) {
+  const bool fold_obs = io.fold_obs && (io.reward || *io.armed), fold_ret = io.reward != nullptr;
+  double *st = io.stats;
+  double cnt[2] = {st[2 * OBS], st[2 * OBS + 3]}, tot[2] = {cnt[0], cnt[1]};
+#pragma unroll
+  for (int c = 0; c <= OBS; ++c) {
+    if (c < OBS ? !fold_obs : !fold_ret) continue;
+    EsMoments v = {0.0, 0.0, 0.0};
+    for (int64_t b = threadIdx.x; b < blocks; b += kBlock) {
+      const double *p = io.part + (b * (OBS + 1) + c) * 3;
+      v = es_merge(v, {p[0], p[1], p[2]});
+    }
+    v = es_merge_cta(v);
+    if (threadIdx.x == 0) {
+      const int k = c < OBS ? 0 : 1;
+      double *mean = c < OBS ? st + c : st + 2 * OBS + 1, *var = c < OBS ? st + OBS + c : st + 2 * OBS + 2;
+      const double N = v.n, t = __dadd_rn(cnt[k], N), d = v.d;
+      const double m2 = __dadd_rn(__dadd_rn(__dmul_rn(*var, cnt[k]), __dmul_rn(__ddiv_rn(v.m2, N), N)),
+                                  __ddiv_rn(__dmul_rn(__dmul_rn(__dmul_rn(d, d), cnt[k]), N), t));
+      *mean = __dadd_rn(*mean, __ddiv_rn(__dmul_rn(d, N), t));
+      *var = __ddiv_rn(m2, t);
+      tot[k] = t;
+    }
+  }
+  if (threadIdx.x == 0) {
+    st[2 * OBS] = tot[0]; st[2 * OBS + 3] = tot[1];
+    if (!fold_ret) *io.armed = 0;
+  }
+}
+// tb_set_vecnorm: the record from `src` (nullptr: fresh, RunningMeanStd(epsilon=1e-4)), returns zeroed, the fold armed
+template <int OBS>
+__global__ void __launch_bounds__(kBlock) vecnorm_init_kernel(const __grid_constant__ VecNormIO io, const double *src) {
+  const int64_t i = (int64_t)blockIdx.x * kBlock + threadIdx.x;
+  if (i < io.n) io.ret[i] = 0.0;
+  if (i < 2 * OBS + 4) io.stats[i] = src ? src[i] : (i < OBS || i == 2 * OBS + 1) ? 0.0 : (i == 2 * OBS || i == 2 * OBS + 3) ? 1e-4 : 1.0;
+  if (i == 0) *io.armed = 1;
+}
+// tb_reset / tb_reset_from with a normaliser in training: returns of the reset envs zeroed; a full reset arms the fold
+__global__ void __launch_bounds__(kBlock) vecnorm_reset_kernel(const __grid_constant__ VecNormIO io, const uint8_t *mask) {
+  const int64_t i = (int64_t)blockIdx.x * kBlock + threadIdx.x;
+  if (i < io.n && (!mask || mask[i])) io.ret[i] = 0.0;
+  if (i == 0 && !mask) *io.armed = 1;
 }
 
 // ------------------------------------------------------------------------------------------------ SAC actor and replay ring
@@ -2734,6 +2864,11 @@ struct PolicyBufs {           // tb_set_policy
   DevPtr<float> params;       // tb_policy_floats(env_kind) parameters
   DevPtr<float> act;          // [N, act_dim] clipped actions handed from policy_kernel to step_kernel
 };
+struct VecNormBufs {          // tb_set_vecnorm (see VecNormIO)
+  DevPtr<double> stats, ret, part;
+  DevPtr<float> raw;          // [N, obs_dim] raw observation handed from step_kernel to policy_kernel<.., true>
+  DevPtr<uint8_t> armed;
+};
 
 struct tb_ctx {
   tb_config cfg;
@@ -2763,7 +2898,9 @@ struct tb_ctx {
   int control_mode = TB_CONTROL_FORCE;
   DevPtr<void> pid;                          // controller memory, allocated by tb_set_control_mode(TB_CONTROL_PID)
   PolicyBufs policy;
-  SacActorBufs sac_actor;                    // SAC actor and ring (tb_set_sac_actor / tb_sac_begin / tb_sac_rollout)
+  VecNormBufs vn;                            // the policy rollout's normaliser (tb_set_vecnorm), kept when detached
+  tb_vecnorm vn_cfg{};                       // its configuration; vn_cfg.struct_size == 0: none attached
+  SacActorBufs sac_actor;                   // SAC actor and ring (tb_set_sac_actor / tb_sac_begin / tb_sac_rollout)
   SacBufs sac;
   int sac_grid = 0;                          // persistent grid of sac_kernel: SMs
   // ES fitness rollout (tb_es_begin / tb_es_rollout); see EsIO
@@ -2957,6 +3094,30 @@ static int launch_reset(tb_ctx *c, const StepIO &io, const double *d_init, const
   });
 }
 
+// CTAs of es_norm_partial_kernel and vecnorm_partial_kernel
+static int64_t es_norm_blocks(int64_t n) { return (n + kBlock * kEsStatsPer - 1) / (kBlock * kEsStatsPer); }
+// The normaliser's kernels: VecNormIO over the context's buffers, and f(VecNormIO, Kind<env_kind>())
+static bool vecnorm_training(const tb_ctx *c) { return c->vn_cfg.struct_size && c->vn_cfg.training; }
+static VecNormIO vecnorm_io(tb_ctx *c) {
+  VecNormIO io;
+  std::memset(&io, 0, sizeof io);
+  io.stats = c->vn.stats.get(); io.ret = c->vn.ret.get(); io.part = c->vn.part.get(); io.armed = c->vn.armed.get();
+  io.n = c->cfg.num_envs; io.gamma = c->vn_cfg.gamma; io.fold_obs = c->vn_cfg.training && c->vn_cfg.norm_obs;
+  return io;
+}
+// One statistics pass (vecnorm_partial_kernel, and vecnorm_final_kernel when the context trains): the entry pass when
+// reward is nullptr (copy obs to the raw buffer, fold it if armed), else the step pass.
+static int vecnorm_pass(tb_ctx *c, const float *obs, const float *reward, const uint8_t *done, cudaStream_t s) {
+  VecNormIO io = vecnorm_io(c);
+  io.obs = obs; io.reward = reward; io.done = done;
+  io.copy = reward ? nullptr : c->vn.raw.get();
+  const int64_t blocks = es_norm_blocks(io.n);
+  return with_kind(c->cfg.env_kind, [&](auto kind) {
+    if (launch(c, kPlain, vecnorm_partial_kernel<Dims<kind>::obs>, (unsigned)blocks, kBlock, s, io)) return 1;
+    return vecnorm_training(c) ? launch(c, kPlain, vecnorm_final_kernel<Dims<kind>::obs>, 1, kBlock, s, io, blocks) : 0;
+  });
+}
+
 extern "C" {
 
 const char *tb_last_error(void) { return g_err; }
@@ -3137,10 +3298,19 @@ static int reset_impl(tb_ctx *c, const double *d_init, const uint8_t *d_mask, fl
   io.obs = d_obs;
   return launch_reset(c, io, d_init, d_mask, (cudaStream_t)stream);
 }
-int tb_reset(tb_ctx *c, const uint8_t *d_mask, float *d_obs, void *stream) { return reset_impl(c, nullptr, d_mask, d_obs, stream); }
+// tb_reset / tb_reset_from with a normaliser in training: the reset envs' returns are zeroed, and a full reset arms the fold
+static int vecnorm_reset(tb_ctx *c, const uint8_t *d_mask, void *stream) {
+  if (!vecnorm_training(c)) return 0;
+  return launch(c, kPlain, vecnorm_reset_kernel, grid_for(c->cfg.num_envs, kBlock), kBlock, (cudaStream_t)stream, vecnorm_io(c), d_mask);
+}
+int tb_reset(tb_ctx *c, const uint8_t *d_mask, float *d_obs, void *stream) {
+  if (reset_impl(c, nullptr, d_mask, d_obs, stream)) return 1;
+  return vecnorm_reset(c, d_mask, stream);
+}
 int tb_reset_from(tb_ctx *c, const double *d_init, const uint8_t *d_mask, float *d_obs, void *stream) {
   if (!d_init) return fail("tb_reset_from: d_init is NULL");
-  return reset_impl(c, d_init, d_mask, d_obs, stream);
+  if (reset_impl(c, d_init, d_mask, d_obs, stream)) return 1;
+  return vecnorm_reset(c, d_mask, stream);
 }
 
 static int step_impl(tb_ctx *c, const float *d_actions, float *d_obs, float *d_reward, uint8_t *d_done,
@@ -3197,30 +3367,89 @@ int tb_policy_rollout(tb_ctx *c, int k_steps, int deterministic, uint64_t noise_
   if (check_fault(c, "tb_policy_rollout")) return 1;
   const int64_t n = c->cfg.num_envs;
   const int od = tb_obs_dim(c->cfg.env_kind), ad = tb_act_dim(c->cfg.env_kind);
+  // with a normaliser: policy_kernel<.., true> reads the raw observation from vn.raw (from d_last_obs after the last step)
+  const bool vn = c->vn_cfg.struct_size != 0, train = vecnorm_training(c);
   void (*kernel)(PolicyIO) = nullptr;
-  with_kind(c->cfg.env_kind, [&](auto kind) { kernel = policy_kernel<Dims<kind>::obs, Dims<kind>::act>; return 0; });
+  with_kind(c->cfg.env_kind, [&](auto kind) {
+    kernel = vn ? policy_kernel<Dims<kind>::obs, Dims<kind>::act, true> : policy_kernel<Dims<kind>::obs, Dims<kind>::act, false>;
+    return 0;
+  });
   cudaStream_t s = (cudaStream_t)stream;
   PolicyIO pio;
   std::memset(&pio, 0, sizeof pio);
   pio.params = c->policy.params.get(); pio.n = n; pio.id_offset = c->cfg.env_id_offset; pio.seed = noise_seed; pio.deterministic = deterministic;
   pio.act_env = c->policy.act.get(); pio.tick = step_counter(c);
+  if (vn) {
+    pio.vn_stats = c->vn.stats.get(); pio.vn_clip_obs = c->vn_cfg.clip_obs; pio.vn_clip_reward = c->vn_cfg.clip_reward;
+    pio.vn_eps = c->vn_cfg.epsilon; pio.vn_norm_obs = c->vn_cfg.norm_obs; pio.vn_norm_reward = c->vn_cfg.norm_reward;
+    if (vecnorm_pass(c, d_obs, nullptr, nullptr, s)) return 1;  // d_obs[0] -> vn.raw, folded when armed
+  }
   const unsigned grid = grid_for(n, kBlock);
   for (int t = 0; t < k_steps; ++t) {
-    pio.obs = d_obs + (size_t)t * n * od;
+    pio.obs = vn ? c->vn.raw.get() : d_obs + (size_t)t * n * od;
     pio.act_raw = d_actions ? d_actions + (size_t)t * n * ad : nullptr;
     pio.logp = d_logp ? d_logp + (size_t)t * n : nullptr;
     pio.value = d_value ? d_value + (size_t)t * n : nullptr;
+    if (vn) { pio.vn_obs = d_obs + (size_t)t * n * od; pio.vn_reward = t ? d_reward + (size_t)(t - 1) * n : nullptr; }
     if (launch(c, kPdl, kernel, dim3(grid, 2), kBlock, s, pio)) return 1;
     StepIO io = make_io(c);
     io.actions = c->policy.act.get();
-    io.obs = t + 1 < k_steps ? d_obs + (size_t)(t + 1) * n * od : d_last_obs;
+    io.obs = t + 1 < k_steps ? (vn ? c->vn.raw.get() : d_obs + (size_t)(t + 1) * n * od) : d_last_obs;
     io.reward = d_reward + (size_t)t * n; io.done = d_done + (size_t)t * n;
     if (launch_step(c, io, s)) return 1;
+    if (train && vecnorm_pass(c, io.obs, io.reward, io.done, s)) return 1;
   }
-  if (d_last_value) {  // bootstrap value of the observation the rollout ends with
+  if (d_last_value || vn) {  // bootstrap value of the observation the rollout ends with; the last step's normalised reward
     pio.obs = d_last_obs; pio.act_raw = nullptr; pio.act_env = nullptr; pio.logp = nullptr; pio.value = d_last_value;
+    pio.vn_obs = nullptr; pio.vn_reward = vn ? d_reward + (size_t)(k_steps - 1) * n : nullptr;
     if (launch(c, kPdl, kernel, dim3(grid, 2), kBlock, s, pio)) return 1;
   }
+  return 0;
+}
+
+int tb_set_vecnorm(tb_ctx *c, const tb_vecnorm *cfg, const double *d_stats, void *stream) {
+  GUARD(c);
+  if (check_fault(c, "tb_set_vecnorm")) return 1;
+  if (!cfg) { c->vn_cfg = tb_vecnorm{}; return 0; }
+  if (cfg->struct_size != sizeof(tb_vecnorm)) return fail("tb_set_vecnorm: tb_vecnorm.struct_size mismatch");
+  if (!(std::isfinite(cfg->clip_obs) && cfg->clip_obs > 0) || !(std::isfinite(cfg->clip_reward) && cfg->clip_reward > 0))
+    return fail("tb_set_vecnorm: clip_obs and clip_reward must be finite and above 0");
+  if (!(cfg->gamma >= 0 && cfg->gamma <= 1)) return fail("tb_set_vecnorm: gamma must be in [0, 1]");
+  if (!(std::isfinite(cfg->epsilon) && cfg->epsilon > 0)) return fail("tb_set_vecnorm: epsilon must be finite and above 0");
+  const int od = tb_obs_dim(c->cfg.env_kind), words = TB_VECNORM_WORDS(od);
+  cudaStream_t s = (cudaStream_t)stream;
+  if (d_stats) {  // the record is read on the device: copy it back and check it first (synchronises `stream`)
+    double h[TB_VECNORM_WORDS(12)];
+    CU(cudaMemcpyAsync(h, d_stats, words * sizeof(double), cudaMemcpyDeviceToHost, s));
+    CU(cudaStreamSynchronize(s));
+    for (int i = 0; i < words; ++i) {
+      const bool count = i == 2 * od || i == 2 * od + 3, var = (i >= od && i < 2 * od) || i == 2 * od + 2;
+      if (!std::isfinite(h[i]) || (count && !(h[i] > 0)) || (var && h[i] < 0))
+        return fail("tb_set_vecnorm: stats[%d] = %g: counts must be above 0, variances at least 0, every entry finite", i, h[i]);
+    }
+  }
+  if (!c->vn.stats) {
+    const int64_t n = c->cfg.num_envs;
+    VecNormBufs b;
+    CU(dev_alloc(b.stats, (size_t)words * sizeof(double)));
+    CU(dev_alloc(b.ret, (size_t)n * sizeof(double)));
+    CU(dev_alloc(b.part, (size_t)es_norm_blocks(n) * (od + 1) * 3 * sizeof(double)));
+    CU(dev_alloc(b.raw, (size_t)n * od * sizeof(float)));
+    CU(dev_alloc(b.armed, 1));
+    c->vn = std::move(b);
+  }
+  c->vn_cfg = *cfg;
+  return with_kind(c->cfg.env_kind, [&](auto kind) {
+    return launch(c, kPlain, vecnorm_init_kernel<Dims<kind>::obs>, grid_for(c->cfg.num_envs, kBlock), kBlock, s, vecnorm_io(c), d_stats);
+  });
+}
+
+int tb_get_vecnorm(tb_ctx *c, double *d_stats, void *stream) {
+  GUARD(c);
+  if (!c->vn_cfg.struct_size) return fail("tb_get_vecnorm: no normaliser attached (tb_set_vecnorm)");
+  if (!d_stats) return fail("tb_get_vecnorm: d_stats is NULL");
+  const size_t bytes = TB_VECNORM_WORDS(tb_obs_dim(c->cfg.env_kind)) * sizeof(double);
+  CU(cudaMemcpyAsync(d_stats, c->vn.stats.get(), bytes, cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
   return 0;
 }
 
@@ -3237,7 +3466,6 @@ static EsIO es_io(tb_ctx *c) {
   return io;
 }
 
-static int64_t es_norm_blocks(int64_t n) { return (n + kBlock * kEsStatsPer - 1) / (kBlock * kEsStatsPer); }
 
 // The checks tb_es_begin and tb_es_begin_noise share once the context is current, then the per-env state (once per context)
 // and room for the population in es_w.

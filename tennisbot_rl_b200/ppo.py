@@ -10,7 +10,8 @@ torch code at all: tb_policy_rollout evaluates the policy in a CUDA kernel of th
 log-density, value), so the 26-step episode is 26 x (policy_kernel, step_kernel, ff_kernel) issued by one C call; the call
 is captured once as a CUDA graph and replayed per update (nothing in it synchronises; the queue tags of ff_kernel advance
 on the device).  `fused_policy=False` keeps the eager torch policy of round 1 for comparison.  Target: the mean episodic
-return stored in backup_models/ppo_swing.zip, 31.5.
+return stored in backup_models/ppo_swing.zip, 31.5.  `normalize=True` puts SB3's VecNormalize on the device rollout
+(tb_set_vecnorm): the policy learns on normalised observations and rewards, the reported returns stay raw.
 
 HitPPO trains Tennisbot-v0 (train.py) the same way with the same hyper-parameters and the same towers on the env's 12
 inputs and 2 outputs (train.py's net_arch is not recorded); its rollouts are K steps of episodes up to 1001 steps long.
@@ -18,6 +19,7 @@ inputs and 2 outputs (train.py's net_arch is not recorded); its rollouts are K s
 import math
 import time
 
+import numpy as np
 import torch
 import torch.nn as nn
 
@@ -97,8 +99,12 @@ class GpuPPO:
     need not hold whole episodes."""
 
     def __init__(self, env_id, num_envs, rollout_len, precision="f64", seed=0, lr=3e-4, epochs=10, minibatches=8, device=0,
-                 use_graph=True, fused_policy=True):
+                 use_graph=True, fused_policy=True, normalize=False):
+        if normalize and not fused_policy:
+            raise ValueError("normalize=True needs fused_policy=True: the normaliser runs inside tb_policy_rollout, and the eager "
+                             "torch policy has none")
         torch.manual_seed(seed)
+        self.normalize = bool(normalize)
         self.fused_policy = fused_policy
         self.seed = seed
         self.dev = torch.device("cuda", device)
@@ -115,7 +121,9 @@ class GpuPPO:
         self.logp_buf, self.rew_buf, self.done_buf, self.val_buf = z(K, n), z(K, n), z(K, n), z(K + 1, n)
         self.done_u8 = torch.zeros((K, n), dtype=torch.uint8, device=self.dev)
         self.params = z(POLICY_FLOATS_BY_DIMS[(od, ad)])
-        self.obs = self.env.reset().clone()
+        self.obs = self.env.reset().clone()  # raw: with normalize, obs_buf / rew_buf receive the normalised values
+        if self.normalize:  # SB3 VecNormalize's defaults, with PPO's gamma; the first rollout folds the reset observation
+            self.env.set_vecnorm(gamma=self.gamma)
         self.graph = None
         self.warmed_up = False
         self.use_graph = use_graph
@@ -229,6 +237,21 @@ class GpuPPO:
                                     v.zero_()
                 self.upd_graph.replay()
 
+    def state_dict(self):
+        """The trained run as numpy arrays: `policy`, tb_set_policy's vector, and with normalize the normaliser's record
+        under load_vecnormalize_npz's keys."""
+        out = {"policy": self.ac.packed().cpu().numpy()}
+        if self.normalize:
+            od, st = self.od, self.env.vecnorm_stats().cpu().numpy()
+            out.update(obs_mean=st[:od], obs_var=st[od:2 * od], obs_count=st[2 * od], ret_mean=st[2 * od + 1],
+                       ret_var=st[2 * od + 2], ret_count=st[2 * od + 3], clip_obs=10.0, clip_reward=10.0, gamma=self.gamma,
+                       epsilon=1e-8)
+        return out
+
+    def save(self, path):
+        """state_dict() as an npz: tools/record_episode.py takes it as --policy (and as --vecnormalize with normalize)."""
+        np.savez(path, **self.state_dict())
+
     def _minibatch_step(self):
         ac = self.ac
         ratio = (ac.log_prob(self.mb_obs, self.mb_act) - self.mb_logp).exp()
@@ -247,9 +270,9 @@ class SwingPPO(GpuPPO):
     """PPO on SwingRacket-v0, one whole episode (26 steps) per env per update."""
 
     def __init__(self, num_envs=16384, precision="f64", seed=0, lr=3e-4, epochs=10, minibatches=8, device=0, use_graph=True,
-                 fused_policy=True):
+                 fused_policy=True, normalize=False):
         super().__init__("SwingRacket-v0", num_envs, EPISODE, precision, seed, lr, epochs, minibatches, device, use_graph,
-                         fused_policy)
+                         fused_policy, normalize)
 
     def train(self, iters=150, target=31.5, log=None):
         history, reached, t0 = [], None, time.time()
@@ -282,9 +305,9 @@ class HitPPO(GpuPPO):
     which a captured graph holds by value.  None: the env's racket scale is left as it is."""
 
     def __init__(self, num_envs=16384, rollout_len=128, curriculum_total_timesteps=None, precision="f64", seed=0, lr=3e-4,
-                 epochs=10, minibatches=8, device=0, use_graph=True, fused_policy=True):
+                 epochs=10, minibatches=8, device=0, use_graph=True, fused_policy=True, normalize=False):
         super().__init__("Tennisbot-v0", num_envs, rollout_len, precision, seed, lr, epochs, minibatches, device, use_graph,
-                         fused_policy)
+                         fused_policy, normalize)
         self.curriculum_total = curriculum_total_timesteps
         self.env_steps = 0   # env steps of the rollouts taken so far (the curriculum's num_timesteps)
         self.scale = None    # racket scale set by the curriculum
@@ -298,7 +321,7 @@ class HitPPO(GpuPPO):
         if s == self.scale:
             return False
         self.env.set_param("racket_scale", s)
-        self.obs.copy_(self.env.reset())
+        self.obs.copy_(self.env.reset())  # (a full reset: a normaliser zeroes its returns and folds this observation next)
         self.graph = None
         self.scale = s
         self.stages.append((self.env_steps, s))
@@ -346,3 +369,29 @@ def load_sb3_policy_npz(path):
     tower = lambda net: [(t(f"mlp_extractor__{net}__{i}__weight"), t(f"mlp_extractor__{net}__{i}__bias")) for i in (0, 2, 4)]  # noqa: E731
     return pack_policy(tower("policy_net"), (t("action_net__weight"), t("action_net__bias")), tower("value_net"),
                        (t("value_net__weight"), t("value_net__bias")), t("log_std"))
+
+
+VECNORMALIZE_KEYS = ("obs_mean", "obs_var", "obs_count", "ret_mean", "ret_var", "ret_count", "clip_obs", "clip_reward", "gamma",
+                     "epsilon")
+
+
+def load_vecnormalize_npz(path, obs_dim=None):
+    """(stats, config) of a saved VecNormalize: stats, float64 [2 obs_dim + 4] in tb_set_vecnorm's record layout; config, the
+    keyword arguments of TennisBatch.set_vecnorm (clip_obs, clip_reward, gamma, epsilon).  The npz holds obs_mean, obs_var
+    [obs_dim] and the scalars obs_count, ret_mean, ret_var, ret_count, clip_obs, clip_reward, gamma, epsilon (INTEGRATION.md
+    section 2 writes one from SB3's vec_normalize.pkl).  Deploy with set_vecnorm(training=False, stats=..., **config)."""
+    w = np.load(path)
+    missing = [k for k in VECNORMALIZE_KEYS if k not in w]
+    if missing:
+        raise ValueError(f"{path}: missing VecNormalize keys {missing}")
+    mean, var = np.asarray(w["obs_mean"], np.float64), np.asarray(w["obs_var"], np.float64)
+    od = mean.size if obs_dim is None else int(obs_dim)
+    if mean.shape != (od,) or var.shape != (od,):
+        raise ValueError(f"{path}: obs_mean and obs_var must have shape ({od},), got {mean.shape} and {var.shape}")
+    scalars = {k: np.asarray(w[k], np.float64) for k in VECNORMALIZE_KEYS[2:]}
+    bad = [k for k, v in scalars.items() if v.shape != ()]
+    if bad:
+        raise ValueError(f"{path}: {bad} must be scalars")
+    stats = np.concatenate([mean, var, [scalars["obs_count"], scalars["ret_mean"], scalars["ret_var"], scalars["ret_count"]]])
+    config = {k: float(scalars[k]) for k in ("clip_obs", "clip_reward", "gamma", "epsilon")}
+    return torch.from_numpy(stats), config

@@ -3,7 +3,9 @@
 
 Action sources: uniform random (default); the scripted ball tracker (--tracker, Tennisbot-v0); or a policy in tb_set_policy's
 layout, rolled by tb_policy_rollout with K = 1 (--policy: a .npy flat vector, or an .npz of an SB3 MlpPolicy state dict such
-as the reference's trained policy tests/golden/ppo_swing_policy.npz).  Frames exist per env step: a SwingRacket-v0 episode is
+as the reference's trained policy tests/golden/ppo_swing_policy.npz, or GpuPPO.save's npz).  A policy trained under VecNormalize
+acts on normalised observations: --vecnormalize FILE attaches that record, frozen (ppo.load_vecnormalize_npz's keys; a
+GpuPPO.save npz of a normalize=True run holds them too).  Frames exist per env step: a SwingRacket-v0 episode is
 26 frames, and its 26th step fast-forwards the ball's whole flight (about 106 physics substeps, at most 776).  With
 --flight-every K that step is also traced substep by substep (tb_trace_step, from the states saved before it and the actions
 it took), and every K-th flight substep plus the last is drawn between frame 25 and the episode's final frame.
@@ -11,6 +13,7 @@ it took), and every K-th flight substep plus the last is drawn between frame 25 
   python tools/record_episode.py SwingRacket-v0 --policy tests/golden/ppo_swing_policy.npz --out frames/swing
   python tools/record_episode.py SwingRacket-v0 --policy tests/golden/ppo_swing_policy.npz --flight-every 4 --out frames/shot
   python tools/record_episode.py Tennisbot-v0 --tracker --out frames/hit
+  python tools/record_episode.py Tennisbot-v0 --policy run.npz --vecnormalize run.npz --out frames/hit_norm
 """
 import argparse
 import struct
@@ -45,6 +48,9 @@ def load_policy(path):
     if path.suffix == ".npz":
         from tennisbot_rl_b200.ppo import load_sb3_policy_npz
 
+        w = np.load(path)
+        if "policy" in w:  # GpuPPO.save
+            return torch.from_numpy(np.ascontiguousarray(w["policy"], np.float32))
         return load_sb3_policy_npz(path)
     return torch.from_numpy(np.load(path).astype(np.float32))
 
@@ -57,6 +63,7 @@ def main():
     ap.add_argument("--steps", type=int, default=450, help="Tennisbot-v0: env steps per recorded episode")
     ap.add_argument("--tracker", action="store_true", help="Tennisbot-v0: the scripted ball tracker (TB_ACT_TRACK)")
     ap.add_argument("--policy", type=Path, help=".npy parameter vector or .npz SB3 MlpPolicy state dict")
+    ap.add_argument("--vecnormalize", type=Path, help="with --policy: the VecNormalize record (npz) it was trained under")
     ap.add_argument("--stochastic", action="store_true", help="sample the policy's actions instead of taking the mean")
     ap.add_argument("--width", type=int, default=320)
     ap.add_argument("--height", type=int, default=240)
@@ -74,6 +81,8 @@ def main():
         ap.error("--tracker is Tennisbot-v0's scripted tracker")
     if a.tracker and a.policy:
         ap.error("--tracker and --policy are two action sources")
+    if a.vecnormalize and not a.policy:
+        ap.error("--vecnormalize normalises a --policy's observations")
 
     m = a.envs
     swing = a.env_id == "SwingRacket-v0"
@@ -87,6 +96,11 @@ def main():
     obs = torch.zeros((1, m, b.obs_dim), device=b.device)
     if a.policy:
         b.set_policy(load_policy(a.policy).to(b.device))
+        if a.vecnormalize:  # frozen: the statistics the policy was trained with
+            from tennisbot_rl_b200.ppo import load_vecnormalize_npz
+
+            stats, cfg = load_vecnormalize_npz(a.vecnormalize, b.obs_dim)
+            b.set_vecnorm(training=False, stats=stats.to(b.device), **cfg)
         rew, done = torch.zeros((1, m), device=b.device), torch.zeros((1, m), dtype=torch.uint8, device=b.device)
         last = torch.zeros((m, b.obs_dim), device=b.device)
         act = torch.zeros((1, m, b.act_dim), device=b.device)
@@ -101,7 +115,7 @@ def main():
             before = b.get_state()
         if a.policy:
             b.policy_rollout(obs, rew, done, last, actions=act, deterministic=not a.stochastic, noise_seed=a.seed)
-            obs[0].copy_(last)
+            obs[0].copy_(last)  # raw, also with a normaliser (obs[0] now holds the normalised observation)
             taken = act[0].clamp(-1, 1)  # policy_rollout returns the unclipped action; the env step took it clipped
         elif a.tracker:
             b.rollout(1, _lib.ACT_TRACK)

@@ -5,15 +5,21 @@ learns to hit the ball: longer flights, contact chains), and the per-kernel spli
 Tennisbot-v0: env-steps/s of the K-step rollout (CUDA graph replay, CUDA events) at each batch size, with the untrained
 policy and with the weights of `iters` PPO updates at 16 384 envs, and the split: step_kernel time from the library's
 per-step CUDA events (tb_set_kernel_timing, an eager run), the rest of the graph's time is policy_kernel and two copies.
+--normalize: the cost of the device VecNormalize (tb_set_vecnorm): for both envs (SwingRacket-v0 K = 26, Tennisbot-v0
+K = 128) and each batch size, the same policy rollout captured as two CUDA graphs, without and with a training normaliser,
+replayed alternately in the same run (CUDA events); ms per rollout step of each and the difference.
 usage: time_policy_rollout.py [n_envs] [iters]
-       time_policy_rollout.py Tennisbot-v0 [iters] [K] [n_envs ...]      (default n_envs: 16384 1048576)"""
+       time_policy_rollout.py Tennisbot-v0 [iters] [K] [n_envs ...]      (default n_envs: 16384 1048576)
+       time_policy_rollout.py --normalize [n_envs ...]                  (default n_envs: 16384 1048576)"""
+import statistics
 import subprocess
 import sys
 
 import torch
 
 sys.path.insert(0, ".")
-from tennisbot_rl_b200.ppo import EPISODE, HitPPO, SwingPPO  # noqa: E402
+from tennisbot_rl_b200.batch import TennisBatch  # noqa: E402
+from tennisbot_rl_b200.ppo import EPISODE, ActorCritic, HitPPO, SwingPPO  # noqa: E402
 
 
 def card():
@@ -93,8 +99,64 @@ def swing(argv):
     print("last fast-forward: server visits %d, flights over after %.3f ms" % (d[1], d[2] * 1e-6))
 
 
+def normalize_cost(argv, rounds=7, reps=5):
+    sizes = [int(a) for a in argv] or [16384, 1048576]
+    print("card (name, power limit, max SM clock):", card(), flush=True)
+    for env_id, K in (("SwingRacket-v0", EPISODE), ("Tennisbot-v0", 128)):
+        for n in sizes:
+            torch.manual_seed(0)
+            b = TennisBatch(env_id, n, seed=0)
+            dev, od, ad = b.device, b.obs_dim, b.act_dim
+            b.set_policy(ActorCritic(od, ad).to(dev).packed())
+            z = lambda *s: torch.zeros(s, device=dev)  # noqa: E731
+            obs, act, logp, val, rew, last, last_v = z(K, n, od), z(K, n, ad), z(K, n), z(K, n), z(K, n), z(n, od), z(n)
+            done = torch.zeros((K, n), dtype=torch.uint8, device=dev)
+            cur = b.reset().clone()
+
+            def body():
+                obs[0].copy_(cur)
+                b.policy_rollout(obs, rew, done, last, actions=act, logp=logp, value=val, last_value=last_v, noise_seed=1)
+                cur.copy_(last)
+
+            graphs = {}
+            for label in ("plain", "vecnorm"):  # a graph keeps the kernels it was captured with
+                if label == "vecnorm":
+                    b.set_vecnorm()
+                s = torch.cuda.Stream(dev)
+                s.wait_stream(torch.cuda.current_stream(dev))
+                with torch.cuda.stream(s):
+                    body()
+                torch.cuda.current_stream(dev).wait_stream(s)
+                g = torch.cuda.CUDAGraph()
+                with torch.cuda.graph(g):
+                    body()
+                graphs[label] = g
+            times = {k: [] for k in graphs}
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            for _ in range(rounds):
+                for label, g in graphs.items():
+                    g.replay()  # one untimed replay after the switch
+                    e0.record()
+                    for _ in range(reps):
+                        g.replay()
+                    e1.record()
+                    torch.cuda.synchronize()
+                    times[label].append(e0.elapsed_time(e1) / reps / K * 1e3)
+            med = {k: statistics.median(v) for k, v in times.items()}
+            spread = {k: (min(v), max(v)) for k, v in times.items()}
+            print(f"{env_id} {n:8d} envs K={K}: per rollout step plain {med['plain']:9.2f} us "
+                  f"[{spread['plain'][0]:.2f}, {spread['plain'][1]:.2f}], with vecnorm {med['vecnorm']:9.2f} us "
+                  f"[{spread['vecnorm'][0]:.2f}, {spread['vecnorm'][1]:.2f}]: +{med['vecnorm'] - med['plain']:.2f} us "
+                  f"({(med['vecnorm'] / med['plain'] - 1) * 100:+.1f} %); medians of {rounds} x {reps} replays", flush=True)
+            del graphs
+            b.close()
+            torch.cuda.empty_cache()
+
+
 if __name__ == "__main__":
-    if len(sys.argv) > 1 and sys.argv[1] in ("Tennisbot-v0", "hit"):
+    if len(sys.argv) > 1 and sys.argv[1] == "--normalize":
+        normalize_cost(sys.argv[2:])
+    elif len(sys.argv) > 1 and sys.argv[1] in ("Tennisbot-v0", "hit"):
         hit(sys.argv[2:])
     else:
         swing(sys.argv[1:])

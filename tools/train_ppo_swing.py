@@ -4,6 +4,7 @@ its racket-scale curriculum over --curriculum TOTAL env steps).
 
     python tools/train_ppo_swing.py --iters 150 --out gpurun_out/ppo_swing_b200.json
     python tools/train_ppo_swing.py --env Tennisbot-v0 --rollout-len 128 --curriculum 200000000 --iters 100
+    python tools/train_ppo_swing.py --env Tennisbot-v0 --iters 60 --normalize --save hit_norm.npz
 """
 import argparse
 import json
@@ -30,18 +31,23 @@ def main():
                     help="Tennisbot-v0: train.py's racket-scale curriculum over TOTAL env steps (0: none)")
     ap.add_argument("--no-graph", action="store_true")
     ap.add_argument("--eager-policy", action="store_true", help="torch policy in the rollout instead of tb_policy_rollout")
+    ap.add_argument("--normalize", action="store_true", help="SB3 VecNormalize on the device rollout (tb_set_vecnorm)")
     ap.add_argument("--out", default="")
+    ap.add_argument("--save", default="", help="npz of the trained policy (and the normaliser's record): GpuPPO.save")
     args = ap.parse_args()
     log = lambda s: print(s, flush=True)  # noqa: E731
     if args.env == "SwingRacket-v0":
         ppo = SwingPPO(args.envs, args.precision, args.seed, args.lr, args.epochs, args.minibatches, use_graph=not args.no_graph,
-                       fused_policy=not args.eager_policy)
+                       fused_policy=not args.eager_policy, normalize=args.normalize)
         summary = ppo.train(args.iters, args.target, log=log)
     else:
         ppo = HitPPO(args.envs, args.rollout_len, args.curriculum or None, args.precision, args.seed, args.lr, args.epochs,
-                     args.minibatches, use_graph=not args.no_graph, fused_policy=not args.eager_policy)
+                     args.minibatches, use_graph=not args.no_graph, fused_policy=not args.eager_policy, normalize=args.normalize)
         summary = ppo.train(args.iters, log=log)
+    summary["normalize"] = args.normalize
     print(json.dumps({k: v for k, v in summary.items() if k != "history"}))
+    if args.save:
+        ppo.save(args.save)
     if args.out:
         Path(args.out).write_text(json.dumps(summary, indent=1))
 
