@@ -204,7 +204,8 @@ int tb_policy_rollout(tb_ctx *ctx, int k_steps, int deterministic, uint64_t nois
  * d_obs[0] when armed, and two statistics launches after each step), K (1 + s) + 2 when not; s = 2 for SwingRacket-v0 and 1 for
  * Tennisbot-v0 (tb_step's launches), and the last launch (bootstrap value, last normalised reward) always runs.  tb_reset /
  * tb_reset_from add one launch while a training normaliser is attached.  The int64 statistics (tb_read_stats) stay raw;
- * tb_step, tb_rollout, tb_reset_host, tb_step_host and the ES and SAC entry points ignore the normaliser.  Each context keeps its
+ * tb_step, tb_rollout, tb_reset_host, tb_step_host and the ES entry points ignore the normaliser, and so does tb_sac_rollout
+ * unless its mode carries TB_SAC_VECNORM (see there; tb_vecnorm_apply normalises replay samples).  Each context keeps its
  * own statistics: shards with env_id_offset do not reproduce the statistics of one batch. */
 typedef struct tb_vecnorm {
   uint32_t struct_size; /* sizeof(tb_vecnorm) */
@@ -221,6 +222,15 @@ int tb_set_vecnorm(tb_ctx *ctx, const tb_vecnorm *cfg, const double *d_stats, vo
 /* d_stats double [TB_VECNORM_WORDS(obs_dim)] = the current record (stream-ordered copy, never synchronises).  Fails when no
  * normaliser is attached. */
 int tb_get_vecnorm(tb_ctx *ctx, double *d_stats, void *stream);
+/* d_out = rule 4's o^ of d_in float32 [rows, obs_dim] (what = TB_VECNORM_OBS), or rule 3's r^ of d_in float32 [rows]
+ * (TB_VECNORM_REWARD), with the record as it stands when the kernel runs (a replayed graph sees the current statistics);
+ * norm_obs = 0 (norm_reward = 0) copies.  What SB3's ReplayBuffer.sample(env=vec_normalize_env) does to a raw batch.  d_out
+ * may be d_in.  One kernel launch (rows = 0 included, which reads nothing), never synchronises.  Fails when no normaliser is
+ * attached, what is unknown, rows < 0 (or the grid would exceed 2^31 - 1 CTAs of 128 floats), d_in or d_out is NULL while
+ * rows > 0, or the context is faulted. */
+#define TB_VECNORM_OBS 0
+#define TB_VECNORM_REWARD 1
+int tb_vecnorm_apply(tb_ctx *ctx, const float *d_in, int64_t rows, int what, float *d_out, void *stream);
 
 /* ---- ES fitness rollout (SURVEY 8(f)-2): fitness_static (fitness_functions.py:18-158) for a whole population in one context.
  * Env i evaluates individual i / (N / individuals) with the reference's GatedCNN (policies.py:59-128) on an 8-step history of
@@ -322,7 +332,17 @@ int tb_sac_begin(tb_ctx *ctx, void *stream);
  * received, reward, done (a time-out is a done like any other: the reference returns {} and SB3 does not bootstrap), next_obs
  * = the terminal observation when done, else the step's observation.  ring = NULL stores nothing (evaluation).  d_last_obs
  * float32 [N, obs_dim] (may be NULL) receives the observation after the last step.  mode TB_SAC_SAMPLE and TB_SAC_MEAN need
- * tb_set_sac_actor.  Never synchronises: capturable in a CUDA graph. */
+ * tb_set_sac_actor.  Never synchronises: capturable in a CUDA graph.
+ * mode | TB_SAC_VECNORM (fails when no normaliser is attached): SB3 SAC under VecNormalize, with the normaliser of tb_set_vecnorm.
+ * After every env step (TB_SAC_UNIFORM included) a training normaliser folds the step's observation of all N envs (rule 1),
+ * the return (rule 2) and zeroes the returns of done envs (rule 3); the actor acts on o^ (rule 4) with the statistics after
+ * that fold.  The ring, d_last_obs and tb_read_stats stay RAW (SB3's get_original_obs / get_original_reward; a terminal
+ * next_obs is the exact raw value, where SB3 stores unnormalize(normalize(.)), which differs where clip_obs bites).  The first
+ * such rollout with a training normaliser after tb_sac_begin zeroes the returns and folds the reset observation of all envs
+ * (a flag of tb_sac_begin, kept on the device); training = 0: statistics and returns never change.  Launches: (K + 1) + K s
+ * frozen; training adds 2 K (the statistics pass after each step) + 3 (the entry pass, which folds only while the reset is
+ * pending). */
+#define TB_SAC_VECNORM 0x100
 int tb_sac_rollout(tb_ctx *ctx, int k_steps, int mode, uint64_t noise_seed, const tb_sac_ring *ring, float *d_last_obs,
                    void *stream);
 

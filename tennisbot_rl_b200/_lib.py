@@ -23,6 +23,8 @@ SAC_FLOATS = 70672         # SwingRacket-v0's SAC actor (TB_SAC_FLOATS)
 SAC_FLOATS_HIT = 70152     # Tennisbot-v0's (TB_SAC_FLOATS_HIT)
 SAC_HIDDEN = 256           # TB_SAC_HIDDEN
 SAC_SAMPLE, SAC_MEAN, SAC_UNIFORM = 0, 1, 2
+SAC_VECNORM = 0x100        # TB_SAC_VECNORM: OR'd into tb_sac_rollout's mode, the normaliser of tb_set_vecnorm applies
+VECNORM_OBS, VECNORM_REWARD = 0, 1  # tb_vecnorm_apply's `what`
 CONTROL_FORCE, CONTROL_PID = 0, 1
 BODY_NONE, BODY_COURT, BODY_NET, BODY_GOAL, BODY_RACKET, BODY_BALL = 0, 1, 2, 3, 4, 5  # TB_BODY_*
 RENDER_SKY = (170, 200, 235)                                                           # TB_RENDER_SKY
@@ -75,6 +77,7 @@ SIGNATURES = {
     "tb_set_policy": [_vp, _vp, _i64, _vp],
     "tb_policy_rollout": [_vp, _i32, _i32, _u64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
     "tb_set_vecnorm": [_vp, C.POINTER(TbVecNorm), _vp, _vp], "tb_get_vecnorm": [_vp, _vp, _vp],
+    "tb_vecnorm_apply": [_vp, _vp, _i64, _i32, _vp, _vp],
     "tb_es_begin": [_vp, _vp, _i64, _i64, _vp, _vp], "tb_es_rollout": [_vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
     "tb_es_begin_noise": [_vp, _vp, _i64, _i64, C.c_float, _u64, _u32, _vp, _vp],
     "tb_es_noise_combine": [_vp, _vp, _vp, _i64, _u64, _u32, _vp, _vp], "tb_es_normalizer_stats": [_vp, _vp, _vp],

@@ -184,6 +184,26 @@ class TennisBatch:
         _lib.check(self.lib.tb_get_vecnorm(self.h, _dptr(out), self._stream()))
         return out
 
+    def vecnorm_apply(self, x, what="obs", out=None):
+        """The normaliser's formula on a batch of raw values (tb_vecnorm_apply), with the record as it stands when the kernel
+        runs: what 'obs' (VECNORM_OBS), x float32 [rows, obs_dim]; 'reward' (VECNORM_REWARD), x float32 [rows].  out: None (a
+        new tensor) or a tensor of x's shape, x itself included.  One launch on the current stream; returns out."""
+        what = {"obs": _lib.VECNORM_OBS, "reward": _lib.VECNORM_REWARD}.get(what, what)
+        if what not in (_lib.VECNORM_OBS, _lib.VECNORM_REWARD):
+            raise ValueError(f"vecnorm_apply: what must be 'obs' or 'reward', got {what!r}")
+        obs = what == _lib.VECNORM_OBS
+        rows = int(x.shape[0]) if torch.is_tensor(x) and x.dim() == (2 if obs else 1) else -1
+        shape = (rows, self.obs_dim) if obs else (rows,)
+        if rows < 0:
+            raise ValueError(f"vecnorm_apply: x must have shape {('rows', self.obs_dim) if obs else ('rows',)}, got "
+                             f"{None if x is None else tuple(x.shape)}")
+        self._need("vecnorm_apply", x, "x", shape)
+        if out is None:
+            out = torch.empty_like(x)
+        self._need("vecnorm_apply", out, "out", shape)
+        _lib.check(self.lib.tb_vecnorm_apply(self.h, _dptr(x), rows, int(what), _dptr(out), self._stream()))
+        return out
+
     # ------------------------------------------------------------------ ES fitness rollout (tb_es_begin / tb_es_rollout)
     def es_begin(self, weights, normalizer=None):
         """Start an ES generation: weights float32 [individuals, es_floats] (individuals divides num_envs; env i evaluates
@@ -266,11 +286,13 @@ class TennisBatch:
         """Reset every env and start the ring at slot 0 (needs force control and auto_reset)."""
         _lib.check(self.lib.tb_sac_begin(self.h, self._stream()))
 
-    def sac_rollout(self, k, mode=_lib.SAC_SAMPLE, ring=None, noise_seed=0, last_obs=None):
+    def sac_rollout(self, k, mode=_lib.SAC_SAMPLE, ring=None, noise_seed=0, last_obs=None, normalize=False):
         """k env steps with in-kernel SAC actions.  mode: SAC_SAMPLE, SAC_MEAN or SAC_UNIFORM (or 'sample', 'mean', 'uniform').
         ring: None or a dict of tensors obs / next_obs float32 [slots, N, obs_dim], act float32 [slots, N, act_dim], reward
         float32 [slots, N], done uint8 [slots, N]; step j since sac_begin goes to slot j % slots.  last_obs float32 [N, obs_dim]
-        receives the observation after the last step.  The library writes through raw pointers, so every buffer is checked here."""
+        receives the observation after the last step.  normalize: the normaliser of set_vecnorm applies (TB_SAC_VECNORM: the
+        actor acts on normalised observations, a training normaliser folds every step; ring and last_obs stay raw).  The
+        library writes through raw pointers, so every buffer is checked here."""
         k, n = int(k), self.num_envs
         if k < 1:
             raise ValueError(f"sac_rollout: k must be >= 1, got {k}")
@@ -289,7 +311,8 @@ class TennisBatch:
             need(ring.get("done"), "ring['done']", (slots, n), dtype=torch.uint8)
             r = _lib.TbSacRing(C.sizeof(_lib.TbSacRing), 0, slots, *(ring[key].data_ptr() for key in
                                                                      ("obs", "act", "reward", "next_obs", "done")))
-        _lib.check(self.lib.tb_sac_rollout(self.h, k, int(mode), int(noise_seed) & (2 ** 64 - 1), None if r is None else C.byref(r),
+        mode = int(mode) | (_lib.SAC_VECNORM if normalize else 0)
+        _lib.check(self.lib.tb_sac_rollout(self.h, k, mode, int(noise_seed) & (2 ** 64 - 1), None if r is None else C.byref(r),
                                            _dptr(last_obs), self._stream()))
 
     # ------------------------------------------------------------------ frames (tb_render)

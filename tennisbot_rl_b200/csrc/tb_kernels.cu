@@ -1942,6 +1942,24 @@ __global__ void __launch_bounds__(kBlock) vecnorm_reset_kernel(const __grid_cons
   if (i < io.n && (!mask || mask[i])) io.ret[i] = 0.0;
   if (i == 0 && !mask) *io.armed = 1;
 }
+// tb_sac_rollout with TB_SAC_VECNORM and a training normaliser, first launch: while the reset of tb_sac_begin is pending
+// (io.armed = the SAC flag, cleared by the entry pass that follows and folds the reset observation), every return starts at 0
+__global__ void __launch_bounds__(kBlock) vecnorm_sac_entry_kernel(const __grid_constant__ VecNormIO io) {
+  const int64_t i = (int64_t)blockIdx.x * kBlock + threadIdx.x;
+  if (i < io.n && *io.armed) io.ret[i] = 0.0;
+}
+// tb_vecnorm_apply: out = vn_apply of `in` with the record as it is when the kernel runs; reward rows use mean 0 and the
+// return variance.  norm = 0 copies.  Element-wise, so in == out is allowed.
+template <int OBS>
+__global__ void __launch_bounds__(kBlock) vecnorm_apply_kernel(const double *stats, const float *in, float *out, int64_t count,
+                                                               int reward, int norm, double clip, double eps) {
+  const int64_t e = (int64_t)blockIdx.x * kBlock + threadIdx.x;
+  if (e >= count) return;
+  const float v = in[e];
+  if (!norm) { out[e] = v; return; }
+  const int c = reward ? 0 : (int)(e % OBS);
+  out[e] = reward ? vn_apply(v, 0.0, stats[2 * OBS + 2], eps, clip) : vn_apply(v, stats[c], stats[OBS + c], eps, clip);
+}
 
 // ------------------------------------------------------------------------------------------------ SAC actor and replay ring
 // SURVEY 8(f)-5: the actor of SB3 SAC's MlpPolicy (latent_pi = Linear(obs, 256), ReLU, Linear(256, 256), ReLU; mu and log_std
@@ -2002,6 +2020,10 @@ struct SacIO {
   float *r_obs, *r_act, *r_reward, *r_next;
   uint8_t *r_done;
   float *last_obs;              // optional: `cur` after the fold (the launch ending a rollout)
+  // NORM instances only (TB_SAC_VECNORM): the network acts on vn_apply of the raw observation; ring and `cur` stay raw
+  const double *vn_stats;       // the running record, TB_VECNORM_WORDS(OBS) doubles
+  double vn_clip_obs, vn_eps;
+  int vn_norm_obs;
 };
 
 // Fold step j = tick - base - 1 of env i into the ring and `cur`; x receives the observation the next action is computed from.
@@ -2068,7 +2090,9 @@ template <int ACT> __device__ __forceinline__ void sac_store_act(const SacIO &io
 //   thread 0 issues 16 x tcgen05.mma (M 128, N 256, K 16) into 256 TMEM columns and commits to an mbarrier;
 //   each warp reads its 32 lanes back (tcgen05.ld 32x32b), adds b2, ReLU, and forms both heads in float32;
 //   clamp, noise, accurate tanhf.
-template <int OBS, int ACT>
+// NORM: the instance of tb_sac_rollout with TB_SAC_VECNORM; the network's input is normalised in registers before layer 1 (the
+// one-thread-per-env shape evaluates no network, so it is the same code in both instances).
+template <int OBS, int ACT, bool NORM>
 __global__ void __launch_bounds__(kBlock, 1) sac_kernel(const __grid_constant__ SacIO io) {
   using L = SacLayout<OBS, ACT>;
   static_assert(OBS % 2 == 0 && ACT % 2 == 0, "observation and action rows are accessed as float2");
@@ -2121,6 +2145,10 @@ __global__ void __launch_bounds__(kBlock, 1) sac_kernel(const __grid_constant__ 
 #pragma unroll
     for (int c = 0; c < OBS; ++c) x[c] = 0.0f;
     if (mine) sac_fold<OBS, ACT>(io, i, x);
+    if (NORM && mine && io.vn_norm_obs) {
+#pragma unroll
+      for (int c = 0; c < OBS; ++c) x[c] = vn_apply(x[c], io.vn_stats[c], io.vn_stats[OBS + c], io.vn_eps, io.vn_clip_obs);
+    }
     // layer 1: acc = b1, then + W1[j][c] x[c] for c = 0 .. OBS - 1, each product and sum rounded (no fused multiply-add)
 #pragma unroll 1
     for (int kc = 0; kc < L::H / 8; ++kc) {
@@ -2859,6 +2887,7 @@ struct SacBufs {              // tb_sac_begin: per-env staging between sac_kerne
   DevPtr<float> cur, act, obs, term, rew;
   DevPtr<uint8_t> done;
   DevPtr<unsigned> base;
+  DevPtr<uint8_t> pending;    // 1 from tb_sac_begin until a TB_SAC_VECNORM rollout with a training normaliser folds the reset
 };
 struct PolicyBufs {           // tb_set_policy
   DevPtr<float> params;       // tb_policy_floats(env_kind) parameters
@@ -3106,16 +3135,19 @@ static VecNormIO vecnorm_io(tb_ctx *c) {
   return io;
 }
 // One statistics pass (vecnorm_partial_kernel, and vecnorm_final_kernel when the context trains): the entry pass when
-// reward is nullptr (copy obs to the raw buffer, fold it if armed), else the step pass.
-static int vecnorm_pass(tb_ctx *c, const float *obs, const float *reward, const uint8_t *done, cudaStream_t s) {
-  VecNormIO io = vecnorm_io(c);
-  io.obs = obs; io.reward = reward; io.done = done;
-  io.copy = reward ? nullptr : c->vn.raw.get();
+// io.reward is nullptr (copy obs to io.copy if set, fold it if *io.armed), else the step pass.
+static int vecnorm_pass(tb_ctx *c, VecNormIO io, cudaStream_t s) {
   const int64_t blocks = es_norm_blocks(io.n);
   return with_kind(c->cfg.env_kind, [&](auto kind) {
     if (launch(c, kPlain, vecnorm_partial_kernel<Dims<kind>::obs>, (unsigned)blocks, kBlock, s, io)) return 1;
     return vecnorm_training(c) ? launch(c, kPlain, vecnorm_final_kernel<Dims<kind>::obs>, 1, kBlock, s, io, blocks) : 0;
   });
+}
+static int vecnorm_pass(tb_ctx *c, const float *obs, const float *reward, const uint8_t *done, cudaStream_t s) {
+  VecNormIO io = vecnorm_io(c);
+  io.obs = obs; io.reward = reward; io.done = done;
+  io.copy = reward ? nullptr : c->vn.raw.get();
+  return vecnorm_pass(c, io, s);
 }
 
 extern "C" {
@@ -3453,6 +3485,26 @@ int tb_get_vecnorm(tb_ctx *c, double *d_stats, void *stream) {
   return 0;
 }
 
+int tb_vecnorm_apply(tb_ctx *c, const float *d_in, int64_t rows, int what, float *d_out, void *stream) {
+  GUARD(c);
+  if (!c->vn_cfg.struct_size) return fail("tb_vecnorm_apply: no normaliser attached (tb_set_vecnorm)");
+  if (what != TB_VECNORM_OBS && what != TB_VECNORM_REWARD) return fail("tb_vecnorm_apply: unknown what %d", what);
+  const int od = tb_obs_dim(c->cfg.env_kind), width = what == TB_VECNORM_OBS ? od : 1;
+  if (rows < 0 || rows > (int64_t)INT32_MAX * kBlock / width)  // (one thread per float, a grid of at most 2^31 - 1 CTAs)
+    return fail("tb_vecnorm_apply: rows must be in 0 .. %lld, got %lld", (long long)((int64_t)INT32_MAX * kBlock / width),
+                (long long)rows);
+  if (rows > 0 && (!d_in || !d_out)) return fail("tb_vecnorm_apply: d_in and d_out are required");  // (an empty tensor's is NULL)
+  if (check_fault(c, "tb_vecnorm_apply")) return 1;
+  const tb_vecnorm &v = c->vn_cfg;
+  const bool obs = what == TB_VECNORM_OBS;
+  const int64_t count = rows * width;
+  const unsigned grid = std::max<unsigned>(1u, grid_for(count, kBlock));  // one launch, rows = 0 included
+  return with_kind(c->cfg.env_kind, [&](auto kind) {
+    return launch(c, kPlain, vecnorm_apply_kernel<Dims<kind>::obs>, grid, kBlock, (cudaStream_t)stream, (const double *)c->vn.stats.get(),
+                  d_in, d_out, count, (int)!obs, obs ? v.norm_obs : v.norm_reward, obs ? v.clip_obs : v.clip_reward, v.epsilon);
+  });
+}
+
 static EsIO es_io(tb_ctx *c) {
   EsIO io;
   std::memset(&io, 0, sizeof io);
@@ -3655,13 +3707,15 @@ int tb_sac_begin(tb_ctx *c, void *stream) {
     CU(dev_alloc(b.rew, n * sizeof(float)));
     CU(dev_alloc(b.done, n));
     CU(dev_alloc(b.base, sizeof(unsigned)));
+    CU(dev_alloc(b.pending, 1));
     c->sac = std::move(b);
   }
   if (!c->sac_grid) {  // (configuration calls, kept out of tb_sac_rollout so that it can be captured in any capture mode)
     CU(cudaDeviceGetAttribute(&c->sac_grid, cudaDevAttrMultiProcessorCount, c->cfg.device));
     if (with_kind(c->cfg.env_kind, [&](auto kind) {
-          constexpr int OBS = Dims<kind>::obs, ACT = Dims<kind>::act;
-          CU(cudaFuncSetAttribute(sac_kernel<OBS, ACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, SacLayout<OBS, ACT>::Smem));
+          constexpr int OBS = Dims<kind>::obs, ACT = Dims<kind>::act, smem = SacLayout<OBS, ACT>::Smem;
+          CU(cudaFuncSetAttribute(sac_kernel<OBS, ACT, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+          CU(cudaFuncSetAttribute(sac_kernel<OBS, ACT, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
           return 0;
         }))
       return 1;
@@ -3671,12 +3725,16 @@ int tb_sac_begin(tb_ctx *c, void *stream) {
   io.obs = c->sac.cur.get();
   if (launch_reset(c, io, nullptr, nullptr, s)) return 1;
   CU(cudaMemcpyAsync(c->sac.base.get(), step_counter(c), sizeof(unsigned), cudaMemcpyDeviceToDevice, s));
+  CU(cudaMemsetAsync(c->sac.pending.get(), 1, 1, s));  // the next TB_SAC_VECNORM rollout folds the reset (SB3's reset())
   return 0;
 }
 
 int tb_sac_rollout(tb_ctx *c, int k_steps, int mode, uint64_t noise_seed, const tb_sac_ring *ring, float *d_last_obs, void *stream) {
   if (k_steps < 1) return fail("tb_sac_rollout: k_steps must be >= 1");
-  if (mode != TB_SAC_SAMPLE && mode != TB_SAC_MEAN && mode != TB_SAC_UNIFORM) return fail("tb_sac_rollout: unknown mode %d", mode);
+  const bool norm = (mode & TB_SAC_VECNORM) != 0;
+  const int flags = mode;
+  mode &= ~TB_SAC_VECNORM;
+  if (mode != TB_SAC_SAMPLE && mode != TB_SAC_MEAN && mode != TB_SAC_UNIFORM) return fail("tb_sac_rollout: unknown mode %d", flags);
   if (ring) {
     if (ring->struct_size != sizeof(tb_sac_ring)) return fail("tb_sac_rollout: tb_sac_ring.struct_size mismatch");
     if (ring->slots < 1) return fail("tb_sac_rollout: ring slots must be >= 1");
@@ -3688,7 +3746,9 @@ int tb_sac_rollout(tb_ctx *c, int k_steps, int mode, uint64_t noise_seed, const 
   if (!c->cfg.auto_reset) return fail("tb_sac_rollout: the ring needs auto_reset = 1");
   if (!c->sac.cur) return fail("tb_sac_rollout: no tb_sac_begin on this context");
   if (mode != TB_SAC_UNIFORM && !c->sac_actor.w2) return fail("tb_sac_rollout: no actor (tb_set_sac_actor)");
+  if (norm && !c->vn_cfg.struct_size) return fail("tb_sac_rollout: TB_SAC_VECNORM needs a normaliser (tb_set_vecnorm)");
   if (check_fault(c, "tb_sac_rollout")) return 1;
+  const bool train = norm && vecnorm_training(c);
   const int64_t n = c->cfg.num_envs;
   cudaStream_t s = (cudaStream_t)stream;
   SacIO sio;
@@ -3700,9 +3760,19 @@ int tb_sac_rollout(tb_ctx *c, int k_steps, int mode, uint64_t noise_seed, const 
     sio.slots = ring->slots; sio.r_obs = ring->obs; sio.r_act = ring->act; sio.r_reward = ring->reward; sio.r_next = ring->next_obs;
     sio.r_done = ring->done;
   }
+  if (norm) {
+    sio.vn_stats = c->vn.stats.get(); sio.vn_clip_obs = c->vn_cfg.clip_obs; sio.vn_eps = c->vn_cfg.epsilon;
+    sio.vn_norm_obs = c->vn_cfg.norm_obs;
+  }
+  if (train) {  // the entry pass: while tb_sac_begin's reset is pending, zero the returns and fold the current observation
+    VecNormIO vio = vecnorm_io(c);
+    vio.obs = c->sac.cur.get(); vio.armed = c->sac.pending.get();
+    if (launch(c, kPlain, vecnorm_sac_entry_kernel, grid_for(n, kBlock), kBlock, s, vio)) return 1;
+    if (vecnorm_pass(c, vio, s)) return 1;
+  }
   return with_kind(c->cfg.env_kind, [&](auto kind) {
     constexpr int OBS = Dims<kind>::obs, ACT = Dims<kind>::act;
-    auto kernel = sac_kernel<OBS, ACT>;
+    auto kernel = norm ? sac_kernel<OBS, ACT, true> : sac_kernel<OBS, ACT, false>;
     constexpr int smem = SacLayout<OBS, ACT>::Smem;
     const int64_t tiles = (n + kBlock - 1) / kBlock;
     for (int t = 0; t <= k_steps; ++t) {  // launch t folds step t - 1 (t > 0) and acts for step t (t < K)
@@ -3717,6 +3787,7 @@ int tb_sac_rollout(tb_ctx *c, int k_steps, int mode, uint64_t noise_seed, const 
       io.actions = c->sac.act.get(); io.obs = c->sac.obs.get(); io.reward = c->sac.rew.get(); io.done = c->sac.done.get();
       io.term_obs = c->sac.term.get();
       if (launch_step(c, io, s)) return 1;
+      if (train && vecnorm_pass(c, io.obs, io.reward, io.done, s)) return 1;  // fold the step's raw observation and reward
     }
     return 0;
   });

@@ -242,10 +242,7 @@ class GpuPPO:
         under load_vecnormalize_npz's keys."""
         out = {"policy": self.ac.packed().cpu().numpy()}
         if self.normalize:
-            od, st = self.od, self.env.vecnorm_stats().cpu().numpy()
-            out.update(obs_mean=st[:od], obs_var=st[od:2 * od], obs_count=st[2 * od], ret_mean=st[2 * od + 1],
-                       ret_var=st[2 * od + 2], ret_count=st[2 * od + 3], clip_obs=10.0, clip_reward=10.0, gamma=self.gamma,
-                       epsilon=1e-8)
+            out.update(vecnormalize_entries(self.env, self.gamma))
         return out
 
     def save(self, path):
@@ -373,6 +370,14 @@ def load_sb3_policy_npz(path):
 
 VECNORMALIZE_KEYS = ("obs_mean", "obs_var", "obs_count", "ret_mean", "ret_var", "ret_count", "clip_obs", "clip_reward", "gamma",
                      "epsilon")
+
+
+def vecnormalize_entries(env, gamma):
+    """The record of env's normaliser (attached with SB3's VecNormalize defaults and this gamma) as numpy values under
+    load_vecnormalize_npz's keys."""
+    od, st = env.obs_dim, env.vecnorm_stats().cpu().numpy()
+    return dict(obs_mean=st[:od], obs_var=st[od:2 * od], obs_count=st[2 * od], ret_mean=st[2 * od + 1], ret_var=st[2 * od + 2],
+                ret_count=st[2 * od + 3], clip_obs=10.0, clip_reward=10.0, gamma=gamma, epsilon=1e-8)
 
 
 def load_vecnormalize_npz(path, obs_dim=None):

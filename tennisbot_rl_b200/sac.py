@@ -10,9 +10,16 @@ not fit 16 k envs stepping in lock step.  DESIGN.md section 4.2 records the swee
 
 One collection (pack the actor, tb_set_sac_actor, tb_sac_rollout of K steps) is captured once as a CUDA graph and replayed;
 one gradient step (batch indices drawn on the device, uniform over the filled rows) is captured as another.
+
+normalize=True is SB3's SAC on a VecNormalize env (its defaults, SAC's gamma): the in-kernel actor acts on normalised
+observations and the statistics are folded on the device after every env step (TB_SAC_VECNORM); the ring stays raw, and each
+gradient step normalises its sampled batch with the record as it stands (tb_vecnorm_apply), as SB3's ReplayBuffer.sample(env=...)
+does.  Reported returns stay raw.
 """
 import math
 import time
+
+import numpy as np
 
 import torch
 import torch.nn as nn
@@ -20,6 +27,7 @@ import torch.nn.functional as F
 
 from . import _lib
 from .batch import TennisBatch
+from .ppo import vecnormalize_entries
 
 LOG_STD_MIN, LOG_STD_MAX = -20.0, 2.0  # SB3 sac/policies.py
 HIDDEN = _lib.SAC_HIDDEN
@@ -146,12 +154,16 @@ class GpuSAC:
     rows of the ring (slots x num_envs transitions)."""
 
     def __init__(self, env_id="SwingRacket-v0", num_envs=1024, steps=1, batch_size=1024, gradient_steps=8, slots=1024,
-                 precision="f64", seed=0, lr=3e-4, gamma=0.99, tau=0.005, learning_starts=100, device=0, eval_envs=1024):
+                 precision="f64", seed=0, lr=3e-4, gamma=0.99, tau=0.005, learning_starts=100, device=0, eval_envs=1024,
+                 normalize=False):
         torch.manual_seed(seed)
         self.env_id, self.seed = env_id, seed
         self.dev = torch.device("cuda", device)
         self.n, self.K, self.B, self.G, self.slots = int(num_envs), int(steps), int(batch_size), int(gradient_steps), int(slots)
         self.env = TennisBatch(env_id, self.n, device=device, seed=seed, precision=precision)
+        self.normalize = bool(normalize)
+        if self.normalize:  # attached before any graph capture; the first rollout folds tb_sac_begin's reset observation
+            self.env.set_vecnorm(gamma=gamma)
         self.od, self.ad = od, ad = self.env.obs_dim, self.env.act_dim
         self.actor = SacActor(od, ad).to(self.dev)
         self.critic = TwinCritic(od, ad).to(self.dev)
@@ -176,7 +188,7 @@ class GpuSAC:
         self.env.set_sac_actor(self.params)  # (allocates the library's image outside the graph capture)
         self.env.sac_begin()
         warm = max(1, math.ceil(learning_starts / n))  # SB3's learning_starts counts transitions of all envs
-        self.env.sac_rollout(warm, "uniform", self.ring, noise_seed=seed + 1)
+        self.env.sac_rollout(warm, "uniform", self.ring, noise_seed=seed + 1, normalize=self.normalize)
         self.steps_taken += warm
         self.collect_graph = self.update_graph = None
         self.losses = z(3)
@@ -188,7 +200,7 @@ class GpuSAC:
     def _collect_body(self):
         self.params.copy_(pack_sac_actor(self.actor))
         self.env.set_sac_actor(self.params)
-        self.env.sac_rollout(self.K, "sample", self.ring, noise_seed=self.seed + 1)
+        self.env.sac_rollout(self.K, "sample", self.ring, noise_seed=self.seed + 1, normalize=self.normalize)
 
     @torch.no_grad()
     def collect(self):
@@ -204,6 +216,9 @@ class GpuSAC:
         idx = (torch.rand(self.B, device=self.dev) * self.fill).long()
         f = self.flat
         batch = (f["obs"][idx], f["act"][idx], f["reward"][idx], f["next_obs"][idx], f["done"][idx].float())
+        if self.normalize:  # the gathered copies, in place, with the record at replay time
+            for x, what in ((batch[0], "obs"), (batch[2], "reward"), (batch[3], "obs")):
+                self.env.vecnorm_apply(x, what, out=x)
         noise = torch.randn(self.B, self.ad, device=self.dev)
         next_noise = torch.randn(self.B, self.ad, device=self.dev)
         a_loss, c_loss, pi, logp, alpha = sac_losses(self.actor, self.critic, self.critic_target, self.log_alpha, batch,
@@ -290,22 +305,38 @@ class GpuSAC:
                 "eval_mean_return": evals[-1]["eval_mean_return"] if evals else None, "evaluations": evals,
                 "wall_s": time.time() - t0, "collect_s": self.collect_s, "update_s": self.update_s, "history": history}
 
+    def state_dict(self):
+        """The trained actor as numpy arrays: `policy`, tb_set_sac_actor's vector, and with normalize the normaliser's record
+        under load_vecnormalize_npz's keys."""
+        out = {"policy": pack_sac_actor(self.actor).cpu().numpy()}
+        if self.normalize:
+            out.update(vecnormalize_entries(self.env, self.gamma))
+        return out
+
+    def save(self, path):
+        """state_dict() as an npz.  Deploy: set_sac_actor(policy), and with normalize set_vecnorm(training=False, ...) from
+        load_vecnormalize_npz, then sac_rollout(..., normalize=True)."""
+        np.savez(path, **self.state_dict())
+
     @torch.no_grad()
     def evaluate(self, episodes=1):
         """Mean return of `episodes` whole episodes per env of eval_envs envs with the deterministic action tanh(mu), on a
-        context of its own with ring = NULL (so training's envs and ring are untouched)."""
+        context of its own with ring = NULL (so training's envs and ring are untouched).  With normalize, that context gets a
+        frozen copy of the training record first (SB3's sync_envs_normalization)."""
         if self._eval is None:
             self._eval = TennisBatch(self.env_id, self.eval_envs, device=self.dev.index, seed=self.seed + 1000,
                                      precision=self.env.precision)
         e = self._eval
         e.set_sac_actor(pack_sac_actor(self.actor).contiguous())
+        if self.normalize:
+            e.set_vecnorm(training=False, gamma=self.gamma, stats=self.env.vecnorm_stats())
         e.sac_begin()
         e.read_stats(clear=True)
         done = 0
         chunk = 26 if e.kind == _lib.ENV_SWING else 100
         # the statistics vector counts every episode that ends; stop once episodes x eval_envs of them have ended
         while done < episodes * self.eval_envs:
-            e.sac_rollout(chunk, "mean", None, noise_seed=0)
+            e.sac_rollout(chunk, "mean", None, noise_seed=0, normalize=self.normalize)
             done = int(e.read_stats()[0])
         st = e.read_stats(clear=True)
         return float(st[6] / 2 ** 20 / max(int(st[0]), 1))

@@ -1,7 +1,8 @@
 """Train with GpuSAC and time the in-kernel SAC actor.
 
 usage: train_sac.py ENV [--envs N] [--steps K] [--batch B] [--gradient-steps G] [--slots S] [--iters I] [--eval-every E]
-                        [--seed N] [--sweep] [--throughput] [--sizes N ...] [--no-train] [--out FILE.json]
+                        [--seed N] [--normalize] [--save FILE.npz] [--sweep] [--throughput] [--sizes N ...] [--no-train]
+                        [--out FILE.json]
 
 Prints the card's name and power limit, then:
   - training (unless --no-train): the curve (collection returns and deterministic evaluations) and the per-phase split of an
@@ -10,7 +11,11 @@ Prints the card's name and power limit, then:
   - --throughput: at each size, collection env-steps/s of tb_sac_rollout (in-kernel actor) against SacActor in torch float32 with
     TennisBatch.step in one CUDA graph (K steps per graph), the actor kernel's own time from torch.profiler (sac_kernel launches
     that evaluate the network) and its achieved TFLOP/s on the tensor cores (2 x N x 256 x 256 per step) against the BF16
-    data-sheet rate of one B200 (2250 dense TFLOP/s at 1000 W).
+    data-sheet rate of one B200 (2250 dense TFLOP/s at 1000 W);
+  - --throughput --normalize: instead, at each size, collection env-steps/s of tb_sac_rollout with and without TB_SAC_VECNORM
+    (a training normaliser: the statistics pass after every step), alternating the two graphs, and once the GpuSAC update
+    graph's time per gradient step with and without tb_vecnorm_apply on the sampled batch.
+--normalize trains with GpuSAC(normalize=True); --save writes GpuSAC.save's npz (actor, and the record with --normalize).
 """
 import argparse
 import json
@@ -39,8 +44,11 @@ def card():
 
 
 def train(args, envs, steps, batch, grad, slots, iters, eval_every):
-    s = GpuSAC(args.env, num_envs=envs, steps=steps, batch_size=batch, gradient_steps=grad, slots=slots, seed=args.seed)
+    s = GpuSAC(args.env, num_envs=envs, steps=steps, batch_size=batch, gradient_steps=grad, slots=slots, seed=args.seed,
+               normalize=args.normalize)
     out = s.train(iters, log=lambda m: print(m, flush=True), eval_every=eval_every)
+    if args.save:
+        s.save(args.save)
     s.env.close()
     out.pop("history")
     per_it = iters or 1
@@ -103,6 +111,68 @@ def throughput(env_id, n, K=26, reps=5):
     return fused, eager, kernel_ms
 
 
+def _graph_rate(b, K, reps, normalize):
+    """Captures K steps of tb_sac_rollout (sample, no ring) and returns a function timing `reps` replays: env-steps/s."""
+    b.sac_rollout(K, "sample", None, normalize=normalize)
+    torch.cuda.synchronize()
+    g = torch.cuda.CUDAGraph()
+    with torch.cuda.graph(g):
+        b.sac_rollout(K, "sample", None, normalize=normalize)
+    g.replay()
+    torch.cuda.synchronize()
+
+    def rate():
+        t0 = time.perf_counter()
+        for _ in range(reps):
+            g.replay()
+        torch.cuda.synchronize()
+        return reps * K * b.num_envs / (time.perf_counter() - t0)
+    return rate
+
+
+def throughput_normalize(env_id, n, K=26, reps=5, rounds=5):
+    """(env-steps/s without, with the normaliser): two contexts, the same actor, best of `rounds` alternating timings."""
+    torch.manual_seed(0)
+    rates = []
+    for normalize in (False, True):
+        b = TennisBatch(env_id, n, seed=1)
+        actor = SacActor(b.obs_dim, b.act_dim).cuda()
+        b.set_sac_actor(pack_sac_actor(actor).cuda())
+        if normalize:
+            b.set_vecnorm()
+        b.sac_begin()
+        rates.append((b, _graph_rate(b, K, reps, normalize)))
+    best = [0.0, 0.0]
+    for _ in range(rounds):
+        for j, (_, rate) in enumerate(rates):
+            best[j] = max(best[j], rate())
+    for b, _ in rates:
+        b.close()
+    return best
+
+
+def update_ms(env_id, rounds=5, reps=50):
+    """GpuSAC's update graph (the defaults: batch 1024), ms per gradient step without and with tb_vecnorm_apply, best of
+    `rounds` alternating timings of `reps` gradient steps."""
+    runs = []
+    for normalize in (False, True):
+        s = GpuSAC(env_id, seed=0, normalize=normalize)
+        s.update()  # captures the graph
+        torch.cuda.synchronize()
+        runs.append(s)
+    best = [float("inf")] * 2
+    for _ in range(rounds):
+        for j, s in enumerate(runs):
+            t0 = time.perf_counter()
+            for _ in range(reps):
+                s.update_graph.replay()
+            torch.cuda.synchronize()
+            best[j] = min(best[j], (time.perf_counter() - t0) / reps * 1e3)
+    for s in runs:
+        s.env.close()
+    return best
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("env", nargs="?", default="SwingRacket-v0")
@@ -114,6 +184,8 @@ def main():
     ap.add_argument("--iters", type=int, default=5000)
     ap.add_argument("--eval-every", type=int, default=1000)
     ap.add_argument("--seed", type=int, default=0)
+    ap.add_argument("--normalize", action="store_true")
+    ap.add_argument("--save", default=None)
     ap.add_argument("--sweep", action="store_true")
     ap.add_argument("--throughput", action="store_true")
     ap.add_argument("--no-train", action="store_true")
@@ -136,7 +208,19 @@ def main():
                                      "evaluations", "wall_s", "collect_s", "update_s")}
             print(json.dumps(row), flush=True)
             results["sweep"].append(row)
-    if args.throughput:
+    if args.throughput and args.normalize:
+        results["throughput_normalize"] = []
+        for n in args.sizes:
+            plain, norm = throughput_normalize(args.env, n)
+            row = {"envs": n, "env_steps_per_s": plain, "env_steps_per_s_normalize": norm,
+                   "us_per_step": 1e6 * n / plain, "us_per_step_normalize": 1e6 * n / norm}
+            print(json.dumps(row), flush=True)
+            results["throughput_normalize"].append(row)
+        plain, norm = update_ms(args.env)
+        row = {"update_ms_per_gradient_step": plain, "update_ms_per_gradient_step_normalize": norm}
+        print(json.dumps(row), flush=True)
+        results["update_normalize"] = row
+    elif args.throughput:
         results["throughput"] = []
         for n in args.sizes:
             fused, eager, kms = throughput(args.env, n)
