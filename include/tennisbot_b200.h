@@ -162,8 +162,17 @@ int tb_rollout(tb_ctx *ctx, int action_mode, int k_steps, float *d_obs, float *d
  *   log_std[2 -> 4]                                                                                          (4 floats) */
 #define TB_POLICY_FLOATS 9076
 #define TB_POLICY_FLOATS_HIT 9324
-/* count must be tb_policy_floats(env_kind) */
+/* count must be tb_policy_floats(env_kind).  Returns the context to one policy after tb_set_policies. */
 int tb_set_policy(tb_ctx *ctx, const float *d_params, int64_t count, void *stream);
+/* A population of policies for one context: d_params float32 [agents, tb_policy_floats(env_kind)], rows in tb_set_policy's
+ * layout.  agents >= 1 must divide N; env i acts with agent i / (N / agents).  Like tb_set_policy, a stream-ordered device to
+ * device copy into a library-owned buffer: it never synchronises, can be captured, and a replayed graph copies the weights
+ * d_params holds at replay time.  A call that needs more floats than the buffer holds allocates a larger one (cudaMalloc, and
+ * cudaFree of the old one, which waits for the device): make the largest call before capturing, and capture again after a
+ * call that grew the buffer, since graphs captured earlier refer to the old one.  Fails on a NULL d_params, agents < 1,
+ * agents not dividing N, count != agents x tb_policy_floats(env_kind), and on a faulted context.  agents = 1 is
+ * tb_set_policy. */
+int tb_set_policies(tb_ctx *ctx, const float *d_params, int64_t agents, int64_t count, void *stream);
 /* K env steps with actions sampled from the policy: per step one policy_kernel launch (forward, Philox Gaussian noise,
  * log-density, value) followed by tb_step's launches, all on `stream`, nothing synchronises - capturable in a CUDA graph.
  * d_obs float32 [K, N, obs_dim]: d_obs[0] must hold the current observation (from tb_reset or the previous rollout's
@@ -173,7 +182,11 @@ int tb_set_policy(tb_ctx *ctx, const float *d_params, int64_t count, void *strea
  * value (GAE bootstrap).  d_actions, d_logp, d_value, d_last_value may be NULL.  deterministic = 1: action = mean
  * (model.predict(deterministic=True)); else stochastic, as validate_swing.py:35 rolls the policy.  The noise streams
  * are keyed (noise_seed, global env id, the context's env-step counter, a device word): independent of the env's own streams
- * and of the sharding, and fresh on every replay of a captured graph. */
+ * and of the sharding, and fresh on every replay of a captured graph.
+ * After tb_set_policies with agents > 1, env i acts with agent i / (N / agents): every buffer, the noise and the launch count
+ * stay as they are, so agent p's envs give what a context of N / agents envs with env_id_offset = p N / agents and the same
+ * seeds gives with that agent's policy.  tb_read_stats still sums over the whole context.  Such a rollout fails while a
+ * normaliser is attached (tb_set_vecnorm keeps one record per context). */
 int tb_policy_rollout(tb_ctx *ctx, int k_steps, int deterministic, uint64_t noise_seed, float *d_obs, float *d_actions,
                       float *d_logp, float *d_value, float *d_reward, uint8_t *d_done, float *d_last_obs,
                       float *d_last_value, void *stream);

@@ -74,7 +74,7 @@ SIGNATURES = {
     "tb_set_param": [_vp, _str, _dbl], "tb_get_param": [_vp, _str, _dblp], "tb_set_control_mode": [_vp, _i32],
     "tb_reset": [_vp, _vp, _vp, _vp], "tb_reset_from": [_vp, _vp, _vp, _vp, _vp],
     "tb_step": [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp], "tb_rollout": [_vp, _i32, _i32, _vp, _vp, _vp, _vp],
-    "tb_set_policy": [_vp, _vp, _i64, _vp],
+    "tb_set_policy": [_vp, _vp, _i64, _vp], "tb_set_policies": [_vp, _vp, _i64, _i64, _vp],
     "tb_policy_rollout": [_vp, _i32, _i32, _u64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
     "tb_set_vecnorm": [_vp, C.POINTER(TbVecNorm), _vp, _vp], "tb_get_vecnorm": [_vp, _vp, _vp],
     "tb_vecnorm_apply": [_vp, _vp, _i64, _i32, _vp, _vp],

@@ -139,9 +139,22 @@ class TennisBatch:
             raise ValueError(f"policy parameter vector must have {want} floats for this env, got {p.numel()}")
         _lib.check(self.lib.tb_set_policy(self.h, _dptr(p), p.numel(), self._stream()))
 
+    def set_policies(self, params):
+        """A population: params float32 CUDA tensor [P, policy_floats] on this batch's device, rows in set_policy's layout, P
+        dividing num_envs.  Env i acts with row i // (num_envs // P) in the next policy_rollout; set_policy returns to one
+        policy.  A stream-ordered copy, capturable once the library's buffer holds P rows (tb_set_policies)."""
+        want = _lib.POLICY_FLOATS if self.kind == _lib.ENV_SWING else _lib.POLICY_FLOATS_HIT
+        agents = int(params.shape[0]) if torch.is_tensor(params) and params.dim() == 2 else -1
+        if agents < 1 or self.num_envs % agents:
+            raise ValueError(f"set_policies: params must have shape (P, {want}) with P dividing {self.num_envs}, got "
+                             f"{tuple(params.shape) if torch.is_tensor(params) else type(params).__name__}")
+        self._need("set_policies", params, "params", (agents, want))
+        _lib.check(self.lib.tb_set_policies(self.h, _dptr(params), agents, agents * want, self._stream()))
+
     def policy_rollout(self, obs, reward, done, last_obs, actions=None, logp=None, value=None, last_value=None,
                        deterministic=False, noise_seed=0):
-        """K = obs.shape[0] env steps with actions sampled in-kernel from the policy set by set_policy.  obs[0] must hold
+        """K = obs.shape[0] env steps with actions sampled in-kernel from the policy set by set_policy (or, after
+        set_policies, env i from row i // (num_envs // P)).  obs[0] must hold
         the current observation.  obs [K, N, obs_dim], actions [K, N, act_dim], reward / logp / value [K, N], last_obs
         [N, obs_dim], last_value [N]: contiguous float32 tensors on this batch's device; done [K, N] uint8.  The library
         writes through raw pointers, so every buffer is checked here."""

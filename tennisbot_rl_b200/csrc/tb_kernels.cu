@@ -1382,6 +1382,8 @@ struct PolicyIO {
   float *vn_reward;        // [N] the previous step's raw reward, replaced by its normalised value (policy tower), may be nullptr
   double vn_clip_obs, vn_clip_reward, vn_eps;
   int vn_norm_obs, vn_norm_reward;
+  // POP instances only (tb_set_policies): params holds one PolLayout row per agent; env i acts with agent i / envs_per_agent
+  int64_t envs_per_agent;
 };
 // VecNormalize's two formulas in float64 with each operation rounded (no contraction), so that numpy reproduces them bit for
 // bit: clip((o - mean) / sqrt(var + eps), -clip, clip), and the same for a reward with mean 0
@@ -1391,101 +1393,116 @@ __device__ __forceinline__ float vn_apply(float v, double mean, double var, doub
 }
 // grid (ceil(N / 128), 2): blockIdx.y = 0 the policy tower (action, log-density), 1 the value tower.  NORM: the normalising
 // instance of tb_policy_rollout with a normaliser attached; the policy tower also writes vn_obs and vn_reward.
-template <int OBS, int ACT, bool NORM>
+// POP: the population instance (tb_set_policies, agents > 1).  A CTA stages the tower of each agent its 128 envs belong to in
+// turn, and only that agent's threads compute with it: one pass when envs_per_agent is a multiple of 128, up to 128 passes
+// (one env per agent) when agents straddle the CTA.
+template <int OBS, int ACT, bool NORM, bool POP>
 __global__ void __launch_bounds__(kBlock) policy_kernel(const __grid_constant__ PolicyIO io) {
   using L = PolLayout<OBS, ACT>;
   static_assert(OBS % 2 == 0 && ACT % 2 == 0, "observation rows are read as float2 / float4, actions written as float2");
+  static_assert(!(NORM && POP), "the normaliser keeps one record per context: no population instance");
   __shared__ __align__(16) float P[L::PiTower + pad4(ACT)];
   const bool vf = blockIdx.y != 0;
   pdl_wait();
   if (vf ? io.value == nullptr : (!io.act_raw && !io.act_env && !io.logp) && !(NORM && (io.vn_obs || io.vn_reward))) return;
-  {
-    const float4 *src = reinterpret_cast<const float4 *>(io.params + (vf ? L::PiTower : 0));
-    const int nv = (vf ? L::VfTower : L::PiTower) / 4;
-    for (int i = threadIdx.x; i < nv; i += kBlock) reinterpret_cast<float4 *>(P)[i] = src[i];
-    if (!vf && threadIdx.x < pad4(ACT) / 4) reinterpret_cast<float4 *>(P + L::PiTower)[threadIdx.x] = reinterpret_cast<const float4 *>(io.params + L::LogStd)[threadIdx.x];
+  int64_t agent = 0, last_agent = 0;  // POP: the agents of this CTA's first and last env
+  if (POP) {
+    const int64_t first = (int64_t)blockIdx.x * kBlock;
+    agent = first / io.envs_per_agent;
+    last_agent = (min(first + kBlock, io.n) - 1) / io.envs_per_agent;
   }
-  __syncthreads();
-  const int64_t me = (int64_t)blockIdx.x * kBlock + threadIdx.x;
-  if (me < io.n) {
-    float x[OBS];
-    if (OBS % 4 == 0) {  // 48 B rows (Tennisbot-v0): three float4
-#pragma unroll
-      for (int j = 0; j < OBS / 4; ++j) {
-        const float4 a = reinterpret_cast<const float4 *>(io.obs + me * OBS)[j];
-        x[4 * j] = a.x; x[4 * j + 1] = a.y; x[4 * j + 2] = a.z; x[4 * j + 3] = a.w;
-      }
-    } else {  // 24 B rows (SwingRacket-v0): three float2
-#pragma unroll
-      for (int j = 0; j < OBS / 2; ++j) {
-        const float2 a = reinterpret_cast<const float2 *>(io.obs + me * OBS)[j];
-        x[2 * j] = a.x; x[2 * j + 1] = a.y;
-      }
+  for (;; ++agent) {
+    {
+      const float *par = POP ? io.params + agent * L::Floats : io.params;
+      const float4 *src = reinterpret_cast<const float4 *>(par + (vf ? L::PiTower : 0));
+      const int nv = (vf ? L::VfTower : L::PiTower) / 4;
+      for (int i = threadIdx.x; i < nv; i += kBlock) reinterpret_cast<float4 *>(P)[i] = src[i];
+      if (!vf && threadIdx.x < pad4(ACT) / 4) reinterpret_cast<float4 *>(P + L::PiTower)[threadIdx.x] = reinterpret_cast<const float4 *>(par + L::LogStd)[threadIdx.x];
     }
-    if (NORM) {
-      if (io.vn_norm_obs) {
+    __syncthreads();
+    const int64_t me = (int64_t)blockIdx.x * kBlock + threadIdx.x;
+    if (me < io.n && (!POP || (me >= agent * io.envs_per_agent && me < (agent + 1) * io.envs_per_agent))) {
+      float x[OBS];
+      if (OBS % 4 == 0) {  // 48 B rows (Tennisbot-v0): three float4
 #pragma unroll
-        for (int c = 0; c < OBS; ++c) x[c] = vn_apply(x[c], io.vn_stats[c], io.vn_stats[OBS + c], io.vn_eps, io.vn_clip_obs);
-      }
-      if (!vf && io.vn_obs) {
-        float2 *q = reinterpret_cast<float2 *>(io.vn_obs + me * OBS);
-#pragma unroll
-        for (int j = 0; j < OBS / 2; ++j) q[j] = make_float2(x[2 * j], x[2 * j + 1]);
-      }
-      if (!vf && io.vn_reward && io.vn_norm_reward)
-        io.vn_reward[me] = vn_apply(io.vn_reward[me], 0.0, io.vn_stats[2 * OBS + 2], io.vn_eps, io.vn_clip_reward);
-      if (!vf && !io.act_raw && !io.act_env && !io.logp) return;  // the last launch: normalised reward only
-    }
-    float h[32];
-    tower<OBS, ACT>(P, x, h);
-    if (!vf) {
-      const float *Wa = P + L::Head, *ba = P + L::Head + ACT * 32, *ls = P + L::PiTower;
-      // one Box-Muller pair (two uniforms) per two components: one Philox call per four components
-      constexpr int NR = (ACT + 3) / 4;
-      uint32_t rr[4 * NR];
-      const uint32_t tick = *io.tick;
-#pragma unroll
-      for (int j = 0; j < NR; ++j) philox4x32(io.seed, (uint64_t)(io.id_offset + me), tick, stream_word(kStreamPolicy, 0, j), rr + 4 * j);
-      float raw[ACT], lp = 0.0f;
-#pragma unroll
-      for (int o = 0; o < ACT; ++o) {
-        float mu = ba[o];
-#pragma unroll
-        for (int i = 0; i < 32; ++i) mu = fmaf(Wa[o * 32 + i], h[i], mu);
-        // Box-Muller on a pair of uniforms: component o takes the cosine (o even) or sine (o odd) branch of pair o / 2
-        const float u1 = ((float)(rr[2 * (o / 2)] >> 8) + 0.5f) * (1.0f / 16777216.0f), u2 = (float)(rr[2 * (o / 2) + 1] >> 8) * (1.0f / 16777216.0f);
-        const float rad = sqrtf(-2.0f * logf(u1));
-        float sc;
-        if (OBS == 6 && ACT == 6) {  // SwingRacket-v0 keeps sinf / cosf, so its rollouts stay what they were (their
-          const float ang = 6.283185307179586f * u2;  // large-argument range reduction costs a 32-byte stack frame)
-          sc = (o & 1) ? sinf(ang) : cosf(ang);
-        } else {  // sin / cos of pi * 2 u2, 2 u2 in [0, 2): exact range reduction, nothing in local memory
-          sc = (o & 1) ? sinpif(2.0f * u2) : cospif(2.0f * u2);
+        for (int j = 0; j < OBS / 4; ++j) {
+          const float4 a = reinterpret_cast<const float4 *>(io.obs + me * OBS)[j];
+          x[4 * j] = a.x; x[4 * j + 1] = a.y; x[4 * j + 2] = a.z; x[4 * j + 3] = a.w;
         }
-        const float eps = io.deterministic ? 0.0f : rad * sc;
-        raw[o] = fmaf(expf(ls[o]), eps, mu);
-        lp += -0.5f * eps * eps - ls[o] - 0.9189385332046727f;
+      } else {  // 24 B rows (SwingRacket-v0): three float2
+#pragma unroll
+        for (int j = 0; j < OBS / 2; ++j) {
+          const float2 a = reinterpret_cast<const float2 *>(io.obs + me * OBS)[j];
+          x[2 * j] = a.x; x[2 * j + 1] = a.y;
+        }
       }
-      if (io.act_raw) {
-        float2 *q = reinterpret_cast<float2 *>(io.act_raw + me * ACT);
+      if (NORM) {
+        if (io.vn_norm_obs) {
 #pragma unroll
-        for (int j = 0; j < ACT / 2; ++j) q[j] = make_float2(raw[2 * j], raw[2 * j + 1]);
+          for (int c = 0; c < OBS; ++c) x[c] = vn_apply(x[c], io.vn_stats[c], io.vn_stats[OBS + c], io.vn_eps, io.vn_clip_obs);
+        }
+        if (!vf && io.vn_obs) {
+          float2 *q = reinterpret_cast<float2 *>(io.vn_obs + me * OBS);
+#pragma unroll
+          for (int j = 0; j < OBS / 2; ++j) q[j] = make_float2(x[2 * j], x[2 * j + 1]);
+        }
+        if (!vf && io.vn_reward && io.vn_norm_reward)
+          io.vn_reward[me] = vn_apply(io.vn_reward[me], 0.0, io.vn_stats[2 * OBS + 2], io.vn_eps, io.vn_clip_reward);
+        if (!vf && !io.act_raw && !io.act_env && !io.logp) return;  // the last launch: normalised reward only
       }
-      if (io.act_env) {
-        float2 *q = reinterpret_cast<float2 *>(io.act_env + me * ACT);
+      float h[32];
+      tower<OBS, ACT>(P, x, h);
+      if (!vf) {
+        const float *Wa = P + L::Head, *ba = P + L::Head + ACT * 32, *ls = P + L::PiTower;
+        // one Box-Muller pair (two uniforms) per two components: one Philox call per four components
+        constexpr int NR = (ACT + 3) / 4;
+        uint32_t rr[4 * NR];
+        const uint32_t tick = *io.tick;
 #pragma unroll
-        for (int o = 0; o < ACT; ++o) raw[o] = fminf(fmaxf(raw[o], -1.0f), 1.0f);
+        for (int j = 0; j < NR; ++j) philox4x32(io.seed, (uint64_t)(io.id_offset + me), tick, stream_word(kStreamPolicy, 0, j), rr + 4 * j);
+        float raw[ACT], lp = 0.0f;
 #pragma unroll
-        for (int j = 0; j < ACT / 2; ++j) q[j] = make_float2(raw[2 * j], raw[2 * j + 1]);
+        for (int o = 0; o < ACT; ++o) {
+          float mu = ba[o];
+#pragma unroll
+          for (int i = 0; i < 32; ++i) mu = fmaf(Wa[o * 32 + i], h[i], mu);
+          // Box-Muller on a pair of uniforms: component o takes the cosine (o even) or sine (o odd) branch of pair o / 2
+          const float u1 = ((float)(rr[2 * (o / 2)] >> 8) + 0.5f) * (1.0f / 16777216.0f), u2 = (float)(rr[2 * (o / 2) + 1] >> 8) * (1.0f / 16777216.0f);
+          const float rad = sqrtf(-2.0f * logf(u1));
+          float sc;
+          if (OBS == 6 && ACT == 6) {  // SwingRacket-v0 keeps sinf / cosf, so its rollouts stay what they were (their
+            const float ang = 6.283185307179586f * u2;  // large-argument range reduction costs a 32-byte stack frame)
+            sc = (o & 1) ? sinf(ang) : cosf(ang);
+          } else {  // sin / cos of pi * 2 u2, 2 u2 in [0, 2): exact range reduction, nothing in local memory
+            sc = (o & 1) ? sinpif(2.0f * u2) : cospif(2.0f * u2);
+          }
+          const float eps = io.deterministic ? 0.0f : rad * sc;
+          raw[o] = fmaf(expf(ls[o]), eps, mu);
+          lp += -0.5f * eps * eps - ls[o] - 0.9189385332046727f;
+        }
+        if (io.act_raw) {
+          float2 *q = reinterpret_cast<float2 *>(io.act_raw + me * ACT);
+#pragma unroll
+          for (int j = 0; j < ACT / 2; ++j) q[j] = make_float2(raw[2 * j], raw[2 * j + 1]);
+        }
+        if (io.act_env) {
+          float2 *q = reinterpret_cast<float2 *>(io.act_env + me * ACT);
+#pragma unroll
+          for (int o = 0; o < ACT; ++o) raw[o] = fminf(fmaxf(raw[o], -1.0f), 1.0f);
+#pragma unroll
+          for (int j = 0; j < ACT / 2; ++j) q[j] = make_float2(raw[2 * j], raw[2 * j + 1]);
+        }
+        if (io.logp) io.logp[me] = lp;
+      } else {
+        const float *Wv = P + L::Head;
+        float v = Wv[32];
+#pragma unroll
+        for (int i = 0; i < 32; ++i) v = fmaf(Wv[i], h[i], v);
+        io.value[me] = v;
       }
-      if (io.logp) io.logp[me] = lp;
-    } else {
-      const float *Wv = P + L::Head;
-      float v = Wv[32];
-#pragma unroll
-      for (int i = 0; i < 32; ++i) v = fmaf(Wv[i], h[i], v);
-      io.value[me] = v;
     }
+    if (!POP || agent == last_agent) break;
+    __syncthreads();  // every thread is done with this agent's tower before the next agent's is staged over it
   }
   pdl_trigger();
 }
@@ -2889,9 +2906,11 @@ struct SacBufs {              // tb_sac_begin: per-env staging between sac_kerne
   DevPtr<unsigned> base;
   DevPtr<uint8_t> pending;    // 1 from tb_sac_begin until a TB_SAC_VECNORM rollout with a training normaliser folds the reset
 };
-struct PolicyBufs {           // tb_set_policy
-  DevPtr<float> params;       // tb_policy_floats(env_kind) parameters
+struct PolicyBufs {           // tb_set_policy / tb_set_policies
+  DevPtr<float> params;       // [agents, tb_policy_floats(env_kind)] parameters
   DevPtr<float> act;          // [N, act_dim] clipped actions handed from policy_kernel to step_kernel
+  int64_t params_cap = 0;     // floats params holds
+  int64_t agents = 1;         // rows the rollout uses: env i acts with row i / (N / agents)
 };
 struct VecNormBufs {          // tb_set_vecnorm (see VecNormIO)
   DevPtr<double> stats, ret, part;
@@ -3374,20 +3393,41 @@ int tb_rollout(tb_ctx *c, int action_mode, int k_steps, float *d_obs, float *d_r
   });
 }
 
+// agents policy rows -> the library's buffer, grown when it holds fewer (cudaMalloc / cudaFree: not while capturing)
+static int copy_policies(tb_ctx *c, const float *d_params, int64_t agents, cudaStream_t s) {
+  const int64_t floats = agents * tb_policy_floats(c->cfg.env_kind);
+  if (c->policy.params_cap < floats) {
+    PolicyBufs p;
+    CU(dev_alloc(p.params, (size_t)floats * sizeof(float)));
+    if (c->policy.act) p.act = std::move(c->policy.act);
+    else CU(dev_alloc(p.act, (size_t)c->cfg.num_envs * tb_act_dim(c->cfg.env_kind) * sizeof(float)));
+    p.params_cap = floats;
+    c->policy = std::move(p);
+  }
+  CU(cudaMemcpyAsync(c->policy.params.get(), d_params, (size_t)floats * sizeof(float), cudaMemcpyDeviceToDevice, s));
+  c->policy.agents = agents;
+  return 0;
+}
+
 int tb_set_policy(tb_ctx *c, const float *d_params, int64_t count, void *stream) {
   GUARD(c);
   const int64_t want = tb_policy_floats(c->cfg.env_kind);
   if (!d_params || count != want)
     return fail("tb_set_policy: expected tb_policy_floats(env_kind) = %lld floats in device memory, got %lld", (long long)want,
                 (long long)count);
-  if (!c->policy.params) {
-    PolicyBufs p;
-    CU(dev_alloc(p.params, (size_t)want * sizeof(float)));
-    CU(dev_alloc(p.act, (size_t)c->cfg.num_envs * tb_act_dim(c->cfg.env_kind) * sizeof(float)));
-    c->policy = std::move(p);
-  }
-  CU(cudaMemcpyAsync(c->policy.params.get(), d_params, (size_t)want * sizeof(float), cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
-  return 0;
+  return copy_policies(c, d_params, 1, (cudaStream_t)stream);
+}
+
+int tb_set_policies(tb_ctx *c, const float *d_params, int64_t agents, int64_t count, void *stream) {
+  GUARD(c);
+  const int64_t n = c->cfg.num_envs, floats = tb_policy_floats(c->cfg.env_kind);
+  if (!d_params) return fail("tb_set_policies: d_params is NULL");
+  if (agents < 1 || n % agents) return fail("tb_set_policies: agents must be >= 1 and divide num_envs = %lld, got %lld", (long long)n, (long long)agents);
+  if (count != agents * floats)
+    return fail("tb_set_policies: expected agents x tb_policy_floats(env_kind) = %lld x %lld floats, got %lld", (long long)agents,
+                (long long)floats, (long long)count);
+  if (check_fault(c, "tb_set_policies")) return 1;
+  return copy_policies(c, d_params, agents, (cudaStream_t)stream);
 }
 
 int tb_policy_rollout(tb_ctx *c, int k_steps, int deterministic, uint64_t noise_seed, float *d_obs, float *d_actions, float *d_logp,
@@ -3400,17 +3440,21 @@ int tb_policy_rollout(tb_ctx *c, int k_steps, int deterministic, uint64_t noise_
   const int64_t n = c->cfg.num_envs;
   const int od = tb_obs_dim(c->cfg.env_kind), ad = tb_act_dim(c->cfg.env_kind);
   // with a normaliser: policy_kernel<.., true> reads the raw observation from vn.raw (from d_last_obs after the last step)
-  const bool vn = c->vn_cfg.struct_size != 0, train = vecnorm_training(c);
+  const bool vn = c->vn_cfg.struct_size != 0, train = vecnorm_training(c), pop = c->policy.agents > 1;
+  if (vn && pop)
+    return fail("tb_policy_rollout: a normaliser (tb_set_vecnorm) keeps one record per context, so it cannot serve %lld agents "
+                "(tb_set_policies); detach it or set one policy", (long long)c->policy.agents);
   void (*kernel)(PolicyIO) = nullptr;
   with_kind(c->cfg.env_kind, [&](auto kind) {
-    kernel = vn ? policy_kernel<Dims<kind>::obs, Dims<kind>::act, true> : policy_kernel<Dims<kind>::obs, Dims<kind>::act, false>;
+    constexpr int O = Dims<kind>::obs, A = Dims<kind>::act;
+    kernel = vn ? policy_kernel<O, A, true, false> : pop ? policy_kernel<O, A, false, true> : policy_kernel<O, A, false, false>;
     return 0;
   });
   cudaStream_t s = (cudaStream_t)stream;
   PolicyIO pio;
   std::memset(&pio, 0, sizeof pio);
   pio.params = c->policy.params.get(); pio.n = n; pio.id_offset = c->cfg.env_id_offset; pio.seed = noise_seed; pio.deterministic = deterministic;
-  pio.act_env = c->policy.act.get(); pio.tick = step_counter(c);
+  pio.act_env = c->policy.act.get(); pio.tick = step_counter(c); pio.envs_per_agent = n / c->policy.agents;
   if (vn) {
     pio.vn_stats = c->vn.stats.get(); pio.vn_clip_obs = c->vn_cfg.clip_obs; pio.vn_clip_reward = c->vn_cfg.clip_reward;
     pio.vn_eps = c->vn_cfg.epsilon; pio.vn_norm_obs = c->vn_cfg.norm_obs; pio.vn_norm_reward = c->vn_cfg.norm_reward;
