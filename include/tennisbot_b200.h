@@ -185,11 +185,21 @@ int tb_set_policies(tb_ctx *ctx, const float *d_params, int64_t agents, int64_t 
  * and of the sharding, and fresh on every replay of a captured graph.
  * After tb_set_policies with agents > 1, env i acts with agent i / (N / agents): every buffer, the noise and the launch count
  * stay as they are, so agent p's envs give what a context of N / agents envs with env_id_offset = p N / agents and the same
- * seeds gives with that agent's policy.  tb_read_stats still sums over the whole context.  Such a rollout fails while a
- * normaliser is attached (tb_set_vecnorm keeps one record per context). */
+ * seeds gives with that agent's policy.  tb_read_stats still sums over the whole context.  With a normaliser attached, the
+ * P policies and the A records of tb_set_vecnorms must agree: P = A = 1 is the one-record rollout, P = A > 1 normalises env i
+ * with record i / (N / A), so agent p's envs also give what the shard gives with record p attached by tb_set_vecnorm; any
+ * other pair fails, naming both counts. */
 int tb_policy_rollout(tb_ctx *ctx, int k_steps, int deterministic, uint64_t noise_seed, float *d_obs, float *d_actions,
                       float *d_logp, float *d_value, float *d_reward, uint8_t *d_done, float *d_last_obs,
                       float *d_last_value, void *stream);
+/* tb_policy_rollout that also returns the env's reward before normalisation: d_raw_reward float32 [K, N] (may be NULL, which is
+ * tb_policy_rollout).  Each step's raw reward is copied there with one cudaMemcpyAsync device to device right after the step,
+ * which is not a kernel launch: the launch count is tb_policy_rollout's.  Without a normaliser it equals d_reward.  With
+ * norm_reward, d_reward comes back normalised by each agent's own record, so per-agent episode returns are summed from
+ * d_raw_reward. */
+int tb_policy_rollout_raw(tb_ctx *ctx, int k_steps, int deterministic, uint64_t noise_seed, float *d_obs, float *d_actions,
+                          float *d_logp, float *d_value, float *d_reward, float *d_raw_reward, uint8_t *d_done,
+                          float *d_last_obs, float *d_last_value, void *stream);
 
 /* ---- observation and reward normalisation of the policy rollout: SB3 1.8 VecNormalize, on the device.
  * Statistics, float64, RunningMeanStd layout: obs mean [obs_dim], obs var [obs_dim], obs count, ret mean, ret var, ret count
@@ -219,7 +229,12 @@ int tb_policy_rollout(tb_ctx *ctx, int k_steps, int deterministic, uint64_t nois
  * tb_reset_from add one launch while a training normaliser is attached.  The int64 statistics (tb_read_stats) stay raw;
  * tb_step, tb_rollout, tb_reset_host, tb_step_host and the ES entry points ignore the normaliser, and so does tb_sac_rollout
  * unless its mode carries TB_SAC_VECNORM (see there; tb_vecnorm_apply normalises replay samples).  Each context keeps its
- * own statistics: shards with env_id_offset do not reproduce the statistics of one batch. */
+ * own statistics: shards with env_id_offset do not reproduce the statistics of one batch.
+ * A population (tb_set_policies) normalises with one record per agent (tb_set_vecnorms): every rule above holds per agent,
+ * over that agent's N / A envs, and the statistics pass stays two launches (a segmented pass: es_norm_blocks(N / A) CTAs per
+ * agent, laid out as a context of N / A envs lays them out, then one CTA per agent), so record p is bit for bit the record of a
+ * context of N / A envs at env_id_offset p N / A.  The launch counts above hold for any A.  One armed byte serves the context:
+ * a full reset resets every agent. */
 typedef struct tb_vecnorm {
   uint32_t struct_size; /* sizeof(tb_vecnorm) */
   int32_t training, norm_obs, norm_reward;
@@ -232,15 +247,32 @@ typedef struct tb_vecnorm {
  * clip_reward or epsilon that is not finite and above 0, gamma outside [0, 1], stats with a count <= 0, a variance < 0 or an
  * entry that is not finite, and on a faulted context.  Detaching keeps the buffers; attaching again starts from d_stats. */
 int tb_set_vecnorm(tb_ctx *ctx, const tb_vecnorm *cfg, const double *d_stats, void *stream);
+/* One record per agent: `agents` records of one configuration cfg.  d_stats double [agents, TB_VECNORM_WORDS(obs_dim)]: the
+ * records to start from (NULL: all fresh); each row is checked as tb_set_vecnorm checks its record, and a failure names the
+ * row; with d_stats the call synchronises `stream`.  agents >= 1 must divide N; agents = 1 is tb_set_vecnorm, with its kernels
+ * and launches, and cfg NULL detaches.  Zeroes the returns of all N envs and arms the reset fold (one launch).  A call that
+ * needs more records or partials than the buffers hold allocates larger ones (cudaMalloc, and cudaFree of the old ones, which
+ * waits for the device): as with tb_set_policies, make the largest call before capturing, and capture again after a call that
+ * grew them.  A rejected call leaves the context as it was. */
+int tb_set_vecnorms(tb_ctx *ctx, const tb_vecnorm *cfg, int64_t agents, const double *d_stats, void *stream);
 /* d_stats double [TB_VECNORM_WORDS(obs_dim)] = the current record (stream-ordered copy, never synchronises).  Fails when no
- * normaliser is attached. */
+ * normaliser is attached, and when more than one record is (tb_get_vecnorms reads them). */
 int tb_get_vecnorm(tb_ctx *ctx, double *d_stats, void *stream);
+/* d_stats double [agents, TB_VECNORM_WORDS(obs_dim)] = every record (stream-ordered copy, never synchronises).  Fails when no
+ * normaliser is attached or agents is not the number of records attached. */
+int tb_get_vecnorms(tb_ctx *ctx, double *d_stats, int64_t agents, void *stream);
+/* The library's record buffer, double [*agents, TB_VECNORM_WORDS(obs_dim)], and the number of records attached.  The kernels
+ * read a record when they run, so a stream-ordered write into a row (a PBT copy of one agent's record over another's) is seen
+ * by the next kernel that reads it, a replayed graph included; unlike tb_set_vecnorms it zeroes no return and arms no fold.
+ * The pointer stays valid until a tb_set_vecnorms call grows the buffer or the context is destroyed.  Fails when no normaliser
+ * is attached. */
+int tb_vecnorm_device_ptr(tb_ctx *ctx, double **d_records, int64_t *agents);
 /* d_out = rule 4's o^ of d_in float32 [rows, obs_dim] (what = TB_VECNORM_OBS), or rule 3's r^ of d_in float32 [rows]
  * (TB_VECNORM_REWARD), with the record as it stands when the kernel runs (a replayed graph sees the current statistics);
  * norm_obs = 0 (norm_reward = 0) copies.  What SB3's ReplayBuffer.sample(env=vec_normalize_env) does to a raw batch.  d_out
  * may be d_in.  One kernel launch (rows = 0 included, which reads nothing), never synchronises.  Fails when no normaliser is
  * attached, what is unknown, rows < 0 (or the grid would exceed 2^31 - 1 CTAs of 128 floats), d_in or d_out is NULL while
- * rows > 0, or the context is faulted. */
+ * rows > 0, or the context is faulted, or more than one record is attached (tb_set_vecnorms). */
 #define TB_VECNORM_OBS 0
 #define TB_VECNORM_REWARD 1
 int tb_vecnorm_apply(tb_ctx *ctx, const float *d_in, int64_t rows, int what, float *d_out, void *stream);
@@ -346,7 +378,7 @@ int tb_sac_begin(tb_ctx *ctx, void *stream);
  * = the terminal observation when done, else the step's observation.  ring = NULL stores nothing (evaluation).  d_last_obs
  * float32 [N, obs_dim] (may be NULL) receives the observation after the last step.  mode TB_SAC_SAMPLE and TB_SAC_MEAN need
  * tb_set_sac_actor.  Never synchronises: capturable in a CUDA graph.
- * mode | TB_SAC_VECNORM (fails when no normaliser is attached): SB3 SAC under VecNormalize, with the normaliser of tb_set_vecnorm.
+ * mode | TB_SAC_VECNORM (fails when no normaliser is attached, or more than one record is): SB3 SAC under VecNormalize, with the normaliser of tb_set_vecnorm.
  * After every env step (TB_SAC_UNIFORM included) a training normaliser folds the step's observation of all N envs (rule 1),
  * the return (rule 2) and zeroes the returns of done envs (rule 3); the actor acts on o^ (rule 4) with the statistics after
  * that fold.  The ring, d_last_obs and tb_read_stats stay RAW (SB3's get_original_obs / get_original_reward; a terminal

@@ -76,7 +76,10 @@ SIGNATURES = {
     "tb_step": [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp], "tb_rollout": [_vp, _i32, _i32, _vp, _vp, _vp, _vp],
     "tb_set_policy": [_vp, _vp, _i64, _vp], "tb_set_policies": [_vp, _vp, _i64, _i64, _vp],
     "tb_policy_rollout": [_vp, _i32, _i32, _u64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
+    "tb_policy_rollout_raw": [_vp, _i32, _i32, _u64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
     "tb_set_vecnorm": [_vp, C.POINTER(TbVecNorm), _vp, _vp], "tb_get_vecnorm": [_vp, _vp, _vp],
+    "tb_set_vecnorms": [_vp, C.POINTER(TbVecNorm), _i64, _vp, _vp], "tb_get_vecnorms": [_vp, _vp, _i64, _vp],
+    "tb_vecnorm_device_ptr": [_vp, C.POINTER(_vp), _i64p],
     "tb_vecnorm_apply": [_vp, _vp, _i64, _i32, _vp, _vp],
     "tb_es_begin": [_vp, _vp, _i64, _i64, _vp, _vp], "tb_es_rollout": [_vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
     "tb_es_begin_noise": [_vp, _vp, _i64, _i64, C.c_float, _u64, _u32, _vp, _vp],

@@ -152,12 +152,13 @@ class TennisBatch:
         _lib.check(self.lib.tb_set_policies(self.h, _dptr(params), agents, agents * want, self._stream()))
 
     def policy_rollout(self, obs, reward, done, last_obs, actions=None, logp=None, value=None, last_value=None,
-                       deterministic=False, noise_seed=0):
+                       deterministic=False, noise_seed=0, raw_reward=None):
         """K = obs.shape[0] env steps with actions sampled in-kernel from the policy set by set_policy (or, after
         set_policies, env i from row i // (num_envs // P)).  obs[0] must hold
         the current observation.  obs [K, N, obs_dim], actions [K, N, act_dim], reward / logp / value [K, N], last_obs
-        [N, obs_dim], last_value [N]: contiguous float32 tensors on this batch's device; done [K, N] uint8.  The library
-        writes through raw pointers, so every buffer is checked here."""
+        [N, obs_dim], last_value [N]: contiguous float32 tensors on this batch's device; done [K, N] uint8.  raw_reward
+        [K, N] (optional) receives the env's reward before normalisation (tb_policy_rollout_raw; reward itself without a
+        normaliser).  The library writes through raw pointers, so every buffer is checked here."""
         k, n = int(obs.shape[0]) if obs.dim() == 3 else -1, self.num_envs
         if k < 1:
             raise ValueError(f"policy_rollout: obs must have shape (K >= 1, {n}, {self.obs_dim}), got {tuple(obs.shape)}")
@@ -170,32 +171,65 @@ class TennisBatch:
         need(done, "done", (k, n), dtype=torch.uint8)
         need(last_obs, "last_obs", (n, self.obs_dim))
         need(last_value, "last_value", (n,), optional=True)
-        _lib.check(self.lib.tb_policy_rollout(self.h, k, int(bool(deterministic)), int(noise_seed) & (2 ** 64 - 1), _dptr(obs),
-                                              _dptr(actions), _dptr(logp), _dptr(value), _dptr(reward), _dptr(done), _dptr(last_obs),
-                                              _dptr(last_value), self._stream()))
+        need(raw_reward, "raw_reward", (k, n), optional=True)
+        _lib.check(self.lib.tb_policy_rollout_raw(self.h, k, int(bool(deterministic)), int(noise_seed) & (2 ** 64 - 1), _dptr(obs),
+                                                  _dptr(actions), _dptr(logp), _dptr(value), _dptr(reward), _dptr(raw_reward),
+                                                  _dptr(done), _dptr(last_obs), _dptr(last_value), self._stream()))
 
     # ------------------------------------------------------------------ normaliser of the policy rollout (tb_set_vecnorm)
     def set_vecnorm(self, training=True, norm_obs=True, norm_reward=True, clip_obs=10.0, clip_reward=10.0, gamma=0.99,
-                    epsilon=1e-8, stats=None):
+                    epsilon=1e-8, agents=1, stats=None):
         """Attach SB3 VecNormalize's observation / reward normalisation to policy_rollout (semantics in the header at
         tb_set_vecnorm).  stats: float64 [2 obs_dim + 4] to start from (obs mean, obs var, obs count, ret mean, ret var, ret
-        count), None = fresh; a given record is checked on the host, which synchronises the stream."""
-        self._need("set_vecnorm", stats, "stats", (_lib.vecnorm_words(self.obs_dim),), torch.float64, optional=True)
+        count), None = fresh; a given record is checked on the host, which synchronises the stream.  agents > 1: one record
+        per agent of a population (tb_set_vecnorms; env i uses record i // (num_envs // agents)), all with this
+        configuration, and stats is [agents, 2 obs_dim + 4]."""
+        words, agents = _lib.vecnorm_words(self.obs_dim), int(agents)
         cfg = _lib.TbVecNorm(C.sizeof(_lib.TbVecNorm), int(bool(training)), int(bool(norm_obs)), int(bool(norm_reward)),
                              float(clip_obs), float(clip_reward), float(gamma), float(epsilon))
-        _lib.check(self.lib.tb_set_vecnorm(self.h, C.byref(cfg), _dptr(stats), self._stream()))
+        if agents == 1:
+            self._need("set_vecnorm", stats, "stats", (words,), torch.float64, optional=True)
+            _lib.check(self.lib.tb_set_vecnorm(self.h, C.byref(cfg), _dptr(stats), self._stream()))
+            return
+        if agents < 1 or self.num_envs % agents:
+            raise ValueError(f"set_vecnorm: agents must be >= 1 and divide {self.num_envs}, got {agents}")
+        self._need("set_vecnorm", stats, "stats", (agents, words), torch.float64, optional=True)
+        _lib.check(self.lib.tb_set_vecnorms(self.h, C.byref(cfg), agents, _dptr(stats), self._stream()))
 
     def clear_vecnorm(self):
         """Detach the normaliser: policy_rollout behaves as if none had been attached."""
         _lib.check(self.lib.tb_set_vecnorm(self.h, None, None, self._stream()))
 
+    def _vecnorm_buffer(self):
+        """(device address, records) of the library's record buffer; (None, 1) when no normaliser is attached."""
+        p, agents = C.c_void_p(), C.c_int64()
+        if self.lib.tb_vecnorm_device_ptr(self.h, C.byref(p), C.byref(agents)) != 0:
+            return None, 1
+        return p.value, agents.value
+
     def vecnorm_stats(self, out=None):
-        """float64 device tensor [2 obs_dim + 4]: the normaliser's current record (stream-ordered copy)."""
+        """float64 device tensor [2 obs_dim + 4]: the normaliser's current record (stream-ordered copy); [A, 2 obs_dim + 4]
+        with A > 1 records (set_vecnorm(agents=A))."""
+        agents = self._vecnorm_buffer()[1]
+        shape = (_lib.vecnorm_words(self.obs_dim),) if agents == 1 else (agents, _lib.vecnorm_words(self.obs_dim))
         if out is None:
-            out = torch.empty(_lib.vecnorm_words(self.obs_dim), dtype=torch.float64, device=self.device)
-        self._need("vecnorm_stats", out, "out", (_lib.vecnorm_words(self.obs_dim),), torch.float64)
-        _lib.check(self.lib.tb_get_vecnorm(self.h, _dptr(out), self._stream()))
+            out = torch.empty(shape, dtype=torch.float64, device=self.device)
+        self._need("vecnorm_stats", out, "out", shape, torch.float64)
+        if agents == 1:
+            _lib.check(self.lib.tb_get_vecnorm(self.h, _dptr(out), self._stream()))
+        else:
+            _lib.check(self.lib.tb_get_vecnorms(self.h, _dptr(out), agents, self._stream()))
         return out
+
+    def vecnorm_records(self):
+        """float64 [A, 2 obs_dim + 4] view of the library's record buffer (tb_vecnorm_device_ptr): the kernels read a record
+        when they run, so an in-place write to a row (copying one agent's record over another's) is seen by the next
+        policy_rollout, a replayed graph included, without zeroing returns or arming the reset fold.  Valid until a
+        set_vecnorm call with more records than before, or close()."""
+        ptr, agents = self._vecnorm_buffer()
+        if ptr is None:
+            raise _lib.TennisbotLibraryError("vecnorm_records: no normaliser attached (set_vecnorm)")
+        return _wrap_device(ptr, (agents, _lib.vecnorm_words(self.obs_dim)), "<f8", self.device, owner=self)
 
     def vecnorm_apply(self, x, what="obs", out=None):
         """The normaliser's formula on a batch of raw values (tb_vecnorm_apply), with the record as it stands when the kernel
@@ -394,7 +428,7 @@ class TennisBatch:
         """int64[10] statistics vector living in HBM, as a torch view (all-reduce it over NCCL)."""
         p = C.c_void_p()
         _lib.check(self.lib.tb_stats_device_ptr(self.h, C.byref(p)))
-        return _wrap_device_int64(p.value, _lib.NUM_STATS, self.device, owner=self)
+        return _wrap_device(p.value, (_lib.NUM_STATS,), "<i8", self.device, owner=self)
 
     def read_stats(self, clear=False):
         out = np.zeros(_lib.NUM_STATS, np.int64)
@@ -458,13 +492,14 @@ class TennisBatch:
         return hb
 
 
-def _wrap_device_int64(ptr, n, device, owner):
-    """View `n` int64 at raw device address `ptr` as a torch tensor through __cuda_array_interface__."""
+def _wrap_device(ptr, shape, typestr, device, owner):
+    """View a C-contiguous array of `shape` and numpy `typestr` at raw device address `ptr` as a torch tensor through
+    __cuda_array_interface__."""
 
     class _Holder:
         pass
 
     h = _Holder()
-    h.__cuda_array_interface__ = {"shape": (n,), "typestr": "<i8", "data": (int(ptr), False), "version": 3}
+    h.__cuda_array_interface__ = {"shape": tuple(shape), "typestr": typestr, "data": (int(ptr), False), "version": 3}
     h._owner = owner
     return torch.as_tensor(h, device=device)

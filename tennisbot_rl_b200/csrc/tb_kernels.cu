@@ -20,6 +20,7 @@
 #include <new>
 #include <type_traits>
 #include <utility>
+#include <vector>
 
 #include "tb_device.cuh"
 
@@ -1395,12 +1396,12 @@ __device__ __forceinline__ float vn_apply(float v, double mean, double var, doub
 // instance of tb_policy_rollout with a normaliser attached; the policy tower also writes vn_obs and vn_reward.
 // POP: the population instance (tb_set_policies, agents > 1).  A CTA stages the tower of each agent its 128 envs belong to in
 // turn, and only that agent's threads compute with it: one pass when envs_per_agent is a multiple of 128, up to 128 passes
-// (one env per agent) when agents straddle the CTA.
+// (one env per agent) when agents straddle the CTA.  NORM && POP (tb_set_vecnorms): each agent pass normalises with that
+// agent's record, vn_stats + agent TB_VECNORM_WORDS(OBS).
 template <int OBS, int ACT, bool NORM, bool POP>
 __global__ void __launch_bounds__(kBlock) policy_kernel(const __grid_constant__ PolicyIO io) {
   using L = PolLayout<OBS, ACT>;
   static_assert(OBS % 2 == 0 && ACT % 2 == 0, "observation rows are read as float2 / float4, actions written as float2");
-  static_assert(!(NORM && POP), "the normaliser keeps one record per context: no population instance");
   __shared__ __align__(16) float P[L::PiTower + pad4(ACT)];
   const bool vf = blockIdx.y != 0;
   pdl_wait();
@@ -1437,9 +1438,10 @@ __global__ void __launch_bounds__(kBlock) policy_kernel(const __grid_constant__ 
         }
       }
       if (NORM) {
+        const double *st = POP ? io.vn_stats + agent * (2 * OBS + 4) : io.vn_stats;
         if (io.vn_norm_obs) {
 #pragma unroll
-          for (int c = 0; c < OBS; ++c) x[c] = vn_apply(x[c], io.vn_stats[c], io.vn_stats[OBS + c], io.vn_eps, io.vn_clip_obs);
+          for (int c = 0; c < OBS; ++c) x[c] = vn_apply(x[c], st[c], st[OBS + c], io.vn_eps, io.vn_clip_obs);
         }
         if (!vf && io.vn_obs) {
           float2 *q = reinterpret_cast<float2 *>(io.vn_obs + me * OBS);
@@ -1447,8 +1449,11 @@ __global__ void __launch_bounds__(kBlock) policy_kernel(const __grid_constant__ 
           for (int j = 0; j < OBS / 2; ++j) q[j] = make_float2(x[2 * j], x[2 * j + 1]);
         }
         if (!vf && io.vn_reward && io.vn_norm_reward)
-          io.vn_reward[me] = vn_apply(io.vn_reward[me], 0.0, io.vn_stats[2 * OBS + 2], io.vn_eps, io.vn_clip_reward);
-        if (!vf && !io.act_raw && !io.act_env && !io.logp) return;  // the last launch: normalised reward only
+          io.vn_reward[me] = vn_apply(io.vn_reward[me], 0.0, st[2 * OBS + 2], io.vn_eps, io.vn_clip_reward);
+        if (!vf && !io.act_raw && !io.act_env && !io.logp) {  // the last launch: normalised reward only
+          if (POP) goto next_agent;  // (the CTA's other agents' threads still meet the __syncthreads below)
+          return;
+        }
       }
       float h[32];
       tower<OBS, ACT>(P, x, h);
@@ -1501,6 +1506,7 @@ __global__ void __launch_bounds__(kBlock) policy_kernel(const __grid_constant__ 
         io.value[me] = v;
       }
     }
+  next_agent:
     if (!POP || agent == last_agent) break;
     __syncthreads();  // every thread is done with this agent's tower before the next agent's is staged over it
   }
@@ -1863,6 +1869,10 @@ __global__ void __launch_bounds__(kBlock) es_norm_final_kernel(const double *par
 // each) and of their discounted returns, in the fixed order of es_norm_partial_kernel (kEsStatsPer envs per thread in order,
 // then es_merge_cta); vecnorm_final_kernel merges the partials in one CTA and updates the record in place.  The moments are
 // kept as offsets from the record's current mean, so the batch's delta of Chan's update is the merged offset itself.
+// SEG (tb_set_vecnorms, A > 1 records): the segmented pass over A agents of io.n envs each, env i belonging to record i / io.n.
+// The partial kernel runs es_norm_blocks(io.n) CTAs per agent, CTA k covering block k % blocks of agent k / blocks's slice
+// (one flat grid: blockIdx.y would cap A at 65 535), with the geometry block b of a context of io.n envs has; the final kernel
+// runs one CTA per agent.  So record p comes out bit-identical to the record of a context of io.n envs at env_id_offset p io.n.
 struct VecNormIO {
   double *stats;           // the running record, TB_VECNORM_WORDS(OBS) doubles
   double *ret;             // [N] discounted returns
@@ -1876,38 +1886,46 @@ struct VecNormIO {
   double gamma;
   int fold_obs;            // training && norm_obs
 };
-template <int OBS>
+template <int OBS, bool SEG = false>
 __global__ void __launch_bounds__(kBlock) vecnorm_partial_kernel(const __grid_constant__ VecNormIO io) {
-  const int64_t n = io.n, e0 = (int64_t)blockIdx.x * kBlock * kEsStatsPer + threadIdx.x;
+  // SEG: this CTA's agent, its block b within the agent, and the agent's first env
+  const int64_t blocks = SEG ? (io.n + kBlock * kEsStatsPer - 1) / (kBlock * kEsStatsPer) : 1;
+  const int64_t agent = SEG ? blockIdx.x / blocks : 0, b = SEG ? blockIdx.x - agent * blocks : blockIdx.x, first = agent * io.n;
+  const double *st = SEG ? io.stats + agent * (2 * OBS + 4) : io.stats;
+  const int64_t n = io.n, e0 = b * kBlock * kEsStatsPer + threadIdx.x;
   const bool fold_obs = io.fold_obs && (io.reward || *io.armed), fold_ret = io.reward != nullptr;
   double m0[OBS + 1];
   EsMoments v[OBS + 1];
 #pragma unroll
-  for (int c = 0; c <= OBS; ++c) { m0[c] = io.stats[c < OBS ? c : 2 * OBS + 1]; v[c] = {0.0, 0.0, 0.0}; }
+  for (int c = 0; c <= OBS; ++c) { m0[c] = st[c < OBS ? c : 2 * OBS + 1]; v[c] = {0.0, 0.0, 0.0}; }
   for (int r = 0; r < kEsStatsPer; ++r) {
-    const int64_t e = e0 + (int64_t)r * kBlock;
+    const int64_t e = e0 + (int64_t)r * kBlock, g = SEG ? first + e : e;
     if (e >= n) break;
     float x[OBS];
 #pragma unroll
     for (int j = 0; j < OBS / 2; ++j) {
-      const float2 a = reinterpret_cast<const float2 *>(io.obs + e * OBS)[j];
+      const float2 a = reinterpret_cast<const float2 *>(io.obs + g * OBS)[j];
       x[2 * j] = a.x; x[2 * j + 1] = a.y;
-      if (io.copy) reinterpret_cast<float2 *>(io.copy + e * OBS)[j] = a;
+      if (io.copy) reinterpret_cast<float2 *>(io.copy + g * OBS)[j] = a;
     }
     if (fold_obs) {
 #pragma unroll
       for (int c = 0; c < OBS; ++c) v[c] = es_merge(v[c], {1.0, __dsub_rn((double)x[c], m0[c]), 0.0});
     }
     if (fold_ret) {  // returns = returns * gamma + reward, folded; then returns[done] = 0
-      const double R = __dadd_rn(__dmul_rn(io.ret[e], io.gamma), (double)io.reward[e]);
+      const double R = __dadd_rn(__dmul_rn(io.ret[g], io.gamma), (double)io.reward[g]);
       v[OBS] = es_merge(v[OBS], {1.0, __dsub_rn(R, m0[OBS]), 0.0});
-      io.ret[e] = io.done[e] ? 0.0 : R;
+      io.ret[g] = io.done[g] ? 0.0 : R;
     }
   }
   double *p = io.part + (int64_t)blockIdx.x * (OBS + 1) * 3;
 #pragma unroll
   for (int c = 0; c <= OBS; ++c) {
-    if (c < OBS ? !fold_obs : !fold_ret) continue;  // (uniform over the CTA)
+    if (c < OBS ? !fold_obs : !fold_ret) {  // (uniform over the CTA)
+      // SEG: an empty partial tells the final kernel not to fold (it cannot read *io.armed: its CTA 0 clears it)
+      if (SEG && c < OBS && io.fold_obs && threadIdx.x == 0) { p[3 * c] = 0.0; p[3 * c + 1] = 0.0; p[3 * c + 2] = 0.0; }
+      continue;
+    }
     const EsMoments s = es_merge_cta(v[c]);
     if (threadIdx.x == 0) { p[3 * c] = s.n; p[3 * c + 1] = s.d; p[3 * c + 2] = s.m2; }
   }
@@ -1915,21 +1933,22 @@ __global__ void __launch_bounds__(kBlock) vecnorm_partial_kernel(const __grid_co
 // One CTA: merge the `blocks` partials of each channel (each thread a strided subset in order, then the fixed tree) and apply
 // RunningMeanStd.update_from_moments with batch mean = mean + d, batch variance M2 / N, batch count N:
 //   tot = count + N, mean += d N / tot, var = (var count + M2 / N N + d^2 count N / tot) / tot, count = tot.
-template <int OBS>
+// SEG: CTA p merges agent p's `blocks` partials into record p; an obs channel whose partials are empty is not folded.
+template <int OBS, bool SEG = false>
 __global__ void __launch_bounds__(kBlock) vecnorm_final_kernel(const __grid_constant__ VecNormIO io, int64_t blocks) {
-  const bool fold_obs = io.fold_obs && (io.reward || *io.armed), fold_ret = io.reward != nullptr;
-  double *st = io.stats;
+  const bool fold_obs = io.fold_obs && (SEG || io.reward || *io.armed), fold_ret = io.reward != nullptr;
+  double *st = SEG ? io.stats + (int64_t)blockIdx.x * (2 * OBS + 4) : io.stats;
   double cnt[2] = {st[2 * OBS], st[2 * OBS + 3]}, tot[2] = {cnt[0], cnt[1]};
 #pragma unroll
   for (int c = 0; c <= OBS; ++c) {
     if (c < OBS ? !fold_obs : !fold_ret) continue;
     EsMoments v = {0.0, 0.0, 0.0};
     for (int64_t b = threadIdx.x; b < blocks; b += kBlock) {
-      const double *p = io.part + (b * (OBS + 1) + c) * 3;
+      const double *p = io.part + ((SEG ? (int64_t)blockIdx.x * blocks + b : b) * (OBS + 1) + c) * 3;
       v = es_merge(v, {p[0], p[1], p[2]});
     }
     v = es_merge_cta(v);
-    if (threadIdx.x == 0) {
+    if (threadIdx.x == 0 && (!SEG || v.n != 0.0)) {
       const int k = c < OBS ? 0 : 1;
       double *mean = c < OBS ? st + c : st + 2 * OBS + 1, *var = c < OBS ? st + OBS + c : st + 2 * OBS + 2;
       const double N = v.n, t = __dadd_rn(cnt[k], N), d = v.d;
@@ -1942,7 +1961,7 @@ __global__ void __launch_bounds__(kBlock) vecnorm_final_kernel(const __grid_cons
   }
   if (threadIdx.x == 0) {
     st[2 * OBS] = tot[0]; st[2 * OBS + 3] = tot[1];
-    if (!fold_ret) *io.armed = 0;
+    if (!fold_ret && (!SEG || blockIdx.x == 0)) *io.armed = 0;
   }
 }
 // tb_set_vecnorm: the record from `src` (nullptr: fresh, RunningMeanStd(epsilon=1e-4)), returns zeroed, the fold armed
@@ -1951,6 +1970,18 @@ __global__ void __launch_bounds__(kBlock) vecnorm_init_kernel(const __grid_const
   const int64_t i = (int64_t)blockIdx.x * kBlock + threadIdx.x;
   if (i < io.n) io.ret[i] = 0.0;
   if (i < 2 * OBS + 4) io.stats[i] = src ? src[i] : (i < OBS || i == 2 * OBS + 1) ? 0.0 : (i == 2 * OBS || i == 2 * OBS + 3) ? 1e-4 : 1.0;
+  if (i == 0) *io.armed = 1;
+}
+// tb_set_vecnorms with A > 1: `records` records from `src` ([records][TB_VECNORM_WORDS(OBS)], nullptr: all fresh), returns
+// zeroed, the fold armed
+template <int OBS>
+__global__ void __launch_bounds__(kBlock) vecnorm_init_records_kernel(const __grid_constant__ VecNormIO io, const double *src,
+                                                                      int64_t records) {
+  constexpr int W = 2 * OBS + 4;
+  const int64_t i = (int64_t)blockIdx.x * kBlock + threadIdx.x;
+  const int w = (int)(i % W);
+  if (i < io.n) io.ret[i] = 0.0;
+  if (i < records * W) io.stats[i] = src ? src[i] : (w < OBS || w == 2 * OBS + 1) ? 0.0 : (w == 2 * OBS || w == 2 * OBS + 3) ? 1e-4 : 1.0;
   if (i == 0) *io.armed = 1;
 }
 // tb_reset / tb_reset_from with a normaliser in training: returns of the reset envs zeroed; a full reset arms the fold
@@ -2912,10 +2943,12 @@ struct PolicyBufs {           // tb_set_policy / tb_set_policies
   int64_t params_cap = 0;     // floats params holds
   int64_t agents = 1;         // rows the rollout uses: env i acts with row i / (N / agents)
 };
-struct VecNormBufs {          // tb_set_vecnorm (see VecNormIO)
-  DevPtr<double> stats, ret, part;
-  DevPtr<float> raw;          // [N, obs_dim] raw observation handed from step_kernel to policy_kernel<.., true>
+struct VecNormBufs {          // tb_set_vecnorm / tb_set_vecnorms (see VecNormIO)
+  DevPtr<double> stats, ret, part;  // stats: [records][TB_VECNORM_WORDS(obs_dim)]
+  DevPtr<float> raw;          // [N, obs_dim] raw observation handed from step_kernel to policy_kernel<.., true, ..>
   DevPtr<uint8_t> armed;
+  int64_t stats_cap = 0, part_cap = 0;  // doubles stats and part hold
+  int64_t records = 1;        // records attached: env i uses record i / (N / records)
 };
 
 struct tb_ctx {
@@ -3153,13 +3186,26 @@ static VecNormIO vecnorm_io(tb_ctx *c) {
   io.n = c->cfg.num_envs; io.gamma = c->vn_cfg.gamma; io.fold_obs = c->vn_cfg.training && c->vn_cfg.norm_obs;
   return io;
 }
+// Doubles of the partials buffer a pass over `records` records of num_envs / records envs each needs
+static int64_t vecnorm_part_doubles(int64_t num_envs, int64_t records, int od) {
+  return records * es_norm_blocks(num_envs / records) * (od + 1) * 3;
+}
 // One statistics pass (vecnorm_partial_kernel, and vecnorm_final_kernel when the context trains): the entry pass when
-// io.reward is nullptr (copy obs to io.copy if set, fold it if *io.armed), else the step pass.
+// io.reward is nullptr (copy obs to io.copy if set, fold it if *io.armed), else the step pass.  With A > 1 records, the
+// segmented instances: still two launches, A es_norm_blocks(N / A) CTAs and A CTAs.
 static int vecnorm_pass(tb_ctx *c, VecNormIO io, cudaStream_t s) {
-  const int64_t blocks = es_norm_blocks(io.n);
+  const int64_t records = c->vn.records;
   return with_kind(c->cfg.env_kind, [&](auto kind) {
-    if (launch(c, kPlain, vecnorm_partial_kernel<Dims<kind>::obs>, (unsigned)blocks, kBlock, s, io)) return 1;
-    return vecnorm_training(c) ? launch(c, kPlain, vecnorm_final_kernel<Dims<kind>::obs>, 1, kBlock, s, io, blocks) : 0;
+    constexpr int O = Dims<kind>::obs;
+    if (records == 1) {
+      const int64_t blocks = es_norm_blocks(io.n);
+      if (launch(c, kPlain, vecnorm_partial_kernel<O>, (unsigned)blocks, kBlock, s, io)) return 1;
+      return vecnorm_training(c) ? launch(c, kPlain, vecnorm_final_kernel<O>, 1, kBlock, s, io, blocks) : 0;
+    }
+    io.n /= records;  // envs per record
+    const int64_t blocks = es_norm_blocks(io.n);
+    if (launch(c, kPlain, vecnorm_partial_kernel<O, true>, (unsigned)(records * blocks), kBlock, s, io)) return 1;
+    return vecnorm_training(c) ? launch(c, kPlain, vecnorm_final_kernel<O, true>, (unsigned)records, kBlock, s, io, blocks) : 0;
   });
 }
 static int vecnorm_pass(tb_ctx *c, const float *obs, const float *reward, const uint8_t *done, cudaStream_t s) {
@@ -3430,8 +3476,9 @@ int tb_set_policies(tb_ctx *c, const float *d_params, int64_t agents, int64_t co
   return copy_policies(c, d_params, agents, (cudaStream_t)stream);
 }
 
-int tb_policy_rollout(tb_ctx *c, int k_steps, int deterministic, uint64_t noise_seed, float *d_obs, float *d_actions, float *d_logp,
-                      float *d_value, float *d_reward, uint8_t *d_done, float *d_last_obs, float *d_last_value, void *stream) {
+int tb_policy_rollout_raw(tb_ctx *c, int k_steps, int deterministic, uint64_t noise_seed, float *d_obs, float *d_actions,
+                          float *d_logp, float *d_value, float *d_reward, float *d_raw_reward, uint8_t *d_done, float *d_last_obs,
+                          float *d_last_value, void *stream) {
   GUARD(c);
   if (!c->policy.params) return fail("tb_policy_rollout: no policy (tb_set_policy)");
   if (c->control_mode != TB_CONTROL_FORCE) return fail("tb_policy_rollout: the policy's actions are forces (TB_CONTROL_FORCE)");
@@ -3441,13 +3488,19 @@ int tb_policy_rollout(tb_ctx *c, int k_steps, int deterministic, uint64_t noise_
   const int od = tb_obs_dim(c->cfg.env_kind), ad = tb_act_dim(c->cfg.env_kind);
   // with a normaliser: policy_kernel<.., true> reads the raw observation from vn.raw (from d_last_obs after the last step)
   const bool vn = c->vn_cfg.struct_size != 0, train = vecnorm_training(c), pop = c->policy.agents > 1;
-  if (vn && pop)
+  if (vn && c->vn.records == 1 && pop)
     return fail("tb_policy_rollout: a normaliser (tb_set_vecnorm) keeps one record per context, so it cannot serve %lld agents "
-                "(tb_set_policies); detach it or set one policy", (long long)c->policy.agents);
+                "(tb_set_policies); detach it or set one policy, or attach one record per agent (tb_set_vecnorms)",
+                (long long)c->policy.agents);
+  if (vn && c->vn.records != c->policy.agents)
+    return fail("tb_policy_rollout: %lld policies (tb_set_policies) and %lld normaliser records (tb_set_vecnorms) differ; env i "
+                "uses policy and record i / (N / agents), so the counts must be equal", (long long)c->policy.agents,
+                (long long)c->vn.records);
   void (*kernel)(PolicyIO) = nullptr;
   with_kind(c->cfg.env_kind, [&](auto kind) {
     constexpr int O = Dims<kind>::obs, A = Dims<kind>::act;
-    kernel = vn ? policy_kernel<O, A, true, false> : pop ? policy_kernel<O, A, false, true> : policy_kernel<O, A, false, false>;
+    kernel = vn ? (pop ? policy_kernel<O, A, true, true> : policy_kernel<O, A, true, false>)
+                : pop ? policy_kernel<O, A, false, true> : policy_kernel<O, A, false, false>;
     return 0;
   });
   cudaStream_t s = (cudaStream_t)stream;
@@ -3473,6 +3526,8 @@ int tb_policy_rollout(tb_ctx *c, int k_steps, int deterministic, uint64_t noise_
     io.obs = t + 1 < k_steps ? (vn ? c->vn.raw.get() : d_obs + (size_t)(t + 1) * n * od) : d_last_obs;
     io.reward = d_reward + (size_t)t * n; io.done = d_done + (size_t)t * n;
     if (launch_step(c, io, s)) return 1;
+    if (d_raw_reward)  // the step's reward before the next policy launch normalises it in place (a copy, not a launch)
+      CU(cudaMemcpyAsync(d_raw_reward + (size_t)t * n, io.reward, (size_t)n * sizeof(float), cudaMemcpyDeviceToDevice, s));
     if (train && vecnorm_pass(c, io.obs, io.reward, io.done, s)) return 1;
   }
   if (d_last_value || vn) {  // bootstrap value of the observation the rollout ends with; the last step's normalised reward
@@ -3483,55 +3538,118 @@ int tb_policy_rollout(tb_ctx *c, int k_steps, int deterministic, uint64_t noise_
   return 0;
 }
 
-int tb_set_vecnorm(tb_ctx *c, const tb_vecnorm *cfg, const double *d_stats, void *stream) {
+int tb_policy_rollout(tb_ctx *c, int k_steps, int deterministic, uint64_t noise_seed, float *d_obs, float *d_actions, float *d_logp,
+                      float *d_value, float *d_reward, uint8_t *d_done, float *d_last_obs, float *d_last_value, void *stream) {
+  return tb_policy_rollout_raw(c, k_steps, deterministic, noise_seed, d_obs, d_actions, d_logp, d_value, d_reward, nullptr, d_done,
+                               d_last_obs, d_last_value, stream);
+}
+
+// tb_set_vecnorm (who = "tb_set_vecnorm", agents = 1) and tb_set_vecnorms: `agents` records of one configuration
+static int set_vecnorms(tb_ctx *c, const char *who, const tb_vecnorm *cfg, int64_t agents, const double *d_stats, void *stream) {
   GUARD(c);
-  if (check_fault(c, "tb_set_vecnorm")) return 1;
+  if (check_fault(c, who)) return 1;
   if (!cfg) { c->vn_cfg = tb_vecnorm{}; return 0; }
-  if (cfg->struct_size != sizeof(tb_vecnorm)) return fail("tb_set_vecnorm: tb_vecnorm.struct_size mismatch");
+  const int64_t n = c->cfg.num_envs;
+  if (agents < 1 || n % agents) return fail("%s: agents must be >= 1 and divide num_envs = %lld, got %lld", who, (long long)n, (long long)agents);
+  if (cfg->struct_size != sizeof(tb_vecnorm)) return fail("%s: tb_vecnorm.struct_size mismatch", who);
   if (!(std::isfinite(cfg->clip_obs) && cfg->clip_obs > 0) || !(std::isfinite(cfg->clip_reward) && cfg->clip_reward > 0))
-    return fail("tb_set_vecnorm: clip_obs and clip_reward must be finite and above 0");
-  if (!(cfg->gamma >= 0 && cfg->gamma <= 1)) return fail("tb_set_vecnorm: gamma must be in [0, 1]");
-  if (!(std::isfinite(cfg->epsilon) && cfg->epsilon > 0)) return fail("tb_set_vecnorm: epsilon must be finite and above 0");
+    return fail("%s: clip_obs and clip_reward must be finite and above 0", who);
+  if (!(cfg->gamma >= 0 && cfg->gamma <= 1)) return fail("%s: gamma must be in [0, 1]", who);
+  if (!(std::isfinite(cfg->epsilon) && cfg->epsilon > 0)) return fail("%s: epsilon must be finite and above 0", who);
   const int od = tb_obs_dim(c->cfg.env_kind), words = TB_VECNORM_WORDS(od);
+  const bool rows = std::strcmp(who, "tb_set_vecnorm") != 0;  // tb_set_vecnorms' messages name the row
   cudaStream_t s = (cudaStream_t)stream;
-  if (d_stats) {  // the record is read on the device: copy it back and check it first (synchronises `stream`)
-    double h[TB_VECNORM_WORDS(12)];
-    CU(cudaMemcpyAsync(h, d_stats, words * sizeof(double), cudaMemcpyDeviceToHost, s));
+  if (d_stats) {  // the records are read on the device: copy them back and check them first (synchronises `stream`)
+    std::vector<double> h((size_t)(agents * words));
+    CU(cudaMemcpyAsync(h.data(), d_stats, h.size() * sizeof(double), cudaMemcpyDeviceToHost, s));
     CU(cudaStreamSynchronize(s));
-    for (int i = 0; i < words; ++i) {
-      const bool count = i == 2 * od || i == 2 * od + 3, var = (i >= od && i < 2 * od) || i == 2 * od + 2;
-      if (!std::isfinite(h[i]) || (count && !(h[i] > 0)) || (var && h[i] < 0))
-        return fail("tb_set_vecnorm: stats[%d] = %g: counts must be above 0, variances at least 0, every entry finite", i, h[i]);
-    }
+    for (int64_t r = 0; r < agents; ++r)
+      for (int i = 0; i < words; ++i) {
+        const double v = h[(size_t)(r * words + i)];
+        const bool count = i == 2 * od || i == 2 * od + 3, var = (i >= od && i < 2 * od) || i == 2 * od + 2;
+        if (!std::isfinite(v) || (count && !(v > 0)) || (var && v < 0)) {
+          if (rows)
+            return fail("%s: stats[%lld][%d] = %g: counts must be above 0, variances at least 0, every entry finite", who,
+                        (long long)r, i, v);
+          return fail("%s: stats[%d] = %g: counts must be above 0, variances at least 0, every entry finite", who, i, v);
+        }
+      }
   }
-  if (!c->vn.stats) {
-    const int64_t n = c->cfg.num_envs;
+  if (!c->vn.ret) {
     VecNormBufs b;
-    CU(dev_alloc(b.stats, (size_t)words * sizeof(double)));
     CU(dev_alloc(b.ret, (size_t)n * sizeof(double)));
-    CU(dev_alloc(b.part, (size_t)es_norm_blocks(n) * (od + 1) * 3 * sizeof(double)));
     CU(dev_alloc(b.raw, (size_t)n * od * sizeof(float)));
     CU(dev_alloc(b.armed, 1));
     c->vn = std::move(b);
   }
+  // records and partials grow to the largest call (cudaMalloc / cudaFree: not while capturing)
+  const int64_t stats_need = agents * words, part_need = vecnorm_part_doubles(n, agents, od);
+  if (c->vn.stats_cap < stats_need) {
+    DevPtr<double> p;
+    CU(dev_alloc(p, (size_t)stats_need * sizeof(double)));
+    c->vn.stats = std::move(p);
+    c->vn.stats_cap = stats_need;
+  }
+  if (c->vn.part_cap < part_need) {
+    DevPtr<double> p;
+    CU(dev_alloc(p, (size_t)part_need * sizeof(double)));
+    c->vn.part = std::move(p);
+    c->vn.part_cap = part_need;
+  }
   c->vn_cfg = *cfg;
+  c->vn.records = agents;
   return with_kind(c->cfg.env_kind, [&](auto kind) {
-    return launch(c, kPlain, vecnorm_init_kernel<Dims<kind>::obs>, grid_for(c->cfg.num_envs, kBlock), kBlock, s, vecnorm_io(c), d_stats);
+    constexpr int O = Dims<kind>::obs;
+    if (agents == 1)
+      return launch(c, kPlain, vecnorm_init_kernel<O>, grid_for(n, kBlock), kBlock, s, vecnorm_io(c), d_stats);
+    return launch(c, kPlain, vecnorm_init_records_kernel<O>, grid_for(std::max<int64_t>(n, stats_need), kBlock), kBlock, s,
+                  vecnorm_io(c), d_stats, agents);
   });
+}
+
+int tb_set_vecnorm(tb_ctx *c, const tb_vecnorm *cfg, const double *d_stats, void *stream) {
+  return set_vecnorms(c, "tb_set_vecnorm", cfg, 1, d_stats, stream);
+}
+
+int tb_set_vecnorms(tb_ctx *c, const tb_vecnorm *cfg, int64_t agents, const double *d_stats, void *stream) {
+  return set_vecnorms(c, "tb_set_vecnorms", cfg, agents, d_stats, stream);
 }
 
 int tb_get_vecnorm(tb_ctx *c, double *d_stats, void *stream) {
   GUARD(c);
   if (!c->vn_cfg.struct_size) return fail("tb_get_vecnorm: no normaliser attached (tb_set_vecnorm)");
+  if (c->vn.records != 1)
+    return fail("tb_get_vecnorm: %lld records are attached; read them with tb_get_vecnorms", (long long)c->vn.records);
   if (!d_stats) return fail("tb_get_vecnorm: d_stats is NULL");
   const size_t bytes = TB_VECNORM_WORDS(tb_obs_dim(c->cfg.env_kind)) * sizeof(double);
   CU(cudaMemcpyAsync(d_stats, c->vn.stats.get(), bytes, cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
   return 0;
 }
 
+int tb_get_vecnorms(tb_ctx *c, double *d_stats, int64_t agents, void *stream) {
+  GUARD(c);
+  if (!c->vn_cfg.struct_size) return fail("tb_get_vecnorms: no normaliser attached (tb_set_vecnorms)");
+  if (agents != c->vn.records)
+    return fail("tb_get_vecnorms: %lld records are attached, got agents = %lld", (long long)c->vn.records, (long long)agents);
+  if (!d_stats) return fail("tb_get_vecnorms: d_stats is NULL");
+  const size_t bytes = (size_t)agents * TB_VECNORM_WORDS(tb_obs_dim(c->cfg.env_kind)) * sizeof(double);
+  CU(cudaMemcpyAsync(d_stats, c->vn.stats.get(), bytes, cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
+  return 0;
+}
+
+int tb_vecnorm_device_ptr(tb_ctx *c, double **d_records, int64_t *agents) {
+  if (!c || !d_records || !agents) return fail("tb_vecnorm_device_ptr: bad argument");
+  if (!c->vn_cfg.struct_size) return fail("tb_vecnorm_device_ptr: no normaliser attached (tb_set_vecnorms)");
+  *d_records = c->vn.stats.get();
+  *agents = c->vn.records;
+  return 0;
+}
+
 int tb_vecnorm_apply(tb_ctx *c, const float *d_in, int64_t rows, int what, float *d_out, void *stream) {
   GUARD(c);
   if (!c->vn_cfg.struct_size) return fail("tb_vecnorm_apply: no normaliser attached (tb_set_vecnorm)");
+  if (c->vn.records != 1)
+    return fail("tb_vecnorm_apply: %lld records are attached (tb_set_vecnorms); it applies one", (long long)c->vn.records);
   if (what != TB_VECNORM_OBS && what != TB_VECNORM_REWARD) return fail("tb_vecnorm_apply: unknown what %d", what);
   const int od = tb_obs_dim(c->cfg.env_kind), width = what == TB_VECNORM_OBS ? od : 1;
   if (rows < 0 || rows > (int64_t)INT32_MAX * kBlock / width)  // (one thread per float, a grid of at most 2^31 - 1 CTAs)
@@ -3791,6 +3909,8 @@ int tb_sac_rollout(tb_ctx *c, int k_steps, int mode, uint64_t noise_seed, const 
   if (!c->sac.cur) return fail("tb_sac_rollout: no tb_sac_begin on this context");
   if (mode != TB_SAC_UNIFORM && !c->sac_actor.w2) return fail("tb_sac_rollout: no actor (tb_set_sac_actor)");
   if (norm && !c->vn_cfg.struct_size) return fail("tb_sac_rollout: TB_SAC_VECNORM needs a normaliser (tb_set_vecnorm)");
+  if (norm && c->vn.records != 1)
+    return fail("tb_sac_rollout: TB_SAC_VECNORM uses one record, and %lld are attached (tb_set_vecnorms)", (long long)c->vn.records);
   if (check_fault(c, "tb_sac_rollout")) return 1;
   const bool train = norm && vecnorm_training(c);
   const int64_t n = c->cfg.num_envs;

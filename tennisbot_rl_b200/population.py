@@ -5,6 +5,8 @@ tb_policy_rollout collects the rollouts of every agent.  The learner is GpuPPO's
 parameters carry a leading agent dimension and go through batched matmuls, and every reduction of the loss (advantage
 normalisation, means, gradient norm) is taken per agent, so agent p's update depends on agent p's samples only.  The
 hyper-parameters live in [P] device tensors that the captured minibatch graph reads, so PBT changes them in place.
+With normalize=True every agent trains under its own SB3 VecNormalize record (tb_set_vecnorms), which PBT copies with the
+weights.
 """
 import math
 import time
@@ -13,7 +15,7 @@ import numpy as np
 import torch
 
 from .batch import TennisBatch
-from .ppo import POLICY_FLOATS_BY_DIMS, ActorCritic
+from .ppo import POLICY_FLOATS_BY_DIMS, ActorCritic, vecnormalize_entries
 
 # GpuPPO's hyper-parameters and their defaults (the reference's SB3 settings, train_swing.py:80-91, and lr 3e-4)
 HYPER_DEFAULTS = {"lr": 3e-4, "ent_coef": 0.002, "clip": 0.2, "vf_coef": 0.5, "max_grad_norm": 0.5, "gamma": 0.99,
@@ -176,11 +178,14 @@ class PopulationPPO:
     weights GpuPPO(seed=seeds[p]) starts from and takes exactly GpuPPO's update on its own samples: its own GAE, permutation,
     minibatches, advantage normalisation, loss coefficients, gradient-norm clipping and Adam learning rate.  The rollout is
     the fused one only (tb_set_policies + tb_policy_rollout in one CUDA graph).  The context's env seed is seeds[0] and the
-    policy noise seed seeds[0] + 1.  pbt_interval: run exploit_explore() after every pbt_interval updates (None: never)."""
+    policy noise seed seeds[0] + 1.  pbt_interval: run exploit_explore() after every pbt_interval updates (None: never).
+    normalize: each agent's envs run under that agent's own VecNormalize record (SB3's defaults, PPO's gamma, which must then
+    be one value for every agent), as GpuPPO(normalize=True) runs its envs: the agent learns on normalised observations and
+    rewards, while its episode statistics and PBT scores come from the raw rewards."""
 
     def __init__(self, env_id, agents, envs_per_agent, rollout_len, seeds=None, lr=3e-4, ent_coef=0.002, clip=0.2, vf_coef=0.5,
                  max_grad_norm=0.5, gamma=0.99, gae_lambda=0.95, epochs=10, minibatches=8, precision="f64", device=0,
-                 use_graph=True, pbt_interval=None, pbt_seed=0):
+                 use_graph=True, pbt_interval=None, pbt_seed=0, normalize=False):
         P = self.P = int(agents)
         if P < 1:
             raise ValueError(f"agents must be >= 1, got {agents}")
@@ -188,6 +193,10 @@ class PopulationPPO:
         given = dict(lr=lr, ent_coef=ent_coef, clip=clip, vf_coef=vf_coef, max_grad_norm=max_grad_norm, gamma=gamma,
                      gae_lambda=gae_lambda)
         values = {k: agent_values(k, v, P) for k, v in given.items()}
+        self.normalize = bool(normalize)
+        if self.normalize and len(set(values["gamma"])) != 1:
+            raise ValueError(f"normalize=True needs one gamma for every agent (the records share one configuration, and PBT "
+                             f"does not perturb gamma), got {values['gamma']}")
         if pbt_interval is not None and (int(pbt_interval) < 1 or P < 2):
             raise ValueError("pbt_interval needs at least 2 agents and must be >= 1")
         self.pbt_interval, self.pbt_rng, self.pbt_log = pbt_interval, np.random.default_rng(pbt_seed), []
@@ -207,7 +216,11 @@ class PopulationPPO:
         self.logp_buf, self.rew_buf, self.done_buf, self.val_buf = z(K, N), z(K, N), z(K, N), z(K + 1, N)
         self.done_u8 = torch.zeros((K, N), dtype=torch.uint8, device=self.dev)
         self.params = z(P, POLICY_FLOATS_BY_DIMS[(od, ad)])
-        self.obs = self.env.reset().clone()
+        self.obs = self.env.reset().clone()  # raw: with normalize, obs_buf / rew_buf receive the normalised values
+        self.vn_gamma = values["gamma"][0]  # the records' gamma (the [P] hyper tensor holds it rounded to float32)
+        if self.normalize:  # one record per agent; the first rollout folds the reset observation
+            self.env.set_vecnorm(gamma=self.vn_gamma, agents=P)
+        self.raw_buf = z(K, N) if self.normalize else None  # the raw rewards the episode statistics are summed from
         self.ep_ret = torch.zeros(N, dtype=torch.float64, device=self.dev)  # return / length of each env's episode in progress
         self.ep_len = torch.zeros(N, dtype=torch.float64, device=self.dev)
         self.graph, self.upd_graph, self.warmed_up = None, None, False
@@ -223,11 +236,12 @@ class PopulationPPO:
         self.env.set_policies(self.params)
         self.obs_buf[0].copy_(self.obs)
         self.env.policy_rollout(self.obs_buf, self.rew_buf, self.done_u8, self.obs, actions=self.act_buf, logp=self.logp_buf,
-                                value=self.val_buf[:self.K], last_value=self.val_buf[self.K], noise_seed=self.seeds[0] + 1)
+                                value=self.val_buf[:self.K], last_value=self.val_buf[self.K], noise_seed=self.seeds[0] + 1,
+                                raw_reward=self.raw_buf)
         self.done_buf.copy_(self.done_u8)
 
     def _episode_stats(self):
-        return episode_stats(self.rew_buf, self.done_u8, self.ep_ret, self.ep_len, self.P)
+        return episode_stats(self.rew_buf if self.raw_buf is None else self.raw_buf, self.done_u8, self.ep_ret, self.ep_len, self.P)
 
     @torch.no_grad()
     def rollout(self):
@@ -338,13 +352,16 @@ class PopulationPPO:
 
     # ------------------------------------------------------------------ PBT
     def exploit_explore(self, scores=None):
-        """One PBT round (module function exploit_explore) on parameters, Adam moments and step counts, and hyper-parameters;
-        env state is not copied.  scores: None ranks by the mean training return since the previous round.  The events are
-        appended to pbt_log as (update, destination, source, new hyper-parameters) and returned."""
+        """One PBT round (module function exploit_explore) on parameters, Adam moments and step counts, hyper-parameters and,
+        with normalize, the VecNormalize record the weights were trained against (a row copy in the library's buffer, which
+        the next rollout reads); env state, the per-env discounted returns included, is not copied.  scores: None ranks by
+        the mean training return since the previous round.  The events are appended to pbt_log as (update, destination,
+        source, new hyper-parameters) and returned."""
         if scores is None:
             r, e = self._interval
             scores = [float(r[p] / e[p]) if e[p] else None for p in range(self.P)]
-        ev = exploit_explore(scores, self.ac.params + self.opt.state_tensors(), self.hyper, self.pbt_rng)
+        rows = self.ac.params + self.opt.state_tensors() + ([self.env.vecnorm_records()] if self.normalize else [])
+        ev = exploit_explore(scores, rows, self.hyper, self.pbt_rng)
         ev = [(self.updates, dst, src, hp) for dst, src, hp in ev]
         self.pbt_log += ev
         self._interval[:] = 0
@@ -390,8 +407,13 @@ class PopulationPPO:
 
     def state_dict(self):
         """numpy arrays: `policies` [P, floats] (tb_set_policies' rows), `seeds`, one [P] array per hyper-parameter, and
-        `pbt_events` [E, len(PBT_COLUMNS)] float64 with the column names in `pbt_columns`."""
+        `pbt_events` [E, len(PBT_COLUMNS)] float64 with the column names in `pbt_columns`.  With normalize also `vecnorm`
+        [P, 2 obs_dim + 4] (tb_get_vecnorms' rows) and their configuration, `vecnorm_clip_obs`, `vecnorm_clip_reward`,
+        `vecnorm_gamma` and `vecnorm_epsilon`: set_vecnorm(agents=P, stats=...) attaches them again."""
         out = {"policies": self.ac.packed().cpu().numpy(), "seeds": np.array(self.seeds)}
+        if self.normalize:
+            out.update(vecnorm=self.env.vecnorm_stats().cpu().numpy(), vecnorm_clip_obs=10.0, vecnorm_clip_reward=10.0,
+                       vecnorm_gamma=self.vn_gamma, vecnorm_epsilon=1e-8)
         out.update({k: v.cpu().numpy() for k, v in self.hyper.items()})
         out["pbt_events"] = np.array([[u, d, s] + [hp[k] for k in HYPER_DEFAULTS] for u, d, s, hp in self.pbt_log],
                                      np.float64).reshape(-1, len(self.PBT_COLUMNS))
@@ -402,6 +424,10 @@ class PopulationPPO:
         np.savez(path, **self.state_dict())
 
     def agent_state_dict(self, p):
-        """Agent p in GpuPPO.state_dict()'s layout ({"policy": tb_set_policy's vector}): tools/record_episode.py plays it."""
-        return {"policy": self.ac.packed()[p].cpu().numpy()}
+        """Agent p in GpuPPO.state_dict()'s layout ({"policy": tb_set_policy's vector}, and with normalize agent p's record
+        under load_vecnormalize_npz's keys): tools/record_episode.py plays it (--policy, and --vecnormalize with normalize)."""
+        out = {"policy": self.ac.packed()[p].cpu().numpy()}
+        if self.normalize:
+            out.update(vecnormalize_entries(self.env.vecnorm_stats()[p], self.vn_gamma))
+        return out
 

@@ -242,7 +242,7 @@ class GpuPPO:
         under load_vecnormalize_npz's keys."""
         out = {"policy": self.ac.packed().cpu().numpy()}
         if self.normalize:
-            out.update(vecnormalize_entries(self.env, self.gamma))
+            out.update(vecnormalize_entries(self.env.vecnorm_stats(), self.gamma))
         return out
 
     def save(self, path):
@@ -372,10 +372,11 @@ VECNORMALIZE_KEYS = ("obs_mean", "obs_var", "obs_count", "ret_mean", "ret_var", 
                      "epsilon")
 
 
-def vecnormalize_entries(env, gamma):
-    """The record of env's normaliser (attached with SB3's VecNormalize defaults and this gamma) as numpy values under
-    load_vecnormalize_npz's keys."""
-    od, st = env.obs_dim, env.vecnorm_stats().cpu().numpy()
+def vecnormalize_entries(record, gamma):
+    """A normaliser's record (float64 [2 obs_dim + 4], tb_get_vecnorm's layout, attached with SB3's VecNormalize defaults and
+    this gamma) as numpy values under load_vecnormalize_npz's keys."""
+    st = np.asarray(record.cpu() if torch.is_tensor(record) else record, np.float64)
+    od = (st.size - 4) // 2
     return dict(obs_mean=st[:od], obs_var=st[od:2 * od], obs_count=st[2 * od], ret_mean=st[2 * od + 1], ret_var=st[2 * od + 2],
                 ret_count=st[2 * od + 3], clip_obs=10.0, clip_reward=10.0, gamma=gamma, epsilon=1e-8)
 

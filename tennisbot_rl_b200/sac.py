@@ -310,7 +310,7 @@ class GpuSAC:
         under load_vecnormalize_npz's keys."""
         out = {"policy": pack_sac_actor(self.actor).cpu().numpy()}
         if self.normalize:
-            out.update(vecnormalize_entries(self.env, self.gamma))
+            out.update(vecnormalize_entries(self.env.vecnorm_stats(), self.gamma))
         return out
 
     def save(self, path):

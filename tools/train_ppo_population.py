@@ -4,12 +4,17 @@
     python tools/train_ppo_population.py SwingRacket-v0 --agents 4 --envs-per-agent 4096 --iters 25
     python tools/train_ppo_population.py Tennisbot-v0 --agents 8 --envs-per-agent 16384 --rollout-len 128 --iters 60 --pbt 10
     python tools/train_ppo_population.py SwingRacket-v0 --throughput
+    python tools/train_ppo_population.py Tennisbot-v0 --agents 8 --envs-per-agent 16384 --throughput --normalize
 
 Prints the card's name and power limit, then per-agent curves (mean training return of the episodes that ended in each
-rollout).  --throughput instead times, at 16 384 envs per agent, for P in 1, 4, 8:
+rollout; raw returns with --normalize, which gives every agent its own VecNormalize record).  --throughput instead times, at
+16 384 envs per agent, for P in 1, 4, 8:
   - the wall time of one population update (rollout + update, synchronised host clock) against P GpuPPO updates in turn;
   - the rollout time per env step (CUDA events) of P policies against one policy over the same P x 16 384 envs;
 and the rollout time per step at 16 384 envs when agents straddle the 128-env CTAs of policy_kernel.
+--throughput --normalize times the rollout per env step over --agents x --envs-per-agent envs with P policies and P training
+records, with P policies and no normaliser, and with one policy and one training record; the same two normalised setups with
+frozen records give the cost of the statistics pass per step (training minus frozen), segmented and with one record.
 """
 import argparse
 import json
@@ -44,23 +49,27 @@ def wall_per_update(step, warm=2, reps=3):
 
 
 def rollout_ms_per_step(env_id, N, agents_list, K, reps=5):
-    """{agents: ms per env step} of tb_policy_rollout over N envs, agents = 0 meaning set_policy; runs alternate."""
+    """{key: ms per env step} of tb_policy_rollout over N envs; runs alternate.  agents_list: agents (0 meaning set_policy),
+    or (key, agents, records, training) tuples that also attach a normaliser of `records` records (0: none)."""
     od, ad = (6, 6) if env_id == "SwingRacket-v0" else (12, 2)
     torch.manual_seed(0)
     row = ActorCritic(od, ad).packed().cuda()
     setups = {}
-    for a in agents_list:
+    for spec in agents_list:
+        key, a, rec, training = spec if isinstance(spec, tuple) else (spec, spec, 0, True)
         b = TennisBatch(env_id, N, seed=1)
         if a:
             b.set_policies((row + 1e-3 * torch.randn(a, row.numel(), device="cuda")).contiguous())
         else:
             b.set_policy(row)
+        if rec:
+            b.set_vecnorm(training=training, agents=rec)
         z = lambda *s: torch.zeros(s, device="cuda")  # noqa: E731
         bufs = dict(obs=z(K, N, od), rew=z(K, N), done=torch.zeros((K, N), dtype=torch.uint8, device="cuda"), last=z(N, od),
                     act=z(K, N, ad), logp=z(K, N), val=z(K, N), lv=z(N))
         bufs["obs"][0].copy_(b.reset())
-        setups[a] = (b, bufs)
-    times = {a: [] for a in agents_list}
+        setups[key] = (b, bufs)
+    times = {a: [] for a in setups}
     ev = [torch.cuda.Event(enable_timing=True) for _ in range(2)]
     for r in range(reps + 1):
         for a, (b, q) in setups.items():
@@ -105,6 +114,21 @@ def throughput(args, log):
     return out
 
 
+def throughput_normalize(args, log):
+    P, n, K = args.agents, args.envs_per_agent, args.rollout_len
+    out = {"card": card(), "env": args.env, "agents": P, "envs_per_agent": n, "rollout_len": K}
+    log(f"card: {out['card']}")
+    r = rollout_ms_per_step(args.env, P * n, [("records", P, P, True), ("none", P, 0, True), ("one", 0, 1, True),
+                                              ("records_frozen", P, P, False), ("one_frozen", 0, 1, False)], K)
+    out["ms_per_step"] = r
+    out["stats_pass_ms_per_step"] = {"segmented": r["records"] - r["records_frozen"], "one_record": r["one"] - r["one_frozen"]}
+    log(f"{P} x {n} envs, rollout per step: {P} policies with {P} records {r['records'] * 1e3:.1f} us, without a normaliser "
+        f"{r['none'] * 1e3:.1f} us, one policy with one record {r['one'] * 1e3:.1f} us; statistics pass per step (training - "
+        f"frozen): segmented {out['stats_pass_ms_per_step']['segmented'] * 1e3:.1f} us, one record "
+        f"{out['stats_pass_ms_per_step']['one_record'] * 1e3:.1f} us")
+    return out
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("env", choices=("SwingRacket-v0", "Tennisbot-v0"))
@@ -119,17 +143,18 @@ def main():
     ap.add_argument("--save", default=None, help="npz of PopulationPPO.state_dict()")
     ap.add_argument("--out", default=None, help="JSON of the result")
     ap.add_argument("--throughput", action="store_true")
+    ap.add_argument("--normalize", action="store_true", help="one VecNormalize record per agent")
     args = ap.parse_args()
     if args.rollout_len is None:
         args.rollout_len = 26 if args.env == "SwingRacket-v0" else 128
     log = lambda m: print(m, flush=True)  # noqa: E731
     if args.throughput:
-        res = throughput(args, log)
+        res = throughput_normalize(args, log) if args.normalize else throughput(args, log)
     else:
         log(f"card: {card()}")
         pop = PopulationPPO(args.env, args.agents, args.envs_per_agent, args.rollout_len,
                             seeds=[args.seed + p for p in range(args.agents)], precision=args.precision, pbt_interval=args.pbt,
-                            pbt_seed=args.pbt_seed)
+                            pbt_seed=args.pbt_seed, normalize=args.normalize)
         res = pop.train(args.iters, log=log)
         res["card"] = card()
         for a in res["per_agent"]:
