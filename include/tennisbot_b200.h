@@ -356,8 +356,18 @@ int tb_es_normalizer_stats(tb_ctx *ctx, double *d_out, void *stream);
 int tb_sac_floats(int env_kind); /* TB_SAC_FLOATS / TB_SAC_FLOATS_HIT (-1: unknown kind); callable without a GPU */
 /* Converts d_params (count = tb_sac_floats(env_kind)) on the device into the library's own image of the actor (W2 as BF16 in
  * the tensor cores' shared-memory layout): one kernel on `stream`, so it is capturable and a replayed graph sees the weights the
- * buffer holds at replay time. */
+ * buffer holds at replay time.  Returns the context to one actor after tb_set_sac_actors. */
 int tb_set_sac_actor(tb_ctx *ctx, const float *d_params, int64_t count, void *stream);
+/* A population of SAC actors for one context: d_params float32 [agents, tb_sac_floats(env_kind)], rows in tb_set_sac_actor's
+ * layout; env i acts with actor i / (N / agents).  One kernel launch converts every row into the library's image, stream-ordered
+ * like tb_set_sac_actor: capturable, and a replayed graph converts the weights d_params holds at replay time.  A call with more
+ * agents than the image buffer holds allocates a larger one (cudaMalloc, and cudaFree of the old one, which waits for the
+ * device): make the largest call before capturing, and capture again after a call that grew the buffer, since graphs captured
+ * earlier refer to the old one.  Fails on a NULL d_params, agents < 1, agents not dividing N, count != agents x
+ * tb_sac_floats(env_kind), a faulted context, and, for agents > 1, N / agents not a multiple of 128 (a 128-env tile of
+ * sac_kernel multiplies against one W2 image in shared memory, and two 128 KB images do not fit beside its A tile).  A
+ * rejected call leaves the actors as they were.  agents = 1 is tb_set_sac_actor (the same image and launch). */
+int tb_set_sac_actors(tb_ctx *ctx, const float *d_params, int64_t agents, int64_t count, void *stream);
 /* Replay ring, caller-owned device arrays: obs, next_obs float32 [slots, N, obs_dim]; act float32 [slots, N, act_dim]; reward
  * float32 [slots, N]; done uint8 [slots, N]. */
 typedef struct tb_sac_ring {
@@ -378,7 +388,12 @@ int tb_sac_begin(tb_ctx *ctx, void *stream);
  * = the terminal observation when done, else the step's observation.  ring = NULL stores nothing (evaluation).  d_last_obs
  * float32 [N, obs_dim] (may be NULL) receives the observation after the last step.  mode TB_SAC_SAMPLE and TB_SAC_MEAN need
  * tb_set_sac_actor.  Never synchronises: capturable in a CUDA graph.
- * mode | TB_SAC_VECNORM (fails when no normaliser is attached, or more than one record is): SB3 SAC under VecNormalize, with the normaliser of tb_set_vecnorm.
+ * After tb_set_sac_actors with agents P > 1, env i acts with actor i / n, n = N / P; the ring's layout, the noise keys,
+ * d_last_obs and the launch count stay as they are (TB_SAC_UNIFORM ignores the actors).  Agent p's transitions are columns
+ * [p n, (p + 1) n) of every ring slot, and agent p's envs give, bit for bit, what a context of n envs with env_id_offset = p n
+ * and the same seed gives with tb_set_sac_actor(row p): actions, ring columns and d_last_obs.
+ * mode | TB_SAC_VECNORM (fails when no normaliser is attached, when more than one record is, and when more than one actor is set,
+ * naming the counts): SB3 SAC under VecNormalize, with the normaliser of tb_set_vecnorm.
  * After every env step (TB_SAC_UNIFORM included) a training normaliser folds the step's observation of all N envs (rule 1),
  * the return (rule 2) and zeroes the returns of done envs (rule 3); the actor acts on o^ (rule 4) with the statistics after
  * that fold.  The ring, d_last_obs and tb_read_stats stay RAW (SB3's get_original_obs / get_original_reward; a terminal

@@ -84,7 +84,8 @@ SIGNATURES = {
     "tb_es_begin": [_vp, _vp, _i64, _i64, _vp, _vp], "tb_es_rollout": [_vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
     "tb_es_begin_noise": [_vp, _vp, _i64, _i64, C.c_float, _u64, _u32, _vp, _vp],
     "tb_es_noise_combine": [_vp, _vp, _vp, _i64, _u64, _u32, _vp, _vp], "tb_es_normalizer_stats": [_vp, _vp, _vp],
-    "tb_sac_floats": [_i32], "tb_set_sac_actor": [_vp, _vp, _i64, _vp], "tb_sac_begin": [_vp, _vp],
+    "tb_sac_floats": [_i32], "tb_set_sac_actor": [_vp, _vp, _i64, _vp], "tb_set_sac_actors": [_vp, _vp, _i64, _i64, _vp],
+    "tb_sac_begin": [_vp, _vp],
     "tb_sac_rollout": [_vp, _i32, _i32, _u64, C.POINTER(TbSacRing), _vp, _vp],
     "tb_render": [_vp, C.POINTER(TbCamera), _vp, _i64, _vp, _vp, _vp, _vp],
     "tb_trace_max_substeps": [_i32], "tb_trace_step": [_vp, _vp, _vp, _i64, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp],

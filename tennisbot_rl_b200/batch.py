@@ -329,6 +329,22 @@ class TennisBatch:
         self._need("set_sac_actor", params, "params", (want,))
         _lib.check(self.lib.tb_set_sac_actor(self.h, _dptr(params), want, self._stream()))
 
+    def set_sac_actors(self, params):
+        """A population: params float32 CUDA tensor [P, sac_floats] on this batch's device, rows in set_sac_actor's layout, P
+        dividing num_envs and, for P > 1, num_envs // P a multiple of 128.  Env i acts with row i // (num_envs // P) in the
+        next sac_rollout; set_sac_actor returns to one actor.  One capturable launch once the library's image buffer holds P
+        actors (tb_set_sac_actors)."""
+        want = _lib.SAC_FLOATS if self.kind == _lib.ENV_SWING else _lib.SAC_FLOATS_HIT
+        agents = int(params.shape[0]) if torch.is_tensor(params) and params.dim() == 2 else -1
+        if agents < 1 or self.num_envs % agents:
+            raise ValueError(f"set_sac_actors: params must have shape (P, {want}) with P dividing {self.num_envs}, got "
+                             f"{tuple(params.shape) if torch.is_tensor(params) else type(params).__name__}")
+        if agents > 1 and (self.num_envs // agents) % 128:
+            raise ValueError(f"set_sac_actors: with P > 1, envs per agent ({self.num_envs} / {agents}) must be a multiple of "
+                             f"128: a 128-env tile multiplies against one actor's W2 image in shared memory")
+        self._need("set_sac_actors", params, "params", (agents, want))
+        _lib.check(self.lib.tb_set_sac_actors(self.h, _dptr(params), agents, agents * want, self._stream()))
+
     def sac_begin(self):
         """Reset every env and start the ring at slot 0 (needs force control and auto_reset)."""
         _lib.check(self.lib.tb_sac_begin(self.h, self._stream()))

@@ -2072,6 +2072,9 @@ struct SacIO {
   const double *vn_stats;       // the running record, TB_VECNORM_WORDS(OBS) doubles
   double vn_clip_obs, vn_eps;
   int vn_norm_obs;
+  // POP instances only (tb_set_sac_actors): w2 and small hold one image per agent, image_w2 uint4 and image_small floats
+  // apart; env i acts with agent i / per_agent, a multiple of 128 so that every tile belongs to one agent
+  int64_t image_w2, image_small, per_agent;
 };
 
 // Fold step j = tick - base - 1 of env i into the ring and `cur`; x receives the observation the next action is computed from.
@@ -2140,7 +2143,11 @@ template <int ACT> __device__ __forceinline__ void sac_store_act(const SacIO &io
 //   clamp, noise, accurate tanhf.
 // NORM: the instance of tb_sac_rollout with TB_SAC_VECNORM; the network's input is normalised in registers before layer 1 (the
 // one-thread-per-env shape evaluates no network, so it is the same code in both instances).
-template <int OBS, int ACT, bool NORM>
+// POP: the population instance (tb_set_sac_actors, agents > 1).  Tile t belongs to agent t * 128 / per_agent.  Each CTA runs a
+// contiguous chunk of tiles instead of the stride loop, so that its tiles are agent-contiguous, and loads an agent's image
+// into shared memory only when its next tile belongs to another agent than the image it holds: once per CTA while tiles <=
+// SMs, and about once per agent boundary a chunk crosses beyond that.
+template <int OBS, int ACT, bool NORM, bool POP>
 __global__ void __launch_bounds__(kBlock, 1) sac_kernel(const __grid_constant__ SacIO io) {
   using L = SacLayout<OBS, ACT>;
   static_assert(OBS % 2 == 0 && ACT % 2 == 0, "observation and action rows are accessed as float2");
@@ -2166,10 +2173,18 @@ __global__ void __launch_bounds__(kBlock, 1) sac_kernel(const __grid_constant__ 
   uint64_t *bar = reinterpret_cast<uint64_t *>(S + L::Small);
   uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(bar + 1);
   const int tid = threadIdx.x, warp = tid >> 5;
+  int64_t held = 0;  // POP: the agent whose image shared memory holds, first that of this CTA's first tile
   {
+    const uint4 *src = io.w2;
+    const float *small = io.small;
+    if constexpr (POP) {
+      held = (n + kBlock - 1) / kBlock * blockIdx.x / gridDim.x * kBlock / io.per_agent;
+      src += held * io.image_w2;
+      small += held * io.image_small;
+    }
     uint4 *w = reinterpret_cast<uint4 *>(W2);
-    for (int q = tid; q < L::W2Bytes / 16; q += kBlock) w[q] = io.w2[q];
-    for (int q = tid; q < L::Small; q += kBlock) S[q] = io.small[q];
+    for (int q = tid; q < L::W2Bytes / 16; q += kBlock) w[q] = src[q];
+    for (int q = tid; q < L::Small; q += kBlock) S[q] = small[q];
   }
   if (warp == 0) {
     asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 256;" ::"r"(smem_u32(tmem_slot)));
@@ -2186,7 +2201,25 @@ __global__ void __launch_bounds__(kBlock, 1) sac_kernel(const __grid_constant__ 
   const uint32_t tmem = *tmem_slot, a_base = smem_u32(A), b_base = smem_u32(W2), bar_a = smem_u32(bar);
   const int64_t tiles = (n + kBlock - 1) / kBlock;
   uint32_t phase = 0;
-  for (int64_t tile = blockIdx.x; tile < tiles; tile += gridDim.x, phase ^= 1u) {
+  int64_t tile = blockIdx.x, last = tiles;
+  if constexpr (POP) {  // this CTA's chunk of tiles [tile, last)
+    tile = tiles * blockIdx.x / gridDim.x;
+    last = tiles * (blockIdx.x + 1) / gridDim.x;
+  }
+  for (; tile < last; tile += POP ? 1 : gridDim.x, phase ^= 1u) {
+    if (POP && tile * kBlock / io.per_agent != held) {
+      // every warp is past its tcgen05.ld of the previous tile and every thread past its reads of S, and the previous MMA,
+      // which read W2, has completed (the mbarrier wait); then the new image, and the proxy fence before the next MMA
+      __syncthreads();
+      held = tile * kBlock / io.per_agent;
+      const uint4 *src = io.w2 + held * io.image_w2;
+      const float *small = io.small + held * io.image_small;
+      uint4 *w = reinterpret_cast<uint4 *>(W2);
+      for (int q = tid; q < L::W2Bytes / 16; q += kBlock) w[q] = src[q];
+      for (int q = tid; q < L::Small; q += kBlock) S[q] = small[q];
+      asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+      __syncthreads();
+    }
     const int64_t i = tile * kBlock + tid;
     const bool mine = i < n;
     float x[OBS];
@@ -2273,9 +2306,17 @@ __global__ void __launch_bounds__(kBlock, 1) sac_kernel(const __grid_constant__ 
 }
 
 // tb_set_sac_actor: the caller's float32 vector -> W2 in BF16 at its canonical-layout offset, everything else to `small`.
-template <int OBS, int ACT> __global__ void __launch_bounds__(256) sac_image_kernel(const float *p, uint16_t *w2, float *small) {
+// POP (tb_set_sac_actors): a flat grid of agents x kSacImageBlocks CTAs; CTA b converts row b / kSacImageBlocks into image
+// b / kSacImageBlocks of w2 (H x H halves apart) and small (SacLayout::Small floats apart).
+template <int OBS, int ACT> constexpr int kSacImageBlocks = (SacLayout<OBS, ACT>::Floats + 255) / 256;
+template <int OBS, int ACT, bool POP>
+__global__ void __launch_bounds__(256) sac_image_kernel(const float *p, uint16_t *w2, float *small) {
   using L = SacLayout<OBS, ACT>;
-  const int f = blockIdx.x * 256 + threadIdx.x;
+  if (POP) {
+    const int agent = blockIdx.x / kSacImageBlocks<OBS, ACT>;
+    p += (int64_t)agent * L::Floats; w2 += (int64_t)agent * L::H * L::H; small += (int64_t)agent * L::Small;
+  }
+  const int f = (POP ? blockIdx.x % kSacImageBlocks<OBS, ACT> : blockIdx.x) * 256 + threadIdx.x;
   if (f >= L::Floats) return;
   if (f < L::W2) small[f] = p[f];
   else if (f < L::B2) {
@@ -2927,9 +2968,11 @@ struct StagingBufs {          // device copies of the host-buffer entry points' 
   DevPtr<float> actions, obs, reward, term;
   DevPtr<uint8_t> done, events, mask;
 };
-struct SacActorBufs {         // tb_set_sac_actor: the actor's image (see SacLayout)
-  DevPtr<uint4> w2;           // W2, 128 KB
-  DevPtr<float> small;        // the other tensors
+struct SacActorBufs {         // tb_set_sac_actor / tb_set_sac_actors: the actors' images (see SacLayout)
+  DevPtr<uint4> w2;           // [agents] W2, 128 KB each
+  DevPtr<float> small;        // [agents] the other tensors
+  int64_t cap = 0;            // images the buffers hold
+  int64_t agents = 1;         // images the rollout uses: env i acts with image i / (N / agents)
 };
 struct SacBufs {              // tb_sac_begin: per-env staging between sac_kernel and the env step (see SacIO)
   DevPtr<float> cur, act, obs, term, rew;
@@ -3834,24 +3877,52 @@ int tb_es_rollout(tb_ctx *c, int k_steps, double *d_return, uint8_t *d_alive, fl
   return 0;
 }
 
+// agents actor rows -> the library's images, one launch; the buffers grow when they hold fewer (cudaMalloc / cudaFree: not
+// while capturing).  agents = 1 is tb_set_sac_actor's launch.
+static int convert_sac_actors(tb_ctx *c, const float *d_params, int64_t agents, cudaStream_t s) {
+  const int64_t floats = tb_sac_floats(c->cfg.env_kind), small = floats - TB_SAC_HIDDEN * TB_SAC_HIDDEN;
+  if (c->sac_actor.cap < agents) {
+    SacActorBufs b;
+    CU(dev_alloc(b.w2, (size_t)agents * TB_SAC_HIDDEN * TB_SAC_HIDDEN * 2));
+    CU(dev_alloc(b.small, (size_t)(agents * small) * sizeof(float)));
+    b.cap = agents;
+    c->sac_actor = std::move(b);
+  }
+  c->sac_actor.agents = agents;
+  uint16_t *w2 = reinterpret_cast<uint16_t *>(c->sac_actor.w2.get());
+  return with_kind(c->cfg.env_kind, [&](auto kind) {
+    constexpr int OBS = Dims<kind>::obs, ACT = Dims<kind>::act;
+    if (agents == 1)
+      return launch(c, kPlain, sac_image_kernel<OBS, ACT, false>, grid_for(floats, 256), 256, s, d_params, w2, c->sac_actor.small.get());
+    return launch(c, kPlain, sac_image_kernel<OBS, ACT, true>, (unsigned)(agents * kSacImageBlocks<OBS, ACT>), 256, s, d_params, w2,
+                  c->sac_actor.small.get());
+  });
+}
+
 int tb_set_sac_actor(tb_ctx *c, const float *d_params, int64_t count, void *stream) {
   GUARD(c);
   const int64_t want = tb_sac_floats(c->cfg.env_kind);
   if (!d_params || count != want)
     return fail("tb_set_sac_actor: expected tb_sac_floats(env_kind) = %lld floats in device memory, got %lld", (long long)want,
                 (long long)count);
-  if (!c->sac_actor.w2) {
-    SacActorBufs b;
-    CU(dev_alloc(b.w2, TB_SAC_HIDDEN * TB_SAC_HIDDEN * 2));
-    CU(dev_alloc(b.small, (size_t)(want - TB_SAC_HIDDEN * TB_SAC_HIDDEN) * sizeof(float)));
-    c->sac_actor = std::move(b);
-  }
-  if (with_kind(c->cfg.env_kind, [&](auto kind) {
-        return launch(c, kPlain, sac_image_kernel<Dims<kind>::obs, Dims<kind>::act>, grid_for(want, 256), 256, (cudaStream_t)stream,
-                      d_params, reinterpret_cast<uint16_t *>(c->sac_actor.w2.get()), c->sac_actor.small.get());
-      }))
-    return 1;
-  return 0;
+  return convert_sac_actors(c, d_params, 1, (cudaStream_t)stream);
+}
+
+int tb_set_sac_actors(tb_ctx *c, const float *d_params, int64_t agents, int64_t count, void *stream) {
+  GUARD(c);
+  const int64_t n = c->cfg.num_envs, floats = tb_sac_floats(c->cfg.env_kind);
+  if (!d_params) return fail("tb_set_sac_actors: d_params is NULL");
+  if (agents < 1 || n % agents)
+    return fail("tb_set_sac_actors: agents must be >= 1 and divide num_envs = %lld, got %lld", (long long)n, (long long)agents);
+  if (count != agents * floats)
+    return fail("tb_set_sac_actors: expected agents x tb_sac_floats(env_kind) = %lld x %lld floats, got %lld", (long long)agents,
+                (long long)floats, (long long)count);
+  if (agents > 1 && (n / agents) % kBlock)
+    return fail("tb_set_sac_actors: with agents > 1, envs per agent (%lld / %lld = %lld) must be a multiple of %d: a %d-env "
+                "tile multiplies against one actor's W2 image in shared memory, and two 128 KB images do not fit beside the A "
+                "tile", (long long)n, (long long)agents, (long long)(n / agents), kBlock, kBlock);
+  if (check_fault(c, "tb_set_sac_actors")) return 1;
+  return convert_sac_actors(c, d_params, agents, (cudaStream_t)stream);
 }
 
 int tb_sac_begin(tb_ctx *c, void *stream) {
@@ -3876,8 +3947,9 @@ int tb_sac_begin(tb_ctx *c, void *stream) {
     CU(cudaDeviceGetAttribute(&c->sac_grid, cudaDevAttrMultiProcessorCount, c->cfg.device));
     if (with_kind(c->cfg.env_kind, [&](auto kind) {
           constexpr int OBS = Dims<kind>::obs, ACT = Dims<kind>::act, smem = SacLayout<OBS, ACT>::Smem;
-          CU(cudaFuncSetAttribute(sac_kernel<OBS, ACT, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-          CU(cudaFuncSetAttribute(sac_kernel<OBS, ACT, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+          CU(cudaFuncSetAttribute(sac_kernel<OBS, ACT, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+          CU(cudaFuncSetAttribute(sac_kernel<OBS, ACT, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+          CU(cudaFuncSetAttribute(sac_kernel<OBS, ACT, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
           return 0;
         }))
       return 1;
@@ -3911,7 +3983,12 @@ int tb_sac_rollout(tb_ctx *c, int k_steps, int mode, uint64_t noise_seed, const 
   if (norm && !c->vn_cfg.struct_size) return fail("tb_sac_rollout: TB_SAC_VECNORM needs a normaliser (tb_set_vecnorm)");
   if (norm && c->vn.records != 1)
     return fail("tb_sac_rollout: TB_SAC_VECNORM uses one record, and %lld are attached (tb_set_vecnorms)", (long long)c->vn.records);
+  if (norm && c->sac_actor.agents > 1)
+    return fail("tb_sac_rollout: TB_SAC_VECNORM normalises with one record, and %lld actors are set (tb_set_sac_actors); a "
+                "population of SAC actors has no per-agent normaliser: set one actor (tb_set_sac_actor) or drop the flag",
+                (long long)c->sac_actor.agents);
   if (check_fault(c, "tb_sac_rollout")) return 1;
+  const bool pop = c->sac_actor.agents > 1;
   const bool train = norm && vecnorm_training(c);
   const int64_t n = c->cfg.num_envs;
   cudaStream_t s = (cudaStream_t)stream;
@@ -3928,6 +4005,10 @@ int tb_sac_rollout(tb_ctx *c, int k_steps, int mode, uint64_t noise_seed, const 
     sio.vn_stats = c->vn.stats.get(); sio.vn_clip_obs = c->vn_cfg.clip_obs; sio.vn_eps = c->vn_cfg.epsilon;
     sio.vn_norm_obs = c->vn_cfg.norm_obs;
   }
+  if (pop) {
+    sio.image_w2 = TB_SAC_HIDDEN * TB_SAC_HIDDEN * 2 / 16; sio.image_small = tb_sac_floats(c->cfg.env_kind) - TB_SAC_HIDDEN * TB_SAC_HIDDEN;
+    sio.per_agent = n / c->sac_actor.agents;
+  }
   if (train) {  // the entry pass: while tb_sac_begin's reset is pending, zero the returns and fold the current observation
     VecNormIO vio = vecnorm_io(c);
     vio.obs = c->sac.cur.get(); vio.armed = c->sac.pending.get();
@@ -3936,7 +4017,7 @@ int tb_sac_rollout(tb_ctx *c, int k_steps, int mode, uint64_t noise_seed, const 
   }
   return with_kind(c->cfg.env_kind, [&](auto kind) {
     constexpr int OBS = Dims<kind>::obs, ACT = Dims<kind>::act;
-    auto kernel = norm ? sac_kernel<OBS, ACT, true> : sac_kernel<OBS, ACT, false>;
+    auto kernel = norm ? sac_kernel<OBS, ACT, true, false> : pop ? sac_kernel<OBS, ACT, false, true> : sac_kernel<OBS, ACT, false, false>;
     constexpr int smem = SacLayout<OBS, ACT>::Smem;
     const int64_t tiles = (n + kBlock - 1) / kBlock;
     for (int t = 0; t <= k_steps; ++t) {  // launch t folds step t - 1 (t > 0) and acts for step t (t < K)

@@ -149,11 +149,11 @@ def episode_stats(reward, done, carry_ret, carry_len, agents):
 
 
 @torch.no_grad()
-def exploit_explore(scores, tensors, hyper, rng):
+def exploit_explore(scores, tensors, hyper, rng, perturbed=PBT_PERTURBED):
     """One PBT round.  scores: P floats, None for an agent that finished no episode (it ranks last).  Each of the bottom
     max(1, P // 4) agents copies an agent drawn from the top max(1, P // 4) with rng (numpy Generator): row dst of every
-    tensor in `tensors` and of every [P] tensor in `hyper` takes row src; then its PBT_PERTURBED hyper-parameters are each
-    multiplied by 0.8 or 1.2.  Returns [(dst, src, {name: new value})]."""
+    tensor in `tensors` and of every [P] tensor in `hyper` takes row src; then its `perturbed` hyper-parameters (PPO's
+    PBT_PERTURBED by default) are each multiplied by 0.8 or 1.2.  Returns [(dst, src, {name: new value})]."""
     P = len(scores)
     if P < 2:
         raise ValueError("exploit_explore needs at least 2 agents")
@@ -166,7 +166,7 @@ def exploit_explore(scores, tensors, hyper, rng):
             t[dst] = t[src]
         for h in hyper.values():
             h[dst] = h[src]
-        for name in PBT_PERTURBED:
+        for name in perturbed:
             hyper[name][dst] = hyper[name][dst] * float(rng.choice(PBT_FACTORS))
         events.append((dst, src, {name: float(h[dst]) for name, h in hyper.items()}))
     return events
